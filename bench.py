@@ -2,7 +2,7 @@
 """
 bench.py - spin-updates/s of the bit-packed 2-D checkerboard Gibbs path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): 2-D Ising 8192 x 8192, T = 2.269, periodic, 4096 independent
@@ -21,6 +21,8 @@ roofline: HBM bound; algorithmic bytes = 0.25 B per spin update (read 1 neighbou
 cpu_baseline / --impl reference: the UNMODIFIED reference (GibbsSampler.gibbs_sweep of tsu/gibbs.py,
          from oracle/_ref or /root/reference) on the host cores, one process per core, on a bounded
          sample of the workload; the oracle's literal port only if the reference tree is not there.
+--dump-outputs DIR: after the timed steps, rank 0 writes what they computed as DIR/<name>.npy (see dump_outputs()).
+         Inputs come from fixed seeds, so two builds run with the same arguments can be compared file by file.
 secondary: the other BASELINE configurations, timed with CUDA events inside this run:
          C1 (IsingModel2D 50 x 50, 1000 gibbs_update + M + E), C3 (dense SK N = 4096, 2048 chains,
          10 sweeps on tcgen05; tensor roofline), C5 (50-temperature ladders of 1024^2 lattices with
@@ -34,10 +36,12 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 L = 8192
 N_REPLICAS = 4096
@@ -166,7 +170,7 @@ class ClockSampler:
         self.device_index = device_index
         self.period_ms = period_ms
         self.proc = None
-        self.path = f"/tmp/tsu_bench_clocks_{os.getpid()}_{id(self)}.csv"
+        self.path = os.path.join(tempfile.gettempdir(), f"tsu_bench_clocks_{os.getpid()}_{id(self)}.csv")
 
     def start(self):
         try:
@@ -235,6 +239,41 @@ def profiled_kernel():
         return d if d.get("workload") == WORKLOAD else None
     except Exception:
         return None
+
+
+# ----------------------------------------------------------------------------- output dump
+# what --dump-outputs writes stays under 64 MB for any shape: at most 40 MB of sampled spins (argument check in main()),
+# 16 B of observables for each of at most 2^20 replicas, and the sample's indices
+DUMP_REPLICAS = 8
+DUMP_SPIN_BYTES = 40 << 20
+DUMP_OBS_REPLICAS = 1 << 20
+
+
+def dump_outputs(eng, out_dir):
+    """write what the timed sweeps left in `eng`, in the form a caller of Ising2DEngine receives it:
+    magnetization.npy, energy.npy        float64 [M]           magnetisation per spin and energy of the first
+                                                               M = min(n_replicas, 2^20) replicas
+    spins.npy                            float32 [R, K, cols]  +-1 spins of R replicas x K rows, all columns
+    spins_replicas.npy, spins_rows.npy   float64 [R], [K]      the replicas and rows spins.npy holds (seeded sample)"""
+    import numpy as np
+    import torch
+
+    rng = np.random.default_rng(SEED)
+    row_bytes = 4 * eng.cols
+    n_rep = min(DUMP_REPLICAS, eng.n_replicas, DUMP_SPIN_BYTES // row_bytes)
+    n_rows = min(eng.rows, DUMP_SPIN_BYTES // (row_bytes * n_rep))
+    replicas = np.sort(rng.choice(eng.n_replicas, n_rep, replace=False))
+    rows = np.sort(rng.choice(eng.rows, n_rows, replace=False))
+    rows_dev = torch.from_numpy(rows).to(eng.device)
+    spins = np.stack([eng.chunk_view(int(r), 1).spins_tensor(pm1=True)[0].index_select(0, rows_dev).cpu().numpy()
+                      for r in replicas])
+    n_obs = min(eng.n_replicas, DUMP_OBS_REPLICAS)
+    arrays = {"magnetization": eng.magnetization()[:n_obs], "energy": eng.energy()[:n_obs],
+              "spins": spins.astype(np.float32), "spins_replicas": replicas.astype(np.float64),
+              "spins_rows": rows.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------- secondary configurations
@@ -555,6 +594,8 @@ def run_b200_arm(args):
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
     ms = _max_over_ranks(torch, dist, world, ms)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)   # before the end-to-end leg overwrites the lattices
     n_launches = args.steps * SWEEPS_PER_STEP * 2
     value = world * updates_per_step * args.steps / (ms * 1e-3)
     launch_s = ms * 1e-3 / n_launches
@@ -734,7 +775,15 @@ def main():
     ap.add_argument("--size", type=int, default=L)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the state the timed steps computed as DIR/<name>.npy (rank 0's replicas)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 arm")
+    if args.dump_outputs and 4 * args.size > DUMP_SPIN_BYTES:
+        ap.error(f"--dump-outputs: one row of {args.size} spins exceeds the {DUMP_SPIN_BYTES >> 20} MB spin sample")
     if args.warmup < 3:
         args.warmup = 3 if args.impl == "b200" else args.warmup
     if args.impl == "reference":

@@ -48,3 +48,35 @@ def test_b200_arm_needs_a_gpu():
         pytest.skip("a CUDA device is present")
     r = run_bench("--steps", "1", "--warmup", "3", "--no-cpu")
     assert r.returncode != 0 and "no CPU fallback" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_what_the_timed_steps_computed(tmp_path):
+    """--dump-outputs: the same files from run to run, spins equal to the oracle after (warmup + steps) x 10 sweeps on
+    the sampled replicas and rows, observables of every replica consistent with them; --steps sets the timed steps"""
+    import numpy as np
+
+    from oracle import ising2d_oracle as O
+
+    size, n_rep, steps, warmup, seed, T = 64, 16, 2, 3, 1234, 2.269
+    dumps = []
+    for k in range(2):
+        out = tmp_path / str(k)
+        r = run_bench("--size", str(size), "--replicas", str(n_rep), "--steps", str(steps), "--warmup", str(warmup),
+                      "--no-cpu", "--no-secondary", "--dump-outputs", str(out))
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads(r.stdout.strip().splitlines()[-1])
+        assert d["steps"] == steps and d["gpu_launches"] == steps * 10 * 2
+        dumps.append({p.stem: np.load(p) for p in out.glob("*.npy")})
+    a, b = dumps
+    assert sorted(a) == ["energy", "magnetization", "spins", "spins_replicas", "spins_rows"]
+    for name in a:
+        assert a[name].dtype in (np.float32, np.float64) and np.array_equal(a[name], b[name]), name
+    assert a["magnetization"].shape == a["energy"].shape == (n_rep,)
+    rows = a["spins_rows"].astype(np.int64)
+    for i, rep in enumerate(a["spins_replicas"].astype(np.int64)):
+        want = O.checkerboard_sweeps_philox(O.init_bits(seed, rep, size, size), seed, rep, 0, (warmup + steps) * 10,
+                                            1.0, 0.0, T, True)
+        assert np.array_equal(a["spins"][i], 2.0 * want[rows] - 1), rep
+        assert a["magnetization"][rep] == (2.0 * want.sum() - size * size) / (size * size)
+        assert a["energy"][rep] == pytest.approx(O.energy(want, 1.0, 0.0, True), abs=1e-9)
