@@ -54,11 +54,15 @@ def _as_square(coupling) -> np.ndarray:
     return J
 
 
+# csrc/dense_gibbs.cu keeps a chain's uniforms (and their logits with float64 fields), fields, self couplings and bits
+# in at most 227 KB of shared memory: 33 N + 272 bytes with float64 fields, 17 N + 272 with float32
+DENSE_MAX_N = {"float64": 7035, "float32": 13657}
+
+
 class _DenseProblem:
     """coupling matrix + bias resident on the device (transposed, see tsu_b200.h)"""
 
     def __init__(self, coupling, bias, precision: str, device):
-        torch = _lib.require_cuda()
         J = _as_square(coupling)
         self.N = J.shape[0]
         if precision == "bf16":
@@ -66,6 +70,10 @@ class _DenseProblem:
                              "this entry point needs a 'float64' or 'float32' sampler")
         if precision not in ("float64", "float32"):
             raise ValueError("precision must be 'float64', 'float32' or 'bf16'")
+        if self.N > DENSE_MAX_N[precision]:
+            raise ValueError(f"precision='{precision}' (dense kernel) supports at most {DENSE_MAX_N[precision]} bits "
+                             f"(float64: {DENSE_MAX_N['float64']}, float32: {DENSE_MAX_N['float32']}); got {self.N}")
+        torch = _lib.require_cuda()
         self.np_dtype = np.float64 if precision == "float64" else np.float32
         self.code = 1 if precision == "float64" else 0
         self.device = device
