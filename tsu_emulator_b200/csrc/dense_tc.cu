@@ -18,7 +18,7 @@
 //     H[:, later blocks of the panel] += delta . J[later, block]^T  corrects the rest of the panel.
 // The result is identical to a site-by-site sweep with the same fields.
 //
-// One CTA owns M = 128 chains (TMEM lane = chain), or 64 when there are too few chains to give every SM a tile.
+// One CTA owns M = 128 chains (TMEM lane = chain), or 64 while 64-chain tiles still fit in one wave of the SMs.
 // The chain states stay resident in shared memory as bits for the whole call.  Each K-chunk of 128 sites is
 // expanded to bf16 by the thread that owns the chain and written straight into TENSOR MEMORY (tcgen05.st,
 // lane = chain, column = K pair): the spin operand A never touches shared memory.  A spin is encoded as 0.0 / 2.0:
@@ -31,7 +31,7 @@
 // +-20 T (the reference's sigmoid clamp, gibbs.py:65-70), u = 24-bit Philox uniform, logit via lg2.approx in fp32,
 // produced one block ahead by two dedicated warps.  Against the float64 rule the kernel can only disagree where u
 // lies within ~5e-6 (exactly representable J) / ~5e-5 (Gaussian J, N <= 4096) of the acceptance probability; the
-// tests count those sites and check the bound (tests/test_dense_gpu.py).
+// tests count those sites and check the bound (tests/test_dense_gpu.py, tests/test_dense_tc_kernel_gpu.py).
 //
 // Warp roles (16 warps): 0-7 two producer groups (TMA requests + spin expansion), 8-11 epilogue, 12 main MMA
 // issuer, 13 in-panel correction issuer, 14-15 thresholds.
@@ -709,11 +709,14 @@ static int launch_tc(const TcParams& P, cudaStream_t st) {
   int rc = make_j_tensor_map(&tmap, P.J, P.N);
   if (rc != TSU_OK) return rc;
   // chains per CTA: 128 fills the tensor core's M; with few chains 64 per CTA puts twice as many SMs to work (a
-  // tcgen05.mma with M = 64 takes as long as one with M = 128, so this only pays while SMs would otherwise idle)
+  // tcgen05.mma with M = 64 takes as long as one with M = 128, so this only pays while SMs would otherwise idle).
+  // One CTA fits an SM, so 64 is chosen only while its tiles fit one wave: from sm_count * 64 + 1 chains on (9473 on
+  // a B200), 64-chain tiles need two waves where 128-chain tiles need one (B200 at its 1000 W power limit, N = 4096,
+  // 10 sweeps: 12000 chains 8.05 ms at M = 64, 4.38 ms at M = 128; tools/tc_tile_height.py)
   int sm_count = 0, dev = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-  int m = (P.n_chains + 127) / 128 < sm_count ? 64 : 128;
+  int m = (P.n_chains + 63) / 64 <= sm_count ? 64 : 128;
   if (const char* env = getenv("TSU_TC_M")) m = atoi(env) == 64 ? 64 : 128;  // tile height override (tests; same bits)
   cudaError_t e;
   if (m == 64) {
