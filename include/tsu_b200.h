@@ -250,6 +250,20 @@ int tsu_dense_gibbs_tc_run(const void* d_J_bf16, const float* d_bias, uint8_t* d
 int tsu_dense_tc_debug_fields(const void* d_J_bf16, const uint8_t* d_state, int n_chains, int N,
                               float* d_fields, uintptr_t stream);
 
+/* Energy of every chain on the tensor cores (simulated annealing and replica exchange on the bf16 path):
+ *   d_energy[c] = -1/2 s^T J s - b^T s   (tsu/gibbs.py:215-236)
+ * for the bf16 couplings d_J_bf16 ([N][N] row-major, as tsu_dense_gibbs_tc_run) and the float32 bias d_bias (or NULL).
+ * The fields f = S J^T come from the same GEMM as tsu_dense_tc_debug_fields (fp32 accumulation in TMEM); the thread of
+ * chain c then sums s_i f_i and s_i b_i in float64 over the sites i = 0 .. N-1 in order, so the value does not depend on
+ * the tile height or on how the chains are split into launches, and it is exact for couplings and bias of the form
+ * m / 2^k.  d_state is read only.
+ * Best-state tracking (tsu/gibbs.py:387-391): pass d_best_energy [n_chains] and d_best_state [n_chains][N] together
+ * (or both NULL).  Where d_energy[c] < d_best_energy[c] (strict), both are replaced by the chain's energy and state;
+ * rows of the other chains are not written.  N % 128 == 0, N <= 4096. */
+int tsu_dense_tc_energy(const void* d_J_bf16, const float* d_bias, const uint8_t* d_state, int n_chains,
+                        int N, double* d_energy, double* d_best_energy, uint8_t* d_best_state,
+                        uintptr_t stream);
+
 /* Chromatic Gibbs sweeps for SPARSE couplings (csrc/sparse_gibbs.cu): IsingChain (tsu/models/ising.py:265-304),
  * irregular graphs, MAX-CUT instances.  J in CSR (row i = couplings into site i, ascending columns, self term
  * allowed), sites grouped into colour classes such that no two coupled sites share one (d_colour_sites, offsets in

@@ -110,6 +110,9 @@ SIGNATURES = {
          c_uintptr],
     ),
     "tsu_dense_tc_debug_fields": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_uintptr]),
+    "tsu_dense_tc_energy": (
+        c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_uintptr]
+    ),
     "tsu_pt_swap": (
         c_int,
         [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_uint64, c_uint32, c_void_p, c_void_p, c_int,

@@ -189,6 +189,10 @@ struct TcParams {
   uint32_t k0, k1, sweep0, chain0;
   int gemm_only;            // diagnostics: no spin update (fields of the initial state for every site)
   int dbg;                  // knock-out switches of timing experiments; always 0 unless built with -DTSU_TC_DEBUG_SWITCHES
+  // energy pass (dense_tc_kernel<kM, true>): read by that instantiation only
+  double* energy;           // [n_chains] -1/2 s^T J s - b^T s of the state
+  double* best_energy;      // [n_chains] lowest energy so far, or nullptr (then best_state is nullptr too)
+  uint8_t* best_state;      // [n_chains][N] the state that had it
 };
 
 constexpr int kProducers = 128 * kGroups;           // warps 0-7: 4 warps (128 chains) per group
@@ -298,7 +302,25 @@ __device__ __forceinline__ bool chain_lane_active(int t) {
   return kM == 128 || (t & 31) < 16;
 }
 
-template <int kM>
+// bits of row `row` of sm.sbits -> dst[0 .. N-1] as uint8 (the layout of the state arrays).  The sweep's final-state
+// write keeps its own copy of this loop: calling this function there changes the sweep's instruction schedule.
+__device__ __forceinline__ void unpack_bits(const TcSmem& sm, int row, int N, uint8_t* dst) {
+  for (int w = 0; w < N / 32; ++w) {
+    const uint32_t x = sm.sbits[w][row];
+    uint8_t* d = dst + 32 * w;
+#pragma unroll
+    for (int b = 0; b < 32; b += 4) {
+      const uint32_t e2 = x >> (b >> 1), o2 = x >> (16 + (b >> 1));
+      *reinterpret_cast<uint32_t*>(d + b) = (e2 & 1u) | ((o2 & 1u) << 8) | ((e2 & 2u) << 15) | ((o2 & 2u) << 23);
+    }
+  }
+}
+
+// kEnergy = false: the sweep (or, with P.gemm_only, the fields of the initial state for diagnostics).
+// kEnergy = true: the energy pass - the main GEMM of every panel (as gemm_only) and, per chain, the energy
+// -1/2 s.f - s.b summed in float64 over the sites in index order, with optional best-state tracking.  A separate
+// instantiation, so that none of it costs the register-bound sweep anything.
+template <int kM, bool kEnergy>
 __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   // round the base up to 1024 bytes in the SHARED address space (keeps the compiler on LDS/STS)
@@ -307,6 +329,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
   const int N = P.N;
   const int n_panels = N / kPanel;  // = number of K-chunks
   const int total_panels = n_panels * P.n_sweeps;
+  const bool gemm_only = kEnergy || P.gemm_only;
 
   // ---- one-time setup -------------------------------------------------------------------------
   if (tid < kM) {  // pack this chain's bits
@@ -459,7 +482,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
     }
   } else if (warp == kIssuer0 + 1) {
     // ===================== correction issuer: H[:, later blocks] += delta(block b) . J[later, block b]^T ====
-    if (!P.gemm_only) {
+    if (!gemm_only) {
       const uint64_t jd_desc0 = umma_desc_sw128(smem_u32(sm.jdiag.bytes));
       uint32_t ready_phase = 0;
       for (int gp = 0; gp < total_panels; ++gp) {
@@ -491,7 +514,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
     //   u < sigmoid(h / T)  <=>  h > T * logit(u)          (gibbs.py:61-77,126; strict <)
     // and the clamp of gibbs.py:65-70 (|h/T| > 20 -> p = 1 / 0) is the clamp of the threshold to +-20 T.
     // This takes Philox, exp and the division off the epilogue's site-to-site dependency chain.
-    if (!P.gemm_only) {
+    if (!gemm_only) {
       const int t = tid - 32 * kThresh0;  // 0..63: chains t and (M = 128) t + 64 of the tile
       constexpr int kPer = kM / 64;
       float Tc[kPer];
@@ -542,6 +565,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
     const bool chain_ok = chain < P.n_chains && chain_lane_active<kM>(t128);
     const uint32_t tmem_lane = tmem_d + ((uint32_t)((warp & 3) * 32) << 16);
     uint32_t accf_phase = 0, corr_phase = 0, thr_phase = 0;
+    double e1 = 0.0, e2 = 0.0;  // energy pass: sum of s_i f_i and of s_i b_i over the sites visited so far
     // diagonal block J[blk, blk]: 8 bf16 per thread (row i0 + t128/4, columns i0 + 8 (t128%4) ..), fetched one
     // block ahead so that the load latency hides behind the previous block's update
     auto load_diag = [&](int blk) {
@@ -565,7 +589,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
     for (int gp = 0; gp < total_panels; ++gp) {
       const int p = gp % n_panels, buf = gp & 1;
       // J[panel, panel] for this panel's corrections; the previous panel's corrections are all complete
-      if (!P.gemm_only && t128 == 0) {
+      if (!gemm_only && t128 == 0) {
         mbar_arrive_expect_tx(&sm.jdiag_full, kTileBytes);
         tma_load_2d(sm.jdiag.bytes, &tmap, p * kPanel, p * kPanel, &sm.jdiag_full);
         tma_load_2d(sm.jdiag.bytes + kHalfBytes, &tmap, p * kPanel + 64, p * kPanel, &sm.jdiag_full);
@@ -582,7 +606,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
         // compare -> new - old -> packed fma into the fields of the sites still to come.
         float thr[kBlk];
         const uint32_t w_old = sm.sbits[blk][row];
-        if (!P.gemm_only) {
+        if (!gemm_only) {
           mbar_wait(&sm.thr_full, thr_phase);
           thr_phase ^= 1u;
 #pragma unroll
@@ -596,7 +620,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
             mbar_wait(&sm.acc_full[buf], (accf_phase >> buf) & 1u);  // main GEMM of the panel
             accf_phase ^= 1u << buf;
             if (warp == kEpilogue0) TC_ACC(11);
-          } else if (!P.gemm_only) {
+          } else if (!gemm_only) {
             mbar_wait(&sm.corr_done, corr_phase);  // flips of block b - 1 are in the fields of this block
             corr_phase ^= 1u;
             if (warp == kEpilogue0) TC_ACC(13);
@@ -615,10 +639,20 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
         // the next block's diagonal couplings go to the other jblk buffer (its previous user, block gblk - 1, is done)
         stage_jblk(jb ^ 1, jd);
         jd = load_diag((blk + 2) % n_blocks);
+        if constexpr (kEnergy) {
+          // sites in index order: f_i = the field without bias (x0.5 is exact), s_i = the bit as the GEMM saw it
 #pragma unroll
-        for (int i = 0; i < kBlk; ++i) h[i] = fmaf(h[i], 0.5f, P.bias ? __ldg(P.bias + i0 + i) : 0.0f);  // spins were 0 / 2
-        if (P.gemm_only) {
-          if (P.fields_out && chain_ok) {
+          for (int i = 0; i < kBlk; ++i) {
+            const bool s = (w_old >> site_bit(i)) & 1u;
+            e1 += s ? (double)(h[i] * 0.5f) : 0.0;
+            e2 += s && P.bias ? (double)__ldg(P.bias + i0 + i) : 0.0;
+          }
+        } else {
+#pragma unroll
+          for (int i = 0; i < kBlk; ++i) h[i] = fmaf(h[i], 0.5f, P.bias ? __ldg(P.bias + i0 + i) : 0.0f);  // spins were 0 / 2
+        }
+        if (gemm_only) {
+          if (!kEnergy && P.fields_out && chain_ok) {
 #pragma unroll
             for (int i = 0; i < kBlk; ++i) P.fields_out[(size_t)chain * N + i0 + i] = h[i];
           }
@@ -657,7 +691,7 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
             if (warp == kEpilogue0) TC_ACC(12);
       }  // release: the producers may expand the chunk holding this panel
     }
-    if (!P.gemm_only && chain_ok) {  // unpack the final bits of this chain
+    if (!gemm_only && chain_ok) {  // unpack the final bits of this chain
       for (int w = 0; w < N / 32; ++w) {
         const uint32_t x = sm.sbits[w][row];
         uint8_t* dst = P.state + (size_t)chain * N + 32 * w;
@@ -665,6 +699,16 @@ __global__ void __launch_bounds__(kThreads, 1) dense_tc_kernel(TcParams P, const
         for (int b = 0; b < 32; b += 4) {
           const uint32_t e2 = x >> (b >> 1), o2 = x >> (16 + (b >> 1));
           *reinterpret_cast<uint32_t*>(dst + b) = (e2 & 1u) | ((o2 & 1u) << 8) | ((e2 & 2u) << 15) | ((o2 & 2u) << 23);
+        }
+      }
+    }
+    if constexpr (kEnergy) {
+      if (chain_ok) {
+        const double E = -0.5 * e1 - e2;
+        P.energy[chain] = E;
+        if (P.best_energy && E < P.best_energy[chain]) {  // strict: an equal energy keeps the earlier state (gibbs.py:387-391)
+          P.best_energy[chain] = E;
+          unpack_bits(sm, row, N, P.best_state + (size_t)chain * N);
         }
       }
     }
@@ -703,6 +747,15 @@ static int make_j_tensor_map(CUtensorMap* tmap, const void* J, int N) {
   return r == CUDA_SUCCESS ? TSU_OK : TSU_ERR_UNSUPPORTED;
 }
 
+template <int kM, bool kEnergy>
+static cudaError_t launch_tiles(const TcParams& P, const CUtensorMap& tmap, size_t smem, cudaStream_t st) {
+  cudaError_t e = cudaFuncSetAttribute(dense_tc_kernel<kM, kEnergy>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  dense_tc_kernel<kM, kEnergy><<<(P.n_chains + kM - 1) / kM, kThreads, smem, st>>>(P, tmap);
+  return cudaGetLastError();
+}
+
+template <bool kEnergy>
 static int launch_tc(const TcParams& P, cudaStream_t st) {
   const size_t smem = sizeof(TcSmem) + 1024;  // slack: the dynamic shared memory base is only guaranteed 16-byte aligned
   CUtensorMap tmap;
@@ -718,17 +771,7 @@ static int launch_tc(const TcParams& P, cudaStream_t st) {
   cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
   int m = (P.n_chains + 63) / 64 <= sm_count ? 64 : 128;
   if (const char* env = getenv("TSU_TC_M")) m = atoi(env) == 64 ? 64 : 128;  // tile height override (tests; same bits)
-  cudaError_t e;
-  if (m == 64) {
-    e = cudaFuncSetAttribute(dense_tc_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    dense_tc_kernel<64><<<(P.n_chains + 63) / 64, kThreads, smem, st>>>(P, tmap);
-  } else {
-    e = cudaFuncSetAttribute(dense_tc_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    dense_tc_kernel<128><<<(P.n_chains + 127) / 128, kThreads, smem, st>>>(P, tmap);
-  }
-  e = cudaGetLastError();
+  const cudaError_t e = m == 64 ? launch_tiles<64, kEnergy>(P, tmap, smem, st) : launch_tiles<128, kEnergy>(P, tmap, smem, st);
   return e == cudaSuccess ? TSU_OK : (int)e;
 }
 
@@ -755,7 +798,7 @@ extern "C" int tsu_dense_gibbs_tc_run(const void* d_J_bf16, const float* d_bias,
 #ifdef TSU_TC_DEBUG_SWITCHES  // knock-out timing experiments (tools/tc_dbg.py); results are wrong with any bit set
   if (const char* e = getenv("TSU_TC_DEBUG")) P.dbg = atoi(e);
 #endif
-  return launch_tc(P, tsu_stream(stream));
+  return launch_tc<false>(P, tsu_stream(stream));
 }
 
 #ifdef TSU_TC_TIMING
@@ -783,5 +826,24 @@ extern "C" int tsu_dense_tc_debug_fields(const void* d_J_bf16, const uint8_t* d_
 #ifdef TSU_TC_DEBUG_SWITCHES  // knock-out timing experiments (tools/tc_dbg.py); results are wrong with any bit set
   if (const char* e = getenv("TSU_TC_DEBUG")) P.dbg = atoi(e);
 #endif
-  return launch_tc(P, tsu_stream(stream));
+  return launch_tc<false>(P, tsu_stream(stream));
+}
+
+extern "C" int tsu_dense_tc_energy(const void* d_J_bf16, const float* d_bias, const uint8_t* d_state, int n_chains, int N,
+                                   double* d_energy, double* d_best_energy, uint8_t* d_best_state, uintptr_t stream) {
+  TSU_CHECK_ARG(d_J_bf16 && d_state && d_energy && n_chains > 0 && N > 0 && N % 128 == 0 && N <= 4096);
+  TSU_CHECK_ARG((d_best_energy == nullptr) == (d_best_state == nullptr));
+  TcParams P = {};
+  P.J = reinterpret_cast<const __nv_bfloat16*>(d_J_bf16);
+  P.bias = d_bias;
+  P.state = const_cast<uint8_t*>(d_state);  // read only: the energy pass never writes the state
+  P.n_chains = n_chains;
+  P.N = N;
+  P.n_sweeps = 1;
+  P.T = 1.0f;
+  P.gemm_only = 1;
+  P.energy = d_energy;
+  P.best_energy = d_best_energy;
+  P.best_state = d_best_state;
+  return launch_tc<true>(P, tsu_stream(stream));
 }

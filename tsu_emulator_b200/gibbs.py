@@ -66,8 +66,9 @@ class _DenseProblem:
         J = _as_square(coupling)
         self.N = J.shape[0]
         if precision == "bf16":
-            raise ValueError("precision='bf16' (tensor cores) serves sample_boltzmann / sample / sample_chains; "
-                             "this entry point needs a 'float64' or 'float32' sampler")
+            raise ValueError("precision='bf16' (tensor cores) serves sample_boltzmann / sample / sample_chains / "
+                             "simulated_annealing / parallel_tempering; this entry point needs a 'float64' or "
+                             "'float32' sampler")
         if precision not in ("float64", "float32"):
             raise ValueError("precision must be 'float64', 'float32' or 'bf16'")
         if self.N > DENSE_MAX_N[precision]:
@@ -346,17 +347,28 @@ class GibbsSampler:
         """README.md:69-80: `sampler.sample(J, n_samples=1000)` -> (n_samples, n_bits) binary configurations"""
         return self.sample_boltzmann(J, n_samples=n_samples, **kwargs)
 
-    def _tc_sweeps(self, prob: "_TcProblem", st, n_sweeps: int, fields=None):
-        """n_sweeps sequential sweeps of all chains of `st` ([n_chains, Np] uint8, in place) on the tensor cores"""
+    def _tc_sweeps(self, prob: "_TcProblem", st, n_sweeps: int, T, fields=None):
+        """n_sweeps sequential sweeps of all chains of `st` ([n_chains, Np] uint8, in place) on the tensor cores at
+        temperature T: a scalar, or a float64 device tensor [n_chains] of per-chain temperatures"""
         torch = _lib.require_cuda()
         if n_sweeps <= 0:
             return
+        T_chain = T if isinstance(T, torch.Tensor) else None
         with torch.cuda.device(prob.device):
             _lib.call("tsu_dense_gibbs_tc_run", ptr(prob.J), ptr(prob.bias), ptr(st), int(st.shape[0]), prob.Np,
-                      float(self.config.temperature), None, int(n_sweeps), self._seed,
+                      1.0 if T_chain is not None else float(T), ptr(T_chain), int(n_sweeps), self._seed,
                       self._sweep_counter & 0xFFFFFFFF, self._chain_counter & 0xFFFFFFFF, ptr(fields),
                       _lib.current_stream())
         self._sweep_counter += int(n_sweeps)
+
+    @staticmethod
+    def _tc_energy(prob: "_TcProblem", st, energy, best_energy=None, best_state=None):
+        """energy[c] = -1/2 s^T J s - b^T s of every chain of `st` on the tensor cores (bf16 J, float64 sums); with
+        best_energy / best_state, chains whose energy is strictly lower than best_energy take it and their state"""
+        torch = _lib.require_cuda()
+        with torch.cuda.device(prob.device):
+            _lib.call("tsu_dense_tc_energy", ptr(prob.J), ptr(prob.bias), ptr(st), int(st.shape[0]), prob.Np,
+                      ptr(energy), ptr(best_energy), ptr(best_state), _lib.current_stream())
 
     def _sample_boltzmann_tensor(self, coupling, bias, n_samples, burnin, initial_state, n_chains, as_tensor):
         """tsu/gibbs.py:198-211 on csrc/dense_tc.cu: burn-in sweeps, then n_samples x config.n_sweeps sweeps with the
@@ -365,9 +377,10 @@ class GibbsSampler:
         prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
         st = prob.pad_state(self._initial_states(prob, n_chains, initial_state))
         samples = torch.empty((n_samples, n_chains, prob.N), dtype=torch.uint8, device=prob.device)
-        self._tc_sweeps(prob, st, burnin)
+        T = self.config.temperature
+        self._tc_sweeps(prob, st, burnin, T)
         for k in range(n_samples):
-            self._tc_sweeps(prob, st, self.config.n_sweeps)
+            self._tc_sweeps(prob, st, self.config.n_sweeps, T)
             samples[k] = st[:, :prob.N]
         self._chain_counter += n_chains
         self.sample_count += n_samples
@@ -384,18 +397,12 @@ class GibbsSampler:
         prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
         device, N = prob.device, prob.N
         st = prob.pad_state(self._initial_states(prob, int(n_chains), initial_state))
-        self._tc_sweeps(prob, st, int(n_sweeps))
+        self._tc_sweeps(prob, st, int(n_sweeps), self.config.temperature)
         self._chain_counter += int(n_chains)
         energy = None
-        if return_energy:  # E = -1/2 s^T J s - b^T s from one more tensor-core field evaluation
-            H = torch.empty((n_chains, prob.Np), dtype=torch.float32, device=device)
-            with torch.cuda.device(device):
-                _lib.call("tsu_dense_tc_debug_fields", ptr(prob.J), ptr(st), int(n_chains), prob.Np, ptr(H),
-                          _lib.current_stream())
-            sf = st.to(torch.float64)
-            energy = -0.5 * (sf * H.to(torch.float64)).sum(1)
-            if prob.bias is not None:
-                energy = energy - sf @ prob.bias.to(torch.float64)
+        if return_energy:  # E = -1/2 s^T J s - b^T s: one more tensor-core field evaluation, summed on the device
+            energy = torch.empty(int(n_chains), dtype=torch.float64, device=device)
+            self._tc_energy(prob, st, energy)
         st = st[:, :N]
         out = st if as_tensor else _host_int64(st)
         if return_energy:
@@ -423,16 +430,37 @@ class GibbsSampler:
         return out
 
     def parallel_tempering(self, coupling: np.ndarray, temperatures: List[float], bias: Optional[np.ndarray] = None,
-                           n_samples: int = 1000, swap_interval: int = 10, *, _inject=None) -> Tuple[np.ndarray, dict]:
+                           n_samples: int = 1000, swap_interval: int = 10, *, n_ladders: int = 1,
+                           criterion: str = "reference", _inject=None) -> Tuple[np.ndarray, dict]:
         """tsu/gibbs.py:238-338: replicas at `temperatures`, n_sweeps sweeps per iteration, adjacent-pair
         Metropolis swaps every swap_interval iterations, samples from temperature slot 0.
 
-        All replicas advance concurrently (one CTA each); configurations stay in place and the
-        slot -> replica map is permuted by tsu_pt_swap, which reproduces the sequential pair order and
-        the draw-only-if-delta<0 rule of gibbs.py:308-323.  One device->host copy at the end.
+        All replicas advance concurrently (one CTA each on the float64 / float32 kernel, one tensor-core tile row
+        each with precision="bf16"); configurations stay in place and the slot -> replica map is permuted by
+        tsu_pt_swap, which reproduces the sequential pair order and the draw-only-if-delta<0 rule of
+        gibbs.py:308-323.  One device->host copy at the end.
+
+        n_ladders = K independent ladders run in one batch: replica k R + j starts in slot j of ladder k.  With K > 1
+        the samples are (K, n_samples, n_bits) (slot 0 of each ladder), the swap counts are totals over the ladders,
+        and info["energies"] / info["final_states"] hold one entry per ladder, each shaped as for one ladder.
+
+        criterion="reference" keeps the swap expression of gibbs.py:317, which favours moving high-energy
+        configurations to cold slots; "metropolis" is the detailed-balance rule, under which slot 0 samples the
+        Boltzmann distribution at temperatures[0].
         """
         torch = _lib.require_cuda()
-        prob = _DenseProblem(coupling, bias, self.precision, self._dev())
+        K = int(n_ladders)
+        if K < 1:
+            raise ValueError("n_ladders must be at least 1")
+        if criterion not in ("metropolis", "reference"):
+            raise ValueError("criterion must be 'metropolis' or 'reference'")
+        tc = self.precision == "bf16"
+        if _inject is not None and (tc or K > 1):
+            raise ValueError("injected draws are a float64 / float32 parity mode of one ladder")
+        if tc:
+            prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
+        else:
+            prob = _DenseProblem(coupling, bias, self.precision, self._dev())
         device = prob.device
         temps = np.asarray(list(temperatures), dtype=np.float64)
         R = temps.size
@@ -440,28 +468,37 @@ class GibbsSampler:
             raise ValueError("Temperature must be positive")
         n_sweeps = self.config.n_sweeps
         T_slot = torch.from_numpy(temps).to(device)
-        slot_replica = torch.arange(R, dtype=torch.int32, device=device)
-        T_chain = T_slot.clone()
+        slot_replica = torch.arange(K * R, dtype=torch.int32, device=device).view(K, R)
+        T_chain = T_slot.repeat(K)                         # replica k R + j starts at slot j of ladder k
         stats = torch.zeros(2, dtype=torch.int64, device=device)
         inj = _inject
-        states = self._initial_states(prob, R, None if inj is None else np.asarray(inj["inits"]))
-        bu = None
-        if inj is not None:  # parity mode: draws are given per temperature slot; slot i starts on replica i
-            bu = torch.from_numpy(np.ascontiguousarray(np.asarray(inj["burn_uniforms"]).transpose(1, 0, 2))).to(device)
-        self._run(prob, states, n_burnin=self.config.n_burnin, n_samples=0, sweeps_per_sample=0, T_chain=T_chain,
-                  uniforms=bu)
-        samples = torch.empty((n_samples, prob.N), dtype=torch.uint8, device=device)
-        energies = torch.empty((n_samples, R), dtype=torch.float64, device=device)
+        states = self._initial_states(prob, K * R, None if inj is None else np.asarray(inj["inits"]))
+        if tc:
+            states = prob.pad_state(states)
+            e = torch.empty(K * R, dtype=torch.float64, device=device)
+            self._tc_sweeps(prob, states, self.config.n_burnin, T_chain)
+        else:
+            bu = None
+            if inj is not None:  # parity mode: draws are given per temperature slot; slot i starts on replica i
+                bu = torch.from_numpy(np.ascontiguousarray(np.asarray(inj["burn_uniforms"]).transpose(1, 0, 2))).to(device)
+            self._run(prob, states, n_burnin=self.config.n_burnin, n_samples=0, sweeps_per_sample=0, T_chain=T_chain,
+                      uniforms=bu)
+        samples = torch.empty((n_samples, K, prob.N), dtype=torch.uint8, device=device)
+        energies = torch.empty((n_samples, K, R), dtype=torch.float64, device=device)
         for it in range(n_samples):
-            su = None
-            if inj is not None:
-                sr_host = slot_replica.cpu().numpy()
-                u_slot = np.asarray(inj["sweep_uniforms"][it])            # [slot, sweep, N]
-                u_rep = np.empty_like(u_slot)
-                u_rep[sr_host] = u_slot                                    # replica sr_host[i] sits at slot i
-                su = torch.from_numpy(np.ascontiguousarray(u_rep.transpose(1, 0, 2))).to(device)
-            _, e, _, _ = self._run(prob, states, n_burnin=n_sweeps, n_samples=0, sweeps_per_sample=0,
-                                   T_chain=T_chain, want_energy=True, uniforms=su)
+            if tc:
+                self._tc_sweeps(prob, states, n_sweeps, T_chain)
+                self._tc_energy(prob, states, e)
+            else:
+                su = None
+                if inj is not None:
+                    sr_host = slot_replica[0].cpu().numpy()
+                    u_slot = np.asarray(inj["sweep_uniforms"][it])            # [slot, sweep, N]
+                    u_rep = np.empty_like(u_slot)
+                    u_rep[sr_host] = u_slot                                    # replica sr_host[i] sits at slot i
+                    su = torch.from_numpy(np.ascontiguousarray(u_rep.transpose(1, 0, 2))).to(device)
+                _, e, _, _ = self._run(prob, states, n_burnin=n_sweeps, n_samples=0, sweeps_per_sample=0,
+                                       T_chain=T_chain, want_energy=True, uniforms=su)
             energies[it] = e[slot_replica.long()]          # history is kept per temperature slot (gibbs.py:302-303)
             if (it + 1) % swap_interval == 0:
                 wu = None
@@ -469,23 +506,27 @@ class GibbsSampler:
                     wu = torch.from_numpy(np.ascontiguousarray(np.asarray(inj["swap_uniforms"][it], dtype=np.float64))).to(device)
                 self._swap_counter += 1
                 with torch.cuda.device(device):
-                    _lib.call("tsu_pt_swap", ptr(e), ptr(T_slot), ptr(slot_replica), None, 1, R, self._seed,
-                              self._swap_counter & 0xFFFFFFFF, ptr(stats), ptr(wu), 0, _lib.current_stream())
-                T_chain[slot_replica.long()] = T_slot
-            samples[it] = states[slot_replica[0].long()]
-        self._chain_counter += R
+                    _lib.call("tsu_pt_swap", ptr(e), ptr(T_slot), ptr(slot_replica), None, K, R, self._seed,
+                              self._swap_counter & 0xFFFFFFFF, ptr(stats), ptr(wu), 1 if criterion == "metropolis" else 0,
+                              _lib.current_stream())
+                T_chain[slot_replica.long()] = T_slot      # every replica takes the temperature of its new slot
+            samples[it] = states[slot_replica[:, 0].long(), :prob.N]
+        self._chain_counter += K * R
         st = stats.cpu().numpy()
         sr = slot_replica.cpu().numpy()
-        states_np = _host_int64(states)
+        states_np = _host_int64(states[:, :prob.N])
         en = energies.cpu().numpy()
+        energy_lists = [[list(en[:, k, i]) for i in range(R)] for k in range(K)]
+        final_states = [[states_np[sr[k, i]] for i in range(R)] for k in range(K)]
         info = {
             "swap_acceptance_rate": (st[1] / st[0]) if st[0] > 0 else 0,
             "swap_attempts": int(st[0]),
             "swap_accepts": int(st[1]),
-            "energies": [list(en[:, i]) for i in range(R)],
-            "final_states": [states_np[sr[i]] for i in range(R)],
+            "energies": energy_lists[0] if K == 1 else energy_lists,
+            "final_states": final_states[0] if K == 1 else final_states,
         }
-        return _host_int64(samples), info
+        out = _host_int64(samples)                         # (n_samples, K, N)
+        return (out[:, 0, :], info) if K == 1 else (np.ascontiguousarray(out.transpose(1, 0, 2)), info)
 
     def simulated_annealing(self, coupling: np.ndarray, bias: Optional[np.ndarray] = None, T_initial: float = 10.0,
                             T_final: float = 0.1, n_steps: int = 1000, cooling_schedule: str = "exponential", *,
@@ -495,16 +536,41 @@ class GibbsSampler:
 
         The whole anneal is one kernel launch (per-sweep temperature array, on-device best tracking).
         With n_chains > 1 that many independent anneals run concurrently and the best is returned.
+
+        precision="bf16": every step is one tensor-core sweep launch at Ts[k] and one tensor-core energy pass that
+        keeps each chain's best state on the device.  The best chain is chosen by the energies of the bf16 model
+        (the model this path samples); the returned energy is that state's energy under the caller's float64
+        couplings and bias.  The two coincide when the couplings are exact in bf16.
         """
         torch = _lib.require_cuda()
-        prob = self._sparse(coupling, bias) if chromatic else _DenseProblem(coupling, bias, self.precision, self._dev())
+        tc = self.precision == "bf16" and not chromatic
+        if tc:
+            if _uniforms is not None:
+                raise ValueError("injected draws are a float64 / float32 parity mode; precision='bf16' draws Philox")
+            prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
+        elif chromatic:
+            prob = self._sparse(coupling, bias)
+        else:
+            prob = _DenseProblem(coupling, bias, self.precision, self._dev())
         steps = np.arange(n_steps, dtype=np.float64)
         if cooling_schedule == "exponential":
             Ts = T_initial * (T_final / T_initial) ** (steps / n_steps)
         else:  # linear
             Ts = T_initial + (T_final - T_initial) * steps / n_steps
         st = self._initial_states(prob, int(n_chains), _initial_state)
-        if n_steps > 0:
+        if tc and n_steps > 0:
+            st = prob.pad_state(st)
+            energy = torch.empty(int(n_chains), dtype=torch.float64, device=prob.device)
+            best_energy = torch.full((int(n_chains),), float("inf"), dtype=torch.float64, device=prob.device)
+            best_state = torch.empty_like(st)
+            self._tc_energy(prob, st, energy, best_energy, best_state)   # the initial state is the first best
+            for k in range(int(n_steps)):
+                self._tc_sweeps(prob, st, 1, float(Ts[k]))
+                self._tc_energy(prob, st, energy, best_energy, best_state)
+            self.config.temperature = float(Ts[-1])
+            k = int(np.argmin(best_energy.cpu().numpy()))
+            state = _host_int64(best_state[k, :prob.N])
+        elif n_steps > 0:
             T_sweep = torch.from_numpy(Ts).to(prob.device)
             self.config.temperature = float(Ts[-1])  # the reference leaves the last T in the config (gibbs.py:382)
             if chromatic:
