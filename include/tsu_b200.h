@@ -313,6 +313,19 @@ int tsu_pt_swap(const double* d_energy, const double* d_T_slot, int32_t* d_slot_
  *   d_traj: [n_chains][n_steps][dim] sampling-phase trajectory or NULL (core.py:155-156).
  *   d_normals: [n_chains][1 + n_burnin + n_steps][dim] injected N(0,1) draws (parity mode; row 0
  *     is the start jitter) or NULL (Philox + Box-Muller, counter = (chain, pair, step, 'LANG')).
+ *   dim <= 64: one thread per chain, state in registers (every kind; MIXTURE needs n_params <= 20000).
+ *   dim > 64 (csrc/langevin_wide.cu), TSU_ERR_INVALID_ARG past a cap:
+ *     QUADRATIC, DOUBLE_WELL   dim <= 131072 (float64), 262144 (float32): the 16-bit Philox block field
+ *     MIXTURE                  the same, with K <= 16 centres (K = (n_params - 1) / (dim + 1))
+ *     QUADRATIC_FORM           dim <= 2048; A need not be symmetric
+ *   Two rules make the wide kernels the same sampler as the register kernels:
+ *     1. coordinate i takes element i % PER of Philox block b = i / PER, counter
+ *        (chain lo, chain hi & 0xFFFF | b << 16, step, 'LANG'), PER = 2 (float64) or 4 (float32): its draw does not
+ *        depend on dim;
+ *     2. the gradient of coordinate i and its update are the same expressions in the same summation order
+ *        (QUADRATIC_FORM: -b_i, then acc = fma(A_ij, x_j, acc) for ascending j; MIXTURE: d2_k over ascending i, tot and
+ *        g_i over ascending k).
+ *   So a coordinate that does not couple to the others gets the same bits at any dim.
  */
 int tsu_langevin_run(void* d_x, int dtype, int64_t n_chains, int dim, int energy_kind,
                      const double* d_params, int n_params, const void* d_x_init, double jitter,

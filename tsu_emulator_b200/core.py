@@ -69,6 +69,13 @@ class TSUConfig:
 # ----------------------------------------------------------------------------- built-in energies
 ENERGY_QUADRATIC, ENERGY_MIXTURE, ENERGY_DOUBLE_WELL, ENERGY_QUADRATIC_FORM = 0, 1, 2, 3
 
+# Dimension limits (csrc/langevin_wide.cuh).  Up to 64 coordinates every energy runs on the register kernels; above
+# that built-in energies and quadratic forms run on the wide kernels, traced energies do not run.
+MAX_TRACED_DIM = 64
+MAX_DIM = {"float64": 131072, "float32": 262144}  # 16-bit Philox block field x 2 (float64) or 4 (float32) normals
+MAX_QUADRATIC_FORM_DIM = 2048                      # shared-memory chain tile of the wide QUADRATIC_FORM kernel
+MAX_MIXTURE_CENTRES = 16                           # wide MIXTURE kernel: one thread per (chain, centre)
+
 
 class BuiltinEnergy:
     """analytic energy evaluated (and differentiated) inside the fused Langevin kernel"""
@@ -193,6 +200,9 @@ def recognise_quadratic(energy_fn: Callable, dim: int, x0: np.ndarray, rtol: flo
 
     Probes are taken around x0 with unit offsets; the fit is accepted only if it reproduces the callable on
     16 random points (relative 1e-8) - a wrong guess is a SamplingError upstream, never a silent approximation.
+
+    The probes cost 1 + 2d + d(d-1)/2 Python calls: about 5 000 at d = 100 and 525 000 at d = 1024.  For large d
+    pass the form itself as QuadraticFormEnergy(A, b) (or a QuadraticEnergy when it is diagonal).
     """
     x0 = np.asarray(x0, dtype=np.float64).reshape(dim)
 
@@ -253,6 +263,12 @@ class TracedEnergy(BuiltinEnergy):
         return float(self.fn(np.atleast_1d(np.asarray(x, dtype=np.float64))))
 
 
+def _traced_dim_message(dim: int) -> str:
+    return (f"traced Python energies are limited to {MAX_TRACED_DIM} coordinates, got {dim}; built-in energies "
+            "(QuadraticEnergy, GaussianEnergy, MixtureEnergy, DoubleWellEnergy) and quadratic forms "
+            "(QuadraticFormEnergy, or a callable recognised as one) are not")
+
+
 # ----------------------------------------------------------------------------- the sampler
 class ThermalSamplingUnit:
     """tsu/core.py:54-267 with the Langevin loop fused into one CUDA kernel (one thread per chain)."""
@@ -303,6 +319,8 @@ class ThermalSamplingUnit:
             q = recognise_quadratic(energy_fn, x_init.size, x_init)
             if q is not None:
                 return q.as_diagonal() or q
+            if x_init.size > MAX_TRACED_DIM:
+                raise SamplingError(_traced_dim_message(x_init.size))
             from .trace import TraceError
 
             try:
@@ -314,14 +332,31 @@ class ThermalSamplingUnit:
                     ".  Arbitrary Python control flow cannot run on the GPU and this engine has no CPU fallback")
         raise SamplingError("energy must be a built-in energy object, its name, or a Python callable")
 
+    def _check_dim(self, energy: BuiltinEnergy, dim: int):
+        """SamplingError for an energy / dim the kernels do not serve (checked before any device work)"""
+        if dim <= MAX_TRACED_DIM:
+            return
+        if isinstance(energy, TracedEnergy):
+            raise SamplingError(_traced_dim_message(dim))
+        cap = MAX_DIM[self.dtype]
+        if dim > cap:
+            raise SamplingError(f"{type(energy).__name__} supports at most {cap} coordinates in {self.dtype} "
+                                f"(16-bit Philox block index), got {dim}")
+        if energy.kind == ENERGY_QUADRATIC_FORM and dim > MAX_QUADRATIC_FORM_DIM:
+            raise SamplingError(f"a quadratic form with more than 64 coordinates supports at most "
+                                f"{MAX_QUADRATIC_FORM_DIM} coordinates, got {dim} (a diagonal form runs as a "
+                                f"QuadraticEnergy, which has no such limit)")
+        if energy.kind == ENERGY_MIXTURE and len(energy.weights) > MAX_MIXTURE_CENTRES:
+            raise SamplingError(f"a mixture with more than 64 coordinates supports at most {MAX_MIXTURE_CENTRES} "
+                                f"centres, got {len(energy.weights)}")
+
     def _launch(self, energy: BuiltinEnergy, x_init: np.ndarray, n_chains: int, return_trajectory: bool,
                 normals=None, as_tensor: bool = False):
+        dim = x_init.size
+        self._check_dim(energy, dim)
         torch = _lib.require_cuda()
         cfg = self.config
         device = torch.device(self._device) if self._device is not None else torch.device("cuda", torch.cuda.current_device())
-        dim = x_init.size
-        if dim > 64:
-            raise SamplingError("the fused Langevin kernel supports dim <= 64")
         tdt = torch.float32 if self.dtype == "float32" else torch.float64
         code = 0 if self.dtype == "float32" else 1
         params = torch.from_numpy(np.ascontiguousarray(energy.params(dim), dtype=np.float64)).to(device)

@@ -9,7 +9,11 @@
 //   state in registers: gradient + noise + update are one fused loop, HBM is touched only for the
 //   final state (and the optional trajectory).
 //
-// Noise: Philox4x32-10 + Box-Muller, counter = (chain lo, chain hi | call << 16, step, 'LANG').
+// Noise: Philox4x32-10 + Box-Muller, counter = (chain lo, chain hi & 0xFFFF | block << 16, step, 'LANG'); block b of a
+// chain holds coordinates b * PER .. b * PER + PER - 1 (PER = 2 in float64, 4 in float32).
+// dim <= 64 runs here; dim > 64 (built-in energies only) runs on the kernels of langevin_wide.cu, which draw the same
+// normal for every coordinate and evaluate the per-coordinate expressions of langevin_body.cuh in the same order (caps
+// in langevin_wide.cuh and include/tsu_b200.h).
 // Parity mode reads the N(0,1) draws from a caller tensor so that the reference (with
 // numpy.random.randn patched to the same draws) can be compared step for step.
 
@@ -21,6 +25,7 @@
 #include "common.cuh"
 #include "jit.cuh"
 #include "langevin_body.cuh"
+#include "langevin_wide.cuh"
 
 namespace {
 
@@ -38,13 +43,13 @@ __device__ __forceinline__ void gradient(int kind, int dim, const real* __restri
     const real two_a = (real)2 * sp[0];
 #pragma unroll
     for (int i = 0; i < MAXD; ++i)
-      if (i < dim) g[i] = two_a * sp[1 + dim + i] * (x[i] - sp[1 + i]);
+      if (i < dim) g[i] = tsu_langevin::grad_quadratic(two_a, sp[1 + dim + i], x[i], sp[1 + i]);
   } else if (kind == ENERGY_DOUBLE_WELL) {
     // E = sum a (x^2 - b)^2
     const real a4 = (real)4 * sp[0], b = sp[1];
 #pragma unroll
     for (int i = 0; i < MAXD; ++i)
-      if (i < dim) g[i] = a4 * x[i] * (x[i] * x[i] - b);
+      if (i < dim) g[i] = tsu_langevin::grad_double_well(a4, b, x[i]);
   } else if (kind == ENERGY_QUADRATIC_FORM) {
     // E = 1/2 x^T A x - b^T x ; sp = [A[dim][dim], b[dim]] ; grad = A x - b
 #pragma unroll
@@ -53,7 +58,7 @@ __device__ __forceinline__ void gradient(int kind, int dim, const real* __restri
         real acc = -sp[dim * dim + i];
 #pragma unroll
         for (int j = 0; j < MAXD; ++j)
-          if (j < dim) acc += sp[i * dim + j] * x[j];
+          if (j < dim) acc = tsu_langevin::qform_term(acc, sp[i * dim + j], x[j]);
         g[i] = acc;
       }
   } else {
@@ -68,17 +73,14 @@ __device__ __forceinline__ void gradient(int kind, int dim, const real* __restri
       real d2 = (real)0;
 #pragma unroll
       for (int i = 0; i < MAXD; ++i)
-        if (i < dim) {
-          real d = x[i] - c[i];
-          d2 += d * d;
-        }
-      const real e = sp[1 + k] * (real)exp((real)-0.5 * d2);
+        if (i < dim) d2 = tsu_langevin::mixture_d2_term(d2, x[i], c[i]);
+      const real e = tsu_langevin::mixture_weight(sp[1 + k], d2);
       tot += e;
 #pragma unroll
       for (int i = 0; i < MAXD; ++i)
-        if (i < dim) g[i] += e * (x[i] - c[i]);
+        if (i < dim) g[i] = tsu_langevin::mixture_grad_term(g[i], e, x[i], c[i]);
     }
-    const real inv = (real)1 / (tot + (real)1e-10);
+    const real inv = tsu_langevin::mixture_inv(tot);
 #pragma unroll
     for (int i = 0; i < MAXD; ++i)
       if (i < dim) g[i] *= inv;
@@ -137,14 +139,25 @@ extern "C" int tsu_langevin_run(void* d_x, int dtype, int64_t n_chains, int dim,
                                 const double* d_params, int n_params, const void* d_x_init, double jitter,
                                 int first_chain_exact, double T, double dt, double gamma, int n_burnin, int n_steps, uint64_t seed, uint64_t chain0,
                                 const void* d_normals, void* d_traj, uintptr_t stream) {
-  TSU_CHECK_ARG(d_x && d_params && n_chains > 0 && dim > 0 && dim <= kMaxDynDim);
+  TSU_CHECK_ARG(d_x && d_params && n_chains > 0 && dim > 0);
   TSU_CHECK_ARG(dtype == 0 || dtype == 1);
   TSU_CHECK_ARG(T > 0 && dt > 0 && gamma > 0 && n_burnin >= 0 && n_steps >= 0);
   TSU_CHECK_ARG(energy_kind >= 0 && energy_kind <= 3);
+  const bool wide = dim > kMaxDynDim;
+  // dim > 64: the wide kernels (langevin_wide.cu), capped by the 16-bit Philox block field and, for QUADRATIC_FORM, by
+  // the shared-memory chain tile
+  if (wide) TSU_CHECK_ARG(dim <= (dtype == 1 ? tsu_langevin::kWideMaxDimF64 : tsu_langevin::kWideMaxDimF32));
+  if (wide && energy_kind == ENERGY_QUADRATIC_FORM) TSU_CHECK_ARG(dim <= tsu_langevin::kWideMaxDimQForm);
   if (energy_kind == ENERGY_QUADRATIC_FORM) TSU_CHECK_ARG(n_params == dim * dim + dim);
   if (energy_kind == ENERGY_QUADRATIC) TSU_CHECK_ARG(n_params == 1 + 2 * dim);
   if (energy_kind == ENERGY_DOUBLE_WELL) TSU_CHECK_ARG(n_params == 2);
-  if (energy_kind == ENERGY_MIXTURE) TSU_CHECK_ARG(n_params >= 2 + dim && n_params <= 20000);
+  if (energy_kind == ENERGY_MIXTURE && !wide) TSU_CHECK_ARG(n_params >= 2 + dim && n_params <= 20000);
+  int mixture_k = 0;  // wide MIXTURE: params = [K, p[K], c[K][dim]] fixes K = (n_params - 1) / (dim + 1)
+  if (energy_kind == ENERGY_MIXTURE && wide) {
+    TSU_CHECK_ARG(n_params > 1 && (n_params - 1) % (dim + 1) == 0);
+    mixture_k = (n_params - 1) / (dim + 1);
+    TSU_CHECK_ARG(mixture_k <= tsu_langevin::kWideMaxCentres);
+  }
   LangevinParams P;
   P.x = d_x;
   P.x_init = d_x_init;
@@ -164,6 +177,7 @@ extern "C" int tsu_langevin_run(void* d_x, int dtype, int64_t n_chains, int dim,
   P.noise = sqrt(2.0 * T * dt / gamma);
   P.k0 = (uint32_t)seed;
   P.k1 = (uint32_t)(seed >> 32);
+  if (wide) return tsu_langevin::langevin_wide_launch(P, dtype, mixture_k, stream);
   return dtype == 0 ? dispatch_dim<float>(P, tsu_stream(stream)) : dispatch_dim<double>(P, tsu_stream(stream));
 }
 

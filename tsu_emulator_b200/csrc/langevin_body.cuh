@@ -79,6 +79,51 @@ struct BoxMuller<double> {
   }
 };
 
+// The PER = BoxMuller<real>::kPerCall normals of Philox block b of (chain, step): coordinates b*PER .. b*PER+PER-1.
+// The counter does not involve dim, so a coordinate draws the same normal at every dim; the 16-bit block field
+// bounds dim at 65536 * PER.
+template <typename real>
+__device__ __forceinline__ void philox_normals(const LangevinParams& P, unsigned long long chain_g, int b, int step,
+                                               real* t) {
+  tsu_u32x4 o = tsu_philox4x32_10((uint32_t)chain_g, ((uint32_t)(chain_g >> 32) & 0xFFFFu) | ((uint32_t)b << 16),
+                                  (uint32_t)step, TSU_STREAM_LANGEVIN, P.k0, P.k1);
+  BoxMuller<real>::draw(o, t);
+}
+
+// Per-coordinate arithmetic of the built-in energies and of the Euler-Maruyama update.  The register kernels
+// (langevin.cu) and the wide kernels (langevin_wide.cu) both evaluate through these, in the same summation order,
+// so nvcc contracts them the same way in both and a coordinate gets the same bits at every dim.
+// QUADRATIC: dE/dx_i = 2a w_i (x_i - mu_i)
+template <typename real>
+__device__ __forceinline__ real grad_quadratic(real two_a, real w, real x, real mu) { return two_a * w * (x - mu); }
+// DOUBLE_WELL: dE/dx_i = 4a x_i (x_i^2 - b)
+template <typename real>
+__device__ __forceinline__ real grad_double_well(real a4, real b, real x) { return a4 * x * (x * x - b); }
+// QUADRATIC_FORM: g_i = -b_i + sum_j A_ij x_j over ascending j; each term contracts to acc = fma(A_ij, x_j, acc)
+template <typename real>
+__device__ __forceinline__ real qform_term(real acc, real a, real x) { return acc + a * x; }
+// MIXTURE: d2_k = sum_i (x_i - c_ki)^2 over ascending i; e_k = p_k exp(-d2_k / 2); tot = sum_k e_k over ascending k;
+// g_i = (sum_k e_k (x_i - c_ki) over ascending k) / (tot + 1e-10)
+template <typename real>
+__device__ __forceinline__ real mixture_d2_term(real d2, real x, real c) {
+  real d = x - c;
+  return d2 + d * d;
+}
+template <typename real>
+__device__ __forceinline__ real mixture_weight(real p, real d2) { return p * (real)exp((real)-0.5 * d2); }
+template <typename real>
+__device__ __forceinline__ real mixture_grad_term(real g, real e, real x, real c) { return g + e * (x - c); }
+template <typename real>
+__device__ __forceinline__ real mixture_inv(real tot) { return (real)1 / (tot + (real)1e-10); }
+// restart jitter: x <- x_init + jitter z  (core.py:142-143)
+template <typename real>
+__device__ __forceinline__ real jitter_start(real x, real jitter, real z) { return x + jitter * z; }
+// x <- x - g dt/gamma + sqrt(2 T dt/gamma) z  (core.py:74-80 order of operations)
+template <typename real>
+__device__ __forceinline__ real em_update(real x, real g, real z, real drift, real noise) {
+  return x + (-g * drift) + noise * z;
+}
+
 // N(0,1) vector for (chain, step): injected rows or Philox + Box-Muller
 template <typename real, int DIM>
 __device__ __forceinline__ void normal_vector(const LangevinParams& P, unsigned long long chain_g, long long chain_l,
@@ -96,10 +141,8 @@ __device__ __forceinline__ void normal_vector(const LangevinParams& P, unsigned 
 #pragma unroll
   for (int b = 0; b < (MAXD + PER - 1) / PER; ++b) {
     if (b * PER < dim) {
-      tsu_u32x4 o = tsu_philox4x32_10((uint32_t)chain_g, ((uint32_t)(chain_g >> 32) & 0xFFFFu) | ((uint32_t)b << 16),
-                                      (uint32_t)step, TSU_STREAM_LANGEVIN, P.k0, P.k1);
       real t[PER];
-      BoxMuller<real>::draw(o, t);
+      philox_normals<real>(P, chain_g, b, step, t);
 #pragma unroll
       for (int q = 0; q < PER; ++q)
         if (b * PER + q < MAXD && b * PER + q < dim) z[b * PER + q] = t[q];
@@ -127,7 +170,7 @@ __device__ __forceinline__ void langevin_chain(const LangevinParams& P, const Gr
     normal_vector<real, DIM>(P, chain_g, chain, 0, dim, z);
 #pragma unroll
     for (int i = 0; i < MAXD; ++i)
-      if (i < dim) x[i] = x[i] + (real)P.jitter * z[i];
+      if (i < dim) x[i] = jitter_start(x[i], (real)P.jitter, z[i]);
   }
   const real drift = (real)P.drift, noise = (real)P.noise;
   const int total = P.n_burnin + P.n_steps;
@@ -137,7 +180,7 @@ __device__ __forceinline__ void langevin_chain(const LangevinParams& P, const Gr
     normal_vector<real, DIM>(P, chain_g, chain, s + 1, dim, z);
 #pragma unroll
     for (int i = 0; i < MAXD; ++i)
-      if (i < dim) x[i] = x[i] + (-g[i] * drift) + noise * z[i];  // core.py:74-80 order of operations
+      if (i < dim) x[i] = em_update(x[i], g[i], z[i], drift, noise);
     if (traj && s >= P.n_burnin) {
       real* dst = traj + ((size_t)chain * P.n_steps + (s - P.n_burnin)) * dim;
 #pragma unroll
