@@ -184,6 +184,49 @@ int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_r
                                         double h, int64_t n_bonds, int64_t n_sites,
                                         double* d_energy, uintptr_t stream);
 
+/* Edwards-Anderson +-J lattices: coupling J_ij = J sigma_ij with a sign sigma_ij = +-1 per nearest-neighbour bond.
+ * The field of the bit model is 4J u' + 2h - 2J d, with u' the number of neighbours j with b_j XOR [sigma_ij = -1]:
+ * the ferromagnet's threshold tables (bias "physical") serve it unchanged, so every rule above (Philox stream, ties,
+ * kernels chosen) holds; the neighbour words are XOR-ed with bond words before the up-count.  Whole lattices only
+ * (no row slabs or halos); the run-time specialised kernel has no bonded form.
+ *
+ * d_signs: int8 [n_real][2][rows][cols]; [k][0][i][j] is the bond (i,j)-(i,(j+1) mod cols), [k][1][i][j] the bond
+ *   (i,j)-((i+1) mod rows,j); a value < 0 is antiferromagnetic.  Bonds the wiring does not create (open edges, a
+ *   wrap that is off) are ignored.
+ * d_bonds: uint32 [n_real][colour][4: N, S, W, E][rows][wpr], aligned with the state words: bit b of word w is 1 iff
+ *   the bond between own-colour lane 32w+b and that neighbour is antiferromagnetic (absent neighbours and padding
+ *   lanes 0).  8 * rows * wpr words per realisation.
+ * d_bond_index: [n_replicas] realisation of each replica, or NULL (all use realisation 0). */
+int tsu_ising2d_pack_bonds(const int8_t* d_signs, uint32_t* d_bonds, int n_real, int rows, int cols,
+                           int wrap_rows, int wrap_cols, uintptr_t stream);
+/* tsu_ising2d_sweeps with bonds (same launch paths: resident, wide + rim, generic, row ranges, replica chunks) */
+int tsu_ising2d_sweeps_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
+                              int wrap_cols, const uint32_t* d_lut, const int32_t* d_lut_index,
+                              const uint32_t* d_bonds, const int32_t* d_bond_index, uint64_t seed,
+                              uint32_t sweep0, int n_sweeps, uint32_t replica0, uintptr_t stream);
+/* one half-sweep of `colour` restricted to rows [row_begin, row_end) (0, rows: all) */
+int tsu_ising2d_half_sweep_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
+                                  int wrap_cols, int colour, const uint32_t* d_lut,
+                                  const int32_t* d_lut_index, const uint32_t* d_bonds,
+                                  const int32_t* d_bond_index, uint64_t seed, uint32_t sweep,
+                                  uint32_t replica0, int row_begin, int row_end, uintptr_t stream);
+int tsu_ising2d_half_sweep_injected_bonded(uint32_t* d_state, int n_replicas, int rows, int cols,
+                                           int wrap_rows, int wrap_cols, int colour,
+                                           const uint32_t* d_lut, const int32_t* d_lut_index,
+                                           const uint32_t* d_bonds, const int32_t* d_bond_index,
+                                           const uint32_t* d_uniforms, uintptr_t stream);
+/* d_out[replica][0] = up spins, d_out[replica][1] = UNSATISFIED bonds (sigma_ij s_i s_j = -1), so that
+ * tsu_ising2d_energy_from_observables gives E = -J sum sigma_ij s_i s_j - h sum s_i unchanged */
+int tsu_ising2d_observables_bonded(const uint32_t* d_state, int n_replicas, int rows, int cols,
+                                   int wrap_rows, int wrap_cols, const uint32_t* d_bonds,
+                                   const int32_t* d_bond_index, unsigned long long* d_out,
+                                   uintptr_t stream);
+/* spin overlap: d_out[q] = number of sites where replicas d_pairs[2q] and d_pairs[2q+1] differ
+ * (q_ab = 1 - 2 d_out / (rows cols)); 1 <= n_pairs <= 65535, indices in [0, n_replicas) */
+int tsu_ising2d_overlap(const uint32_t* d_state, int n_replicas, int rows, int cols,
+                        const int32_t* d_pairs, int n_pairs, unsigned long long* d_out,
+                        uintptr_t stream);
+
 /* ------------------------------------------------------------------ dense-J Gibbs ----- */
 /*
  * Replaces GibbsSampler.gibbs_sweep / sample_boltzmann / compute_energy and the sweep part of

@@ -90,6 +90,26 @@ SIGNATURES = {
         c_int,
         [c_void_p, c_int, c_double, c_double, c_int64, c_int64, c_void_p, c_uintptr],
     ),
+    "tsu_ising2d_pack_bonds": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_uintptr]),
+    "tsu_ising2d_sweeps_bonded": (
+        c_int,
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_uint64, c_uint32, c_int,
+         c_uint32, c_uintptr],
+    ),
+    "tsu_ising2d_half_sweep_bonded": (
+        c_int,
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_uint64, c_uint32,
+         c_uint32, c_int, c_int, c_uintptr],
+    ),
+    "tsu_ising2d_half_sweep_injected_bonded": (
+        c_int,
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_uintptr],
+    ),
+    "tsu_ising2d_observables_bonded": (
+        c_int,
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_uintptr],
+    ),
+    "tsu_ising2d_overlap": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_uintptr]),
     "tsu_dense_gibbs_run": (
         c_int,
         [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_void_p, c_int, c_int, c_int,

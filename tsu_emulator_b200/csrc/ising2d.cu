@@ -42,6 +42,13 @@ using tsu_fast::opp_row;
 using tsu_fast::Coords;
 using tsu_fast::lattice_call;
 using tsu_fast::SweepParams;
+using tsu_fast::BondParams;
+using tsu_fast::kBondN;
+using tsu_fast::kBondS;
+using tsu_fast::kBondW;
+using tsu_fast::kBondE;
+
+constexpr BondParams kNoBonds = {nullptr, nullptr};
 
 __device__ __forceinline__ uint32_t lane_mask_lt(int n) {  // lanes [0, n), n clamped to [0, 32]
   return n >= 32 ? 0xffffffffu : (n <= 0 ? 0u : ((1u << n) - 1u));
@@ -97,6 +104,18 @@ __device__ __forceinline__ Hood load_hood(const Planes& P, const Geom& g, int co
     if (last >= 0 && (last >> 5) == w && 2 * last + 1 >= g.cols) h.missE = 1u << (last & 31);  // odd cols
   }
   return h;
+}
+
+// Bonded lattices: XOR the four neighbour words of (colour, local row i, word w) with their bond words, so that every
+// count taken from the hood counts bond-satisfying neighbours (absent neighbours keep reading 0: their bits are 0)
+__device__ __forceinline__ void apply_bonds(Hood& h, const BondParams& B, const Geom& g, int rep, int colour, int i, int w) {
+  const size_t plane = (size_t)g.rows * g.wpr;
+  const uint32_t* b = tsu_fast::bond_base(B, g, rep, colour) + (size_t)i * g.wpr + w;
+  const int p = (g.row0 + i + colour) & 1;  // own columns odd: the centre word is the west neighbour
+  h.n ^= b[kBondN * plane];
+  h.s ^= b[kBondS * plane];
+  h.c ^= b[(p ? kBondW : kBondE) * plane];
+  h.side ^= b[(p ? kBondE : kBondW) * plane];
 }
 
 // ---- bit-sliced acceptance -------------------------------------------------------------
@@ -214,12 +233,12 @@ __device__ __forceinline__ unsigned long long trace_now() {
 }
 #endif
 
-template <int W, int MINB>
-__global__ void __launch_bounds__(128, MINB) half_sweep_fast_kernel(SweepParams P) {
+template <int W, int MINB, bool BONDED>
+__global__ void __launch_bounds__(128, MINB) half_sweep_fast_kernel(SweepParams P, BondParams B) {
 #ifdef TSU_LATTICE_TRACE
   const unsigned long long t_start = trace_now();
 #endif
-  tsu_fast::half_sweep_fast_body<W>(P);
+  tsu_fast::half_sweep_fast_body<W, BONDED>(P, B);
 #ifdef TSU_LATTICE_TRACE
   __syncthreads();
   if (threadIdx.x == 0 && blockIdx.x < kTraceCtas) {
@@ -234,7 +253,9 @@ __global__ void __launch_bounds__(128, MINB) half_sweep_fast_kernel(SweepParams 
 }
 
 // One word of (replica rep, colour, local row i): any size, open or periodic edges, ragged last word.
-__device__ __forceinline__ void generic_update_one(const SweepParams& P, int colour, uint32_t sweep, int rep, int i, int w) {
+template <bool BONDED>
+__device__ __forceinline__ void generic_update_one(const SweepParams& P, const BondParams& B, int colour, uint32_t sweep,
+                                                   int rep, int i, int w) {
   const Geom& g = P.g;
   const size_t plane = (size_t)g.rows * g.wpr;
   uint32_t* own = P.state + ((size_t)rep * 2 + colour) * plane;
@@ -244,8 +265,9 @@ __device__ __forceinline__ void generic_update_one(const SweepParams& P, int col
   pl.halo_bot = P.halo_bot ? P.halo_bot + (size_t)rep * g.wpr : nullptr;
   const uint32_t* lut = P.lut + (P.lut_index ? (size_t)P.lut_index[rep] * 32 : 0);
 
-  const Hood h = load_hood(pl, g, colour, i, w);
+  Hood h = load_hood(pl, g, colour, i, w);
   if (h.valid == 0u) return;  // padding word (stays 0)
+  if constexpr (BONDED) apply_bonds(h, B, g, rep, colour, i, w);
   const int d_row = 2 + h.has_n + h.has_s;
   LutRegs L;
   load_lut_regs(L, lut, d_row);
@@ -260,7 +282,8 @@ __device__ __forceinline__ void generic_update_one(const SweepParams& P, int col
 }
 
 // Generic path: one thread per word, one launch per half-sweep.
-__global__ void __launch_bounds__(128) half_sweep_generic_kernel(SweepParams P) {
+template <bool BONDED>
+__global__ void __launch_bounds__(128) half_sweep_generic_kernel(SweepParams P, BondParams B) {
   // rows [P.row_begin, P.row_end) of every replica
   const Geom& g = P.g;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -269,7 +292,7 @@ __global__ void __launch_bounds__(128) half_sweep_generic_kernel(SweepParams P) 
   const int rep = (int)(tid / per_rep);
   const int rem = (int)(tid - (long long)rep * per_rep);
   const int i = rem / g.wpr;
-  generic_update_one(P, P.colour, P.sweep, rep, P.row_begin + i, rem - i * g.wpr);
+  generic_update_one<BONDED>(P, B, P.colour, P.sweep, rep, P.row_begin + i, rem - i * g.wpr);
 }
 
 // Small lattices (C1: 50 x 50): the whole replica belongs to ONE thread block, which runs both colours of
@@ -277,7 +300,8 @@ __global__ void __launch_bounds__(128) half_sweep_generic_kernel(SweepParams P) 
 // coordinates, same bits as the per-half-sweep launches - it only removes 2 n_sweeps - 1 kernel launches,
 // which is all the time there is at this size.
 constexpr int kResidentThreads = 256;
-__global__ void __launch_bounds__(kResidentThreads) sweeps_resident_kernel(SweepParams P, int n_sweeps) {
+template <bool BONDED>
+__global__ void __launch_bounds__(kResidentThreads) sweeps_resident_kernel(SweepParams P, int n_sweeps, BondParams B) {
   const Geom& g = P.g;
   const int rep = blockIdx.x;
   const int per_rep = g.rows * g.wpr;
@@ -285,7 +309,7 @@ __global__ void __launch_bounds__(kResidentThreads) sweeps_resident_kernel(Sweep
     for (int colour = 0; colour < 2; ++colour) {
       for (int rem = threadIdx.x; rem < per_rep; rem += kResidentThreads) {
         const int i = rem / g.wpr;
-        generic_update_one(P, colour, P.sweep + (uint32_t)t, rep, i, rem - i * g.wpr);
+        generic_update_one<BONDED>(P, B, colour, P.sweep + (uint32_t)t, rep, i, rem - i * g.wpr);
       }
       __syncthreads();  // the other colour reads what this half-sweep wrote (same SM: L1 is coherent for its own stores)
     }
@@ -303,7 +327,8 @@ struct RimRows {
   int head, tail_begin;
 };
 
-__global__ void __launch_bounds__(128) half_sweep_rim_kernel(SweepParams P, RimRows R) {
+template <bool BONDED>
+__global__ void __launch_bounds__(128) half_sweep_rim_kernel(SweepParams P, RimRows R, BondParams B) {
   const Geom& g = P.g;
   const int na = R.a1 - R.a0, nb = R.b1 - R.b0;
   const int full_rows = na + nb;
@@ -324,11 +349,13 @@ __global__ void __launch_bounds__(128) half_sweep_rim_kernel(SweepParams P, RimR
     i = R.p0 + r;
     w = (R.head && k == 0) ? 0 : R.tail_begin + (k - R.head);
   }
-  generic_update_one(P, P.colour, P.sweep, rep, i, w);
+  generic_update_one<BONDED>(P, B, P.colour, P.sweep, rep, i, w);
 }
 
 // Parity mode: uniforms injected per site.  One thread per word, one lane at a time.
-__global__ void __launch_bounds__(128) half_sweep_injected_kernel(SweepParams P, const uint32_t* __restrict__ uniforms) {
+template <bool BONDED>
+__global__ void __launch_bounds__(128) half_sweep_injected_kernel(SweepParams P, const uint32_t* __restrict__ uniforms,
+                                                                  BondParams B) {
   const Geom& g = P.g;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long per_rep = (long long)g.rows * g.wpr;
@@ -344,8 +371,9 @@ __global__ void __launch_bounds__(128) half_sweep_injected_kernel(SweepParams P,
   pl.halo_top = P.halo_top ? P.halo_top + (size_t)rep * g.wpr : nullptr;
   pl.halo_bot = P.halo_bot ? P.halo_bot + (size_t)rep * g.wpr : nullptr;
   const uint32_t* lut = P.lut + (P.lut_index ? (size_t)P.lut_index[rep] * 32 : 0);
-  const Hood h = load_hood(pl, g, P.colour, i, w);
+  Hood h = load_hood(pl, g, P.colour, i, w);
   if (h.valid == 0u) return;
+  if constexpr (BONDED) apply_bonds(h, B, g, rep, P.colour, i, w);
   const int p = (g.row0 + i + P.colour) & 1;
   const uint32_t* urow = uniforms + ((size_t)rep * g.rows + i) * g.cols;
   uint32_t out = 0u;
@@ -422,10 +450,11 @@ __global__ void unpack_kernel(const uint32_t* __restrict__ state, int8_t* spins,
   }
 }
 
-// up-spin count and anti-aligned (right + down) bond count per replica
+// up-spin count and anti-aligned (right + down) bond count per replica; bonded: unsatisfied bonds (sigma s_i s_j = -1)
+template <bool BONDED>
 __global__ void __launch_bounds__(256) observables_kernel(const uint32_t* __restrict__ state, Geom g,
                                                          const uint32_t* __restrict__ next_rows,
-                                                         unsigned long long* out) {
+                                                         unsigned long long* out, BondParams B) {
   const int rep = blockIdx.y;
   const size_t plane = (size_t)g.rows * g.wpr;
   const long long n_words = 2LL * g.rows * g.wpr;
@@ -441,8 +470,9 @@ __global__ void __launch_bounds__(256) observables_kernel(const uint32_t* __rest
     pl.opp = state + ((size_t)rep * 2 + (1 - colour)) * plane;
     pl.halo_top = nullptr;
     pl.halo_bot = next_rows ? next_rows + ((size_t)rep * 2 + (1 - colour)) * g.wpr : nullptr;
-    const Hood h = load_hood(pl, g, colour, i, w);
+    Hood h = load_hood(pl, g, colour, i, w);
     if (h.valid == 0u) continue;
+    if constexpr (BONDED) apply_bonds(h, B, g, rep, colour, i, w);
     const uint32_t x = own[(size_t)i * g.wpr + w];
     const int p = (g.row0 + i + colour) & 1;
     ups += __popc(x & h.valid);
@@ -464,9 +494,11 @@ __global__ void __launch_bounds__(256) observables_kernel(const uint32_t* __rest
 // loaded once as a 16-byte vector.  In a row exactly one colour has odd own columns (east neighbour = next lane of
 // the other plane, i.e. a 1-bit funnel shift that needs one extra word); the other colour's east neighbour is the
 // same lane.  The south neighbour of (colour, row i, lane) is (other colour, row i+1, same lane).
+// Bonded: the east and south bond words of both colours are XOR-ed into the pairs, which counts unsatisfied bonds.
+template <bool BONDED>
 __global__ void __launch_bounds__(128) observables_fast_kernel(const uint32_t* __restrict__ state, Geom g,
                                                               const uint32_t* __restrict__ next_rows, int strip_rows,
-                                                              int n_strips, unsigned long long* out) {
+                                                              int n_strips, unsigned long long* out, BondParams B) {
   const int nvec = g.wpr >> 2;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int per_rep = n_strips * nvec;
@@ -502,6 +534,18 @@ __global__ void __launch_bounds__(128) observables_fast_kernel(const uint32_t* _
       const uint32_t x0[4] = {a[0].x, a[0].y, a[0].z, a[0].w}, x1[4] = {a[1].x, a[1].y, a[1].z, a[1].w};
       const uint32_t* own_odd = odd ? x1 : x0;   // colour with the shifted east neighbour
       const uint32_t* own_even = odd ? x0 : x1;
+      // bond words of row i: east of either colour, south of colour 0 / 1 (all 0 for the ferromagnet)
+      uint4 be_odd = make_uint4(0u, 0u, 0u, 0u), be_even = be_odd, bs0 = be_odd, bs1 = be_odd;
+      if constexpr (BONDED) {
+        const size_t off = (size_t)i * g.wpr + w0;
+        const uint32_t* b0 = tsu_fast::bond_base(B, g, rep, 0) + off;
+        const uint32_t* b1 = tsu_fast::bond_base(B, g, rep, 1) + off;
+        be_odd = *reinterpret_cast<const uint4*>((odd ? b1 : b0) + kBondE * plane);
+        be_even = *reinterpret_cast<const uint4*>((odd ? b0 : b1) + kBondE * plane);
+        bs0 = *reinterpret_cast<const uint4*>(b0 + kBondS * plane);
+        bs1 = *reinterpret_cast<const uint4*>(b1 + kBondS * plane);
+      }
+      const uint32_t eo[4] = {be_odd.x, be_odd.y, be_odd.z, be_odd.w}, ee[4] = {be_even.x, be_even.y, be_even.z, be_even.w};
       // (own_even is also the plane the odd colour looks at, and vice versa)
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
@@ -510,10 +554,18 @@ __global__ void __launch_bounds__(128) observables_fast_kernel(const uint32_t* _
         // open columns: the last site of a row with odd own columns has no east neighbour
         const uint32_t has_east = (k == 3 && !g.wrap_cols && w0 + 4 == g.wpr) ? 0x7fffffffu : 0xffffffffu;
         ups += __popc(x0[k]) + __popc(x1[k]);
-        anti += __popc((own_odd[k] ^ east_odd) & has_east) + __popc(own_even[k] ^ own_odd[k]);
+        if constexpr (BONDED)
+          anti += __popc((own_odd[k] ^ east_odd ^ eo[k]) & has_east) + __popc(own_even[k] ^ own_odd[k] ^ ee[k]);
+        else
+          anti += __popc((own_odd[k] ^ east_odd) & has_east) + __popc(own_even[k] ^ own_odd[k]);
       }
-      if (s1) anti += __popc(a[0].x ^ b[1].x) + __popc(a[0].y ^ b[1].y) + __popc(a[0].z ^ b[1].z) + __popc(a[0].w ^ b[1].w);
-      if (s0) anti += __popc(a[1].x ^ b[0].x) + __popc(a[1].y ^ b[0].y) + __popc(a[1].z ^ b[0].z) + __popc(a[1].w ^ b[0].w);
+      if constexpr (BONDED) {
+        if (s1) anti += __popc(a[0].x ^ b[1].x ^ bs0.x) + __popc(a[0].y ^ b[1].y ^ bs0.y) + __popc(a[0].z ^ b[1].z ^ bs0.z) + __popc(a[0].w ^ b[1].w ^ bs0.w);
+        if (s0) anti += __popc(a[1].x ^ b[0].x ^ bs1.x) + __popc(a[1].y ^ b[0].y ^ bs1.y) + __popc(a[1].z ^ b[0].z ^ bs1.z) + __popc(a[1].w ^ b[0].w ^ bs1.w);
+      } else {
+        if (s1) anti += __popc(a[0].x ^ b[1].x) + __popc(a[0].y ^ b[1].y) + __popc(a[0].z ^ b[1].z) + __popc(a[0].w ^ b[1].w);
+        if (s0) anti += __popc(a[1].x ^ b[0].x) + __popc(a[1].y ^ b[0].y) + __popc(a[1].z ^ b[0].z) + __popc(a[1].w ^ b[0].w);
+      }
       a[0] = b[0];
       a[1] = b[1];
     }
@@ -532,6 +584,61 @@ __global__ void energy_from_obs_kernel(const unsigned long long* __restrict__ ob
   const double up = (double)obs[2 * r];
   const double anti = (double)obs[2 * r + 1];
   energy[r] = -J * ((double)n_bonds - 2.0 * anti) - h * (2.0 * up - (double)n_sites);
+}
+
+// ---- Edwards-Anderson bonds ---------------------------------------------------------------------------------
+// int8 signs[k][2][rows][cols] ([.,0,i,j]: bond (i,j)-(i,j+1 mod cols), [.,1,i,j]: bond (i,j)-(i+1 mod rows,j); < 0
+// = antiferromagnetic) -> bond words[k][colour][N,S,W,E][rows][wpr].  Bonds the wiring does not create (open edges;
+// a wrap that is off) leave their bits 0, and so do padding lanes.  One thread per word.
+__global__ void pack_bonds_kernel(const int8_t* __restrict__ signs, uint32_t* bonds, int n_real, Geom g) {
+  const long long plane = (long long)g.rows * g.wpr;
+  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (tid >= (long long)n_real * 8 * plane) return;
+  const int k = (int)(tid / (8 * plane));
+  long long rem = tid - (long long)k * 8 * plane;
+  const int colour = (int)(rem / (4 * plane));
+  rem -= (long long)colour * 4 * plane;
+  const int dir = (int)(rem / plane);
+  rem -= (long long)dir * plane;
+  const int i = (int)(rem / g.wpr);
+  const int w = (int)(rem - (long long)i * g.wpr);
+  const int p = (i + colour) & 1;
+  const int nk = colour_count(g.cols, p);
+  const int8_t* horiz = signs + ((size_t)k * 2 * g.rows) * g.cols;
+  const int8_t* vert = horiz + (size_t)g.rows * g.cols;
+  uint32_t x = 0u;
+  for (int j = 0; j < 32; ++j) {
+    const int kk = 32 * w + j;
+    if (kk >= nk) break;
+    const int col = 2 * kk + p;
+    int8_t sgn = 1;
+    if (dir == kBondN) {
+      if (i > 0 || g.wrap_rows) sgn = vert[(size_t)(i > 0 ? i - 1 : g.rows - 1) * g.cols + col];
+    } else if (dir == kBondS) {
+      if (i + 1 < g.rows || g.wrap_rows) sgn = vert[(size_t)i * g.cols + col];
+    } else if (dir == kBondW) {
+      if (col > 0 || g.wrap_cols) sgn = horiz[(size_t)i * g.cols + (col > 0 ? col - 1 : g.cols - 1)];
+    } else {
+      if (col + 1 < g.cols || g.wrap_cols) sgn = horiz[(size_t)i * g.cols + col];
+    }
+    if (sgn < 0) x |= 1u << j;
+  }
+  bonds[tid] = x;
+}
+
+// number of sites at which replicas pairs[2q] and pairs[2q+1] differ, for every pair q (padding bits are 0 in both)
+__global__ void __launch_bounds__(256) overlap_kernel(const uint32_t* __restrict__ state, long long rep_vecs,
+                                                      const int32_t* __restrict__ pairs, unsigned long long* out) {
+  const int q = blockIdx.y;
+  const uint4* a = reinterpret_cast<const uint4*>(state) + (size_t)pairs[2 * q] * rep_vecs;
+  const uint4* b = reinterpret_cast<const uint4*>(state) + (size_t)pairs[2 * q + 1] * rep_vecs;
+  unsigned long long diff = 0;
+  for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < rep_vecs; t += (long long)gridDim.x * blockDim.x) {
+    const uint4 x = a[t], y = b[t];
+    diff += __popc(x.x ^ y.x) + __popc(x.y ^ y.y) + __popc(x.z ^ y.z) + __popc(x.w ^ y.w);
+  }
+  diff = tsu_warp_sum(diff);
+  if ((threadIdx.x & 31) == 0 && diff) atomicAdd(out + q, diff);
 }
 
 // ---- row slabs with peer-mapped halos (tsu_ising2d_slab_sweeps_p2p) ---------------------------------------
@@ -669,8 +776,10 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
                       const uint32_t* d_lut, const int32_t* d_lut_index, uint64_t seed, uint32_t sweep,
                       uint32_t replica0, int row0, const uint32_t* d_halo_top, const uint32_t* d_halo_bot,
                       cudaStream_t st, JitKernel jit = JitKernel{nullptr, 0, 0}, int upd_begin = 0, int upd_end = -1,
-                      int pieces = 1) {
+                      int pieces = 1, BondParams B = kNoBonds) {
   // pieces: this launch is one of `pieces` row ranges of a half-sweep that run concurrently (split_ranges())
+  // B.words: +-J bonds (bonded kernels; the specialised kernel has no bonded form and is never used for them)
+  const bool bonded = B.words != nullptr;
   if (upd_end < 0) upd_end = rows;  // local rows [upd_begin, upd_end) are updated (default: all)
   if (upd_begin >= upd_end) return TSU_OK;
   SweepParams P;
@@ -702,7 +811,7 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
   bool fast = nvec_f >= 1 && re - rb >= 1;
   if (need_rim && tuning().open_generic) fast = false;
   if (fast) {
-    const bool use_jit = jit.fn && !d_lut_index;
+    const bool use_jit = jit.fn && !d_lut_index && !bonded;
     const int W = use_jit ? jit.w : (tuning().w == 2 ? 2 : kDefaultW);
     const int nvec = nvec_f * (4 / W);  // W-word groups per row
     const int frows = re - rb;
@@ -725,10 +834,15 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
     if (use_jit) {  // table-specialised build of the same kernel body
       void* args[] = {&P};
       if (tsu_jit::launch(jit.fn, blocks_for(total, jit.threads), jit.threads, 0, (void*)st, args) != 0) return 999;  // driver-API launch failure
+    } else if (bonded) {  // one CTA per SM fewer: the next row's 4 W bond words stay in registers without spills
+      if (W == 2)
+        half_sweep_fast_kernel<2, 6, true><<<grid, 128, 0, st>>>(P, B);
+      else
+        half_sweep_fast_kernel<4, 3, true><<<grid, 128, 0, st>>>(P, B);
     } else if (W == 2) {
-      half_sweep_fast_kernel<2, 8><<<grid, 128, 0, st>>>(P);
+      half_sweep_fast_kernel<2, 8, false><<<grid, 128, 0, st>>>(P, kNoBonds);
     } else {
-      half_sweep_fast_kernel<4, 4><<<grid, 128, 0, st>>>(P);
+      half_sweep_fast_kernel<4, 4, false><<<grid, 128, 0, st>>>(P, kNoBonds);
     }
     if (need_rim) {
       RimRows R;
@@ -739,7 +853,12 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
       R.tail_begin = ragged ? 4 * nvec_f : (wrap_cols ? P.g.wpr : P.g.wpr - 1);
       const long long per_rep = (long long)((R.a1 - R.a0) + (R.b1 - R.b0)) * P.g.wpr +
                                 (long long)(R.head + P.g.wpr - R.tail_begin) * frows;
-      if (per_rep > 0) half_sweep_rim_kernel<<<blocks_for(per_rep * n_replicas, 128), 128, 0, st>>>(P, R);
+      if (per_rep > 0) {
+        if (bonded)
+          half_sweep_rim_kernel<true><<<blocks_for(per_rep * n_replicas, 128), 128, 0, st>>>(P, R, B);
+        else
+          half_sweep_rim_kernel<false><<<blocks_for(per_rep * n_replicas, 128), 128, 0, st>>>(P, R, kNoBonds);
+      }
     }
   } else {
     P.strip_rows = 1;
@@ -747,7 +866,10 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
     P.row_begin = upd_begin;
     P.row_end = upd_end;
     const long long total = (long long)n_replicas * (upd_end - upd_begin) * P.g.wpr;
-    half_sweep_generic_kernel<<<blocks_for(total, 128), 128, 0, st>>>(P);
+    if (bonded)
+      half_sweep_generic_kernel<true><<<blocks_for(total, 128), 128, 0, st>>>(P, B);
+    else
+      half_sweep_generic_kernel<false><<<blocks_for(total, 128), 128, 0, st>>>(P, kNoBonds);
   }
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? TSU_OK : (int)e;
@@ -781,7 +903,7 @@ int split_replicas(int n_replicas, int rows, int cols) {
 // the whole-lattice sweeps of tsu_ising2d_sweeps / _sweeps_jit (no halos)
 int launch_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols, const uint32_t* d_lut,
                   const int32_t* d_lut_index, uint64_t seed, uint32_t sweep0, int n_sweeps, uint32_t replica0,
-                  cudaStream_t st, JitKernel jit) {
+                  cudaStream_t st, JitKernel jit, BondParams B = kNoBonds) {
   // many replicas: independent chunks of replicas, one stream each, no dependency between them at all
   const int KR = split_replicas(n_replicas, rows, cols);
   if (KR > 1 && n_sweeps > 0) {
@@ -800,10 +922,11 @@ int launch_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wra
       }
       if (k > 0) cudaStreamWaitEvent(sk, ev_join, 0);
       const int r0 = (int)((long long)n_replicas * k / KR), r1 = (int)((long long)n_replicas * (k + 1) / KR);
+      const BondParams Bk = {B.words, B.index ? B.index + r0 : nullptr};
       for (int t = 0; t < 2 * n_sweeps && rc == TSU_OK; ++t)
         rc = launch_half_sweep(d_state + (size_t)r0 * rep_words, r1 - r0, rows, cols, wrap_rows, wrap_cols, t & 1, d_lut,
                                d_lut_index ? d_lut_index + r0 : nullptr, seed, sweep0 + (uint32_t)(t >> 1),
-                               replica0 + (uint32_t)r0, 0, nullptr, nullptr, sk, jit, 0, -1, KR);
+                               replica0 + (uint32_t)r0, 0, nullptr, nullptr, sk, jit, 0, -1, KR, Bk);
     }
     for (int k = 1; k < KR; ++k) {  // also after an error: the caller's stream must not run ahead of what was launched
       cudaStream_t sk = slab_stream(dev, k - 1);
@@ -820,7 +943,7 @@ int launch_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wra
   if (K <= 2 || n_sweeps == 0) {
     for (int t = 0; t < 2 * n_sweeps; ++t) {
       int rc = launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, t & 1, d_lut, d_lut_index, seed,
-                                 sweep0 + (uint32_t)(t >> 1), replica0, 0, nullptr, nullptr, st, jit);
+                                 sweep0 + (uint32_t)(t >> 1), replica0, 0, nullptr, nullptr, st, jit, 0, -1, 1, B);
       if (rc != TSU_OK) return rc;
     }
     return TSU_OK;
@@ -854,7 +977,8 @@ int launch_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wra
         if (k + 1 < K || wrap_rows) cudaStreamWaitEvent(sub[k], ev[below][jp], 0);
       }
       rc = launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, t & 1, d_lut, d_lut_index, seed,
-                             sweep0 + (uint32_t)(t >> 1), replica0, 0, nullptr, nullptr, sub[k], jit, bound[k], bound[k + 1], K);
+                             sweep0 + (uint32_t)(t >> 1), replica0, 0, nullptr, nullptr, sub[k], jit, bound[k], bound[k + 1], K,
+                             B);
       cudaEventRecord(ev[k][j], sub[k]);
     }
   }
@@ -880,7 +1004,7 @@ bool resident_eligible(int n_replicas, int rows, int cols) {
 
 int launch_resident_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
                            const uint32_t* d_lut, const int32_t* d_lut_index, uint64_t seed, uint32_t sweep0, int n_sweeps,
-                           uint32_t replica0, cudaStream_t st) {
+                           uint32_t replica0, cudaStream_t st, BondParams B = kNoBonds) {
   SweepParams P = {};
   P.state = d_state;
   P.lut = d_lut;
@@ -892,9 +1016,74 @@ int launch_resident_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols
   P.k1 = (uint32_t)(seed >> 32);
   P.strip_rows = 1;
   P.n_strips = rows;
-  sweeps_resident_kernel<<<n_replicas, kResidentThreads, 0, st>>>(P, n_sweeps);
+  if (B.words)
+    sweeps_resident_kernel<true><<<n_replicas, kResidentThreads, 0, st>>>(P, n_sweeps, B);
+  else
+    sweeps_resident_kernel<false><<<n_replicas, kResidentThreads, 0, st>>>(P, n_sweeps, kNoBonds);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? TSU_OK : (int)e;
+}
+
+// tsu_ising2d_half_sweep_injected[_bonded]
+int half_sweep_injected(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols, int colour,
+                        const uint32_t* d_lut, const int32_t* d_lut_index, const uint32_t* d_uniforms, int row0,
+                        const uint32_t* d_halo_top, const uint32_t* d_halo_bot, cudaStream_t st, BondParams B) {
+  TSU_CHECK_ARG(d_state && d_lut && d_uniforms && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
+  TSU_CHECK_ARG(colour == 0 || colour == 1);
+  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
+  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2) || d_halo_top || d_halo_bot);
+  SweepParams P;
+  P.state = d_state;
+  P.lut = d_lut;
+  P.lut_index = d_lut_index;
+  P.halo_top = d_halo_top;
+  P.halo_bot = d_halo_bot;
+  P.g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
+  P.colour = colour;
+  P.sweep = 0;
+  P.replica0 = 0;
+  P.k0 = P.k1 = 0;
+  P.strip_rows = 1;
+  P.n_strips = rows;
+  const long long total = (long long)n_replicas * rows * P.g.wpr;
+  if (B.words)
+    half_sweep_injected_kernel<true><<<blocks_for(total, 128), 128, 0, st>>>(P, d_uniforms, B);
+  else
+    half_sweep_injected_kernel<false><<<blocks_for(total, 128), 128, 0, st>>>(P, d_uniforms, kNoBonds);
+  TSU_RETURN_LAUNCH_STATUS();
+}
+
+// tsu_ising2d_observables[_bonded]
+int observables(const uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols, int row0,
+                const uint32_t* d_next_rows, unsigned long long* d_out, cudaStream_t st, BondParams B) {
+  TSU_CHECK_ARG(d_state && d_out && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
+  Geom g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
+  cudaError_t e = cudaMemsetAsync(d_out, 0, sizeof(unsigned long long) * 2 * (size_t)n_replicas, st);
+  if (e != cudaSuccess) return (int)e;
+  if (cols % 256 == 0 && !tuning().obs_generic) {
+    const int nvec = g.wpr / 4;
+    int strip = 64;  // long strips re-read one row in `strip`; short ones fill the GPU for small batches
+    while (strip > 1 && (long long)n_replicas * nvec * ((rows + strip - 1) / strip) < 148LL * 2048) strip >>= 1;
+    const int n_strips = (rows + strip - 1) / strip;
+    const long long per_rep_pad = ((long long)n_strips * nvec + 31) / 32 * 32;
+    const unsigned grid = blocks_for((long long)n_replicas * per_rep_pad, 128);
+    if (B.words)
+      observables_fast_kernel<true><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, B);
+    else
+      observables_fast_kernel<false><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, kNoBonds);
+    TSU_RETURN_LAUNCH_STATUS();
+  }
+  TSU_CHECK_ARG(n_replicas <= 65535);  // gridDim.y of the word-by-word kernel
+  const long long n_words = 2LL * rows * g.wpr;
+  long long bx = (n_words + 255) / 256;
+  const long long cap = (148LL * 8 + n_replicas - 1) / n_replicas;  // about 8 CTAs per SM in total
+  if (bx > cap) bx = cap < 1 ? 1 : cap;
+  dim3 grid((unsigned)bx, (unsigned)n_replicas);
+  if (B.words)
+    observables_kernel<true><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, B);
+  else
+    observables_kernel<false><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, kNoBonds);
+  TSU_RETURN_LAUNCH_STATUS();
 }
 
 }  // namespace
@@ -1091,53 +1280,14 @@ int tsu_ising2d_half_sweep_injected(uint32_t* d_state, int n_replicas, int rows,
                                     int wrap_cols, int colour, const uint32_t* d_lut, const int32_t* d_lut_index,
                                     const uint32_t* d_uniforms, int row0, const uint32_t* d_halo_top,
                                     const uint32_t* d_halo_bot, uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && d_uniforms && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
-  TSU_CHECK_ARG(colour == 0 || colour == 1);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2) || d_halo_top || d_halo_bot);
-  SweepParams P;
-  P.state = d_state;
-  P.lut = d_lut;
-  P.lut_index = d_lut_index;
-  P.halo_top = d_halo_top;
-  P.halo_bot = d_halo_bot;
-  P.g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
-  P.colour = colour;
-  P.sweep = 0;
-  P.replica0 = 0;
-  P.k0 = P.k1 = 0;
-  P.strip_rows = 1;
-  P.n_strips = rows;
-  const long long total = (long long)n_replicas * rows * P.g.wpr;
-  half_sweep_injected_kernel<<<blocks_for(total, 128), 128, 0, tsu_stream(stream)>>>(P, d_uniforms);
-  TSU_RETURN_LAUNCH_STATUS();
+  return half_sweep_injected(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, d_uniforms,
+                             row0, d_halo_top, d_halo_bot, tsu_stream(stream), kNoBonds);
 }
 
 int tsu_ising2d_observables(const uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
                             int row0, const uint32_t* d_next_rows, unsigned long long* d_out, uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_out && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
-  Geom g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
-  cudaStream_t st = tsu_stream(stream);
-  cudaError_t e = cudaMemsetAsync(d_out, 0, sizeof(unsigned long long) * 2 * (size_t)n_replicas, st);
-  if (e != cudaSuccess) return (int)e;
-  if (cols % 256 == 0 && !tuning().obs_generic) {
-    const int nvec = g.wpr / 4;
-    int strip = 64;  // long strips re-read one row in `strip`; short ones fill the GPU for small batches
-    while (strip > 1 && (long long)n_replicas * nvec * ((rows + strip - 1) / strip) < 148LL * 2048) strip >>= 1;
-    const int n_strips = (rows + strip - 1) / strip;
-    const long long per_rep_pad = ((long long)n_strips * nvec + 31) / 32 * 32;
-    observables_fast_kernel<<<blocks_for((long long)n_replicas * per_rep_pad, 128), 128, 0, st>>>(d_state, g, d_next_rows,
-                                                                                                strip, n_strips, d_out);
-    TSU_RETURN_LAUNCH_STATUS();
-  }
-  TSU_CHECK_ARG(n_replicas <= 65535);  // gridDim.y of the word-by-word kernel
-  const long long n_words = 2LL * rows * g.wpr;
-  long long bx = (n_words + 255) / 256;
-  const long long cap = (148LL * 8 + n_replicas - 1) / n_replicas;  // about 8 CTAs per SM in total
-  if (bx > cap) bx = cap < 1 ? 1 : cap;
-  dim3 grid((unsigned)bx, (unsigned)n_replicas);
-  observables_kernel<<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out);
-  TSU_RETURN_LAUNCH_STATUS();
+  return observables(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, row0, d_next_rows, d_out, tsu_stream(stream),
+                     kNoBonds);
 }
 
 int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_replicas, double J, double h,
@@ -1225,6 +1375,79 @@ int tsu_ising2d_sweeps_jit(int jit_handle, uint32_t* d_state, int n_replicas, in
                                   n_sweeps, replica0, tsu_stream(stream));
   return launch_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, nullptr, seed, sweep0, n_sweeps, replica0,
                        tsu_stream(stream), jit_function(jit_handle));
+}
+
+// ---- Edwards-Anderson +-J lattices: the same update with bond words XOR-ed into the neighbour words ----------
+int tsu_ising2d_pack_bonds(const int8_t* d_signs, uint32_t* d_bonds, int n_real, int rows, int cols, int wrap_rows,
+                           int wrap_cols, uintptr_t stream) {
+  TSU_CHECK_ARG(d_signs && d_bonds && geom_ok(n_real, rows, cols));
+  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
+  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
+  const Geom g = make_geom(n_real, rows, cols, wrap_rows, wrap_cols, 0);
+  const long long total = 8LL * n_real * rows * g.wpr;
+  pack_bonds_kernel<<<blocks_for(total, 256), 256, 0, tsu_stream(stream)>>>(d_signs, d_bonds, n_real, g);
+  TSU_RETURN_LAUNCH_STATUS();
+}
+
+int tsu_ising2d_sweeps_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                              const uint32_t* d_lut, const int32_t* d_lut_index, const uint32_t* d_bonds,
+                              const int32_t* d_bond_index, uint64_t seed, uint32_t sweep0, int n_sweeps, uint32_t replica0,
+                              uintptr_t stream) {
+  TSU_CHECK_ARG(d_state && d_lut && d_bonds && geom_ok(n_replicas, rows, cols) && n_sweeps >= 0);
+  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
+  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
+  const BondParams B = {d_bonds, d_bond_index};
+  if (n_sweeps > 0 && resident_eligible(n_replicas, rows, cols))
+    return launch_resident_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, d_lut_index, seed, sweep0,
+                                  n_sweeps, replica0, tsu_stream(stream), B);
+  return launch_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, d_lut_index, seed, sweep0, n_sweeps,
+                       replica0, tsu_stream(stream), JitKernel{nullptr, 0, 0}, B);
+}
+
+int tsu_ising2d_half_sweep_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                                  int colour, const uint32_t* d_lut, const int32_t* d_lut_index, const uint32_t* d_bonds,
+                                  const int32_t* d_bond_index, uint64_t seed, uint32_t sweep, uint32_t replica0,
+                                  int row_begin, int row_end, uintptr_t stream) {
+  TSU_CHECK_ARG(d_state && d_lut && d_bonds && geom_ok(n_replicas, rows, cols));
+  TSU_CHECK_ARG(colour == 0 || colour == 1);
+  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
+  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
+  TSU_CHECK_ARG(row_begin >= 0 && row_begin <= row_end && row_end <= rows);
+  return launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, seed, sweep,
+                           replica0, 0, nullptr, nullptr, tsu_stream(stream), JitKernel{nullptr, 0, 0}, row_begin, row_end,
+                           1, BondParams{d_bonds, d_bond_index});
+}
+
+int tsu_ising2d_half_sweep_injected_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
+                                           int wrap_cols, int colour, const uint32_t* d_lut, const int32_t* d_lut_index,
+                                           const uint32_t* d_bonds, const int32_t* d_bond_index,
+                                           const uint32_t* d_uniforms, uintptr_t stream) {
+  TSU_CHECK_ARG(d_bonds);
+  return half_sweep_injected(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, d_uniforms,
+                             0, nullptr, nullptr, tsu_stream(stream), BondParams{d_bonds, d_bond_index});
+}
+
+int tsu_ising2d_observables_bonded(const uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
+                                   int wrap_cols, const uint32_t* d_bonds, const int32_t* d_bond_index,
+                                   unsigned long long* d_out, uintptr_t stream) {
+  TSU_CHECK_ARG(d_bonds);
+  return observables(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, 0, nullptr, d_out, tsu_stream(stream),
+                     BondParams{d_bonds, d_bond_index});
+}
+
+int tsu_ising2d_overlap(const uint32_t* d_state, int n_replicas, int rows, int cols, const int32_t* d_pairs, int n_pairs,
+                        unsigned long long* d_out, uintptr_t stream) {
+  TSU_CHECK_ARG(d_state && d_pairs && d_out && geom_ok(n_replicas, rows, cols));
+  TSU_CHECK_ARG(n_pairs > 0 && n_pairs <= 65535);  // gridDim.y
+  cudaStream_t st = tsu_stream(stream);
+  cudaError_t e = cudaMemsetAsync(d_out, 0, sizeof(unsigned long long) * (size_t)n_pairs, st);
+  if (e != cudaSuccess) return (int)e;
+  const long long rep_vecs = 2LL * rows * words_per_row(cols) / 4;  // wpr is a multiple of 4
+  long long bx = (rep_vecs + 255) / 256;
+  const long long cap = (148LL * 8 + n_pairs - 1) / n_pairs;
+  if (bx > cap) bx = cap < 1 ? 1 : cap;
+  overlap_kernel<<<dim3((unsigned)bx, (unsigned)n_pairs), 256, 0, st>>>(d_state, rep_vecs, d_pairs, d_out);
+  TSU_RETURN_LAUNCH_STATUS();
 }
 
 }  // extern "C"

@@ -87,6 +87,24 @@ struct SweepParams {
   int nvec_fast;           // 4-word groups per row the wide path updates (all their lanes exist); the rest is rim
 };
 
+// Edwards-Anderson +-J bonds (tsu_ising2d_*_bonded): uint32 words[realisation][colour][4][rows][wpr] aligned with the
+// state words, direction order N, S, W, E.  Bit j of a word is 1 iff the bond between own-colour lane j and that
+// neighbour is antiferromagnetic; absent neighbours and padding lanes have 0.  XOR-ing a neighbour word with its
+// bond word turns the up-count into the count of bond-satisfying neighbours, which the ferromagnet's threshold
+// table then serves unchanged: 4J sigma b + 2h - 2J sigma summed over the bonds = 4J u' + 2h - 2J d.
+enum { kBondN = 0, kBondS = 1, kBondW = 2, kBondE = 3 };
+struct BondParams {
+  const uint32_t* words;  // nullptr: ferromagnet (all bonds +1)
+  const int32_t* index;   // [n_replicas] realisation of each replica, or nullptr (all use realisation 0)
+};
+
+// bond words of (replica rep, colour): direction d of local row i, word w at [d * plane + i * wpr + w]
+__device__ __forceinline__ const uint32_t* bond_base(const BondParams& B, const Geom& g, int rep, int colour) {
+  const size_t plane = (size_t)g.rows * g.wpr;
+  const size_t k = B.index ? (size_t)B.index[rep] : 0;
+  return B.words + (k * 2 + (size_t)colour) * 4 * plane;
+}
+
 // lop3 with a compile-time truth table: out bit = (LUT >> (4a + 2b + c)) & 1
 template <int LUT>
 __device__ __forceinline__ uint32_t lop3_imm(uint32_t a, uint32_t b, uint32_t c) {
@@ -222,8 +240,8 @@ __device__ __forceinline__ uint32_t drain_pass(uint32_t* ring, uint32_t head, ui
 #ifndef TSU_FAST_WARPS
 #define TSU_FAST_WARPS 4  // warps per CTA the kernel is launched with (warps never cooperate: any CTA size works)
 #endif
-template <int W>
-__device__ __forceinline__ void half_sweep_fast_body(const SweepParams& P) {
+template <int W, bool BONDED = false>
+__device__ __forceinline__ void half_sweep_fast_body(const SweepParams& P, const BondParams& B = BondParams{nullptr, nullptr}) {
   constexpr int REC = TieRec<W>::kWords;
   __shared__ __align__(16) uint32_t tie_rings[TSU_FAST_WARPS][kRingSlots * REC];  // one ring per warp of the CTA
   const Geom& g = P.g;
@@ -299,6 +317,21 @@ __device__ __forceinline__ void half_sweep_fast_body(const SweepParams& P) {
     side_c = rc0[((g.row0 + r_begin + P.colour) & 1) ? w_next : w_prev];
     ld_words<W>(opp_row(pl, g, r_begin + 1) + w0, s);
   }
+  // bonded: the N, S, W, E bond words of the current row, and a running pointer to those of the next one
+  uint32_t bd[4][W];
+  const uint32_t* p_bd = nullptr;
+  if constexpr (BONDED) {
+#pragma unroll
+    for (int d = 0; d < 4; ++d)
+#pragma unroll
+      for (int k = 0; k < W; ++k) bd[d][k] = 0u;
+    p_bd = bond_base(B, g, rep, P.colour) + (size_t)r_begin * g.wpr + w0;
+    if (active) {
+#pragma unroll
+      for (int d = 0; d < 4; ++d) ld_words<W>(p_bd + (size_t)d * plane, bd[d]);
+    }
+    p_bd += g.wpr;
+  }
   // running addresses: row it + 2 of the other colour (prefetch), the row being written; the row below the last
   // local row (halo or wrap) replaces the prefetch address in the one iteration that needs it
   const size_t stride = (size_t)g.wpr;
@@ -324,9 +357,20 @@ __device__ __forceinline__ void half_sweep_fast_body(const SweepParams& P) {
 #pragma unroll
     for (int k = 0; k < W; ++k) s2[k] = s[k];
     uint32_t side_s = 0u;
+    uint32_t bd2[4][W];
+    if constexpr (BONDED) {
+#pragma unroll
+      for (int d = 0; d < 4; ++d)
+#pragma unroll
+        for (int k = 0; k < W; ++k) bd2[d][k] = bd[d][k];
+    }
     if (it + 1 < n_rows) {
       side_s = p_s2[p ? d_even : d_odd];  // the next row has the opposite parity
       ld_words<W>(it == it_bottom ? p_bottom : p_s2, s2);
+      if constexpr (BONDED) {
+#pragma unroll
+        for (int d = 0; d < 4; ++d) ld_words<W>(p_bd + (size_t)d * plane, bd2[d]);
+      }
     }
     uint32_t lt[W], eq[W], c0[W], c1[W], c2[W];
     uint32_t any = 0u;
@@ -344,12 +388,24 @@ __device__ __forceinline__ void half_sweep_fast_body(const SweepParams& P) {
       // bit-sliced up-neighbour count of the words
 #pragma unroll
       for (int k = 0; k < W; ++k) {
-        const uint32_t s1 = n[k] ^ s[k] ^ c[k];
-        const uint32_t m1 = lop3_maj(n[k], s[k], c[k]);
-        c0[k] = s1 ^ sd[k];
-        const uint32_t k2 = s1 & sd[k];
-        c1[k] = m1 ^ k2;
-        c2[k] = m1 & k2;
+        if constexpr (BONDED) {  // bond-corrected neighbour bits; the centre word is the west neighbour iff p
+          const uint32_t nn = n[k] ^ bd[kBondN][k], ss = s[k] ^ bd[kBondS][k];
+          const uint32_t cc = c[k] ^ (p ? bd[kBondW][k] : bd[kBondE][k]);
+          const uint32_t sdd = sd[k] ^ (p ? bd[kBondE][k] : bd[kBondW][k]);
+          const uint32_t s1 = nn ^ ss ^ cc;
+          const uint32_t m1 = lop3_maj(nn, ss, cc);
+          c0[k] = s1 ^ sdd;
+          const uint32_t k2 = s1 & sdd;
+          c1[k] = m1 ^ k2;
+          c2[k] = m1 & k2;
+        } else {
+          const uint32_t s1 = n[k] ^ s[k] ^ c[k];
+          const uint32_t m1 = lop3_maj(n[k], s[k], c[k]);
+          c0[k] = s1 ^ sd[k];
+          const uint32_t k2 = s1 & sd[k];
+          c1[k] = m1 ^ k2;
+          c2[k] = m1 & k2;
+        }
       }
       // borrow-chain compare of the top 8 bits of the uniforms against the thresholds, least significant
       // plane first; planes 4-7 (second Philox call) are consumed before planes 0-3 are generated
@@ -450,6 +506,13 @@ __device__ __forceinline__ void half_sweep_fast_body(const SweepParams& P) {
       s[k] = s2[k];
     }
     side_c = side_s;
+    if constexpr (BONDED) {
+#pragma unroll
+      for (int d = 0; d < 4; ++d)
+#pragma unroll
+        for (int k = 0; k < W; ++k) bd[d][k] = bd2[d][k];
+      p_bd += stride;
+    }
     p_s2 += stride;
     p_own += stride;
     p ^= 1;

@@ -69,6 +69,40 @@ def lattice_bond_count(rows: int, cols: int, wrap_rows: bool, wrap_cols: bool) -
     return rows * (cols - 1) + (rows if wrap_cols else 0) + (rows - 1) * cols + (cols if wrap_rows else 0)
 
 
+def check_bonds(bonds, bond_index, rows: int, cols: int, n_replicas: int, bias_mode: str = "physical",
+                is_slab: bool = False):
+    """validated +-1 signs int8 [K, 2, rows, cols] and int32 bond_index [n_replicas] (None: all realisation 0) of an
+    Edwards-Anderson engine (see Ising2DEngine); ValueError for anything the bonded kernels cannot serve"""
+    if bias_mode != "physical":
+        raise ValueError("bonds need bias_mode='physical': the reference bias depends on each site's signed row sum, "
+                         "which the threshold table cannot express")
+    if is_slab:
+        raise ValueError("bonds are not available on row-slab engines")
+    b = np.asarray(bonds)
+    if b.ndim == 3:
+        b = b[None]
+    if b.ndim != 4 or b.shape[1:] != (2, rows, cols) or b.shape[0] < 1:
+        raise ValueError(f"bonds must have shape (2, {rows}, {cols}) or (K, 2, {rows}, {cols}), got {np.shape(bonds)}")
+    if b.dtype == np.bool_ or not np.all((b == 1) | (b == -1)):
+        raise ValueError("bonds must hold +1 or -1 only")
+    K = b.shape[0]
+    if bond_index is None:
+        if K == 1:
+            idx = None
+        elif K == n_replicas:
+            idx = np.arange(K, dtype=np.int32)
+        else:
+            raise ValueError("bond_index is required when the number of realisations is neither 1 nor n_replicas")
+    else:
+        idx = np.asarray(bond_index)
+        if idx.shape != (n_replicas,) or not np.issubdtype(idx.dtype, np.integer):
+            raise ValueError(f"bond_index must hold {n_replicas} integers")
+        if np.any(idx < 0) or np.any(idx >= K):
+            raise ValueError(f"bond_index entries must lie in [0, {K})")
+        idx = idx.astype(np.int32)
+    return b.astype(np.int8), idx
+
+
 class Ising2DEngine:
     """n_replicas independent rows x cols lattices (or one row-slab of each) resident in HBM.
 
@@ -76,6 +110,12 @@ class Ising2DEngine:
     Replica r uses temperature temperatures[r] (scalar = shared).  All randomness is
     Philox(seed; replica0+r, sweep index, global row, word), so a lattice split into row slabs
     (row0/halos) or a replica batch split across GPUs (replica0) reproduces the single-GPU bits.
+
+    Edwards-Anderson +-J spin glasses: `bonds` holds +-1 of shape (2, rows, cols) or (K, 2, rows, cols);
+    [k, 0, i, j] is the bond (i, j)-(i, (j+1) % cols), [k, 1, i, j] the bond (i, j)-((i+1) % rows, j), and the
+    coupling of a bond is coupling * sign.  Entries of bonds the wiring does not create (open edges, the wrap of a
+    periodic dimension of length 2) are ignored.  `bond_index` maps each replica to one of the K realisations
+    (default: all 0 when K = 1, arange when K = n_replicas).  Whole lattices with bias_mode "physical" only.
     """
 
     def __init__(
@@ -93,7 +133,14 @@ class Ising2DEngine:
         replica0: int = 0,
         row0: int = 0,
         global_rows: Optional[int] = None,
+        bonds=None,
+        bond_index=None,
     ):
+        if bonds is not None:  # checked before anything touches the device
+            bonds, bond_index = check_bonds(bonds, bond_index, rows, cols, n_replicas, bias_mode,
+                                            global_rows is not None and int(global_rows) != int(rows))
+        elif bond_index is not None:
+            raise ValueError("bond_index needs bonds")
         torch = _lib.require_cuda()
         self._torch = torch
         self.lib = _lib.load()
@@ -121,7 +168,23 @@ class Ising2DEngine:
             self._obs = torch.zeros((self.n_replicas, 2), dtype=torch.int64, device=self.device)
         self.lut = None
         self.lut_index = None
+        self.bonds = None
+        self.bond_index = None
+        if bonds is not None:
+            self._set_bonds(bonds, bond_index)
         self.set_temperature(temperature)
+
+    def _set_bonds(self, b: np.ndarray, idx: Optional[np.ndarray]):
+        """pack validated signs (check_bonds) into the kernels' bond words [K, 2, 4, rows, wpr]"""
+        torch = self._torch
+        K = b.shape[0]
+        self.n_realisations = K
+        with torch.cuda.device(self.device):
+            signs = torch.from_numpy(np.ascontiguousarray(b.astype(np.int8))).to(self.device)
+            self.bonds = torch.empty((K, 2, 4, self.rows, self.wpr), dtype=torch.int32, device=self.device)
+            _lib.call("tsu_ising2d_pack_bonds", ptr(signs), ptr(self.bonds), K, self.rows, self.cols, int(self.wrap_rows),
+                      int(self.wrap_cols), _lib.current_stream())
+            self.bond_index = None if idx is None else torch.from_numpy(idx).to(self.device)
 
     # ------------------------------------------------------------------ parameters
     def set_temperature(self, temperature):
@@ -149,8 +212,8 @@ class Ising2DEngine:
     def _jit_worthwhile(self, force: bool = False) -> bool:
         import os
 
-        if os.environ.get("TSU_B200_NO_JIT"):
-            return False
+        if os.environ.get("TSU_B200_NO_JIT") or self.bonds is not None:
+            return False  # (the specialised kernel has no bonded form)
         wide = (self.cols // 2) // 32 >= 4 and self.rows >= 3   # at least one 4-word group of full words per row
         if not wide:
             return False  # only the wide full-word kernel has a specialised form (open rims run the generic kernel)
@@ -220,6 +283,7 @@ class Ising2DEngine:
             cache[key] = v
         v.lut = self.lut
         v.lut_index = None if self.lut_index is None else self.lut_index[start:start + count]
+        v.bond_index = None if self.bond_index is None else self.bond_index[start:start + count]
         return v
 
     # ------------------------------------------------------------------ state i/o
@@ -264,7 +328,26 @@ class Ising2DEngine:
         """resample every site of `colour`; halos are [n_replicas, wpr] int32 rows of the other colour.
         rows=(begin, end) restricts the update to those local rows (same bits for any split of the rows)."""
         with self._torch.cuda.device(self.device):
-            if rows is not None:
+            if self.bonds is not None:
+                if halo_top is not None or halo_bot is not None:
+                    raise ValueError("bonded engines have no halos")
+                if uniforms is not None:
+                    if rows is not None:
+                        raise ValueError("row ranges are not available in injected-uniform mode")
+                    _lib.call(
+                        "tsu_ising2d_half_sweep_injected_bonded", ptr(self.state), self.n_replicas, self.rows,
+                        self.cols, int(self.wrap_rows), int(self.wrap_cols), int(colour), ptr(self.lut),
+                        ptr(self.lut_index), ptr(self.bonds), ptr(self.bond_index), ptr(uniforms), _lib.current_stream(),
+                    )
+                else:
+                    begin, end = (0, self.rows) if rows is None else (int(rows[0]), int(rows[1]))
+                    _lib.call(
+                        "tsu_ising2d_half_sweep_bonded", ptr(self.state), self.n_replicas, self.rows, self.cols,
+                        int(self.wrap_rows), int(self.wrap_cols), int(colour), ptr(self.lut), ptr(self.lut_index),
+                        ptr(self.bonds), ptr(self.bond_index), self.seed, self.sweep_index & 0xFFFFFFFF, self.replica0,
+                        begin, end, _lib.current_stream(),
+                    )
+            elif rows is not None:
                 if uniforms is not None:
                     raise ValueError("row ranges are not available in injected-uniform mode")
                 _lib.call(
@@ -301,7 +384,14 @@ class Ising2DEngine:
         if self.is_slab:
             raise RuntimeError("row-slab engines are driven by ShardedIsing2D (halo exchange between half-sweeps)")
         with self._torch.cuda.device(self.device):
-            if self.lut_index is None and getattr(self, "_jit", 0) > 0:
+            if self.bonds is not None:
+                _lib.call(
+                    "tsu_ising2d_sweeps_bonded", ptr(self.state), self.n_replicas, self.rows, self.cols,
+                    int(self.wrap_rows), int(self.wrap_cols), ptr(self.lut), ptr(self.lut_index), ptr(self.bonds),
+                    ptr(self.bond_index), self.seed, self.sweep_index & 0xFFFFFFFF, int(n_sweeps), self.replica0,
+                    _lib.current_stream(),
+                )
+            elif self.lut_index is None and getattr(self, "_jit", 0) > 0:
                 _lib.call(
                     "tsu_ising2d_sweeps_jit", self._jit, ptr(self.state), self.n_replicas, self.rows, self.cols,
                     int(self.wrap_rows), int(self.wrap_cols), ptr(self.lut), self.seed, self.sweep_index & 0xFFFFFFFF,
@@ -331,8 +421,18 @@ class Ising2DEngine:
 
     # ------------------------------------------------------------------ observables
     def observables_tensor(self, next_rows=None):
-        """int64 tensor [n_replicas, 2]: (# up spins, # anti-aligned right+down bonds) of the local rows"""
+        """int64 tensor [n_replicas, 2]: (# up spins, # anti-aligned right+down bonds) of the local rows;
+        with bonds the second column counts unsatisfied bonds (sign * s_i * s_j = -1)"""
         with self._torch.cuda.device(self.device):
+            if self.bonds is not None:
+                if next_rows is not None:
+                    raise ValueError("bonded engines have no halos")
+                _lib.call(
+                    "tsu_ising2d_observables_bonded", ptr(self.state), self.n_replicas, self.rows, self.cols,
+                    int(self.wrap_rows), int(self.wrap_cols), ptr(self.bonds), ptr(self.bond_index), ptr(self._obs),
+                    _lib.current_stream(),
+                )
+                return self._obs
             _lib.call(
                 "tsu_ising2d_observables", ptr(self.state), self.n_replicas, self.rows, self.cols,
                 int(self.wrap_rows and not self.is_slab), int(self.wrap_cols), self.row0, ptr(next_rows),
@@ -347,6 +447,26 @@ class Ising2DEngine:
     @property
     def n_bonds(self) -> int:
         return lattice_bond_count(self.rows, self.cols, self.wrap_rows, self.wrap_cols)
+
+    def overlap_tensor(self, pairs):
+        """float64 device tensor [n_pairs]: spin overlap q_ab = (1/N) sum_i s_i^a s_i^b = 1 - 2 diff_ab / N of every
+        replica pair (a, b) in `pairs` (shape [n_pairs, 2], indices of this engine's replicas)"""
+        torch = self._torch
+        pr = np.asarray(pairs)
+        if pr.ndim != 2 or pr.shape[1] != 2 or pr.shape[0] < 1 or not np.issubdtype(pr.dtype, np.integer):
+            raise ValueError("pairs must be integers of shape [n_pairs, 2]")
+        if np.any(pr < 0) or np.any(pr >= self.n_replicas):
+            raise ValueError(f"pair indices must lie in [0, {self.n_replicas})")
+        with torch.cuda.device(self.device):
+            dev = torch.from_numpy(np.ascontiguousarray(pr.astype(np.int32))).to(self.device)
+            diff = torch.empty(pr.shape[0], dtype=torch.int64, device=self.device)
+            _lib.call("tsu_ising2d_overlap", ptr(self.state), self.n_replicas, self.rows, self.cols, ptr(dev),
+                      int(pr.shape[0]), ptr(diff), _lib.current_stream())
+            return 1.0 - 2.0 * diff.to(torch.float64) / self.n_sites
+
+    def overlap(self, pairs) -> np.ndarray:
+        """spin overlap q_ab of every replica pair (host numpy, see overlap_tensor)"""
+        return self.overlap_tensor(pairs).cpu().numpy()
 
     def magnetization(self) -> np.ndarray:
         """signed magnetisation per spin of every replica (tsu/models/ising.py:183-193 on the current state)"""
