@@ -34,7 +34,7 @@ extern "C" {
 #define TSU_ERR_UNSUPPORTED (-2)
 #define TSU_ERR_NO_DEVICE (-3)
 
-#define TSU_B200_ABI_VERSION 1
+#define TSU_B200_ABI_VERSION 2
 
 int tsu_version(void);
 const char* tsu_error_string(int code);
@@ -96,25 +96,25 @@ int tsu_ising2d_pack(const int8_t* d_spins, uint32_t* d_state, int n_replicas, i
 int tsu_ising2d_unpack(const uint32_t* d_state, int8_t* d_spins, int n_replicas, int rows, int cols,
                        int as_pm1, uintptr_t stream);
 
-/* One half-sweep: every site of `colour` is resampled (heat bath).  Uniforms come from the
- * in-register Philox stream (seed, replica0+replica, sweep, row0+row, word).
+/* One half-sweep: every site of `colour` in the local rows [row_begin, row_end) is resampled (heat bath); the other
+ * rows are neither read for writing nor written (0, rows: all).  Uniforms come from the in-register Philox stream
+ * (seed, replica0+replica, sweep, row0+row, word), so the bits are identical for any split of the rows: a row-slab
+ * driver can update its two boundary rows first, send them to the ring neighbours and update the interior while the
+ * halo exchange is in flight.
  * d_halo_top / d_halo_bot: [n_replicas][wpr] words of the OPPOSITE colour for global rows
  * row0-1 / row0+rows (row-slab sharding); NULL = wrap inside the local array if wrap_rows,
- * else open edge.  wrap_cols: periodic in the column direction (cols must be even). */
-int tsu_ising2d_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                           int wrap_cols, int colour, const uint32_t* d_lut,
-                           const int32_t* d_lut_index, uint64_t seed, uint32_t sweep,
-                           uint32_t replica0, int row0, const uint32_t* d_halo_top,
-                           const uint32_t* d_halo_bot, uintptr_t stream);
-/* The same update restricted to the local rows [row_begin, row_end) (the others are neither read for writing nor
- * written): lets a row-slab driver update its two boundary rows first, send them to the ring neighbours and
- * update the interior while the halo exchange is in flight.  jit_handle > 0 (and d_lut_index == NULL) selects the
- * run-time specialised kernel of tsu_ising2d_jit_prepare; bits are identical for any split of the rows. */
-int tsu_ising2d_half_sweep_rows(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols,
-                                int wrap_rows, int wrap_cols, int colour, const uint32_t* d_lut,
-                                const int32_t* d_lut_index, uint64_t seed, uint32_t sweep,
-                                uint32_t replica0, int row0, const uint32_t* d_halo_top,
-                                const uint32_t* d_halo_bot, int row_begin, int row_end, uintptr_t stream);
+ * else open edge.  wrap_cols: periodic in the column direction (cols must be even).
+ * jit_handle > 0 selects the run-time specialised kernel of tsu_ising2d_jit_prepare where it applies (d_lut_index and
+ * d_bonds NULL), 0 the prebuilt kernels; same bits either way.
+ * d_bonds / d_bond_index: +-J bonds (tsu_ising2d_pack_bonds below) or NULL; bonds serve whole lattices only, so with
+ * bonds a halo or row0 != 0 is TSU_ERR_INVALID_ARG. */
+int tsu_ising2d_half_sweep(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols,
+                           int wrap_rows, int wrap_cols, int colour, const uint32_t* d_lut,
+                           const int32_t* d_lut_index, const uint32_t* d_bonds, const int32_t* d_bond_index,
+                           uint64_t seed, uint32_t sweep, uint32_t replica0, int row0,
+                           const uint32_t* d_halo_top, const uint32_t* d_halo_bot,
+                           int row_begin, int row_end, uintptr_t stream);
+
 /* n_sweeps sweeps of ONE row slab of a lattice that is split over the GPUs of a box, halo exchange included: the
  * compute step and its exchange in one call, no collective library in the data path.  Per half-sweep
  *   side stream: wait for the neighbours' rows of the other colour -> update rows 0 and rows-1 -> copy them into
@@ -135,7 +135,8 @@ int tsu_ising2d_slab_sweeps_p2p(int jit_handle, uint32_t* d_state, int n_replica
                                 uint32_t* d_up_flags, uint32_t* d_down_halo, uint32_t* d_down_flags,
                                 uint32_t msgs_colour0, uint32_t msgs_colour1, uintptr_t main_stream,
                                 uintptr_t side_stream);
-/* n_sweeps full sweeps (black then white), sweep indices sweep0 .. sweep0+n_sweeps-1, no halos.
+/* n_sweeps full sweeps (black then white), sweep indices sweep0 .. sweep0+n_sweeps-1, no halos; jit_handle and
+ * d_bonds / d_bond_index as in tsu_ising2d_half_sweep.
  * Two launches per sweep; lattices of at most 4096 words per replica in batches that would not fill the GPU
  * (BASELINE config 1: 50 x 50) run ALL sweeps of the call in ONE launch, one thread block per replica.  Same
  * bits either way (TSU_LATTICE_RESIDENT=0 disables the single-launch form).
@@ -144,40 +145,37 @@ int tsu_ising2d_slab_sweeps_p2p(int jit_handle, uint32_t* d_state, int n_replica
  * k+1 of the half-sweep before, so that the next half-sweep fills the SMs while this one drains (+3 .. 11 %).  The
  * extra streams fork from `stream` and are joined back into it before the call returns: to the caller the call is
  * still ordered on `stream` alone.  TSU_LATTICE_SPLIT=1 keeps one launch per half-sweep; same bits either way. */
-int tsu_ising2d_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                       int wrap_cols, const uint32_t* d_lut, const int32_t* d_lut_index,
-                       uint64_t seed, uint32_t sweep0, int n_sweeps, uint32_t replica0,
-                       uintptr_t stream);
+int tsu_ising2d_sweeps(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols,
+                       int wrap_rows, int wrap_cols, const uint32_t* d_lut, const int32_t* d_lut_index,
+                       const uint32_t* d_bonds, const int32_t* d_bond_index, uint64_t seed,
+                       uint32_t sweep0, int n_sweeps, uint32_t replica0, uintptr_t stream);
 /* Run-time specialisation (NVRTC) of the fast half-sweep kernel for ONE threshold table (all replicas at the
  * same temperature): the eight 5-bit truth tables of h_lut (host copy of the table, layout above) become
  * literals of csrc/ising2d_fast.cuh, which removes the jump tables from the inner loop (+17 % measured).
- * src_dir = directory that holds ising2d_fast.cuh and philox.cuh.  Returns a handle >= 1, or 0 when NVRTC /
- * the driver API is unavailable or compilation failed (log_buf gets the reason): callers then keep using the
- * prebuilt kernels.  Results are bit-identical to tsu_ising2d_half_sweep / tsu_ising2d_sweeps; geometries
- * outside the fast path silently use the prebuilt generic kernel. */
+ * src_dir = directory that holds ising2d_fast.cuh and philox.cuh.  Returns a handle >= 1 to pass as jit_handle, or
+ * 0 when NVRTC / the driver API is unavailable or compilation failed (log_buf gets the reason): callers then pass 0
+ * and keep using the prebuilt kernels.  Results are bit-identical to the prebuilt kernels; geometries outside the
+ * fast path silently use the prebuilt generic kernel. */
 int tsu_ising2d_jit_prepare(const uint32_t* h_lut, const char* src_dir, char* log_buf, int log_len);
-int tsu_ising2d_half_sweep_jit(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols,
-                               int wrap_rows, int wrap_cols, int colour, const uint32_t* d_lut,
-                               uint64_t seed, uint32_t sweep, uint32_t replica0, int row0,
-                               const uint32_t* d_halo_top, const uint32_t* d_halo_bot, uintptr_t stream);
-int tsu_ising2d_sweeps_jit(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols,
-                           int wrap_rows, int wrap_cols, const uint32_t* d_lut, uint64_t seed,
-                           uint32_t sweep0, int n_sweeps, uint32_t replica0, uintptr_t stream);
 
 /* Parity mode: same update, but the uniform of site (replica,row,col) is read from
- * d_uniforms[replica][row][col] (uint32 k meaning k/2^32) instead of Philox. */
+ * d_uniforms[replica][row][col] (uint32 k meaning k/2^32) instead of Philox.  Bonds as in tsu_ising2d_half_sweep. */
 int tsu_ising2d_half_sweep_injected(uint32_t* d_state, int n_replicas, int rows, int cols,
                                     int wrap_rows, int wrap_cols, int colour, const uint32_t* d_lut,
-                                    const int32_t* d_lut_index, const uint32_t* d_uniforms,
-                                    int row0, const uint32_t* d_halo_top,
-                                    const uint32_t* d_halo_bot, uintptr_t stream);
+                                    const int32_t* d_lut_index, const uint32_t* d_bonds,
+                                    const int32_t* d_bond_index, const uint32_t* d_uniforms, int row0,
+                                    const uint32_t* d_halo_top, const uint32_t* d_halo_bot, uintptr_t stream);
 /* d_out[replica][0] = number of up spins, d_out[replica][1] = number of anti-aligned bonds
  * (right + down bonds of every local site, wiring of tsu/models/ising.py:343-361).
  * d_next_rows: [n_replicas][2][wpr] both colours of global row row0+rows (slab sharding) or NULL.
  * M and E follow on the host: M = (2 up - N)/N, E = -J (n_bonds - 2 anti) - h (2 up - N)
- * (tsu/models/ising.py:98-117,183-193). */
+ * (tsu/models/ising.py:98-117,183-193).
+ * With d_bonds (whole lattices only: d_next_rows NULL, row0 0), d_out[replica][1] counts the UNSATISFIED bonds
+ * (sigma_ij s_i s_j = -1), so that tsu_ising2d_energy_from_observables gives E = -J sum sigma_ij s_i s_j - h sum s_i
+ * unchanged. */
 int tsu_ising2d_observables(const uint32_t* d_state, int n_replicas, int rows, int cols,
-                            int wrap_rows, int wrap_cols, int row0, const uint32_t* d_next_rows,
+                            int wrap_rows, int wrap_cols, const uint32_t* d_bonds,
+                            const int32_t* d_bond_index, int row0, const uint32_t* d_next_rows,
                             unsigned long long* d_out, uintptr_t stream);
 /* d_energy[r] = -J (n_bonds - 2 anti_r) - h (2 up_r - n_sites)   (float64) */
 int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_replicas, double J,
@@ -187,8 +185,8 @@ int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_r
 /* Edwards-Anderson +-J lattices: coupling J_ij = J sigma_ij with a sign sigma_ij = +-1 per nearest-neighbour bond.
  * The field of the bit model is 4J u' + 2h - 2J d, with u' the number of neighbours j with b_j XOR [sigma_ij = -1]:
  * the ferromagnet's threshold tables (bias "physical") serve it unchanged, so every rule above (Philox stream, ties,
- * kernels chosen) holds; the neighbour words are XOR-ed with bond words before the up-count.  Whole lattices only
- * (no row slabs or halos); the run-time specialised kernel has no bonded form.
+ * kernels chosen, launch paths) holds; the neighbour words are XOR-ed with bond words before the up-count.  Whole
+ * lattices only (no row slabs or halos); the run-time specialised kernel has no bonded form.
  *
  * d_signs: int8 [n_real][2][rows][cols]; [k][0][i][j] is the bond (i,j)-(i,(j+1) mod cols), [k][1][i][j] the bond
  *   (i,j)-((i+1) mod rows,j); a value < 0 is antiferromagnetic.  Bonds the wiring does not create (open edges, a
@@ -199,28 +197,6 @@ int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_r
  * d_bond_index: [n_replicas] realisation of each replica, or NULL (all use realisation 0). */
 int tsu_ising2d_pack_bonds(const int8_t* d_signs, uint32_t* d_bonds, int n_real, int rows, int cols,
                            int wrap_rows, int wrap_cols, uintptr_t stream);
-/* tsu_ising2d_sweeps with bonds (same launch paths: resident, wide + rim, generic, row ranges, replica chunks) */
-int tsu_ising2d_sweeps_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                              int wrap_cols, const uint32_t* d_lut, const int32_t* d_lut_index,
-                              const uint32_t* d_bonds, const int32_t* d_bond_index, uint64_t seed,
-                              uint32_t sweep0, int n_sweeps, uint32_t replica0, uintptr_t stream);
-/* one half-sweep of `colour` restricted to rows [row_begin, row_end) (0, rows: all) */
-int tsu_ising2d_half_sweep_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                                  int wrap_cols, int colour, const uint32_t* d_lut,
-                                  const int32_t* d_lut_index, const uint32_t* d_bonds,
-                                  const int32_t* d_bond_index, uint64_t seed, uint32_t sweep,
-                                  uint32_t replica0, int row_begin, int row_end, uintptr_t stream);
-int tsu_ising2d_half_sweep_injected_bonded(uint32_t* d_state, int n_replicas, int rows, int cols,
-                                           int wrap_rows, int wrap_cols, int colour,
-                                           const uint32_t* d_lut, const int32_t* d_lut_index,
-                                           const uint32_t* d_bonds, const int32_t* d_bond_index,
-                                           const uint32_t* d_uniforms, uintptr_t stream);
-/* d_out[replica][0] = up spins, d_out[replica][1] = UNSATISFIED bonds (sigma_ij s_i s_j = -1), so that
- * tsu_ising2d_energy_from_observables gives E = -J sum sigma_ij s_i s_j - h sum s_i unchanged */
-int tsu_ising2d_observables_bonded(const uint32_t* d_state, int n_replicas, int rows, int cols,
-                                   int wrap_rows, int wrap_cols, const uint32_t* d_bonds,
-                                   const int32_t* d_bond_index, unsigned long long* d_out,
-                                   uintptr_t stream);
 /* spin overlap: d_out[q] = number of sites where replicas d_pairs[2q] and d_pairs[2q+1] differ
  * (q_ab = 1 - 2 d_out / (rows cols)); 1 <= n_pairs <= 65535, indices in [0, n_replicas) */
 int tsu_ising2d_overlap(const uint32_t* d_state, int n_replicas, int rows, int cols,

@@ -23,9 +23,9 @@ def test_header_symbols_are_exported_and_typed():
     assert set(_lib.SIGNATURES) == set(syms)
 
 
-def test_version_and_error_strings():
+def test_abi_version_2_and_error_strings():
     lib = _lib.load()
-    assert lib.tsu_version() == 1
+    assert lib.tsu_version() == 2
     assert lib.tsu_error_string(0) == b"ok"
     assert b"invalid" in lib.tsu_error_string(-1)
 
@@ -39,10 +39,10 @@ def test_words_per_row_matches_oracle():
         assert lib.tsu_ising2d_state_words(7, cols) == 2 * 7 * words_per_row(cols)
 
 
-def test_invalid_arguments_return_error_codes_without_gpu():
+def test_invalid_arguments_return_error_codes_before_any_cuda_call():
     lib = _lib.load()
     # NULL state pointer is rejected before any CUDA call
     rc = lib.tsu_ising2d_init_random(None, 1, 4, 4, 0, 0, 0, 0)
     assert rc == _lib.TSU_ERR_INVALID_ARG
-    rc = lib.tsu_ising2d_sweeps(None, 1, 4, 4, 1, 1, None, None, 0, 0, 1, 0, 0)
+    rc = lib.tsu_ising2d_sweeps(0, None, 1, 4, 4, 1, 1, None, None, None, None, 0, 0, 1, 0, 0)
     assert rc == _lib.TSU_ERR_INVALID_ARG

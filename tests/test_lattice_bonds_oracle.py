@@ -132,6 +132,8 @@ def test_reference_bias_and_slabs_are_rejected():
         engine(bonds=ones, bias_mode="reference")
     with pytest.raises(ValueError, match="row-slab"):
         engine(bonds=ones, global_rows=8, periodic=False)
+    with pytest.raises(ValueError, match="row-slab"):
+        engine(bonds=ones, row0=4, periodic=False)
     with pytest.raises(ValueError, match="needs bonds"):
         engine(bond_index=[0, 0])
 
@@ -147,30 +149,37 @@ def test_check_bonds_defaults():
     assert idx.dtype == np.int32 and list(idx) == [1, 0, 1]
 
 
-def test_bonded_abi_rejects_arguments_before_any_cuda_call():
+def test_merged_lattice_abi_rejects_bonded_arguments_before_any_cuda_call():
     from tsu_emulator_b200 import _lib
 
     lib = _lib.load()
     bad = _lib.TSU_ERR_INVALID_ARG
     p = ctypes.c_void_p(256)  # never dereferenced: every call below fails its argument check
-    # missing pointers
+    # missing pointers (a bond index without bond words)
     assert lib.tsu_ising2d_pack_bonds(None, p, 1, 4, 4, 1, 1, 0) == bad
     assert lib.tsu_ising2d_pack_bonds(p, None, 1, 4, 4, 1, 1, 0) == bad
-    assert lib.tsu_ising2d_sweeps_bonded(p, 1, 4, 4, 1, 1, p, None, None, None, 0, 0, 1, 0, 0) == bad
-    assert lib.tsu_ising2d_half_sweep_bonded(p, 1, 4, 4, 1, 1, 0, p, None, None, None, 0, 0, 0, 0, 4, 0) == bad
-    assert lib.tsu_ising2d_half_sweep_injected_bonded(p, 1, 4, 4, 1, 1, 0, p, None, None, None, p, 0) == bad
-    assert lib.tsu_ising2d_observables_bonded(p, 1, 4, 4, 1, 1, None, None, p, 0) == bad
+    assert lib.tsu_ising2d_sweeps(0, p, 1, 4, 4, 1, 1, p, None, None, p, 0, 0, 1, 0, 0) == bad
+    assert lib.tsu_ising2d_half_sweep(0, p, 1, 4, 4, 1, 1, 0, p, None, None, p, 0, 0, 0, 0, None, None, 0, 4, 0) == bad
+    assert lib.tsu_ising2d_half_sweep_injected(p, 1, 4, 4, 1, 1, 0, p, None, None, p, p, 0, None, None, 0) == bad
+    assert lib.tsu_ising2d_observables(p, 1, 4, 4, 1, 1, None, p, 0, None, p, 0) == bad
     assert lib.tsu_ising2d_overlap(p, 2, 4, 4, None, 1, p, 0) == bad
     # geometry, colour, row ranges, wraps, pair counts
     assert lib.tsu_ising2d_pack_bonds(p, p, 0, 4, 4, 0, 0, 0) == bad
     assert lib.tsu_ising2d_pack_bonds(p, p, 1, 4, 2, 0, 1, 0) == bad     # column wrap of length 2
     assert lib.tsu_ising2d_pack_bonds(p, p, 1, 5, 4, 1, 0, 0) == bad     # odd periodic rows
-    assert lib.tsu_ising2d_sweeps_bonded(p, 1, 4, 4, 1, 1, p, None, p, None, 0, 0, -1, 0, 0) == bad
-    assert lib.tsu_ising2d_sweeps_bonded(p, 1, 4, 3, 1, 1, p, None, p, None, 0, 0, 1, 0, 0) == bad
-    assert lib.tsu_ising2d_half_sweep_bonded(p, 1, 4, 4, 1, 1, 2, p, None, p, None, 0, 0, 0, 0, 4, 0) == bad
-    assert lib.tsu_ising2d_half_sweep_bonded(p, 1, 4, 4, 1, 1, 0, p, None, p, None, 0, 0, 0, 3, 2, 0) == bad
-    assert lib.tsu_ising2d_half_sweep_bonded(p, 1, 4, 4, 1, 1, 0, p, None, p, None, 0, 0, 0, 0, 5, 0) == bad
-    assert lib.tsu_ising2d_half_sweep_injected_bonded(p, 1, 4, 4, 1, 1, 0, p, None, p, None, None, 0) == bad
-    assert lib.tsu_ising2d_observables_bonded(p, 0, 4, 4, 1, 1, p, None, p, 0) == bad
+    assert lib.tsu_ising2d_sweeps(0, p, 1, 4, 4, 1, 1, p, None, p, None, 0, 0, -1, 0, 0) == bad
+    assert lib.tsu_ising2d_sweeps(0, p, 1, 4, 3, 1, 1, p, None, p, None, 0, 0, 1, 0, 0) == bad
+    assert lib.tsu_ising2d_half_sweep(0, p, 1, 4, 4, 1, 1, 2, p, None, p, None, 0, 0, 0, 0, None, None, 0, 4, 0) == bad
+    assert lib.tsu_ising2d_half_sweep(0, p, 1, 4, 4, 1, 1, 0, p, None, p, None, 0, 0, 0, 0, None, None, 3, 2, 0) == bad
+    assert lib.tsu_ising2d_half_sweep(0, p, 1, 4, 4, 1, 1, 0, p, None, p, None, 0, 0, 0, 0, None, None, 0, 5, 0) == bad
+    assert lib.tsu_ising2d_half_sweep_injected(p, 1, 4, 4, 1, 1, 0, p, None, p, None, None, 0, None, None, 0) == bad
+    assert lib.tsu_ising2d_observables(p, 0, 4, 4, 1, 1, p, None, 0, None, p, 0) == bad
     assert lib.tsu_ising2d_overlap(p, 2, 4, 4, p, 0, p, 0) == bad
     assert lib.tsu_ising2d_overlap(p, 2, 4, 4, p, 65536, p, 0) == bad
+    # bond words are indexed by local row: no halos, row slabs or next rows with bonds
+    assert lib.tsu_ising2d_half_sweep(0, p, 1, 4, 4, 0, 1, 0, p, None, p, None, 0, 0, 0, 0, p, None, 0, 4, 0) == bad
+    assert lib.tsu_ising2d_half_sweep(0, p, 1, 4, 4, 0, 1, 0, p, None, p, None, 0, 0, 0, 4, None, None, 0, 4, 0) == bad
+    assert lib.tsu_ising2d_half_sweep_injected(p, 1, 4, 4, 0, 1, 0, p, None, p, None, p, 0, None, p, 0) == bad
+    assert lib.tsu_ising2d_half_sweep_injected(p, 1, 4, 4, 0, 1, 0, p, None, p, None, p, 4, None, None, 0) == bad
+    assert lib.tsu_ising2d_observables(p, 1, 4, 4, 0, 1, p, None, 0, p, p, 0) == bad
+    assert lib.tsu_ising2d_observables(p, 1, 4, 4, 0, 1, p, None, 4, None, p, 0) == bad

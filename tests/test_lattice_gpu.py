@@ -338,8 +338,8 @@ def test_resident_small_lattice_kernel_matches_per_half_sweep_launches(rows, col
 @pytest.mark.parametrize("rows,cols,periodic", [(40, 1024, True), (33, 1000, False), (24, 512, False), (12, 70, True),
                                                 (9, 50, False)])
 def test_row_ranges_compose_to_the_full_half_sweep(rows, cols, periodic, tuning):
-    """tsu_ising2d_half_sweep_rows: boundary rows, interior and arbitrary splits, launched in any order, give the bits
-    of the one-launch half-sweep (what the overlapped row-slab driver relies on)"""
+    """tsu_ising2d_half_sweep over row ranges: boundary rows, interior and arbitrary splits, launched in any order, give
+    the bits of the one-launch half-sweep (what the overlapped row-slab driver relies on)"""
     import torch
     tuning.setenv("TSU_LATTICE_RESIDENT", "0")
     kw = dict(n_replicas=2, temperature=2.269, periodic=periodic, seed=19, field=0.05)

@@ -49,13 +49,8 @@ SIGNATURES = {
     "tsu_ising2d_unpack": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_uintptr]),
     "tsu_ising2d_half_sweep": (
         c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_uint64, c_uint32, c_uint32, c_int,
-         c_void_p, c_void_p, c_uintptr],
-    ),
-    "tsu_ising2d_half_sweep_rows": (
-        c_int,
-        [c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_uint64, c_uint32, c_uint32,
-         c_int, c_void_p, c_void_p, c_int, c_int, c_uintptr],
+        [c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_uint64,
+         c_uint32, c_uint32, c_int, c_void_p, c_void_p, c_int, c_int, c_uintptr],
     ),
     "tsu_ising2d_slab_sweeps_p2p": (
         c_int,
@@ -64,51 +59,24 @@ SIGNATURES = {
     ),
     "tsu_ising2d_sweeps": (
         c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_uint64, c_uint32, c_int, c_uint32,
-         c_uintptr],
+        [c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_uint64, c_uint32,
+         c_int, c_uint32, c_uintptr],
     ),
     "tsu_ising2d_jit_prepare": (c_int, [POINTER(c_uint32), c_char_p, c_char_p, c_int]),
-    "tsu_ising2d_half_sweep_jit": (
-        c_int,
-        [c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_uint64, c_uint32, c_uint32, c_int,
-         c_void_p, c_void_p, c_uintptr],
-    ),
-    "tsu_ising2d_sweeps_jit": (
-        c_int,
-        [c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_uint64, c_uint32, c_int, c_uint32, c_uintptr],
-    ),
     "tsu_ising2d_half_sweep_injected": (
         c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
-         c_uintptr],
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+         c_void_p, c_void_p, c_uintptr],
     ),
     "tsu_ising2d_observables": (
         c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_uintptr],
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_uintptr],
     ),
     "tsu_ising2d_energy_from_observables": (
         c_int,
         [c_void_p, c_int, c_double, c_double, c_int64, c_int64, c_void_p, c_uintptr],
     ),
     "tsu_ising2d_pack_bonds": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_uintptr]),
-    "tsu_ising2d_sweeps_bonded": (
-        c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_uint64, c_uint32, c_int,
-         c_uint32, c_uintptr],
-    ),
-    "tsu_ising2d_half_sweep_bonded": (
-        c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_uint64, c_uint32,
-         c_uint32, c_int, c_int, c_uintptr],
-    ),
-    "tsu_ising2d_half_sweep_injected_bonded": (
-        c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_uintptr],
-    ),
-    "tsu_ising2d_observables_bonded": (
-        c_int,
-        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_uintptr],
-    ),
     "tsu_ising2d_overlap": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_uintptr]),
     "tsu_dense_gibbs_run": (
         c_int,
@@ -170,7 +138,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)  # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.tsu_version() != 1:
+    if lib.tsu_version() != 2:
         raise ImportError("libtsu_b200.so ABI version mismatch; rebuild with python -m tsu_emulator_b200.build --force")
     _lib = lib
     return lib
@@ -210,5 +178,6 @@ def current_stream() -> int:
 
 
 def ptr(t):
-    """device pointer of a torch tensor (or None -> NULL)"""
-    return None if t is None else c_void_p(t.data_ptr())
+    """device pointer of a torch tensor (or None -> NULL) for a c_void_p argument.  A plain int: ctypes converts it
+    faster than a c_void_p built here, which matters on latency-bound calls (50 x 50 sweeps)."""
+    return None if t is None else t.data_ptr()

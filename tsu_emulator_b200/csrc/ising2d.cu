@@ -766,53 +766,97 @@ struct JitKernel {
 };
 std::vector<JitKernel> g_jit_functions;  // handle - 1 -> kernel
 
-JitKernel jit_function(int handle) {
+// the kernel of `handle` where it can serve a call: one threshold table for all replicas and no bonds (it has no
+// bonded form); fn == nullptr: the prebuilt kernels
+JitKernel jit_function(int handle, const int32_t* d_lut_index, const uint32_t* d_bonds) {
+  if (handle < 1 || d_lut_index || d_bonds) return JitKernel{nullptr, 0, 0};
   std::lock_guard<std::mutex> lock(g_jit_mutex);
-  if (handle < 1 || handle > (int)g_jit_functions.size()) return JitKernel{nullptr, 0, 0};
+  if (handle > (int)g_jit_functions.size()) return JitKernel{nullptr, 0, 0};
   return g_jit_functions[handle - 1];
 }
 
-int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols, int colour,
-                      const uint32_t* d_lut, const int32_t* d_lut_index, uint64_t seed, uint32_t sweep,
-                      uint32_t replica0, int row0, const uint32_t* d_halo_top, const uint32_t* d_halo_bot,
-                      cudaStream_t st, JitKernel jit = JitKernel{nullptr, 0, 0}, int upd_begin = 0, int upd_end = -1,
-                      int pieces = 1, BondParams B = kNoBonds) {
-  // pieces: this launch is one of `pieces` row ranges of a half-sweep that run concurrently (split_ranges())
-  // B.words: +-J bonds (bonded kernels; the specialised kernel has no bonded form and is never used for them)
-  const bool bonded = B.words != nullptr;
-  if (upd_end < 0) upd_end = rows;  // local rows [upd_begin, upd_end) are updated (default: all)
-  if (upd_begin >= upd_end) return TSU_OK;
-  SweepParams P;
-  P.state = d_state;
-  P.lut = d_lut;
-  P.lut_index = d_lut_index;
-  P.halo_top = d_halo_top;
-  P.halo_bot = d_halo_bot;
-  P.g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
+// What stays fixed over one call of a lattice entry point.
+struct Lattice {
+  uint32_t* state;
+  Geom g;  // geometry, wraps, row0, number of replicas
+  const uint32_t* lut;
+  const int32_t* lut_index;
+  BondParams B;  // B.words == nullptr: ferromagnet
+  uint64_t seed;
+  uint32_t replica0;
+  JitKernel jit;  // jit.fn == nullptr: the prebuilt kernels
+
+  // the same lattices restricted to replicas [r0, r1)
+  Lattice replicas(int r0, int r1) const {
+    Lattice c = *this;
+    c.state += (size_t)r0 * 2 * g.rows * g.wpr;
+    c.g.n_replicas = r1 - r0;
+    if (lut_index) c.lut_index += r0;
+    if (B.index) c.B.index += r0;
+    c.replica0 += (uint32_t)r0;
+    return c;
+  }
+};
+
+// The argument rules of the lattice entry points, checked before any CUDA call.  `halo`: rows next to the local ones
+// are given (halo rows, or the row after the last for the observables); they take the place of a row wrap.  Bond words
+// are indexed by local row, so bonds serve whole lattices only; a bond index needs bond words.
+bool args_ok(const Geom& g, const BondParams& B, bool halo, int colour, int row_begin, int row_end) {
+  return geom_ok(g.n_replicas, g.rows, g.cols) && rows_ok(g.rows, g.row0) && (colour == 0 || colour == 1) &&
+         row_begin >= 0 && row_begin <= row_end && row_end <= g.rows &&
+         (!g.wrap_cols || (g.cols % 2 == 0 && g.cols > 2)) &&
+         (!g.wrap_rows || (g.rows % 2 == 0 && g.rows > 2) || halo) &&
+         (B.words ? !halo && g.row0 == 0 : !B.index);
+}
+
+// kernel parameters of a half-sweep of every local row; the wide path narrows the rows and sets its strips
+SweepParams sweep_params(const Lattice& L, int colour, uint32_t sweep, const uint32_t* halo_top,
+                         const uint32_t* halo_bot) {
+  SweepParams P = {};
+  P.state = L.state;
+  P.lut = L.lut;
+  P.lut_index = L.lut_index;
+  P.halo_top = halo_top;
+  P.halo_bot = halo_bot;
+  P.g = L.g;
   P.colour = colour;
   P.sweep = sweep;
-  P.replica0 = replica0;
-  P.k0 = (uint32_t)seed;
-  P.k1 = (uint32_t)(seed >> 32);
+  P.replica0 = L.replica0;
+  P.k0 = (uint32_t)L.seed;
+  P.k1 = (uint32_t)(L.seed >> 32);
   P.keys = tsu_philox_key_schedule(P.k0, P.k1);
+  P.strip_rows = 1;
+  P.n_strips = L.g.rows;
   P.row_begin = 0;
-  P.row_end = rows;
-  P.nvec_fast = P.g.wpr / 4;
+  P.row_end = L.g.rows;
+  P.nvec_fast = L.g.wpr / 4;
+  return P;
+}
+
+// One half-sweep of `colour` over the local rows [upd_begin, upd_end).  pieces: this launch is one of `pieces` row
+// ranges or replica chunks of a half-sweep that run concurrently (split_ranges(), split_replicas()).
+int launch_half_sweep(const Lattice& L, int colour, uint32_t sweep, const uint32_t* halo_top, const uint32_t* halo_bot,
+                      int upd_begin, int upd_end, int pieces, cudaStream_t st) {
+  if (upd_begin >= upd_end) return TSU_OK;
+  const Geom& g = L.g;
+  const int rows = g.rows, cols = g.cols;
+  const bool bonded = L.B.words != nullptr;
+  SweepParams P = sweep_params(L, colour, sweep, halo_top, halo_bot);
   // rows that have a north / south neighbour (exactly the cases opp_row() resolves): the wide kernel takes those,
   // columns treated as periodic; what that gets wrong on open lattices is redone by the rim pass
-  const bool north_ok = d_halo_top || wrap_rows, south_ok = d_halo_bot || wrap_rows;
+  const bool north_ok = halo_top || g.wrap_rows, south_ok = halo_bot || g.wrap_rows;
   const int rb0 = north_ok ? 0 : 1, re0 = south_ok ? rows : rows - 1;
   const int rb = rb0 > upd_begin ? rb0 : upd_begin, re = re0 < upd_end ? re0 : upd_end;  // rows of the wide kernel
   // words that are full for both row parities: floor(cols / 2) lanes exist in every row of either colour
   const int full_words = (cols / 2) / 32;
   const bool ragged = cols % 256 != 0;
-  const int nvec_f = ragged ? full_words / 4 : P.g.wpr / 4;
-  const bool need_rim = rb > upd_begin || re < upd_end || !wrap_cols || ragged;
+  const int nvec_f = ragged ? full_words / 4 : g.wpr / 4;
+  const bool need_rim = rb > upd_begin || re < upd_end || !g.wrap_cols || ragged;
   bool fast = nvec_f >= 1 && re - rb >= 1;
   if (need_rim && tuning().open_generic) fast = false;
   if (fast) {
-    const bool use_jit = jit.fn && !d_lut_index && !bonded;
-    const int W = use_jit ? jit.w : (tuning().w == 2 ? 2 : kDefaultW);
+    const JitKernel& jit = L.jit;
+    const int W = jit.fn ? jit.w : (tuning().w == 2 ? 2 : kDefaultW);
     const int nvec = nvec_f * (4 / W);  // W-word groups per row
     const int frows = re - rb;
     P.nvec_fast = nvec_f;
@@ -820,7 +864,7 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
     const long long target_threads = 148LL * 2048;
     int strip = 128;
     const long long srows = (long long)frows * pieces;
-    while (strip > 1 && (long long)n_replicas * nvec * ((srows + strip - 1) / strip) < target_threads) strip >>= 1;
+    while (strip > 1 && (long long)g.n_replicas * nvec * ((srows + strip - 1) / strip) < target_threads) strip >>= 1;
     // the tail of one range is filled by the next: longer strips (less set-up per row) cost nothing there
     if (pieces >= 4) strip = strip * 4 < 128 ? strip * 4 : 128;
     if (tuning().strip > 0) strip = tuning().strip;
@@ -829,16 +873,16 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
     P.row_begin = rb;
     P.row_end = re;
     const long long per_rep_pad = ((long long)P.n_strips * nvec + 31) / 32 * 32;  // warps never straddle replicas
-    const long long total = (long long)n_replicas * per_rep_pad;
+    const long long total = (long long)g.n_replicas * per_rep_pad;
     const unsigned grid = blocks_for(total, 128);
-    if (use_jit) {  // table-specialised build of the same kernel body
+    if (jit.fn) {  // table-specialised build of the same kernel body
       void* args[] = {&P};
       if (tsu_jit::launch(jit.fn, blocks_for(total, jit.threads), jit.threads, 0, (void*)st, args) != 0) return 999;  // driver-API launch failure
     } else if (bonded) {  // one CTA per SM fewer: the next row's 4 W bond words stay in registers without spills
       if (W == 2)
-        half_sweep_fast_kernel<2, 6, true><<<grid, 128, 0, st>>>(P, B);
+        half_sweep_fast_kernel<2, 6, true><<<grid, 128, 0, st>>>(P, L.B);
       else
-        half_sweep_fast_kernel<4, 3, true><<<grid, 128, 0, st>>>(P, B);
+        half_sweep_fast_kernel<4, 3, true><<<grid, 128, 0, st>>>(P, L.B);
     } else if (W == 2) {
       half_sweep_fast_kernel<2, 8, false><<<grid, 128, 0, st>>>(P, kNoBonds);
     } else {
@@ -849,30 +893,27 @@ int launch_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int
       R.a0 = upd_begin; R.a1 = rb;   // updated rows above / below the wide kernel's range (no north / south neighbour)
       R.b0 = re; R.b1 = upd_end;
       R.p0 = rb; R.p1 = re;
-      R.head = (ragged || !wrap_cols) ? 1 : 0;
-      R.tail_begin = ragged ? 4 * nvec_f : (wrap_cols ? P.g.wpr : P.g.wpr - 1);
-      const long long per_rep = (long long)((R.a1 - R.a0) + (R.b1 - R.b0)) * P.g.wpr +
-                                (long long)(R.head + P.g.wpr - R.tail_begin) * frows;
+      R.head = (ragged || !g.wrap_cols) ? 1 : 0;
+      R.tail_begin = ragged ? 4 * nvec_f : (g.wrap_cols ? g.wpr : g.wpr - 1);
+      const long long per_rep = (long long)((R.a1 - R.a0) + (R.b1 - R.b0)) * g.wpr +
+                                (long long)(R.head + g.wpr - R.tail_begin) * frows;
       if (per_rep > 0) {
         if (bonded)
-          half_sweep_rim_kernel<true><<<blocks_for(per_rep * n_replicas, 128), 128, 0, st>>>(P, R, B);
+          half_sweep_rim_kernel<true><<<blocks_for(per_rep * g.n_replicas, 128), 128, 0, st>>>(P, R, L.B);
         else
-          half_sweep_rim_kernel<false><<<blocks_for(per_rep * n_replicas, 128), 128, 0, st>>>(P, R, kNoBonds);
+          half_sweep_rim_kernel<false><<<blocks_for(per_rep * g.n_replicas, 128), 128, 0, st>>>(P, R, kNoBonds);
       }
     }
   } else {
-    P.strip_rows = 1;
-    P.n_strips = rows;
     P.row_begin = upd_begin;
     P.row_end = upd_end;
-    const long long total = (long long)n_replicas * (upd_end - upd_begin) * P.g.wpr;
+    const long long total = (long long)g.n_replicas * (upd_end - upd_begin) * g.wpr;
     if (bonded)
-      half_sweep_generic_kernel<true><<<blocks_for(total, 128), 128, 0, st>>>(P, B);
+      half_sweep_generic_kernel<true><<<blocks_for(total, 128), 128, 0, st>>>(P, L.B);
     else
       half_sweep_generic_kernel<false><<<blocks_for(total, 128), 128, 0, st>>>(P, kNoBonds);
   }
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? TSU_OK : (int)e;
+  TSU_RETURN_LAUNCH_STATUS();
 }
 
 // Row ranges a half-sweep is cut into.  One launch per half-sweep loses ~15 us to its tail (launch gap, the last warps
@@ -900,71 +941,93 @@ int split_replicas(int n_replicas, int rows, int cols) {
   return tuning().split > 1 ? (tuning().split < kMaxSplit ? tuning().split : kMaxSplit) : kDefaultSplit;
 }
 
-// the whole-lattice sweeps of tsu_ising2d_sweeps / _sweeps_jit (no halos)
-int launch_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols, const uint32_t* d_lut,
-                  const int32_t* d_lut_index, uint64_t seed, uint32_t sweep0, int n_sweeps, uint32_t replica0,
-                  cudaStream_t st, JitKernel jit, BondParams B = kNoBonds) {
-  // many replicas: independent chunks of replicas, one stream each, no dependency between them at all
-  const int KR = split_replicas(n_replicas, rows, cols);
-  if (KR > 1 && n_sweeps > 0) {
+// The streams of one call that runs row ranges or replica chunks concurrently: s[0] is the caller's stream,
+// s[1 .. K-1] are library streams (slab_stream) and s[K] is the caller's `side` stream if one is given.  They all start
+// after what the caller queued before the call.  join() makes the caller's stream wait for all of them, so that to
+// the caller the call stays ordered on its own stream; the destructor does the same on any other way out.
+// ev[k][j] is for stream k to record after its half-sweep of colour j.
+struct StreamFork {
+  cudaStream_t s[kMaxSplit + 1];
+  cudaEvent_t ev[kMaxSplit + 1][2] = {};
+  cudaEvent_t fork = nullptr;
+  int n = 0;            // streams forked, joined back by release()
+  int status = TSU_OK;  // otherwise nothing was forked: the call returns this
+
+  StreamFork(cudaStream_t caller, int K, const cudaStream_t* side = nullptr) {
     int dev = 0;
     cudaGetDevice(&dev);
-    cudaEvent_t ev_join;
-    if (cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming) != cudaSuccess) return (int)cudaGetLastError();
-    cudaEventRecord(ev_join, st);
-    const size_t rep_words = 2 * (size_t)rows * words_per_row(cols);
+    s[0] = caller;
+    bool ok = true;
+    for (int k = 1; k < K && ok; ++k) ok = (s[k] = slab_stream(dev, k - 1)) != nullptr;
+    const int m = side ? K + 1 : K;
+    if (side) s[K] = *side;
+    ok = ok && cudaEventCreateWithFlags(&fork, cudaEventDisableTiming) == cudaSuccess;
+    for (int k = 0; k < m && ok; ++k)
+      for (int j = 0; j < 2 && ok; ++j) ok = cudaEventCreateWithFlags(&ev[k][j], cudaEventDisableTiming) == cudaSuccess;
+    if (!ok) {  // (a failed slab_stream need not leave an error behind)
+      const cudaError_t e = cudaGetLastError();
+      status = e != cudaSuccess ? (int)e : (int)cudaErrorUnknown;
+      return;
+    }
+    cudaEventRecord(fork, caller);
+    for (int k = 1; k < m; ++k) cudaStreamWaitEvent(s[k], fork, 0);
+    n = m;
+  }
+  ~StreamFork() { release(); }
+
+  void release() {
+    for (int k = 1; k < n; ++k) {
+      cudaEventRecord(fork, s[k]);
+      cudaStreamWaitEvent(s[0], fork, 0);
+    }
+    n = 0;
+    for (auto& evk : ev)
+      for (cudaEvent_t& e : evk) {
+        if (e) cudaEventDestroy(e);
+        e = nullptr;
+      }
+    if (fork) cudaEventDestroy(fork);
+    fork = nullptr;
+  }
+
+  // status of a call whose launches returned rc, after the join
+  int join(int rc) {
+    release();
+    if (rc != TSU_OK) return rc;
+    TSU_RETURN_LAUNCH_STATUS();
+  }
+};
+
+// the whole-lattice sweeps of tsu_ising2d_sweeps (no halos)
+int launch_sweeps(const Lattice& L, uint32_t sweep0, int n_sweeps, cudaStream_t st) {
+  const Geom& g = L.g;
+  if (n_sweeps == 0) return TSU_OK;
+  // many replicas: independent chunks of replicas, one stream each, no dependency between them at all
+  const int KR = split_replicas(g.n_replicas, g.rows, g.cols);
+  if (KR > 1) {
+    StreamFork F(st, KR);
+    if (F.status != TSU_OK) return F.status;
     int rc = TSU_OK;
     for (int k = 0; k < KR && rc == TSU_OK; ++k) {
-      cudaStream_t sk = k == 0 ? st : slab_stream(dev, k - 1);
-      if (k > 0 && !sk) {  // (the caller's stream may be the default stream: a null handle)
-        rc = (int)cudaErrorUnknown;
-        break;
-      }
-      if (k > 0) cudaStreamWaitEvent(sk, ev_join, 0);
-      const int r0 = (int)((long long)n_replicas * k / KR), r1 = (int)((long long)n_replicas * (k + 1) / KR);
-      const BondParams Bk = {B.words, B.index ? B.index + r0 : nullptr};
+      const int r0 = (int)((long long)g.n_replicas * k / KR), r1 = (int)((long long)g.n_replicas * (k + 1) / KR);
+      const Lattice c = L.replicas(r0, r1);
       for (int t = 0; t < 2 * n_sweeps && rc == TSU_OK; ++t)
-        rc = launch_half_sweep(d_state + (size_t)r0 * rep_words, r1 - r0, rows, cols, wrap_rows, wrap_cols, t & 1, d_lut,
-                               d_lut_index ? d_lut_index + r0 : nullptr, seed, sweep0 + (uint32_t)(t >> 1),
-                               replica0 + (uint32_t)r0, 0, nullptr, nullptr, sk, jit, 0, -1, KR, Bk);
+        rc = launch_half_sweep(c, t & 1, sweep0 + (uint32_t)(t >> 1), nullptr, nullptr, 0, g.rows, KR, F.s[k]);
     }
-    for (int k = 1; k < KR; ++k) {  // also after an error: the caller's stream must not run ahead of what was launched
-      cudaStream_t sk = slab_stream(dev, k - 1);
-      if (!sk) break;
-      cudaEventRecord(ev_join, sk);
-      cudaStreamWaitEvent(st, ev_join, 0);
-    }
-    cudaEventDestroy(ev_join);
-    if (rc != TSU_OK) return rc;
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? TSU_OK : (int)e;
+    return F.join(rc);
   }
-  const int K = split_ranges(n_replicas, rows, cols);
-  if (K <= 2 || n_sweeps == 0) {
+  const int K = split_ranges(g.n_replicas, g.rows, g.cols);
+  if (K <= 2) {
     for (int t = 0; t < 2 * n_sweeps; ++t) {
-      int rc = launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, t & 1, d_lut, d_lut_index, seed,
-                                 sweep0 + (uint32_t)(t >> 1), replica0, 0, nullptr, nullptr, st, jit, 0, -1, 1, B);
+      const int rc = launch_half_sweep(L, t & 1, sweep0 + (uint32_t)(t >> 1), nullptr, nullptr, 0, g.rows, 1, st);
       if (rc != TSU_OK) return rc;
     }
     return TSU_OK;
   }
-  int dev = 0;
-  cudaGetDevice(&dev);
-  cudaStream_t sub[kMaxSplit];
-  sub[0] = st;
-  for (int k = 1; k < K; ++k) {
-    sub[k] = slab_stream(dev, k - 1);
-    if (!sub[k]) return (int)cudaGetLastError();
-  }
+  StreamFork F(st, K);
+  if (F.status != TSU_OK) return F.status;
   int bound[kMaxSplit + 1];
-  for (int k = 0; k <= K; ++k) bound[k] = (int)((long long)rows * k / K);
-  cudaEvent_t ev[kMaxSplit][2], ev_join;
-  bool ev_ok = cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming) == cudaSuccess;
-  for (int k = 0; k < K && ev_ok; ++k)
-    for (int j = 0; j < 2 && ev_ok; ++j) ev_ok = cudaEventCreateWithFlags(&ev[k][j], cudaEventDisableTiming) == cudaSuccess;
-  if (!ev_ok) return (int)cudaGetLastError();
-  cudaEventRecord(ev_join, st);
-  for (int k = 1; k < K; ++k) cudaStreamWaitEvent(sub[k], ev_join, 0);
+  for (int k = 0; k <= K; ++k) bound[k] = (int)((long long)g.rows * k / K);
   int rc = TSU_OK;
   for (int t = 0; t < 2 * n_sweeps && rc == TSU_OK; ++t) {
     const int j = t & 1, jp = j ^ 1;
@@ -973,25 +1036,14 @@ int launch_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wra
     for (int i = 0; i < K && rc == TSU_OK; ++i) {
       const int k = (t + i) % K, above = (k + K - 1) % K, below = (k + 1) % K;
       if (t > 0) {
-        if (k > 0 || wrap_rows) cudaStreamWaitEvent(sub[k], ev[above][jp], 0);
-        if (k + 1 < K || wrap_rows) cudaStreamWaitEvent(sub[k], ev[below][jp], 0);
+        if (k > 0 || g.wrap_rows) cudaStreamWaitEvent(F.s[k], F.ev[above][jp], 0);
+        if (k + 1 < K || g.wrap_rows) cudaStreamWaitEvent(F.s[k], F.ev[below][jp], 0);
       }
-      rc = launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, t & 1, d_lut, d_lut_index, seed,
-                             sweep0 + (uint32_t)(t >> 1), replica0, 0, nullptr, nullptr, sub[k], jit, bound[k], bound[k + 1], K,
-                             B);
-      cudaEventRecord(ev[k][j], sub[k]);
+      rc = launch_half_sweep(L, j, sweep0 + (uint32_t)(t >> 1), nullptr, nullptr, bound[k], bound[k + 1], K, F.s[k]);
+      cudaEventRecord(F.ev[k][j], F.s[k]);
     }
   }
-  for (int k = 1; k < K; ++k) {  // the caller's stream continues after everything issued here
-    cudaEventRecord(ev_join, sub[k]);
-    cudaStreamWaitEvent(st, ev_join, 0);
-  }
-  for (int k = 0; k < K; ++k)
-    for (int j = 0; j < 2; ++j) cudaEventDestroy(ev[k][j]);
-  cudaEventDestroy(ev_join);
-  if (rc != TSU_OK) return rc;
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? TSU_OK : (int)e;
+  return F.join(rc);
 }
 
 // true when a replica is small enough that per-half-sweep launches would be pure launch latency
@@ -1002,87 +1054,12 @@ bool resident_eligible(int n_replicas, int rows, int cols) {
   return per_rep <= 16LL * kResidentThreads && (long long)n_replicas * per_rep <= 148LL * 2048;
 }
 
-int launch_resident_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
-                           const uint32_t* d_lut, const int32_t* d_lut_index, uint64_t seed, uint32_t sweep0, int n_sweeps,
-                           uint32_t replica0, cudaStream_t st, BondParams B = kNoBonds) {
-  SweepParams P = {};
-  P.state = d_state;
-  P.lut = d_lut;
-  P.lut_index = d_lut_index;
-  P.g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, 0);
-  P.sweep = sweep0;
-  P.replica0 = replica0;
-  P.k0 = (uint32_t)seed;
-  P.k1 = (uint32_t)(seed >> 32);
-  P.strip_rows = 1;
-  P.n_strips = rows;
-  if (B.words)
-    sweeps_resident_kernel<true><<<n_replicas, kResidentThreads, 0, st>>>(P, n_sweeps, B);
+int launch_resident_sweeps(const Lattice& L, uint32_t sweep0, int n_sweeps, cudaStream_t st) {
+  const SweepParams P = sweep_params(L, 0, sweep0, nullptr, nullptr);
+  if (L.B.words)
+    sweeps_resident_kernel<true><<<L.g.n_replicas, kResidentThreads, 0, st>>>(P, n_sweeps, L.B);
   else
-    sweeps_resident_kernel<false><<<n_replicas, kResidentThreads, 0, st>>>(P, n_sweeps, kNoBonds);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? TSU_OK : (int)e;
-}
-
-// tsu_ising2d_half_sweep_injected[_bonded]
-int half_sweep_injected(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols, int colour,
-                        const uint32_t* d_lut, const int32_t* d_lut_index, const uint32_t* d_uniforms, int row0,
-                        const uint32_t* d_halo_top, const uint32_t* d_halo_bot, cudaStream_t st, BondParams B) {
-  TSU_CHECK_ARG(d_state && d_lut && d_uniforms && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
-  TSU_CHECK_ARG(colour == 0 || colour == 1);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2) || d_halo_top || d_halo_bot);
-  SweepParams P;
-  P.state = d_state;
-  P.lut = d_lut;
-  P.lut_index = d_lut_index;
-  P.halo_top = d_halo_top;
-  P.halo_bot = d_halo_bot;
-  P.g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
-  P.colour = colour;
-  P.sweep = 0;
-  P.replica0 = 0;
-  P.k0 = P.k1 = 0;
-  P.strip_rows = 1;
-  P.n_strips = rows;
-  const long long total = (long long)n_replicas * rows * P.g.wpr;
-  if (B.words)
-    half_sweep_injected_kernel<true><<<blocks_for(total, 128), 128, 0, st>>>(P, d_uniforms, B);
-  else
-    half_sweep_injected_kernel<false><<<blocks_for(total, 128), 128, 0, st>>>(P, d_uniforms, kNoBonds);
-  TSU_RETURN_LAUNCH_STATUS();
-}
-
-// tsu_ising2d_observables[_bonded]
-int observables(const uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols, int row0,
-                const uint32_t* d_next_rows, unsigned long long* d_out, cudaStream_t st, BondParams B) {
-  TSU_CHECK_ARG(d_state && d_out && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
-  Geom g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
-  cudaError_t e = cudaMemsetAsync(d_out, 0, sizeof(unsigned long long) * 2 * (size_t)n_replicas, st);
-  if (e != cudaSuccess) return (int)e;
-  if (cols % 256 == 0 && !tuning().obs_generic) {
-    const int nvec = g.wpr / 4;
-    int strip = 64;  // long strips re-read one row in `strip`; short ones fill the GPU for small batches
-    while (strip > 1 && (long long)n_replicas * nvec * ((rows + strip - 1) / strip) < 148LL * 2048) strip >>= 1;
-    const int n_strips = (rows + strip - 1) / strip;
-    const long long per_rep_pad = ((long long)n_strips * nvec + 31) / 32 * 32;
-    const unsigned grid = blocks_for((long long)n_replicas * per_rep_pad, 128);
-    if (B.words)
-      observables_fast_kernel<true><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, B);
-    else
-      observables_fast_kernel<false><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, kNoBonds);
-    TSU_RETURN_LAUNCH_STATUS();
-  }
-  TSU_CHECK_ARG(n_replicas <= 65535);  // gridDim.y of the word-by-word kernel
-  const long long n_words = 2LL * rows * g.wpr;
-  long long bx = (n_words + 255) / 256;
-  const long long cap = (148LL * 8 + n_replicas - 1) / n_replicas;  // about 8 CTAs per SM in total
-  if (bx > cap) bx = cap < 1 ? 1 : cap;
-  dim3 grid((unsigned)bx, (unsigned)n_replicas);
-  if (B.words)
-    observables_kernel<true><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, B);
-  else
-    observables_kernel<false><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, kNoBonds);
+    sweeps_resident_kernel<false><<<L.g.n_replicas, kResidentThreads, 0, st>>>(P, n_sweeps, kNoBonds);
   TSU_RETURN_LAUNCH_STATUS();
 }
 
@@ -1131,30 +1108,15 @@ int tsu_ising2d_unpack(const uint32_t* d_state, int8_t* d_spins, int n_replicas,
   TSU_RETURN_LAUNCH_STATUS();
 }
 
-int tsu_ising2d_half_sweep(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
-                           int colour, const uint32_t* d_lut, const int32_t* d_lut_index, uint64_t seed,
-                           uint32_t sweep, uint32_t replica0, int row0, const uint32_t* d_halo_top,
-                           const uint32_t* d_halo_bot, uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
-  TSU_CHECK_ARG(colour == 0 || colour == 1);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2) || d_halo_top || d_halo_bot);
-  return launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, seed,
-                           sweep, replica0, row0, d_halo_top, d_halo_bot, tsu_stream(stream));
-}
-
-int tsu_ising2d_half_sweep_rows(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                                int wrap_cols, int colour, const uint32_t* d_lut, const int32_t* d_lut_index, uint64_t seed,
-                                uint32_t sweep, uint32_t replica0, int row0, const uint32_t* d_halo_top,
-                                const uint32_t* d_halo_bot, int row_begin, int row_end, uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
-  TSU_CHECK_ARG(colour == 0 || colour == 1);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2) || d_halo_top || d_halo_bot);
-  TSU_CHECK_ARG(row_begin >= 0 && row_begin <= row_end && row_end <= rows);
-  const JitKernel jit = (jit_handle > 0 && !d_lut_index) ? jit_function(jit_handle) : JitKernel{nullptr, 0, 0};
-  return launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, seed, sweep,
-                           replica0, row0, d_halo_top, d_halo_bot, tsu_stream(stream), jit, row_begin, row_end);
+int tsu_ising2d_half_sweep(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
+                           int wrap_cols, int colour, const uint32_t* d_lut, const int32_t* d_lut_index,
+                           const uint32_t* d_bonds, const int32_t* d_bond_index, uint64_t seed, uint32_t sweep,
+                           uint32_t replica0, int row0, const uint32_t* d_halo_top, const uint32_t* d_halo_bot,
+                           int row_begin, int row_end, uintptr_t stream) {
+  const Lattice L = {d_state, make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0), d_lut, d_lut_index,
+                     {d_bonds, d_bond_index}, seed, replica0, jit_function(jit_handle, d_lut_index, d_bonds)};
+  TSU_CHECK_ARG(d_state && d_lut && args_ok(L.g, L.B, d_halo_top || d_halo_bot, colour, row_begin, row_end));
+  return launch_half_sweep(L, colour, sweep, d_halo_top, d_halo_bot, row_begin, row_end, 1, tsu_stream(stream));
 }
 
 int tsu_ising2d_slab_sweeps_p2p(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_cols,
@@ -1163,13 +1125,13 @@ int tsu_ising2d_slab_sweeps_p2p(int jit_handle, uint32_t* d_state, int n_replica
                                 uint32_t* d_up_halo, uint32_t* d_up_flags, uint32_t* d_down_halo, uint32_t* d_down_flags,
                                 uint32_t msgs_colour0, uint32_t msgs_colour1, uintptr_t main_stream,
                                 uintptr_t side_stream) {
-  TSU_CHECK_ARG(d_state && d_lut && d_halo && d_flags && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
+  const Lattice L = {d_state, make_geom(n_replicas, rows, cols, 0, wrap_cols, row0), d_lut, d_lut_index, kNoBonds, seed,
+                     replica0, jit_function(jit_handle, d_lut_index, nullptr)};
+  TSU_CHECK_ARG(d_state && d_lut && d_halo && d_flags && args_ok(L.g, L.B, false, 0, 0, rows));
   TSU_CHECK_ARG(rows >= 4 && n_sweeps >= 0 && main_stream != side_stream);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
   TSU_CHECK_ARG((d_up_halo == nullptr) == (d_up_flags == nullptr) && (d_down_halo == nullptr) == (d_down_flags == nullptr));
-  const JitKernel jit = (jit_handle > 0 && !d_lut_index) ? jit_function(jit_handle) : JitKernel{nullptr, 0, 0};
   cudaStream_t main = tsu_stream(main_stream), side = tsu_stream(side_stream);
-  const int wpr = words_per_row(cols);
+  const int wpr = L.g.wpr;
   const size_t side_words = (size_t)n_replicas * wpr;  // one halo row set
   auto halo = [&](uint32_t* base, int colour, int which) { return base ? base + ((size_t)colour * 2 + which) * side_words : nullptr; };
   auto flag = [&](uint32_t* base, int colour, int which) { return base ? base + colour * 2 + which : nullptr; };
@@ -1178,25 +1140,13 @@ int tsu_ising2d_slab_sweeps_p2p(int jit_handle, uint32_t* d_state, int n_replica
   // ranges k - 1, k, k + 1 (and, at the ends, on the boundary rows) of the half-sweep before, so the first ranges of
   // the next half-sweep fill the SMs while the last ranges of this one drain.  A single launch per half-sweep loses
   // ~15 us to its tail (launch gap + the last warps finishing alone), 6 % of a 16384 x 131072 slab.
-  int dev = 0;
-  cudaGetDevice(&dev);
   const int K = split_ranges(n_replicas, rows - 2, cols);
-  cudaStream_t sub[kMaxSplit];
-  sub[0] = main;
-  for (int k = 1; k < K; ++k) {
-    sub[k] = slab_stream(dev, k - 1);
-    if (!sub[k]) return (int)cudaGetLastError();
-  }
   int bound[kMaxSplit + 1];  // range k = local rows [bound[k], bound[k + 1])
   for (int k = 0; k <= K; ++k) bound[k] = 1 + (int)((long long)(rows - 2) * k / K);
-  // strips as long as one launch over the whole interior would use
-  cudaEvent_t ev_sub[kMaxSplit][2], ev_bnd[2], ev_join;
-  bool ev_ok = cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming) == cudaSuccess;
-  for (int j = 0; j < 2 && ev_ok; ++j) {
-    ev_ok = cudaEventCreateWithFlags(&ev_bnd[j], cudaEventDisableTiming) == cudaSuccess;
-    for (int k = 0; k < K && ev_ok; ++k) ev_ok = cudaEventCreateWithFlags(&ev_sub[k][j], cudaEventDisableTiming) == cudaSuccess;
-  }
-  if (!ev_ok) return (int)cudaGetLastError();
+  // range k runs on F.s[k]; the boundary rows run on the side stream F.s[K] and record F.ev[K].  Everything the caller
+  // queued on the main stream (e.g. a changed state) precedes the first rows sent and updated.
+  StreamFork F(main, K, &side);
+  if (F.status != TSU_OK) return F.status;
   const unsigned send_grid = blocks_for(2LL * n_replicas * (wpr / 4), 256) < 64u ? blocks_for(2LL * n_replicas * (wpr / 4), 256) : 64u;
   // what a half-sweep of `colour` sends afterwards: my first row to the rank above (its "below" halo), my last row
   // to the rank below (its "above" halo), then the message number
@@ -1207,10 +1157,6 @@ int tsu_ising2d_slab_sweeps_p2p(int jit_handle, uint32_t* d_state, int n_replica
     slab_signal_kernel<<<1, 1, 0, side>>>(flag(d_up_flags, colour, 1), flag(d_down_flags, colour, 0), msgs[colour]);
   };
   int rc = TSU_OK;
-  // everything the caller queued on the main stream (e.g. a changed state) precedes the first rows sent and updated
-  cudaEventRecord(ev_join, main);
-  cudaStreamWaitEvent(side, ev_join, 0);
-  for (int k = 1; k < K; ++k) cudaStreamWaitEvent(sub[k], ev_join, 0);
   send(1);  // colour 0 goes first and reads colour 1
   for (int t = 0; t < 2 * n_sweeps && rc == TSU_OK; ++t) {
     const int colour = t & 1, opp = 1 - colour, j = t & 1, jp = j ^ 1;
@@ -1218,76 +1164,96 @@ int tsu_ising2d_slab_sweeps_p2p(int jit_handle, uint32_t* d_state, int n_replica
     // interior ranges: each reads and overwrites rows next to what its neighbours updated in the half-sweep before
     for (int k = 0; k < K && rc == TSU_OK; ++k) {
       if (t > 0) {
-        if (k > 0) cudaStreamWaitEvent(sub[k], ev_sub[k - 1][jp], 0);
-        if (k + 1 < K) cudaStreamWaitEvent(sub[k], ev_sub[k + 1][jp], 0);
-        if (k == 0 || k + 1 == K) cudaStreamWaitEvent(sub[k], ev_bnd[jp], 0);
+        if (k > 0) cudaStreamWaitEvent(F.s[k], F.ev[k - 1][jp], 0);
+        if (k + 1 < K) cudaStreamWaitEvent(F.s[k], F.ev[k + 1][jp], 0);
+        if (k == 0 || k + 1 == K) cudaStreamWaitEvent(F.s[k], F.ev[K][jp], 0);
       }
-      rc = launch_half_sweep(d_state, n_replicas, rows, cols, 0, wrap_cols, colour, d_lut, d_lut_index, seed, sweep, replica0,
-                             row0, nullptr, nullptr, sub[k], jit, bound[k], bound[k + 1], K);
-      cudaEventRecord(ev_sub[k][j], sub[k]);
+      rc = launch_half_sweep(L, colour, sweep, nullptr, nullptr, bound[k], bound[k + 1], K, F.s[k]);
+      cudaEventRecord(F.ev[k][j], F.s[k]);
     }
     if (rc != TSU_OK) break;
     // boundary rows on the side stream: after the previous update of the rows next to them and the arrival of the
     // neighbours' rows of the other colour
     if (t > 0) {
-      cudaStreamWaitEvent(side, ev_sub[0][jp], 0);
-      if (K > 1) cudaStreamWaitEvent(side, ev_sub[K - 1][jp], 0);
+      cudaStreamWaitEvent(side, F.ev[0][jp], 0);
+      if (K > 1) cudaStreamWaitEvent(side, F.ev[K - 1][jp], 0);
     }
     const uint32_t* top = d_up_halo ? halo(d_halo, opp, 0) : nullptr;
     const uint32_t* bot = d_down_halo ? halo(d_halo, opp, 1) : nullptr;
     if (top || bot)
       slab_wait_kernel<<<1, 1, 0, side>>>(top ? flag(d_flags, opp, 0) : nullptr, bot ? flag(d_flags, opp, 1) : nullptr,
                                           msgs[opp], d_flags + 8);
-    rc = launch_half_sweep(d_state, n_replicas, rows, cols, 0, wrap_cols, colour, d_lut, d_lut_index, seed, sweep, replica0,
-                           row0, top, bot, side, jit, 0, 1);
-    if (rc == TSU_OK)
-      rc = launch_half_sweep(d_state, n_replicas, rows, cols, 0, wrap_cols, colour, d_lut, d_lut_index, seed, sweep, replica0,
-                             row0, top, bot, side, jit, rows - 1, rows);
-    cudaEventRecord(ev_bnd[j], side);
+    rc = launch_half_sweep(L, colour, sweep, top, bot, 0, 1, 1, side);
+    if (rc == TSU_OK) rc = launch_half_sweep(L, colour, sweep, top, bot, rows - 1, rows, 1, side);
+    cudaEventRecord(F.ev[K][j], side);
     send(colour);
   }
-  // the caller's stream continues after everything issued here
-  cudaEventRecord(ev_join, side);
-  cudaStreamWaitEvent(main, ev_join, 0);
-  for (int k = 1; k < K; ++k) {
-    cudaEventRecord(ev_join, sub[k]);
-    cudaStreamWaitEvent(main, ev_join, 0);
-  }
-  for (int j = 0; j < 2; ++j) {
-    cudaEventDestroy(ev_bnd[j]);
-    for (int k = 0; k < K; ++k) cudaEventDestroy(ev_sub[k][j]);
-  }
-  cudaEventDestroy(ev_join);
-  if (rc != TSU_OK) return rc;
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? TSU_OK : (int)e;
+  return F.join(rc);
 }
 
-int tsu_ising2d_sweeps(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
-                       const uint32_t* d_lut, const int32_t* d_lut_index, uint64_t seed, uint32_t sweep0, int n_sweeps,
-                       uint32_t replica0, uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && geom_ok(n_replicas, rows, cols) && n_sweeps >= 0);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
-  if (n_sweeps > 0 && resident_eligible(n_replicas, rows, cols))
-    return launch_resident_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, d_lut_index, seed, sweep0,
-                                  n_sweeps, replica0, tsu_stream(stream));
-  return launch_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, d_lut_index, seed, sweep0, n_sweeps,
-                       replica0, tsu_stream(stream), JitKernel{nullptr, 0, 0});
+int tsu_ising2d_sweeps(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
+                       int wrap_cols, const uint32_t* d_lut, const int32_t* d_lut_index, const uint32_t* d_bonds,
+                       const int32_t* d_bond_index, uint64_t seed, uint32_t sweep0, int n_sweeps, uint32_t replica0,
+                       uintptr_t stream) {
+  const Lattice L = {d_state, make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, 0), d_lut, d_lut_index,
+                     {d_bonds, d_bond_index}, seed, replica0, jit_function(jit_handle, d_lut_index, d_bonds)};
+  TSU_CHECK_ARG(d_state && d_lut && n_sweeps >= 0 && args_ok(L.g, L.B, false, 0, 0, rows));
+  if (n_sweeps > 0 && resident_eligible(n_replicas, rows, cols))  // launch latency dominates: one launch for everything
+    return launch_resident_sweeps(L, sweep0, n_sweeps, tsu_stream(stream));
+  return launch_sweeps(L, sweep0, n_sweeps, tsu_stream(stream));
 }
 
 int tsu_ising2d_half_sweep_injected(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
                                     int wrap_cols, int colour, const uint32_t* d_lut, const int32_t* d_lut_index,
-                                    const uint32_t* d_uniforms, int row0, const uint32_t* d_halo_top,
-                                    const uint32_t* d_halo_bot, uintptr_t stream) {
-  return half_sweep_injected(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, d_uniforms,
-                             row0, d_halo_top, d_halo_bot, tsu_stream(stream), kNoBonds);
+                                    const uint32_t* d_bonds, const int32_t* d_bond_index, const uint32_t* d_uniforms,
+                                    int row0, const uint32_t* d_halo_top, const uint32_t* d_halo_bot,
+                                    uintptr_t stream) {
+  const Lattice L = {d_state, make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0), d_lut, d_lut_index,
+                     {d_bonds, d_bond_index}, 0, 0, JitKernel{nullptr, 0, 0}};
+  TSU_CHECK_ARG(d_state && d_lut && d_uniforms && args_ok(L.g, L.B, d_halo_top || d_halo_bot, colour, 0, rows));
+  const SweepParams P = sweep_params(L, colour, 0, d_halo_top, d_halo_bot);
+  const unsigned grid = blocks_for((long long)n_replicas * rows * L.g.wpr, 128);
+  cudaStream_t st = tsu_stream(stream);
+  if (d_bonds)
+    half_sweep_injected_kernel<true><<<grid, 128, 0, st>>>(P, d_uniforms, L.B);
+  else
+    half_sweep_injected_kernel<false><<<grid, 128, 0, st>>>(P, d_uniforms, kNoBonds);
+  TSU_RETURN_LAUNCH_STATUS();
 }
 
 int tsu_ising2d_observables(const uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
-                            int row0, const uint32_t* d_next_rows, unsigned long long* d_out, uintptr_t stream) {
-  return observables(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, row0, d_next_rows, d_out, tsu_stream(stream),
-                     kNoBonds);
+                            const uint32_t* d_bonds, const int32_t* d_bond_index, int row0, const uint32_t* d_next_rows,
+                            unsigned long long* d_out, uintptr_t stream) {
+  const Geom g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
+  const BondParams B = {d_bonds, d_bond_index};
+  TSU_CHECK_ARG(d_state && d_out && args_ok(g, B, d_next_rows != nullptr, 0, 0, rows));
+  cudaStream_t st = tsu_stream(stream);
+  cudaError_t e = cudaMemsetAsync(d_out, 0, sizeof(unsigned long long) * 2 * (size_t)n_replicas, st);
+  if (e != cudaSuccess) return (int)e;
+  if (cols % 256 == 0 && !tuning().obs_generic) {
+    const int nvec = g.wpr / 4;
+    int strip = 64;  // long strips re-read one row in `strip`; short ones fill the GPU for small batches
+    while (strip > 1 && (long long)n_replicas * nvec * ((rows + strip - 1) / strip) < 148LL * 2048) strip >>= 1;
+    const int n_strips = (rows + strip - 1) / strip;
+    const long long per_rep_pad = ((long long)n_strips * nvec + 31) / 32 * 32;
+    const unsigned grid = blocks_for((long long)n_replicas * per_rep_pad, 128);
+    if (d_bonds)
+      observables_fast_kernel<true><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, B);
+    else
+      observables_fast_kernel<false><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, kNoBonds);
+    TSU_RETURN_LAUNCH_STATUS();
+  }
+  TSU_CHECK_ARG(n_replicas <= 65535);  // gridDim.y of the word-by-word kernel
+  const long long n_words = 2LL * rows * g.wpr;
+  long long bx = (n_words + 255) / 256;
+  const long long cap = (148LL * 8 + n_replicas - 1) / n_replicas;  // about 8 CTAs per SM in total
+  if (bx > cap) bx = cap < 1 ? 1 : cap;
+  dim3 grid((unsigned)bx, (unsigned)n_replicas);
+  if (d_bonds)
+    observables_kernel<true><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, B);
+  else
+    observables_kernel<false><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, kNoBonds);
+  TSU_RETURN_LAUNCH_STATUS();
 }
 
 int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_replicas, double J, double h,
@@ -1352,87 +1318,14 @@ int tsu_ising2d_jit_prepare(const uint32_t* h_lut, const char* src_dir, char* lo
   return handle;
 }
 
-int tsu_ising2d_half_sweep_jit(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                               int wrap_cols, int colour, const uint32_t* d_lut, uint64_t seed, uint32_t sweep,
-                               uint32_t replica0, int row0, const uint32_t* d_halo_top, const uint32_t* d_halo_bot,
-                               uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && geom_ok(n_replicas, rows, cols) && rows_ok(rows, row0));
-  TSU_CHECK_ARG(colour == 0 || colour == 1);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2) || d_halo_top || d_halo_bot);
-  return launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, nullptr, seed, sweep,
-                           replica0, row0, d_halo_top, d_halo_bot, tsu_stream(stream), jit_function(jit_handle));
-}
-
-int tsu_ising2d_sweeps_jit(int jit_handle, uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                           int wrap_cols, const uint32_t* d_lut, uint64_t seed, uint32_t sweep0, int n_sweeps,
-                           uint32_t replica0, uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && geom_ok(n_replicas, rows, cols) && n_sweeps >= 0);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
-  if (n_sweeps > 0 && resident_eligible(n_replicas, rows, cols))  // launch latency dominates: one launch for everything
-    return launch_resident_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, nullptr, seed, sweep0,
-                                  n_sweeps, replica0, tsu_stream(stream));
-  return launch_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, nullptr, seed, sweep0, n_sweeps, replica0,
-                       tsu_stream(stream), jit_function(jit_handle));
-}
-
 // ---- Edwards-Anderson +-J lattices: the same update with bond words XOR-ed into the neighbour words ----------
 int tsu_ising2d_pack_bonds(const int8_t* d_signs, uint32_t* d_bonds, int n_real, int rows, int cols, int wrap_rows,
                            int wrap_cols, uintptr_t stream) {
-  TSU_CHECK_ARG(d_signs && d_bonds && geom_ok(n_real, rows, cols));
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
   const Geom g = make_geom(n_real, rows, cols, wrap_rows, wrap_cols, 0);
+  TSU_CHECK_ARG(d_signs && d_bonds && args_ok(g, kNoBonds, false, 0, 0, rows));
   const long long total = 8LL * n_real * rows * g.wpr;
   pack_bonds_kernel<<<blocks_for(total, 256), 256, 0, tsu_stream(stream)>>>(d_signs, d_bonds, n_real, g);
   TSU_RETURN_LAUNCH_STATUS();
-}
-
-int tsu_ising2d_sweeps_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
-                              const uint32_t* d_lut, const int32_t* d_lut_index, const uint32_t* d_bonds,
-                              const int32_t* d_bond_index, uint64_t seed, uint32_t sweep0, int n_sweeps, uint32_t replica0,
-                              uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && d_bonds && geom_ok(n_replicas, rows, cols) && n_sweeps >= 0);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
-  const BondParams B = {d_bonds, d_bond_index};
-  if (n_sweeps > 0 && resident_eligible(n_replicas, rows, cols))
-    return launch_resident_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, d_lut_index, seed, sweep0,
-                                  n_sweeps, replica0, tsu_stream(stream), B);
-  return launch_sweeps(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, d_lut, d_lut_index, seed, sweep0, n_sweeps,
-                       replica0, tsu_stream(stream), JitKernel{nullptr, 0, 0}, B);
-}
-
-int tsu_ising2d_half_sweep_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
-                                  int colour, const uint32_t* d_lut, const int32_t* d_lut_index, const uint32_t* d_bonds,
-                                  const int32_t* d_bond_index, uint64_t seed, uint32_t sweep, uint32_t replica0,
-                                  int row_begin, int row_end, uintptr_t stream) {
-  TSU_CHECK_ARG(d_state && d_lut && d_bonds && geom_ok(n_replicas, rows, cols));
-  TSU_CHECK_ARG(colour == 0 || colour == 1);
-  TSU_CHECK_ARG(!wrap_cols || (cols % 2 == 0 && cols > 2));
-  TSU_CHECK_ARG(!wrap_rows || (rows % 2 == 0 && rows > 2));
-  TSU_CHECK_ARG(row_begin >= 0 && row_begin <= row_end && row_end <= rows);
-  return launch_half_sweep(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, seed, sweep,
-                           replica0, 0, nullptr, nullptr, tsu_stream(stream), JitKernel{nullptr, 0, 0}, row_begin, row_end,
-                           1, BondParams{d_bonds, d_bond_index});
-}
-
-int tsu_ising2d_half_sweep_injected_bonded(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                                           int wrap_cols, int colour, const uint32_t* d_lut, const int32_t* d_lut_index,
-                                           const uint32_t* d_bonds, const int32_t* d_bond_index,
-                                           const uint32_t* d_uniforms, uintptr_t stream) {
-  TSU_CHECK_ARG(d_bonds);
-  return half_sweep_injected(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, colour, d_lut, d_lut_index, d_uniforms,
-                             0, nullptr, nullptr, tsu_stream(stream), BondParams{d_bonds, d_bond_index});
-}
-
-int tsu_ising2d_observables_bonded(const uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows,
-                                   int wrap_cols, const uint32_t* d_bonds, const int32_t* d_bond_index,
-                                   unsigned long long* d_out, uintptr_t stream) {
-  TSU_CHECK_ARG(d_bonds);
-  return observables(d_state, n_replicas, rows, cols, wrap_rows, wrap_cols, 0, nullptr, d_out, tsu_stream(stream),
-                     BondParams{d_bonds, d_bond_index});
 }
 
 int tsu_ising2d_overlap(const uint32_t* d_state, int n_replicas, int rows, int cols, const int32_t* d_pairs, int n_pairs,

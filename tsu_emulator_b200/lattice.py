@@ -138,7 +138,7 @@ class Ising2DEngine:
     ):
         if bonds is not None:  # checked before anything touches the device
             bonds, bond_index = check_bonds(bonds, bond_index, rows, cols, n_replicas, bias_mode,
-                                            global_rows is not None and int(global_rows) != int(rows))
+                                            global_rows is not None and int(global_rows) != int(rows) or int(row0) != 0)
         elif bond_index is not None:
             raise ValueError("bond_index needs bonds")
         torch = _lib.require_cuda()
@@ -327,82 +327,34 @@ class Ising2DEngine:
     def half_sweep(self, colour: int, halo_top=None, halo_bot=None, uniforms=None, rows=None):
         """resample every site of `colour`; halos are [n_replicas, wpr] int32 rows of the other colour.
         rows=(begin, end) restricts the update to those local rows (same bits for any split of the rows)."""
+        if self.bonds is not None and (halo_top is not None or halo_bot is not None):
+            raise ValueError("bonded engines have no halos")
+        if uniforms is not None and rows is not None:
+            raise ValueError("row ranges are not available in injected-uniform mode")
+        lat = (ptr(self.state), self.n_replicas, self.rows, self.cols, int(self.wrap_rows and not self.is_slab),
+                   int(self.wrap_cols), int(colour), ptr(self.lut), ptr(self.lut_index), ptr(self.bonds),
+                   ptr(self.bond_index))
         with self._torch.cuda.device(self.device):
-            if self.bonds is not None:
-                if halo_top is not None or halo_bot is not None:
-                    raise ValueError("bonded engines have no halos")
-                if uniforms is not None:
-                    if rows is not None:
-                        raise ValueError("row ranges are not available in injected-uniform mode")
-                    _lib.call(
-                        "tsu_ising2d_half_sweep_injected_bonded", ptr(self.state), self.n_replicas, self.rows,
-                        self.cols, int(self.wrap_rows), int(self.wrap_cols), int(colour), ptr(self.lut),
-                        ptr(self.lut_index), ptr(self.bonds), ptr(self.bond_index), ptr(uniforms), _lib.current_stream(),
-                    )
-                else:
-                    begin, end = (0, self.rows) if rows is None else (int(rows[0]), int(rows[1]))
-                    _lib.call(
-                        "tsu_ising2d_half_sweep_bonded", ptr(self.state), self.n_replicas, self.rows, self.cols,
-                        int(self.wrap_rows), int(self.wrap_cols), int(colour), ptr(self.lut), ptr(self.lut_index),
-                        ptr(self.bonds), ptr(self.bond_index), self.seed, self.sweep_index & 0xFFFFFFFF, self.replica0,
-                        begin, end, _lib.current_stream(),
-                    )
-            elif rows is not None:
-                if uniforms is not None:
-                    raise ValueError("row ranges are not available in injected-uniform mode")
-                _lib.call(
-                    "tsu_ising2d_half_sweep_rows", int(getattr(self, "_jit", 0)) if self.lut_index is None else 0,
-                    ptr(self.state), self.n_replicas, self.rows, self.cols,
-                    int(self.wrap_rows and not self.is_slab), int(self.wrap_cols), int(colour), ptr(self.lut),
-                    ptr(self.lut_index), self.seed, self.sweep_index & 0xFFFFFFFF, self.replica0, self.row0,
-                    ptr(halo_top), ptr(halo_bot), int(rows[0]), int(rows[1]), _lib.current_stream(),
-                )
-            elif uniforms is None and self.lut_index is None and getattr(self, "_jit", 0) > 0:
-                _lib.call(
-                    "tsu_ising2d_half_sweep_jit", self._jit, ptr(self.state), self.n_replicas, self.rows, self.cols,
-                    int(self.wrap_rows and not self.is_slab), int(self.wrap_cols), int(colour), ptr(self.lut),
-                    self.seed, self.sweep_index & 0xFFFFFFFF, self.replica0, self.row0, ptr(halo_top), ptr(halo_bot),
-                    _lib.current_stream(),
-                )
-            elif uniforms is None:
-                _lib.call(
-                    "tsu_ising2d_half_sweep", ptr(self.state), self.n_replicas, self.rows, self.cols,
-                    int(self.wrap_rows and not self.is_slab), int(self.wrap_cols), int(colour), ptr(self.lut),
-                    ptr(self.lut_index), self.seed, self.sweep_index & 0xFFFFFFFF, self.replica0, self.row0,
-                    ptr(halo_top), ptr(halo_bot), _lib.current_stream(),
-                )
+            if uniforms is not None:
+                _lib.call("tsu_ising2d_half_sweep_injected", *lat, ptr(uniforms), self.row0, ptr(halo_top),
+                          ptr(halo_bot), _lib.current_stream())
             else:
-                _lib.call(
-                    "tsu_ising2d_half_sweep_injected", ptr(self.state), self.n_replicas, self.rows, self.cols,
-                    int(self.wrap_rows and not self.is_slab), int(self.wrap_cols), int(colour), ptr(self.lut),
-                    ptr(self.lut_index), ptr(uniforms), self.row0, ptr(halo_top), ptr(halo_bot),
-                    _lib.current_stream(),
-                )
+                begin, end = (0, self.rows) if rows is None else (int(rows[0]), int(rows[1]))
+                _lib.call("tsu_ising2d_half_sweep", self._jit if self.lut_index is None else 0, *lat, self.seed,
+                          self.sweep_index & 0xFFFFFFFF, self.replica0, self.row0, ptr(halo_top), ptr(halo_bot), begin,
+                          end, _lib.current_stream())
 
     def sweep(self, n_sweeps: int = 1):
         """n full sweeps: black half-sweep then white half-sweep (one gibbs_update each)."""
         if self.is_slab:
             raise RuntimeError("row-slab engines are driven by ShardedIsing2D (halo exchange between half-sweeps)")
         with self._torch.cuda.device(self.device):
-            if self.bonds is not None:
-                _lib.call(
-                    "tsu_ising2d_sweeps_bonded", ptr(self.state), self.n_replicas, self.rows, self.cols,
-                    int(self.wrap_rows), int(self.wrap_cols), ptr(self.lut), ptr(self.lut_index), ptr(self.bonds),
-                    ptr(self.bond_index), self.seed, self.sweep_index & 0xFFFFFFFF, int(n_sweeps), self.replica0,
-                    _lib.current_stream(),
-                )
-            elif self.lut_index is None and getattr(self, "_jit", 0) > 0:
-                _lib.call(
-                    "tsu_ising2d_sweeps_jit", self._jit, ptr(self.state), self.n_replicas, self.rows, self.cols,
-                    int(self.wrap_rows), int(self.wrap_cols), ptr(self.lut), self.seed, self.sweep_index & 0xFFFFFFFF,
-                    int(n_sweeps), self.replica0, _lib.current_stream(),
-                )
-            else:
-                _lib.call(
-                    "tsu_ising2d_sweeps", ptr(self.state), self.n_replicas, self.rows, self.cols, int(self.wrap_rows),
-                    int(self.wrap_cols), ptr(self.lut), ptr(self.lut_index), self.seed, self.sweep_index & 0xFFFFFFFF,
-                    int(n_sweeps), self.replica0, _lib.current_stream(),
-                )
+            _lib.call(
+                "tsu_ising2d_sweeps", self._jit if self.lut_index is None else 0, ptr(self.state), self.n_replicas,
+                self.rows, self.cols, int(self.wrap_rows), int(self.wrap_cols), ptr(self.lut), ptr(self.lut_index),
+                ptr(self.bonds), ptr(self.bond_index), self.seed, self.sweep_index & 0xFFFFFFFF, int(n_sweeps),
+                self.replica0, _lib.current_stream(),
+            )
         self.sweep_index += int(n_sweeps)
         return self
 
@@ -423,20 +375,13 @@ class Ising2DEngine:
     def observables_tensor(self, next_rows=None):
         """int64 tensor [n_replicas, 2]: (# up spins, # anti-aligned right+down bonds) of the local rows;
         with bonds the second column counts unsatisfied bonds (sign * s_i * s_j = -1)"""
+        if self.bonds is not None and next_rows is not None:
+            raise ValueError("bonded engines have no halos")
         with self._torch.cuda.device(self.device):
-            if self.bonds is not None:
-                if next_rows is not None:
-                    raise ValueError("bonded engines have no halos")
-                _lib.call(
-                    "tsu_ising2d_observables_bonded", ptr(self.state), self.n_replicas, self.rows, self.cols,
-                    int(self.wrap_rows), int(self.wrap_cols), ptr(self.bonds), ptr(self.bond_index), ptr(self._obs),
-                    _lib.current_stream(),
-                )
-                return self._obs
             _lib.call(
                 "tsu_ising2d_observables", ptr(self.state), self.n_replicas, self.rows, self.cols,
-                int(self.wrap_rows and not self.is_slab), int(self.wrap_cols), self.row0, ptr(next_rows),
-                ptr(self._obs), _lib.current_stream(),
+                int(self.wrap_rows and not self.is_slab), int(self.wrap_cols), ptr(self.bonds), ptr(self.bond_index),
+                self.row0, ptr(next_rows), ptr(self._obs), _lib.current_stream(),
             )
         return self._obs
 
