@@ -203,6 +203,27 @@ int tsu_ising2d_overlap(const uint32_t* d_state, int n_replicas, int rows, int c
                         const int32_t* d_pairs, int n_pairs, unsigned long long* d_out,
                         uintptr_t stream);
 
+/* Simulated annealing of whole lattices (tsu/gibbs.py:340-393 on the lattice): n_steps sweeps, step k with the
+ * threshold table d_luts[k] (layout above) and sweep index sweep0 + k, for every replica; no host sync inside.
+ * The initial state and the state after every step are evaluated: d_energy[r] gets E of the final state (formula and
+ * float64 rounding of tsu_ising2d_energy_from_observables, exact integer counts), and with d_best_energy /
+ * d_best_state (in/out, both set or both NULL) a replica whose E is strictly below d_best_energy[r] takes E and
+ * copies its state words [2][rows][wpr] to d_best_state[r].  An anneal split into calls that share the best buffers
+ * therefore equals one call.  The bits equal, step for step, tsu_ising2d_sweeps(n_sweeps = 1) with that table
+ * followed by tsu_ising2d_observables and tsu_ising2d_energy_from_observables.
+ * Bonds as in tsu_ising2d_sweeps; whole lattices only (no halos, row0 = 0); always the prebuilt kernels.
+ * d_obs: [n_replicas][2] scratch (left holding flags, not counts).  n_steps = 0 evaluates the initial state only.
+ * Lattices that tsu_ising2d_sweeps runs in one launch run the whole anneal in one launch, one thread block per
+ * replica (TSU_LATTICE_RESIDENT=0 disables); the others run per step the sweep launches of tsu_ising2d_sweeps, the
+ * counts, one select kernel and, for the replicas that improved, one copy kernel.  Replica chunks anneal on streams
+ * of their own; everything is joined back into `stream` before the call returns. */
+int tsu_ising2d_anneal(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                       const uint32_t* d_luts, int n_steps, const uint32_t* d_bonds,
+                       const int32_t* d_bond_index, uint64_t seed, uint32_t sweep0, uint32_t replica0,
+                       double J, double h, long long n_bonds, long long n_sites,
+                       unsigned long long* d_obs, double* d_energy, double* d_best_energy,
+                       uint32_t* d_best_state, uintptr_t stream);
+
 /* ------------------------------------------------------------------ dense-J Gibbs ----- */
 /*
  * Replaces GibbsSampler.gibbs_sweep / sample_boltzmann / compute_energy and the sweep part of

@@ -78,6 +78,11 @@ SIGNATURES = {
     ),
     "tsu_ising2d_pack_bonds": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_uintptr]),
     "tsu_ising2d_overlap": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_uintptr]),
+    "tsu_ising2d_anneal": (
+        c_int,
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_uint64, c_uint32, c_uint32,
+         c_double, c_double, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_uintptr],
+    ),
     "tsu_dense_gibbs_run": (
         c_int,
         [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_void_p, c_int, c_int, c_int,

@@ -450,6 +450,29 @@ __global__ void unpack_kernel(const uint32_t* __restrict__ state, int8_t* spins,
   }
 }
 
+// Adds to ups / anti the up spins and the anti-aligned (right + down) bonds of word (rep, colour, local row i, w);
+// bonded: unsatisfied bonds (sigma s_i s_j = -1) instead of anti-aligned ones.  plane = rows * wpr.
+template <bool BONDED>
+__device__ __forceinline__ void count_word(const uint32_t* state, const Geom& g, size_t plane, const uint32_t* next_rows,
+                                           const BondParams& B, int rep, int colour, int i, int w,
+                                           unsigned long long& ups, unsigned long long& anti) {
+  const uint32_t* own = state + ((size_t)rep * 2 + colour) * plane;
+  Planes pl;
+  pl.opp = state + ((size_t)rep * 2 + (1 - colour)) * plane;
+  pl.halo_top = nullptr;
+  pl.halo_bot = next_rows ? next_rows + ((size_t)rep * 2 + (1 - colour)) * g.wpr : nullptr;
+  Hood h = load_hood(pl, g, colour, i, w);
+  if (h.valid == 0u) return;
+  if constexpr (BONDED) apply_bonds(h, B, g, rep, colour, i, w);
+  const uint32_t x = own[(size_t)i * g.wpr + w];
+  const int p = (g.row0 + i + colour) & 1;
+  ups += __popc(x & h.valid);
+  // east neighbour: centre word if own col is even (p == 0), shifted word otherwise
+  const uint32_t east = p ? h.side : h.c;
+  anti += __popc((x ^ east) & h.valid & ~h.missE);
+  if (h.has_s) anti += __popc((x ^ h.s) & h.valid);
+}
+
 // up-spin count and anti-aligned (right + down) bond count per replica; bonded: unsatisfied bonds (sigma s_i s_j = -1)
 template <bool BONDED>
 __global__ void __launch_bounds__(256) observables_kernel(const uint32_t* __restrict__ state, Geom g,
@@ -465,21 +488,7 @@ __global__ void __launch_bounds__(256) observables_kernel(const uint32_t* __rest
     const long long rem = t - (long long)colour * g.rows * g.wpr;
     const int i = (int)(rem / g.wpr);
     const int w = (int)(rem - (long long)i * g.wpr);
-    const uint32_t* own = state + ((size_t)rep * 2 + colour) * plane;
-    Planes pl;
-    pl.opp = state + ((size_t)rep * 2 + (1 - colour)) * plane;
-    pl.halo_top = nullptr;
-    pl.halo_bot = next_rows ? next_rows + ((size_t)rep * 2 + (1 - colour)) * g.wpr : nullptr;
-    Hood h = load_hood(pl, g, colour, i, w);
-    if (h.valid == 0u) continue;
-    if constexpr (BONDED) apply_bonds(h, B, g, rep, colour, i, w);
-    const uint32_t x = own[(size_t)i * g.wpr + w];
-    const int p = (g.row0 + i + colour) & 1;
-    ups += __popc(x & h.valid);
-    // east neighbour: centre word if own col is even (p == 0), shifted word otherwise
-    const uint32_t east = p ? h.side : h.c;
-    anti += __popc((x ^ east) & h.valid & ~h.missE);
-    if (h.has_s) anti += __popc((x ^ h.s) & h.valid);
+    count_word<BONDED>(state, g, plane, next_rows, B, rep, colour, i, w, ups, anti);
   }
   ups = tsu_warp_sum(ups);
   anti = tsu_warp_sum(anti);
@@ -577,13 +586,120 @@ __global__ void __launch_bounds__(128) observables_fast_kernel(const uint32_t* _
   }
 }
 
+// E = -J (n_bonds - 2 anti) - h (2 up - n_sites).  The two differences are exact (integers below 2^53); the rounding
+// is spelled out as one product and one fused multiply-add, so that every kernel computing E rounds the same way.
+__device__ __forceinline__ double energy_of_counts(double up, double anti, double J, double h, long long n_bonds,
+                                                   long long n_sites) {
+  return fma(-J, (double)n_bonds - 2.0 * anti, -__dmul_rn(h, 2.0 * up - (double)n_sites));
+}
+
 __global__ void energy_from_obs_kernel(const unsigned long long* __restrict__ obs, int n, double J, double h,
                                        long long n_bonds, long long n_sites, double* energy) {
   int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= n) return;
-  const double up = (double)obs[2 * r];
-  const double anti = (double)obs[2 * r + 1];
-  energy[r] = -J * ((double)n_bonds - 2.0 * anti) - h * (2.0 * up - (double)n_sites);
+  energy[r] = energy_of_counts((double)obs[2 * r], (double)obs[2 * r + 1], J, h, n_bonds, n_sites);
+}
+
+// ---- simulated annealing (tsu_ising2d_anneal) -----------------------------------------------------------------
+// What an anneal step does after its sweep: E of every replica from its counts, and the strict best-so-far update.
+struct AnnealOut {
+  double J, h;
+  long long n_bonds, n_sites;
+  double* energy;       // [replicas] E of the current state
+  double* best_energy;  // [replicas] in/out, or NULL (then best_state is NULL too)
+  uint32_t* best_state; // [replicas][2][rows][wpr]
+};
+
+// obs[r] = (up, anti) -> energy[r]; replicas with E < best_energy[r] take E, and obs[2r] becomes 1 if they did, else 0
+// (the flag anneal_copy_kernel reads)
+__global__ void anneal_select_kernel(unsigned long long* obs, int n, AnnealOut A) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const double e = energy_of_counts((double)obs[2 * r], (double)obs[2 * r + 1], A.J, A.h, A.n_bonds, A.n_sites);
+  A.energy[r] = e;
+  if (!A.best_energy) return;
+  const bool better = e < A.best_energy[r];
+  if (better) A.best_energy[r] = e;
+  obs[2 * r] = better ? 1ull : 0ull;
+}
+
+// best_state[r] = state[r] for the replicas flagged by anneal_select_kernel; blockIdx.y walks the replicas, so the
+// blocks of replicas that did not improve leave at once.  16-byte accesses, four in flight per thread.
+__global__ void __launch_bounds__(256) anneal_copy_kernel(const uint4* __restrict__ state, uint4* best_state,
+                                                          const unsigned long long* __restrict__ flags, int n,
+                                                          long long rep_vecs) {
+  for (int r = blockIdx.y; r < n; r += gridDim.y) {
+    if (!flags[2 * r]) continue;
+    const uint4* src = state + (size_t)r * rep_vecs;
+    uint4* dst = best_state + (size_t)r * rep_vecs;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    for (; t + 3 * stride < rep_vecs; t += 4 * stride) {
+      const uint4 a = src[t], b = src[t + stride], c = src[t + 2 * stride], d = src[t + 3 * stride];
+      dst[t] = a;
+      dst[t + stride] = b;
+      dst[t + 2 * stride] = c;
+      dst[t + 3 * stride] = d;
+    }
+    for (; t < rep_vecs; t += stride) dst[t] = src[t];
+  }
+}
+
+// Small lattices: the whole anneal in one launch, one thread block per replica (as sweeps_resident_kernel).  Step k
+// sweeps with table luts[k] and sweep index P.sweep + k; before the first step and after every step the block counts
+// its replica as count_word does, and takes E and the best state as anneal_select_kernel / anneal_copy_kernel do.
+template <bool BONDED>
+__global__ void __launch_bounds__(kResidentThreads) anneal_resident_kernel(SweepParams P, const uint32_t* __restrict__ luts,
+                                                                           int n_steps, BondParams B, AnnealOut A) {
+  const Geom& g = P.g;
+  const int rep = blockIdx.x;
+  const int per_rep = g.rows * g.wpr;
+  __shared__ unsigned long long part[2][kResidentThreads / 32];
+  __shared__ int better;
+  for (int k = -1; k < n_steps; ++k) {
+    if (k >= 0) {
+      SweepParams Q = P;
+      Q.lut = luts + 32 * (size_t)k;
+      for (int colour = 0; colour < 2; ++colour) {
+        for (int rem = threadIdx.x; rem < per_rep; rem += kResidentThreads) {
+          const int i = rem / g.wpr;
+          generic_update_one<BONDED>(Q, B, colour, P.sweep + (uint32_t)k, rep, i, rem - i * g.wpr);
+        }
+        __syncthreads();
+      }
+    }
+    unsigned long long ups = 0, anti = 0;
+    for (int t = threadIdx.x; t < 2 * per_rep; t += kResidentThreads) {
+      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
+      count_word<BONDED>(P.state, g, (size_t)per_rep, nullptr, B, rep, colour, i, rem - i * g.wpr, ups, anti);
+    }
+    ups = tsu_warp_sum(ups);
+    anti = tsu_warp_sum(anti);
+    if ((threadIdx.x & 31) == 0) {
+      part[0][threadIdx.x >> 5] = ups;
+      part[1][threadIdx.x >> 5] = anti;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      ups = 0;
+      anti = 0;
+      for (int j = 0; j < kResidentThreads / 32; ++j) {
+        ups += part[0][j];
+        anti += part[1][j];
+      }
+      const double e = energy_of_counts((double)ups, (double)anti, A.J, A.h, A.n_bonds, A.n_sites);
+      A.energy[rep] = e;
+      better = A.best_energy && e < A.best_energy[rep];
+      if (better) A.best_energy[rep] = e;
+    }
+    __syncthreads();
+    if (better) {
+      const uint4* src = reinterpret_cast<const uint4*>(P.state + (size_t)rep * 2 * per_rep);
+      uint4* dst = reinterpret_cast<uint4*>(A.best_state + (size_t)rep * 2 * per_rep);
+      for (int t = threadIdx.x; t < per_rep / 2; t += kResidentThreads) dst[t] = src[t];  // 2 per_rep words
+    }
+    __syncthreads();  // the next half-sweep overwrites what the counts and the copy read
+  }
 }
 
 // ---- Edwards-Anderson bonds ---------------------------------------------------------------------------------
@@ -1063,6 +1179,79 @@ int launch_resident_sweeps(const Lattice& L, uint32_t sweep0, int n_sweeps, cuda
   TSU_RETURN_LAUNCH_STATUS();
 }
 
+// full-word lattices count at HBM speed (observables_fast_kernel); the others word by word
+bool obs_fast(int cols) { return cols % 256 == 0 && !tuning().obs_generic; }
+
+// the counts of tsu_ising2d_observables into out[replica][2] (zeroed first)
+int launch_observables(const uint32_t* state, const Geom& g, const BondParams& B, const uint32_t* next_rows,
+                       unsigned long long* out, cudaStream_t st) {
+  const int n_replicas = g.n_replicas, rows = g.rows;
+  cudaError_t e = cudaMemsetAsync(out, 0, sizeof(unsigned long long) * 2 * (size_t)n_replicas, st);
+  if (e != cudaSuccess) return (int)e;
+  if (obs_fast(g.cols)) {
+    const int nvec = g.wpr / 4;
+    int strip = 64;  // long strips re-read one row in `strip`; short ones fill the GPU for small batches
+    while (strip > 1 && (long long)n_replicas * nvec * ((rows + strip - 1) / strip) < 148LL * 2048) strip >>= 1;
+    const int n_strips = (rows + strip - 1) / strip;
+    const long long per_rep_pad = ((long long)n_strips * nvec + 31) / 32 * 32;
+    const unsigned grid = blocks_for((long long)n_replicas * per_rep_pad, 128);
+    if (B.words)
+      observables_fast_kernel<true><<<grid, 128, 0, st>>>(state, g, next_rows, strip, n_strips, out, B);
+    else
+      observables_fast_kernel<false><<<grid, 128, 0, st>>>(state, g, next_rows, strip, n_strips, out, kNoBonds);
+    TSU_RETURN_LAUNCH_STATUS();
+  }
+  TSU_CHECK_ARG(n_replicas <= 65535);  // gridDim.y of the word-by-word kernel
+  const long long n_words = 2LL * rows * g.wpr;
+  long long bx = (n_words + 255) / 256;
+  const long long cap = (148LL * 8 + n_replicas - 1) / n_replicas;  // about 8 CTAs per SM in total
+  if (bx > cap) bx = cap < 1 ? 1 : cap;
+  dim3 grid((unsigned)bx, (unsigned)n_replicas);
+  if (B.words)
+    observables_kernel<true><<<grid, 256, 0, st>>>(state, g, next_rows, out, B);
+  else
+    observables_kernel<false><<<grid, 256, 0, st>>>(state, g, next_rows, out, kNoBonds);
+  TSU_RETURN_LAUNCH_STATUS();
+}
+
+// The anneal of tsu_ising2d_anneal for lattices too large for anneal_resident_kernel, on one stream: the initial state
+// is evaluated, then every step is one sweep (L.lut + 32 k is its table), the counts, anneal_select_kernel and, when
+// the best states are kept, anneal_copy_kernel.  pieces > 1: L is one of that many replica chunks running concurrently.
+int launch_anneal(const Lattice& L, const AnnealOut& A, int n_steps, uint32_t sweep0, unsigned long long* obs, int pieces,
+                  cudaStream_t st) {
+  const Geom& g = L.g;
+  const int n = g.n_replicas;
+  const long long rep_vecs = 2LL * g.rows * g.wpr / 4;  // wpr is a multiple of 4
+  long long bx = (rep_vecs + 255) / 256;
+  const long long cap = (148LL * 8 + n - 1) / n;  // about 8 CTAs per SM when every replica improves
+  if (bx > cap) bx = cap < 1 ? 1 : cap;
+  const dim3 copy_grid((unsigned)bx, (unsigned)(n < 65535 ? n : 65535));
+  for (int k = -1; k < n_steps; ++k) {
+    if (k >= 0) {
+      Lattice Lk = L;
+      Lk.lut = L.lut + 32 * (size_t)k;
+      const uint32_t sweep = sweep0 + (uint32_t)k;
+      int rc;
+      if (pieces > 1) {  // a replica chunk: its half-sweeps back to back, as launch_sweeps runs them
+        rc = launch_half_sweep(Lk, 0, sweep, nullptr, nullptr, 0, g.rows, pieces, st);
+        if (rc == TSU_OK) rc = launch_half_sweep(Lk, 1, sweep, nullptr, nullptr, 0, g.rows, pieces, st);
+      } else {  // row ranges on streams of their own are joined back into st before the counts
+        rc = launch_sweeps(Lk, sweep, 1, st);
+      }
+      if (rc != TSU_OK) return rc;
+    }
+    const int rc = launch_observables(L.state, g, L.B, nullptr, obs, st);
+    if (rc != TSU_OK) return rc;
+    anneal_select_kernel<<<blocks_for(n, 128), 128, 0, st>>>(obs, n, A);
+    if (A.best_energy)
+      anneal_copy_kernel<<<copy_grid, 256, 0, st>>>(reinterpret_cast<const uint4*>(L.state),
+                                                    reinterpret_cast<uint4*>(A.best_state), obs, n, rep_vecs);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return (int)e;
+  }
+  return TSU_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1227,33 +1416,46 @@ int tsu_ising2d_observables(const uint32_t* d_state, int n_replicas, int rows, i
   const Geom g = make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, row0);
   const BondParams B = {d_bonds, d_bond_index};
   TSU_CHECK_ARG(d_state && d_out && args_ok(g, B, d_next_rows != nullptr, 0, 0, rows));
+  return launch_observables(d_state, g, B, d_next_rows, d_out, tsu_stream(stream));
+}
+
+int tsu_ising2d_anneal(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                       const uint32_t* d_luts, int n_steps, const uint32_t* d_bonds, const int32_t* d_bond_index,
+                       uint64_t seed, uint32_t sweep0, uint32_t replica0, double J, double h, long long n_bonds,
+                       long long n_sites, unsigned long long* d_obs, double* d_energy, double* d_best_energy,
+                       uint32_t* d_best_state, uintptr_t stream) {
+  const Lattice L = {d_state, make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, 0), d_luts, nullptr,
+                     {d_bonds, d_bond_index}, seed, replica0, JitKernel{nullptr, 0, 0}};
+  TSU_CHECK_ARG(d_state && args_ok(L.g, L.B, false, 0, 0, rows) && n_steps >= 0 && (d_luts || n_steps == 0));
+  TSU_CHECK_ARG(d_obs && d_energy && (d_best_energy == nullptr) == (d_best_state == nullptr));
+  const AnnealOut A = {J, h, n_bonds, n_sites, d_energy, d_best_energy, d_best_state};
   cudaStream_t st = tsu_stream(stream);
-  cudaError_t e = cudaMemsetAsync(d_out, 0, sizeof(unsigned long long) * 2 * (size_t)n_replicas, st);
-  if (e != cudaSuccess) return (int)e;
-  if (cols % 256 == 0 && !tuning().obs_generic) {
-    const int nvec = g.wpr / 4;
-    int strip = 64;  // long strips re-read one row in `strip`; short ones fill the GPU for small batches
-    while (strip > 1 && (long long)n_replicas * nvec * ((rows + strip - 1) / strip) < 148LL * 2048) strip >>= 1;
-    const int n_strips = (rows + strip - 1) / strip;
-    const long long per_rep_pad = ((long long)n_strips * nvec + 31) / 32 * 32;
-    const unsigned grid = blocks_for((long long)n_replicas * per_rep_pad, 128);
+  if (resident_eligible(n_replicas, rows, cols)) {
+    const SweepParams P = sweep_params(L, 0, sweep0, nullptr, nullptr);
     if (d_bonds)
-      observables_fast_kernel<true><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, B);
+      anneal_resident_kernel<true><<<n_replicas, kResidentThreads, 0, st>>>(P, d_luts, n_steps, L.B, A);
     else
-      observables_fast_kernel<false><<<grid, 128, 0, st>>>(d_state, g, d_next_rows, strip, n_strips, d_out, kNoBonds);
+      anneal_resident_kernel<false><<<n_replicas, kResidentThreads, 0, st>>>(P, d_luts, n_steps, kNoBonds, A);
     TSU_RETURN_LAUNCH_STATUS();
   }
-  TSU_CHECK_ARG(n_replicas <= 65535);  // gridDim.y of the word-by-word kernel
-  const long long n_words = 2LL * rows * g.wpr;
-  long long bx = (n_words + 255) / 256;
-  const long long cap = (148LL * 8 + n_replicas - 1) / n_replicas;  // about 8 CTAs per SM in total
-  if (bx > cap) bx = cap < 1 ? 1 : cap;
-  dim3 grid((unsigned)bx, (unsigned)n_replicas);
-  if (d_bonds)
-    observables_kernel<true><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, B);
-  else
-    observables_kernel<false><<<grid, 256, 0, st>>>(d_state, g, d_next_rows, d_out, kNoBonds);
-  TSU_RETURN_LAUNCH_STATUS();
+  TSU_CHECK_ARG(obs_fast(cols) || n_replicas <= 65535);  // as tsu_ising2d_observables
+  const int KR = split_replicas(n_replicas, rows, cols);
+  if (KR == 1) return launch_anneal(L, A, n_steps, sweep0, d_obs, 1, st);
+  // replica chunks do not depend on each other: each runs its whole anneal on its own stream
+  StreamFork F(st, KR);
+  if (F.status != TSU_OK) return F.status;
+  int rc = TSU_OK;
+  for (int k = 0; k < KR && rc == TSU_OK; ++k) {
+    const int r0 = (int)((long long)n_replicas * k / KR), r1 = (int)((long long)n_replicas * (k + 1) / KR);
+    AnnealOut Ak = A;
+    Ak.energy += r0;
+    if (Ak.best_energy) {
+      Ak.best_energy += r0;
+      Ak.best_state += (size_t)r0 * 2 * rows * L.g.wpr;
+    }
+    rc = launch_anneal(L.replicas(r0, r1), Ak, n_steps, sweep0, d_obs + 2 * (size_t)r0, KR, F.s[k]);
+  }
+  return F.join(rc);
 }
 
 int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_replicas, double J, double h,

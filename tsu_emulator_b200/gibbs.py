@@ -133,6 +133,15 @@ class _TcProblem:
         return out
 
 
+def annealing_temperatures(T_initial: float, T_final: float, n_steps: int, cooling_schedule: str = "exponential"):
+    """float64 [n_steps]: the temperature of every annealing step (tsu/gibbs.py:340-393): T_initial at step 0 towards
+    T_final, which is not reached; "exponential" or, for anything else, "linear" cooling"""
+    steps = np.arange(n_steps, dtype=np.float64)
+    if cooling_schedule == "exponential":
+        return T_initial * (T_final / T_initial) ** (steps / n_steps)
+    return T_initial + (T_final - T_initial) * steps / n_steps  # linear
+
+
 class GibbsSampler:
     """tsu/gibbs.py:39-393 on the GPU.
 
@@ -552,11 +561,7 @@ class GibbsSampler:
             prob = self._sparse(coupling, bias)
         else:
             prob = _DenseProblem(coupling, bias, self.precision, self._dev())
-        steps = np.arange(n_steps, dtype=np.float64)
-        if cooling_schedule == "exponential":
-            Ts = T_initial * (T_final / T_initial) ** (steps / n_steps)
-        else:  # linear
-            Ts = T_initial + (T_final - T_initial) * steps / n_steps
+        Ts = annealing_temperatures(T_initial, T_final, n_steps, cooling_schedule)
         st = self._initial_states(prob, int(n_chains), _initial_state)
         if tc and n_steps > 0:
             st = prob.pad_state(st)

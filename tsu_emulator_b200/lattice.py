@@ -103,6 +103,32 @@ def check_bonds(bonds, bond_index, rows: int, cols: int, n_replicas: int, bias_m
     return b.astype(np.int8), idx
 
 
+class AnnealResult:
+    """What Ising2DEngine.anneal returns; pass it back as `best=` to continue an anneal.
+
+    energy:      float64 device tensor [n_replicas], E of every replica's final state
+    best_energy: float64 device tensor [n_replicas], lowest E seen by each replica (None with track_best=False)
+    best_state:  int32 device tensor [n_replicas, 2, rows, wpr], the packed state that had best_energy (same layout as
+                 Ising2DEngine.state; None with track_best=False)
+    """
+
+    def __init__(self, energy, best_energy, best_state, rows: int, cols: int):
+        self.energy, self.best_energy, self.best_state = energy, best_energy, best_state
+        self.rows, self.cols = int(rows), int(cols)
+
+    def best_spins(self, pm1: bool = True):
+        """int8 device tensor [n_replicas, rows, cols] of the best states ({-1, +1}, or {0, 1} with pm1=False)"""
+        if self.best_state is None:
+            raise ValueError("this anneal kept no best states (track_best=False)")
+        torch = _lib.require_cuda()
+        dev = self.best_state.device
+        with torch.cuda.device(dev):
+            out = torch.empty((self.best_state.shape[0], self.rows, self.cols), dtype=torch.int8, device=dev)
+            _lib.call("tsu_ising2d_unpack", ptr(self.best_state), ptr(out), int(self.best_state.shape[0]), self.rows,
+                      self.cols, 1 if pm1 else 0, _lib.current_stream())
+        return out
+
+
 class Ising2DEngine:
     """n_replicas independent rows x cols lattices (or one row-slab of each) resident in HBM.
 
@@ -370,6 +396,96 @@ class Ising2DEngine:
                 self.half_sweep(colour, uniforms=dev[t])
             self.sweep_index += 1
         return self
+
+    # ------------------------------------------------------------------ annealing
+    def anneal(self, temperatures, *, track_best: bool = True, best: Optional[AnnealResult] = None) -> AnnealResult:
+        """Simulated annealing (tsu/gibbs.py:340-393) of every replica in one call, with no host sync.
+
+        Step k sweeps once at temperatures[k].  The initial state and the state after every step are evaluated, and a
+        replica whose energy is strictly below its best so far takes that energy and a copy of its state.  The result
+        equals, bit for bit, the loop
+
+            E = energy_tensor()                      # initial state: the first best
+            for T in temperatures:
+                set_temperature(T); sweep(1); E = energy_tensor()
+                # replicas with E < best_energy take E and copy their state
+
+        Afterwards sweep_index has advanced by len(temperatures) and the engine is at the scalar temperature
+        temperatures[-1].  Lattices that sweep() runs in one launch anneal in one launch.
+
+        track_best=True keeps a packed copy of every replica's state on the device, which doubles the state memory
+        (34 GB more for 4096 replicas of 8192 x 8192).  best: the AnnealResult of an earlier anneal of this engine; its
+        buffers are compared against and updated in place (and decide whether best states are kept), so an anneal
+        split into calls equals one call.
+        """
+        Ts = np.asarray(temperatures, dtype=np.float64)
+        if Ts.ndim != 1 or Ts.size == 0:
+            raise ValueError("temperatures must be a non-empty 1-D schedule")
+        return self._anneal(Ts, track_best, best)
+
+    def simulated_annealing(self, T_initial: float = 10.0, T_final: float = 0.1, n_steps: int = 1000,
+                            cooling_schedule: str = "exponential", *, track_best: bool = True,
+                            best: Optional[AnnealResult] = None) -> AnnealResult:
+        """anneal() along the schedule of GibbsSampler.simulated_annealing: the same float64 temperatures, from
+        T_initial towards T_final, "exponential" or "linear".  n_steps = 0 evaluates the initial state only."""
+        from .gibbs import annealing_temperatures
+
+        if int(n_steps) < 0:
+            raise ValueError("n_steps must be >= 0")
+        return self._anneal(annealing_temperatures(T_initial, T_final, int(n_steps), cooling_schedule), track_best, best)
+
+    def _anneal(self, Ts: np.ndarray, track_best: bool, best: Optional[AnnealResult]) -> AnnealResult:
+        if self.is_slab:
+            raise ValueError("annealing needs whole lattices; row-slab engines cannot anneal")
+        if not np.all(np.isfinite(Ts)) or np.any(Ts <= 0):
+            raise ValueError("temperatures must be positive and finite")
+        torch = self._torch
+        n = self.n_replicas
+        if best is not None:
+            be, bs = best.best_energy, best.best_state
+            if (be is None) != (bs is None):
+                raise ValueError("best needs both best_energy and best_state, or neither")
+            if be is not None and not (be.dtype == torch.float64 and tuple(be.shape) == (n,) and be.is_contiguous()
+                                       and be.device == self.device and bs.dtype == torch.int32
+                                       and bs.shape == self.state.shape and bs.is_contiguous() and bs.device == self.device):
+                raise ValueError(f"best buffers must be float64 [{n}] and int32 {tuple(self.state.shape)}, contiguous, "
+                                 f"on {self.device}")
+        with torch.cuda.device(self.device):
+            energy = torch.empty(n, dtype=torch.float64, device=self.device)
+            if best is not None:
+                best_energy, best_state = best.best_energy, best.best_state
+            elif track_best:
+                best_energy = torch.full((n,), float("inf"), dtype=torch.float64, device=self.device)
+                best_state = torch.empty_like(self.state)
+            else:
+                best_energy = best_state = None
+            luts = self._schedule_tables(Ts) if Ts.size else None
+            _lib.call(
+                "tsu_ising2d_anneal", ptr(self.state), n, self.rows, self.cols, int(self.wrap_rows), int(self.wrap_cols),
+                ptr(luts), int(Ts.size), ptr(self.bonds), ptr(self.bond_index), self.seed, self.sweep_index & 0xFFFFFFFF,
+                self.replica0, self.coupling, self.field, self.n_bonds, self.n_sites, ptr(self._obs), ptr(energy),
+                ptr(best_energy), ptr(best_state), _lib.current_stream(),
+            )
+        self.sweep_index += int(Ts.size)
+        if Ts.size:
+            self.set_temperature(float(Ts[-1]))  # (host work that overlaps the anneal on the device)
+        if best is not None:
+            best.energy = energy
+            return best
+        return AnnealResult(energy, best_energy, best_state, self.rows, self.cols)
+
+    def _schedule_tables(self, Ts: np.ndarray):
+        """int32 device tensor [len(Ts), 32]: the threshold table of every step; the last schedule's tables are kept,
+        so that repeated anneals along one schedule build and upload nothing"""
+        key = (self.coupling, self.field, self.bias_mode, Ts.tobytes())
+        cached = self.__dict__.get("_anneal_tables")
+        if cached is not None and cached[0] == key:
+            return cached[1]
+        uniq, inv = np.unique(Ts, return_inverse=True)
+        luts = np.stack([build_lut(self.coupling, self.field, float(t), self.bias_mode) for t in uniq])[inv.reshape(-1)]
+        tables = self._torch.from_numpy(np.ascontiguousarray(luts).view(np.int32)).to(self.device)
+        self._anneal_tables = (key, tables)
+        return tables
 
     # ------------------------------------------------------------------ observables
     def observables_tensor(self, next_rows=None):
