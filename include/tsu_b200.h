@@ -224,6 +224,45 @@ int tsu_ising2d_anneal(uint32_t* d_state, int n_replicas, int rows, int cols, in
                        unsigned long long* d_obs, double* d_energy, double* d_best_energy,
                        uint32_t* d_best_state, uintptr_t stream);
 
+/* Population annealing of whole lattices (Hukushima-Iba, Machta): the n_replicas replicas form n_populations equal
+ * contiguous populations of R_p = n_replicas / n_populations replicas, each resampled on its own; no host sync inside.
+ * The caller guarantees one bond realisation per population (d_bond_index constant within each).  Step k of n_steps:
+ *   1. count: exact (up, anti) of every replica as tsu_ising2d_observables, E_i with the rounding of
+ *      tsu_ising2d_energy_from_observables; d_count_sums[k][p] = (sum up, sum anti), d_energy_ref[k][p] = min_i E_i.
+ *   2. weigh: x_i = d_dbeta[k] (E_i - E_ref) (d_dbeta[k] = 1/T_k - 1/T_{k-1} >= 0, float64),
+ *      q_i = floor(exp(-x_i) 2^s) with s = 62 - ceil(log2 R_p) and exp spelled out in float64 adds and multiplies
+ *      rounded to nearest (range reduction, degree-13 polynomial, ldexp: within 1 ulp of exp on [0, 45], exp(0) = 1);
+ *      q_i = 0 when rint(x_i / ln 2) > s + 1.  d_weight_sum[k][p] = W = sum q_i, 2^s <= W <= 2^62.  Dropping
+ *      weights below 2^-s biases ln(W / (R_p 2^s)) by at most R_p 2^-s / W <= 2^-31.
+ *   3. resample, systematically, R_p fixed: u = one 64-bit draw of the lattice stream (kind 3, replica
+ *      replica0 + p R_p, sweep sweep0 + k sweeps_per_step), U = floor(u W / 2^64); with inclusive prefix sums C_i the
+ *      parent of child j is the smallest i with R_p C_i > j W + U (integer arithmetic: any scan order gives the same).
+ *   4. gather: state'[j] = state[parent(j)], family'[j] = d_family[parent(j)] (ping-pong with d_scratch /
+ *      d_family_scratch; the result always ends in d_state / d_family).
+ *   5. sweep: sweeps_per_step sweeps with table d_luts[k] and sweep indices sweep0 + k sweeps_per_step ...; the launches
+ *      of tsu_ising2d_sweeps with the prebuilt kernels (each step's sweeps joined before the next counts).
+ * After the last step the final states are counted into d_count_sums[n_steps] and d_energy[r] = E of replica r.
+ * With d_dbeta all 0 every parent is its child, so the run equals tsu_ising2d_sweeps(n_steps sweeps_per_step).
+ * A block of whole populations run on its own (its replica0, its family entries) equals that block of the whole run.
+ * Buffers: d_scratch [n_replicas][2][rows][wpr], d_family / d_family_scratch int32 [n_replicas],
+ *   d_weight_sum uint64 [n_steps][n_populations], d_energy_ref [n_steps][n_populations],
+ *   d_count_sums uint64 [n_steps + 1][n_populations][2], d_obs [n_replicas][2] scratch, d_energy [n_replicas],
+ *   d_work of at least tsu_ising2d_population_work_bytes(n_replicas, n_populations) bytes, 8-byte aligned (prefix
+ *   sums; the library allocates nothing).  Bonds as in tsu_ising2d_sweeps; whole lattices only.
+ * TSU_ERR_INVALID_ARG before any CUDA call for: n_replicas % n_populations != 0, n_populations outside [1, 65535],
+ *   sweeps_per_step < 1, n_steps < 0, a NULL pointer, d_scratch == d_state, d_family_scratch == d_family, a work
+ *   buffer below the size, and the lattice rules of tsu_ising2d_sweeps.  More than 65535 replicas of a lattice
+ *   without full words (cols % 256 != 0) are counted by one warp per replica. */
+int64_t tsu_ising2d_population_work_bytes(int n_replicas, int n_populations);
+int tsu_ising2d_population_anneal(uint32_t* d_state, uint32_t* d_scratch, int n_replicas, int rows, int cols,
+                                  int wrap_rows, int wrap_cols, const uint32_t* d_luts, const double* d_dbeta,
+                                  int n_steps, int sweeps_per_step, int n_populations, const uint32_t* d_bonds,
+                                  const int32_t* d_bond_index, uint64_t seed, uint32_t sweep0, uint32_t replica0,
+                                  double J, double h, long long n_bonds, long long n_sites, int32_t* d_family,
+                                  int32_t* d_family_scratch, unsigned long long* d_weight_sum, double* d_energy_ref,
+                                  unsigned long long* d_count_sums, unsigned long long* d_obs, double* d_energy,
+                                  void* d_work, size_t work_bytes, uintptr_t stream);
+
 /* ------------------------------------------------------------------ dense-J Gibbs ----- */
 /*
  * Replaces GibbsSampler.gibbs_sweep / sample_boltzmann / compute_energy and the sweep part of

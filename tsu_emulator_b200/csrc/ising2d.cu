@@ -25,6 +25,7 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "common.cuh"
@@ -623,8 +624,21 @@ __global__ void anneal_select_kernel(unsigned long long* obs, int n, AnnealOut A
   obs[2 * r] = better ? 1ull : 0ull;
 }
 
+// dst[t] = src[t] for t = t0, t0 + stride, ... below n_vecs: 16-byte accesses, four in flight per thread
+__device__ __forceinline__ void copy_vecs(const uint4* src, uint4* dst, long long n_vecs, long long t0, long long stride) {
+  long long t = t0;
+  for (; t + 3 * stride < n_vecs; t += 4 * stride) {
+    const uint4 a = src[t], b = src[t + stride], c = src[t + 2 * stride], d = src[t + 3 * stride];
+    dst[t] = a;
+    dst[t + stride] = b;
+    dst[t + 2 * stride] = c;
+    dst[t + 3 * stride] = d;
+  }
+  for (; t < n_vecs; t += stride) dst[t] = src[t];
+}
+
 // best_state[r] = state[r] for the replicas flagged by anneal_select_kernel; blockIdx.y walks the replicas, so the
-// blocks of replicas that did not improve leave at once.  16-byte accesses, four in flight per thread.
+// blocks of replicas that did not improve leave at once.
 __global__ void __launch_bounds__(256) anneal_copy_kernel(const uint4* __restrict__ state, uint4* best_state,
                                                           const unsigned long long* __restrict__ flags, int n,
                                                           long long rep_vecs) {
@@ -633,15 +647,7 @@ __global__ void __launch_bounds__(256) anneal_copy_kernel(const uint4* __restric
     const uint4* src = state + (size_t)r * rep_vecs;
     uint4* dst = best_state + (size_t)r * rep_vecs;
     const long long stride = (long long)gridDim.x * blockDim.x;
-    long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    for (; t + 3 * stride < rep_vecs; t += 4 * stride) {
-      const uint4 a = src[t], b = src[t + stride], c = src[t + 2 * stride], d = src[t + 3 * stride];
-      dst[t] = a;
-      dst[t + stride] = b;
-      dst[t + 2 * stride] = c;
-      dst[t + 3 * stride] = d;
-    }
-    for (; t < rep_vecs; t += stride) dst[t] = src[t];
+    copy_vecs(src, dst, rep_vecs, (long long)blockIdx.x * blockDim.x + threadIdx.x, stride);
   }
 }
 
@@ -699,6 +705,242 @@ __global__ void __launch_bounds__(kResidentThreads) anneal_resident_kernel(Sweep
       for (int t = threadIdx.x; t < per_rep / 2; t += kResidentThreads) dst[t] = src[t];  // 2 per_rep words
     }
     __syncthreads();  // the next half-sweep overwrites what the counts and the copy read
+  }
+}
+
+// ---- population annealing (tsu_ising2d_population_anneal) -------------------------------------------------------
+// The population is n_pop contiguous blocks of rp replicas, each resampled on its own.  Everything after the weights'
+// exp is integer arithmetic, so any decomposition of the sums gives the same bits.  The caller's work buffer holds
+// (uint64): prefix[n_replicas] (inclusive prefix sums of the quantised weights within each tile of kPaTile replicas),
+// tile_off[n_pop][nt] (tile totals, then their exclusive prefix sums within the population), min_key[n_pop] (order key
+// of E_ref) and draw[n_pop] (the step's U).
+constexpr int kPaThreads = 256, kPaPerThread = 4, kPaTile = kPaThreads * kPaPerThread, kPaScanThreads = 1024;
+
+struct PopParams {
+  int rp, n_pop, nt, s;  // replicas per population, populations, tiles per population, weight shift 62 - ceil(log2 rp)
+  unsigned long long* prefix;
+  unsigned long long* tile_off;
+  unsigned long long* min_key;
+  unsigned long long* draw;
+};
+
+// float64 -> uint64 with the same order, so that the lowest E is an integer atomicMin
+__device__ __forceinline__ unsigned long long order_key(double e) {
+  const unsigned long long b = (unsigned long long)__double_as_longlong(e);
+  return (b >> 63) ? ~b : b | 0x8000000000000000ull;
+}
+
+__device__ __forceinline__ double key_value(unsigned long long k) {
+  return __longlong_as_double((long long)((k >> 63) ? k & 0x7fffffffffffffffull : ~k));
+}
+
+__device__ __forceinline__ unsigned long long warp_min(unsigned long long v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+
+__device__ __forceinline__ unsigned long long warp_inclusive_scan(unsigned long long v) {
+  const int lane = threadIdx.x & 31;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const unsigned long long y = __shfl_up_sync(0xffffffffu, v, d);
+    if (lane >= d) v += y;
+  }
+  return v;
+}
+
+// More replicas than the word-by-word observables kernel's grid takes (gridDim.y <= 65535): one warp per replica counts
+// its words with count_word and writes out[rep] (no atomics, no zeroing).
+template <bool BONDED>
+__global__ void __launch_bounds__(256) pa_count_kernel(const uint32_t* __restrict__ state, Geom g,
+                                                      unsigned long long* out, BondParams B) {
+  const long long rep = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (rep >= g.n_replicas) return;
+  const long long plane = (long long)g.rows * g.wpr;
+  unsigned long long ups = 0, anti = 0;
+  for (long long t = threadIdx.x & 31; t < 2 * plane; t += 32) {
+    const int colour = (int)(t / plane);
+    const long long rem = t - colour * plane;
+    const int i = (int)(rem / g.wpr);
+    count_word<BONDED>(state, g, (size_t)plane, nullptr, B, (int)rep, colour, i, (int)(rem - (long long)i * g.wpr), ups,
+                       anti);
+  }
+  ups = tsu_warp_sum(ups);
+  anti = tsu_warp_sum(anti);
+  if ((threadIdx.x & 31) == 0) {
+    out[2 * rep] = ups;
+    out[2 * rep + 1] = anti;
+  }
+}
+
+// E of every replica from its counts (energy_of_counts) into A.energy; per population the sums of the counts
+// (sums[p][2]) and the order key of the lowest E (Q.min_key[p]).  Grid (x, n_pop): blockIdx.x strides over a population.
+__global__ void __launch_bounds__(kPaThreads) pa_reduce_kernel(const unsigned long long* __restrict__ obs, PopParams Q,
+                                                               AnnealOut A, unsigned long long* sums) {
+  const int p = blockIdx.y;
+  unsigned long long ups = 0, anti = 0, key = ~0ull;
+  for (int j = blockIdx.x * kPaThreads + threadIdx.x; j < Q.rp; j += gridDim.x * kPaThreads) {
+    const size_t r = (size_t)p * Q.rp + j;
+    const unsigned long long u = obs[2 * r], a = obs[2 * r + 1];
+    const double e = energy_of_counts((double)u, (double)a, A.J, A.h, A.n_bonds, A.n_sites);
+    A.energy[r] = e;
+    ups += u;
+    anti += a;
+    key = min(key, order_key(e));
+  }
+  __shared__ unsigned long long part[3][kPaThreads / 32];
+  ups = tsu_warp_sum(ups);
+  anti = tsu_warp_sum(anti);
+  key = warp_min(key);
+  if ((threadIdx.x & 31) == 0) {
+    part[0][threadIdx.x >> 5] = ups;
+    part[1][threadIdx.x >> 5] = anti;
+    part[2][threadIdx.x >> 5] = key;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < kPaThreads / 32; ++w) {
+      ups += part[0][w];
+      anti += part[1][w];
+      key = min(key, part[2][w]);
+    }
+    atomicAdd(sums + 2 * p, ups);
+    atomicAdd(sums + 2 * p + 1, anti);
+    atomicMin(Q.min_key + p, key);
+  }
+}
+
+// exp(-x) for x >= 0 with every rounding spelled out (oracle/population_oracle.py, exp_neg, repeats it): n = rint(x / ln 2),
+// r = x - n ln 2 with a two-part ln 2, exp(-r) by a degree-13 Horner polynomial in -r, times 2^(s - n).  Only float64
+// multiplies and adds rounded to nearest, never contracted: within 1 ulp of exp on [0, 45] and exactly 1 at x = 0.
+// q = floor(exp(-x) 2^s); 0 when n > s + 1.
+__device__ __forceinline__ unsigned long long quantised_weight(double x, int s) {
+  constexpr double kInvLn2 = 0x1.71547652b82fep+0, kLn2Hi = 0x1.62e42fee00000p-1, kLn2Lo = 0x1.a39ef35793c76p-33;
+  constexpr double c[14] = {0x1.0p+0, 0x1.0p+0, 0x1.0p-1, 0x1.5555555555555p-3, 0x1.5555555555555p-5,
+                            0x1.1111111111111p-7, 0x1.6c16c16c16c17p-10, 0x1.a01a01a01a01ap-13, 0x1.a01a01a01a01ap-16,
+                            0x1.71de3a556c734p-19, 0x1.27e4fb7789f5cp-22, 0x1.ae64567f544e4p-26, 0x1.1eed8eff8d898p-29,
+                            0x1.6124613a86d09p-33};  // 1/k!
+  const double n = rint(__dmul_rn(x, kInvLn2));
+  if (n > (double)(s + 1)) return 0ull;
+  const double t = -__dsub_rn(__dsub_rn(x, __dmul_rn(n, kLn2Hi)), __dmul_rn(n, kLn2Lo));
+  double p = c[13];
+#pragma unroll
+  for (int k = 12; k >= 0; --k) p = __dadd_rn(__dmul_rn(p, t), c[k]);
+  return __double2ull_rz(ldexp(p, s - (int)n));
+}
+
+// Quantised weights of one tile of kPaTile replicas of population blockIdx.y (x = dbeta (E - E_ref)), their inclusive
+// prefix sums within the tile into Q.prefix and the tile total into Q.tile_off.
+__global__ void __launch_bounds__(kPaThreads) pa_weights_kernel(const double* __restrict__ energy,
+                                                                const double* __restrict__ dbeta, PopParams Q) {
+  const int p = blockIdx.y, tile = blockIdx.x;
+  const double db = *dbeta, e_ref = key_value(Q.min_key[p]);
+  const size_t base = (size_t)p * Q.rp;
+  const int j0 = tile * kPaTile + threadIdx.x * kPaPerThread;
+  unsigned long long q[kPaPerThread], run = 0;
+#pragma unroll
+  for (int m = 0; m < kPaPerThread; ++m) {
+    const int j = j0 + m;
+    run += j < Q.rp ? quantised_weight(__dmul_rn(db, __dsub_rn(energy[base + j], e_ref)), Q.s) : 0ull;
+    q[m] = run;
+  }
+  __shared__ unsigned long long warp_tot[kPaThreads / 32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned long long incl = warp_inclusive_scan(run);
+  if (lane == 31) warp_tot[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    const unsigned long long v = warp_inclusive_scan(lane < kPaThreads / 32 ? warp_tot[lane] : 0ull);
+    if (lane < kPaThreads / 32) warp_tot[lane] = v;
+  }
+  __syncthreads();
+  const unsigned long long excl = incl - run + (warp > 0 ? warp_tot[warp - 1] : 0ull);
+#pragma unroll
+  for (int m = 0; m < kPaPerThread; ++m)
+    if (j0 + m < Q.rp) Q.prefix[base + j0 + m] = excl + q[m];
+  if (threadIdx.x == kPaThreads - 1) Q.tile_off[(size_t)p * Q.nt + tile] = excl + run;
+}
+
+// One block per population: the tile totals become exclusive prefix sums, W = their sum goes to weight_sum[p], E_ref to
+// energy_ref[p] (min_key is reset for the next step), and the population's Philox draw u (kind 3) gives
+// U = floor(u W / 2^64) in Q.draw[p].
+__global__ void __launch_bounds__(kPaScanThreads) pa_scan_kernel(PopParams Q, uint32_t k0, uint32_t k1, uint32_t sweep,
+                                                                 uint32_t replica0, unsigned long long* weight_sum,
+                                                                 double* energy_ref) {
+  const int p = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned long long* off = Q.tile_off + (size_t)p * Q.nt;
+  __shared__ unsigned long long warp_tot[kPaScanThreads / 32];
+  unsigned long long carry = 0;  // the same in every thread
+  for (int c0 = 0; c0 < Q.nt; c0 += kPaScanThreads) {
+    const int t = c0 + threadIdx.x;
+    const unsigned long long v = t < Q.nt ? off[t] : 0ull;
+    const unsigned long long incl = warp_inclusive_scan(v);
+    if (lane == 31) warp_tot[warp] = incl;
+    __syncthreads();
+    if (warp == 0) warp_tot[lane] = warp_inclusive_scan(warp_tot[lane]);
+    __syncthreads();
+    if (t < Q.nt) off[t] = carry + incl - v + (warp > 0 ? warp_tot[warp - 1] : 0ull);
+    carry += warp_tot[kPaScanThreads / 32 - 1];
+    __syncthreads();  // warp_tot is overwritten by the next chunk
+  }
+  if (threadIdx.x == 0) {
+    const unsigned long long W = carry;
+    weight_sum[p] = W;
+    energy_ref[p] = key_value(Q.min_key[p]);
+    Q.min_key[p] = ~0ull;
+    const tsu_u32x4 o = tsu_lattice_philox(0u, 0u, TSU_KIND_RESAMPLE, 0u, sweep, replica0 + (uint32_t)p * (uint32_t)Q.rp,
+                                           k0, k1);
+    Q.draw[p] = __umul64hi((unsigned long long)o.x | ((unsigned long long)o.y << 32), W);
+  }
+}
+
+// Parent of child j of population p: the smallest i with rp C_i > j W + U (128-bit products), C_i the inclusive prefix
+// sum prefix[i] + tile_off[i / kPaTile].  C is non-decreasing and rp C_{rp-1} = rp W > j W + U, so a bisection finds it.
+__device__ __forceinline__ int pa_parent(const PopParams& Q, int p, int j, unsigned long long W) {
+  const unsigned long long U = Q.draw[p];
+  unsigned long long t_lo = (unsigned long long)j * W, t_hi = __umul64hi((unsigned long long)j, W);
+  t_lo += U;
+  t_hi += t_lo < U ? 1ull : 0ull;
+  const unsigned long long* pre = Q.prefix + (size_t)p * Q.rp;
+  const unsigned long long* off = Q.tile_off + (size_t)p * Q.nt;
+  const unsigned long long rp = (unsigned long long)Q.rp;
+  int lo = 0, hi = Q.rp - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    const unsigned long long c = pre[mid] + off[mid / kPaTile];
+    const unsigned long long c_lo = rp * c, c_hi = __umul64hi(rp, c);
+    if (c_hi > t_hi || (c_hi == t_hi && c_lo > t_lo))
+      hi = mid;
+    else
+      lo = mid + 1;
+  }
+  return lo;
+}
+
+// state'[c] = state[parent(c)] and family'[c] = family[parent(c)].  group < 256: `group` threads (a power of two) per
+// child, 256 / group children per block along x; group == 256: blockIdx.y walks the children and blockIdx.x tiles one.
+__global__ void __launch_bounds__(256) pa_gather_kernel(const uint4* __restrict__ src, uint4* dst,
+                                                        const int32_t* __restrict__ fam_src, int32_t* fam_dst,
+                                                        PopParams Q, const unsigned long long* __restrict__ weight_sum,
+                                                        long long rep_vecs, int group) {
+  const int n = Q.rp * Q.n_pop;
+  if (group < 256) {
+    const long long c = (long long)blockIdx.x * (256 / group) + threadIdx.x / group;
+    if (c >= n) return;
+    const int p = (int)(c / Q.rp);
+    const size_t parent = (size_t)p * Q.rp + pa_parent(Q, p, (int)(c - (long long)p * Q.rp), weight_sum[p]);
+    const int t0 = threadIdx.x & (group - 1);
+    copy_vecs(src + parent * rep_vecs, dst + c * rep_vecs, rep_vecs, t0, group);
+    if (t0 == 0) fam_dst[c] = fam_src[parent];
+    return;
+  }
+  for (int c = blockIdx.y; c < n; c += gridDim.y) {
+    const int p = c / Q.rp;
+    const size_t parent = (size_t)p * Q.rp + pa_parent(Q, p, c - p * Q.rp, weight_sum[p]);
+    copy_vecs(src + parent * rep_vecs, dst + (size_t)c * rep_vecs, rep_vecs,
+              (long long)blockIdx.x * blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x);
+    if (blockIdx.x == 0 && threadIdx.x == 0) fam_dst[c] = fam_src[parent];
   }
 }
 
@@ -1252,6 +1494,31 @@ int launch_anneal(const Lattice& L, const AnnealOut& A, int n_steps, uint32_t sw
   return TSU_OK;
 }
 
+// The counts of a population-annealing step into obs[replica][2]: the observables kernels, or one warp per replica where
+// the word-by-word kernel's grid would be too tall (more than 65535 replicas of lattices without full words).
+int launch_population_counts(const Lattice& L, unsigned long long* obs, cudaStream_t st) {
+  const Geom& g = L.g;
+  if (obs_fast(g.cols) || g.n_replicas <= 65535) return launch_observables(L.state, g, L.B, nullptr, obs, st);
+  const unsigned grid = blocks_for(32LL * g.n_replicas, 256);
+  if (L.B.words)
+    pa_count_kernel<true><<<grid, 256, 0, st>>>(L.state, g, obs, L.B);
+  else
+    pa_count_kernel<false><<<grid, 256, 0, st>>>(L.state, g, obs, kNoBonds);
+  TSU_RETURN_LAUNCH_STATUS();
+}
+
+// E of every replica, and per population the count sums and E_ref, of the state L holds now
+int launch_population_reduce(const Lattice& L, const PopParams& Q, const AnnealOut& A, unsigned long long* obs,
+                             unsigned long long* sums, cudaStream_t st) {
+  const int rc = launch_population_counts(L, obs, st);
+  if (rc != TSU_OK) return rc;
+  long long bx = (Q.rp + kPaThreads - 1) / kPaThreads;
+  const long long cap = (148LL * 8 + Q.n_pop - 1) / Q.n_pop;  // about 8 CTAs per SM in total
+  if (bx > cap) bx = cap;
+  pa_reduce_kernel<<<dim3((unsigned)bx, (unsigned)Q.n_pop), kPaThreads, 0, st>>>(obs, Q, A, sums);
+  TSU_RETURN_LAUNCH_STATUS();
+}
+
 }  // namespace
 
 extern "C" {
@@ -1456,6 +1723,94 @@ int tsu_ising2d_anneal(uint32_t* d_state, int n_replicas, int rows, int cols, in
     rc = launch_anneal(L.replicas(r0, r1), Ak, n_steps, sweep0, d_obs + 2 * (size_t)r0, KR, F.s[k]);
   }
   return F.join(rc);
+}
+
+int64_t tsu_ising2d_population_work_bytes(int n_replicas, int n_populations) {
+  if (n_replicas <= 0 || n_populations <= 0 || n_replicas % n_populations) return 0;
+  const long long rp = n_replicas / n_populations, nt = (rp + kPaTile - 1) / kPaTile;
+  return 8LL * (n_replicas + (long long)n_populations * (nt + 2));
+}
+
+int tsu_ising2d_population_anneal(uint32_t* d_state, uint32_t* d_scratch, int n_replicas, int rows, int cols,
+                                  int wrap_rows, int wrap_cols, const uint32_t* d_luts, const double* d_dbeta,
+                                  int n_steps, int sweeps_per_step, int n_populations, const uint32_t* d_bonds,
+                                  const int32_t* d_bond_index, uint64_t seed, uint32_t sweep0, uint32_t replica0,
+                                  double J, double h, long long n_bonds, long long n_sites, int32_t* d_family,
+                                  int32_t* d_family_scratch, unsigned long long* d_weight_sum, double* d_energy_ref,
+                                  unsigned long long* d_count_sums, unsigned long long* d_obs, double* d_energy,
+                                  void* d_work, size_t work_bytes, uintptr_t stream) {
+  Lattice L = {d_state, make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, 0), d_luts, nullptr,
+               {d_bonds, d_bond_index}, seed, replica0, JitKernel{nullptr, 0, 0}};
+  TSU_CHECK_ARG(d_state && d_scratch && d_state != d_scratch && args_ok(L.g, L.B, false, 0, 0, rows));
+  TSU_CHECK_ARG(n_steps >= 0 && sweeps_per_step >= 1 && n_populations >= 1 && n_populations <= 65535 &&
+                n_replicas % n_populations == 0);
+  TSU_CHECK_ARG(n_steps == 0 || (d_luts && d_dbeta && d_weight_sum && d_energy_ref));
+  TSU_CHECK_ARG(d_family && d_family_scratch && d_family != d_family_scratch && d_count_sums && d_obs && d_energy);
+  TSU_CHECK_ARG(d_work && work_bytes >= (size_t)tsu_ising2d_population_work_bytes(n_replicas, n_populations));
+  PopParams Q;
+  Q.rp = n_replicas / n_populations;
+  Q.n_pop = n_populations;
+  Q.nt = (Q.rp + kPaTile - 1) / kPaTile;
+  int lg = 0;
+  while ((1LL << lg) < Q.rp) ++lg;
+  Q.s = 62 - lg;
+  Q.prefix = static_cast<unsigned long long*>(d_work);
+  Q.tile_off = Q.prefix + n_replicas;
+  Q.min_key = Q.tile_off + (size_t)n_populations * Q.nt;
+  Q.draw = Q.min_key + n_populations;
+  const AnnealOut A = {J, h, n_bonds, n_sites, d_energy, nullptr, nullptr};
+  cudaStream_t st = tsu_stream(stream);
+  const size_t sums_per_step = 2 * (size_t)n_populations;
+  cudaError_t e = cudaMemsetAsync(d_count_sums, 0, sizeof(unsigned long long) * sums_per_step * (n_steps + 1), st);
+  if (e == cudaSuccess) e = cudaMemsetAsync(Q.min_key, 0xff, sizeof(unsigned long long) * n_populations, st);
+  if (e != cudaSuccess) return (int)e;
+  // the gather: a group of threads per child, at least 4 vectors per thread, or whole blocks for large replicas
+  const long long rep_vecs = 2LL * rows * L.g.wpr / 4;  // wpr is a multiple of 4
+  int group = 1;
+  while (group < 256 && 4LL * group < rep_vecs) group <<= 1;
+  dim3 gather_grid;
+  if (group < 256) {
+    gather_grid = dim3(blocks_for(n_replicas, 256 / group));
+  } else {
+    long long bx = (rep_vecs + 4 * 256 - 1) / (4 * 256);
+    const long long cap = (148LL * 8 + n_replicas - 1) / n_replicas;  // about 8 CTAs per SM in total
+    if (bx > cap) bx = cap;
+    gather_grid = dim3((unsigned)bx, (unsigned)(n_replicas < 65535 ? n_replicas : 65535));
+  }
+  const bool resident = resident_eligible(n_replicas, rows, cols);
+  uint32_t* other = d_scratch;
+  int32_t* fam = d_family;
+  int32_t* fam_other = d_family_scratch;
+  for (int k = 0; k < n_steps; ++k) {
+    int rc = launch_population_reduce(L, Q, A, d_obs, d_count_sums + sums_per_step * k, st);
+    if (rc != TSU_OK) return rc;
+    const uint32_t sweep = sweep0 + (uint32_t)k * (uint32_t)sweeps_per_step;
+    pa_weights_kernel<<<dim3((unsigned)Q.nt, (unsigned)n_populations), kPaThreads, 0, st>>>(d_energy, d_dbeta + k, Q);
+    pa_scan_kernel<<<n_populations, kPaScanThreads, 0, st>>>(Q, (uint32_t)seed, (uint32_t)(seed >> 32), sweep, replica0,
+                                                             d_weight_sum + (size_t)n_populations * k,
+                                                             d_energy_ref + (size_t)n_populations * k);
+    pa_gather_kernel<<<gather_grid, 256, 0, st>>>(reinterpret_cast<const uint4*>(L.state), reinterpret_cast<uint4*>(other),
+                                                 fam, fam_other, Q, d_weight_sum + (size_t)n_populations * k, rep_vecs,
+                                                 group);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return (int)e;
+    std::swap(L.state, other);
+    std::swap(fam, fam_other);
+    Lattice Lk = L;
+    Lk.lut = d_luts + 32 * (size_t)k;
+    rc = resident ? launch_resident_sweeps(Lk, sweep, sweeps_per_step, st) : launch_sweeps(Lk, sweep, sweeps_per_step, st);
+    if (rc != TSU_OK) return rc;
+  }
+  const int rc = launch_population_reduce(L, Q, A, d_obs, d_count_sums + sums_per_step * n_steps, st);
+  if (rc != TSU_OK) return rc;
+  if (L.state != d_state) {  // an odd number of gathers: the result is in the scratch buffers
+    e = cudaMemcpyAsync(d_state, L.state, sizeof(uint32_t) * 2 * (size_t)rows * L.g.wpr * n_replicas,
+                        cudaMemcpyDeviceToDevice, st);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(d_family, fam, sizeof(int32_t) * (size_t)n_replicas, cudaMemcpyDeviceToDevice, st);
+    if (e != cudaSuccess) return (int)e;
+  }
+  TSU_RETURN_LAUNCH_STATUS();
 }
 
 int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_replicas, double J, double h,

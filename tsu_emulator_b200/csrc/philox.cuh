@@ -102,6 +102,8 @@ __host__ __device__ __forceinline__ tsu_u32x4 tsu_philox4x32_10_keyed(uint32_t c
 //   counter = ( (w >> 2) | colour << 24,  global_row | (w & 3) << 24 | kind << 26,  sweep,  replica ),  key = seed
 //   kind 0,1  : bit-plane calls (planes 0-3 / 4-7 = top 8 bits of every lane's uniform)
 //   kind 2    : initial configuration
+//   kind 3    : population annealing, one call per population and step (w = colour = row = 0, replica = the
+//               population's first replica, sweep = the step's first sweep; words x | y << 32 are the 64-bit draw)
 //   kind 8-15 : low 24 bits, one call per group of 4 lanes (lane b uses word b&3 of call 8+(b>>2))
 // Everything that changes between the calls a thread makes while it walks down its rows (row, word within
 // the 4-word group, kind) sits in counter word 1; words 0, 2, 3 are fixed per thread.  Philox round 1 then
@@ -111,6 +113,7 @@ __host__ __device__ __forceinline__ tsu_u32x4 tsu_philox4x32_10_keyed(uint32_t c
 #define TSU_KIND_PLANE0 0u
 #define TSU_KIND_PLANE1 1u
 #define TSU_KIND_INIT 2u
+#define TSU_KIND_RESAMPLE 3u
 #define TSU_KIND_LOW0 8u
 #define TSU_LATTICE_MAX_ROWS (1 << 24)
 #define TSU_LATTICE_C0(w, colour) (((uint32_t)(w) >> 2) | ((uint32_t)(colour) << 24))

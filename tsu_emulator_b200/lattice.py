@@ -129,6 +129,64 @@ class AnnealResult:
         return out
 
 
+class PopulationResult:
+    """What Ising2DEngine.population_annealing returns; pass it back as `previous=` to continue the run.
+
+    Device tensors (P = n_populations, n = len(temperatures)):
+      energy      float64 [n_replicas], E of every replica's final state
+      family      int32 [n_replicas], the initial replica (replica0 + r) each replica descends from
+      weight_sum  int64 [n, P], W = sum of the quantised weights floor(exp(-dbeta (E_i - E_ref)) 2^s) of step k
+      energy_ref  float64 [n, P], E_ref = lowest E of the population entering step k
+      count_sums  int64 [n + 1, P, 2], (sum of up spins, sum of anti-aligned / unsatisfied bonds) of the states
+                  entering step k; entry n: the final states
+    Host: temperatures, T_start, dbeta, r_pop (R_p), shift (s), rows, cols, J, h, n_bonds, n_sites.
+    """
+
+    def __init__(self, energy, family, weight_sum, energy_ref, count_sums, temperatures, T_start, dbeta, r_pop, shift,
+                 rows, cols, J, h, n_bonds, n_sites):
+        self.energy, self.family = energy, family
+        self.weight_sum, self.energy_ref, self.count_sums = weight_sum, energy_ref, count_sums
+        self.temperatures, self.T_start, self.dbeta = temperatures, float(T_start), dbeta
+        self.r_pop, self.shift = int(r_pop), int(shift)
+        self.rows, self.cols, self.J, self.h = int(rows), int(cols), float(J), float(h)
+        self.n_bonds, self.n_sites = int(n_bonds), int(n_sites)
+
+    @property
+    def n_populations(self) -> int:
+        return int(self.weight_sum.shape[1])
+
+    def log_q(self) -> np.ndarray:
+        """[n, P] float64: ln Q_k = ln Z(T_k) / Z(T_{k-1}) ~ ln(W / (R_p 2^s)) - dbeta_k E_ref"""
+        W = self.weight_sum.cpu().numpy().astype(np.float64)
+        e_ref = self.energy_ref.cpu().numpy()
+        return np.log(W) - math.log(self.r_pop) - self.shift * math.log(2.0) - self.dbeta[:, None] * e_ref
+
+    def log_z_ratio(self) -> np.ndarray:
+        """[n, P]: ln Z(T_k) / Z(T_start), the cumulative sum of log_q"""
+        return np.cumsum(self.log_q(), axis=0)
+
+    def free_energy(self) -> np.ndarray:
+        """[n, P]: free energy per site -T_k ln Z(T_k) / N, with ln Z(T_start = inf) = N ln 2"""
+        if not math.isinf(self.T_start):
+            raise ValueError("free_energy needs a run from T_start = inf (ln Z is known only at infinite temperature)")
+        N = self.n_sites
+        return -self.temperatures[:, None] * (N * math.log(2.0) + self.log_z_ratio()) / N
+
+    def mean_energy(self) -> np.ndarray:
+        """[n, P]: population mean of E at temperatures[k] (after step k's sweeps), from count_sums[1:]"""
+        c = self.count_sums[1:].cpu().numpy().astype(np.float64) / self.r_pop
+        return -self.J * (self.n_bonds - 2.0 * c[..., 1]) - self.h * (2.0 * c[..., 0] - self.n_sites)
+
+    def rho_t(self) -> np.ndarray:
+        """[P]: R_p sum_f (n_f / R_p)^2 over the families f of each population (1 when every family has one member)"""
+        fam = self.family.cpu().numpy().reshape(self.n_populations, self.r_pop)
+        out = np.empty(self.n_populations)
+        for p in range(self.n_populations):
+            n_f = np.unique(fam[p], return_counts=True)[1].astype(np.float64)
+            out[p] = (n_f * n_f).sum() / self.r_pop
+        return out
+
+
 class Ising2DEngine:
     """n_replicas independent rows x cols lattices (or one row-slab of each) resident in HBM.
 
@@ -486,6 +544,91 @@ class Ising2DEngine:
         tables = self._torch.from_numpy(np.ascontiguousarray(luts).view(np.int32)).to(self.device)
         self._anneal_tables = (key, tables)
         return tables
+
+    # ------------------------------------------------------------------ population annealing
+    def population_annealing(self, temperatures, *, sweeps_per_step: int = 10, n_populations: int = 1,
+                             T_start: float = math.inf, previous: Optional[PopulationResult] = None) -> PopulationResult:
+        """Population annealing (Hukushima-Iba, Machta) of every replica in one call, with no host sync.
+
+        The replicas form n_populations equal contiguous populations of R_p replicas, each resampled on its own (one
+        population per disorder realisation: bond_index must be constant within each).  The current state is taken
+        to be an equilibrium sample at T_start (inf: beta = 0, e.g. the states of init_random()).  Step k resamples
+        every population in proportion to exp(-dbeta_k E) with dbeta_k = 1/T_k - 1/T_{k-1} (T_{-1} = T_start), keeping
+        R_p fixed (systematic resampling with integer weights; tsu_ising2d_population_anneal states the exact rule),
+        then sweeps sweeps_per_step times at T_k.  The result gives ln Z ratios, free energies, mean energies and the
+        family statistic rho_t; see PopulationResult.
+
+        temperatures must be non-increasing and at most T_start.  previous: the result of an earlier run of this
+        engine; its last temperature becomes T_start and its family buffer is continued in place, so a run split into
+        calls equals one call.  Afterwards sweep_index has advanced by len(temperatures) * sweeps_per_step and the
+        engine is at the scalar temperature temperatures[-1].
+
+        The call allocates a second state buffer and a small workspace for its duration, so the state memory doubles
+        while it runs.  Always the prebuilt kernels.
+        """
+        if self.is_slab:
+            raise ValueError("population annealing needs whole lattices; row-slab engines cannot run it")
+        if self.bias_mode != "physical":
+            raise ValueError("population annealing needs bias_mode='physical': the sweeps of the reference bias do not "
+                             "sample exp(-E/T), so the resampling weights would be wrong")
+        Ts = np.asarray(temperatures, dtype=np.float64)
+        if Ts.ndim != 1 or Ts.size == 0:
+            raise ValueError("temperatures must be a non-empty 1-D schedule")
+        if not np.all(np.isfinite(Ts)) or np.any(Ts <= 0):
+            raise ValueError("temperatures must be positive and finite")
+        if np.any(np.diff(Ts) > 0):
+            raise ValueError("temperatures must be non-increasing")
+        theta, P, n = int(sweeps_per_step), int(n_populations), self.n_replicas
+        if theta < 1:
+            raise ValueError("sweeps_per_step must be >= 1")
+        if P < 1 or P > 65535 or n % P:
+            raise ValueError(f"n_populations must divide n_replicas = {n} (and lie in [1, 65535])")
+        r_pop = n // P
+        if previous is not None:
+            if (previous.n_populations != P or previous.r_pop != r_pop or tuple(previous.family.shape) != (n,)
+                    or (previous.rows, previous.cols) != (self.rows, self.cols)):
+                raise ValueError(f"previous must come from a run of {P} populations of {r_pop} replicas of "
+                                 f"{self.rows} x {self.cols}")
+            T_start = float(previous.temperatures[-1])
+        T_start = float(T_start)
+        if not T_start > 0 or Ts[0] > T_start:
+            raise ValueError("T_start must be positive and at least temperatures[0]")
+        if self.bond_index is not None:
+            idx = np.asarray(self.bond_index.cpu()).reshape(P, r_pop)
+            if np.any(idx != idx[:, :1]):
+                raise ValueError("bond_index must be constant within each population (one realisation per population)")
+        beta = 1.0 / Ts
+        dbeta = np.diff(np.concatenate([[0.0 if math.isinf(T_start) else 1.0 / T_start], beta]))
+        torch = self._torch
+        dev = self.device
+        with torch.cuda.device(dev):
+            if previous is not None:
+                family = previous.family
+            else:
+                family = torch.arange(self.replica0, self.replica0 + n, dtype=torch.int32, device=dev)
+            scratch = torch.empty_like(self.state)
+            family_scratch = torch.empty_like(family)
+            work_bytes = int(self.lib.tsu_ising2d_population_work_bytes(n, P))
+            work = torch.empty(work_bytes // 8, dtype=torch.int64, device=dev)
+            weight_sum = torch.empty((Ts.size, P), dtype=torch.int64, device=dev)
+            energy_ref = torch.empty((Ts.size, P), dtype=torch.float64, device=dev)
+            count_sums = torch.empty((Ts.size + 1, P, 2), dtype=torch.int64, device=dev)
+            energy = torch.empty(n, dtype=torch.float64, device=dev)
+            d_dbeta = torch.from_numpy(dbeta).to(dev)
+            luts = self._schedule_tables(Ts)
+            _lib.call(
+                "tsu_ising2d_population_anneal", ptr(self.state), ptr(scratch), n, self.rows, self.cols,
+                int(self.wrap_rows), int(self.wrap_cols), ptr(luts), ptr(d_dbeta), int(Ts.size), theta, P,
+                ptr(self.bonds), ptr(self.bond_index), self.seed, self.sweep_index & 0xFFFFFFFF, self.replica0,
+                self.coupling, self.field, self.n_bonds, self.n_sites, ptr(family), ptr(family_scratch),
+                ptr(weight_sum), ptr(energy_ref), ptr(count_sums), ptr(self._obs), ptr(energy), ptr(work), work_bytes,
+                _lib.current_stream(),
+            )
+        self.sweep_index += int(Ts.size) * theta
+        self.set_temperature(float(Ts[-1]))
+        shift = 62 - (r_pop - 1).bit_length()
+        return PopulationResult(energy, family, weight_sum, energy_ref, count_sums, Ts.copy(), T_start, dbeta, r_pop,
+                                shift, self.rows, self.cols, self.coupling, self.field, self.n_bonds, self.n_sites)
 
     # ------------------------------------------------------------------ observables
     def observables_tensor(self, next_rows=None):
