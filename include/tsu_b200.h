@@ -263,6 +263,37 @@ int tsu_ising2d_population_anneal(uint32_t* d_state, uint32_t* d_scratch, int n_
                                   unsigned long long* d_count_sums, unsigned long long* d_obs, double* d_energy,
                                   void* d_work, size_t work_bytes, uintptr_t stream);
 
+/* Swendsen-Wang cluster updates of whole lattices at h = 0 ("physical" bias); no host sync, nothing allocated.
+ * One step at sweep index s, for replica r with threshold t = d_thresholds[d_lut_index ? d_lut_index[r] : 0]:
+ *   1. satisfied bonds: J sigma_ij s_i s_j > 0 (sigma = +-1 bond sign, +1 without bonds; J's sign is
+ *      coupling_sign = +1 or -1), over the bonds tsu_ising2d_observables counts (right and down of every site, wraps
+ *      only where wrap_rows / wrap_cols are set).
+ *   2. activation: a satisfied bond is active iff u < t, t = ceil(p 2^32) with p = -expm1(-2|J| / T) in float64
+ *      (t = 2^32: always active).  u is a 32-bit uniform of the lattice stream built as the Gibbs uniform, for the
+ *      site the bond starts from: bit-planes of kinds 16, 17 and low bits of kinds 24-31 (east bonds), kinds 18, 19
+ *      and 32-39 (south bonds).
+ *   3. clusters: connected components of the active bonds; a cluster's root is its site with the smallest
+ *      row * cols + col.
+ *   4. flip: a cluster flips iff bit b of word x of the lattice call (w, colour, kind 4, row, s, replica0 + r) is 1,
+ *      (colour, row, w, b) being the root's packed position.
+ * n_steps steps use sweep indices sweep0 .. sweep0 + n_steps - 1; n_steps = 0 is a no-op.  The bits depend on neither
+ * the launch path nor the workspace: the replicas run in chunks of work_bytes / tsu_ising2d_cluster_work_bytes(1, ..)
+ * replicas, each chunk through all its steps, all ordered on `stream`.  Lattices of at most 12288 sites run every
+ * step in one launch, one block per replica with the labels in shared memory (TSU_LATTICE_RESIDENT=0 disables);
+ * larger ones run four launches per step: activation and flip words, union-find in shared-memory tiles of 32 x 256
+ * sites, unions across tiles and wraps in global memory, and the flips.
+ * d_work: at least tsu_ising2d_cluster_work_bytes(1, rows, cols) bytes, 16-byte aligned (labels, activation and flip
+ * words: about 4.4 bytes per site and replica); its layout is private.  Bonds as in tsu_ising2d_sweeps.
+ * TSU_ERR_INVALID_ARG before any CUDA call for: n_steps < 0, a NULL d_state / d_thresholds / d_work, a work buffer
+ * below one replica, rows * cols above 2^31 - 1, coupling_sign not +-1, and the lattice rules of tsu_ising2d_sweeps.
+ * tsu_ising2d_cluster_work_bytes returns 0 for a lattice it cannot serve. */
+int64_t tsu_ising2d_cluster_work_bytes(int n_replicas, int rows, int cols);
+int tsu_ising2d_swendsen_wang(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                              const uint64_t* d_thresholds, const int32_t* d_lut_index, int coupling_sign,
+                              const uint32_t* d_bonds, const int32_t* d_bond_index, uint64_t seed,
+                              uint32_t sweep0, int n_steps, uint32_t replica0,
+                              void* d_work, size_t work_bytes, uintptr_t stream);
+
 /* ------------------------------------------------------------------ dense-J Gibbs ----- */
 /*
  * Replaces GibbsSampler.gibbs_sweep / sample_boltzmann / compute_energy and the sweep part of

@@ -139,11 +139,13 @@ __device__ __forceinline__ uint32_t bitsel(uint32_t m, uint32_t a, uint32_t b) {
   return (m & a) | (~m & b);
 }
 
-__device__ __forceinline__ uint32_t lane_uniform(const uint32_t r[8], const Coords& q, uint32_t w, uint32_t row_g, int j) {
+// lane j's 32-bit uniform: the top 8 bits from the bit-planes r, the low 24 from call low0 + (j >> 2)
+__device__ __forceinline__ uint32_t lane_uniform(const uint32_t r[8], const Coords& q, uint32_t w, uint32_t row_g, int j,
+                                                 uint32_t low0 = TSU_KIND_LOW0) {
   uint32_t u = 0;
 #pragma unroll
   for (int k = 0; k < 8; ++k) u |= ((r[k] >> j) & 1u) << (31 - k);
-  tsu_u32x4 lo = lattice_call(q, w, row_g, TSU_KIND_LOW0 + (uint32_t)(j >> 2));
+  tsu_u32x4 lo = lattice_call(q, w, row_g, low0 + (uint32_t)(j >> 2));
   int sel = j & 3;
   uint32_t v = sel == 0 ? lo.x : (sel == 1 ? lo.y : (sel == 2 ? lo.z : lo.w));
   return u | (v >> 8);
@@ -944,6 +946,298 @@ __global__ void __launch_bounds__(256) pa_gather_kernel(const uint4* __restrict_
   }
 }
 
+// ---- Swendsen-Wang cluster updates (tsu_ising2d_swendsen_wang) ------------------------------------------------
+// Per replica the caller's work buffer holds (ClusterParams::rep_bytes apart) labels int32 [rows * cols] (site index
+// row * cols + col, padded to 16 bytes), the activation words uint32 [2 colours][east, south][rows][wpr] and the flip
+// words uint32 [2 colours][rows][wpr], both in the layout of the state.  Labels form a union-find forest in which a
+// site's parent never has a larger index; unions always hang the larger root under the smaller, so every tree's root
+// is its cluster's smallest site index, whatever order the unions run in.
+constexpr int kClusterThreads = 256;
+constexpr int kClusterTileRows = 32, kClusterTileWords = 4;  // tiles of the local pass: 32 rows x 256 columns
+constexpr int kClusterTileCols = 64 * kClusterTileWords;
+constexpr int kClusterResidentSites = 12288;  // labels of a replica in 48 KB of shared memory: one launch per call
+
+struct ClusterParams {
+  const unsigned long long* thresholds;  // [n_tables] t = ceil(p 2^32), p = 1 - exp(-2|J|/T); 2^32: always active
+  int sign;                              // sign of J: +1 satisfied = aligned (after the bond sign), -1 anti-aligned
+  char* work;
+  size_t rep_bytes, act_offset, flip_offset;  // per replica: its share of the work buffer, where its words start
+};
+
+__device__ __forceinline__ int32_t* cluster_labels(const ClusterParams& C, int rep) {
+  return reinterpret_cast<int32_t*>(C.work + (size_t)rep * C.rep_bytes);
+}
+__device__ __forceinline__ uint32_t* cluster_act(const ClusterParams& C, int rep) {  // [colour][dir][rows][wpr]
+  return reinterpret_cast<uint32_t*>(C.work + (size_t)rep * C.rep_bytes + C.act_offset);
+}
+__device__ __forceinline__ uint32_t* cluster_flip(const ClusterParams& C, int rep) {  // [colour][rows][wpr]
+  return reinterpret_cast<uint32_t*>(C.work + (size_t)rep * C.rep_bytes + C.flip_offset);
+}
+
+// lanes of `sat` whose bond uniform u (bit-planes of kinds plane0, plane0 + 1, low bits of kinds low0 ..) is below t:
+// the borrow chain of update_word against one threshold, with the low words drawn only on ties
+__device__ __forceinline__ uint32_t activate_bonds(uint32_t sat, unsigned long long t, const Coords& q, uint32_t w,
+                                                   uint32_t row_g, uint32_t plane0, uint32_t low0) {
+  if (sat == 0u || t >= (1ull << 32)) return sat;
+  const uint32_t t32 = (uint32_t)t;
+  uint32_t r[8];
+  {
+    tsu_u32x4 p0 = lattice_call(q, w, row_g, plane0);
+    tsu_u32x4 p1 = lattice_call(q, w, row_g, plane0 + 1u);
+    r[0] = p0.x; r[1] = p0.y; r[2] = p0.z; r[3] = p0.w;
+    r[4] = p1.x; r[5] = p1.y; r[6] = p1.z; r[7] = p1.w;
+  }
+  uint32_t lt = 0u, eq = 0xffffffffu;
+#pragma unroll
+  for (int k = 7; k >= 0; --k) {
+    const uint32_t tk = 0u - ((t32 >> (31 - k)) & 1u);
+    const uint32_t x = r[k] ^ tk;
+    lt = (~r[k] & tk) | (~x & lt);
+    eq &= ~x;
+  }
+  eq &= sat;
+  while (eq) {
+    const int j = __ffs(eq) - 1;
+    eq &= eq - 1u;
+    const uint32_t bit = lane_uniform(r, q, w, row_g, j, low0) < t32 ? 1u : 0u;
+    lt = (lt & ~(1u << j)) | (bit << j);
+  }
+  return lt & sat;
+}
+
+// Step `sweep` of word (rep, colour, row i, w): its east and south activation words and its flip word.  The hood's
+// neighbour words carry the bond signs (apply_bonds), so x ^ neighbour is 1 where sigma s_i s_j = -1, as count_word counts.
+template <bool BONDED>
+__device__ __forceinline__ void cluster_bond_word(const SweepParams& P, const BondParams& B, const ClusterParams& C,
+                                                  uint32_t sweep, int rep, int colour, int i, int w) {
+  const Geom& g = P.g;
+  const size_t plane = (size_t)g.rows * g.wpr;
+  Planes pl;
+  pl.opp = P.state + ((size_t)rep * 2 + (1 - colour)) * plane;
+  pl.halo_top = nullptr;
+  pl.halo_bot = nullptr;
+  Hood h = load_hood(pl, g, colour, i, w);
+  const size_t off = (size_t)i * g.wpr + w;
+  uint32_t* act = cluster_act(C, rep) + (size_t)colour * 2 * plane + off;
+  uint32_t* flip = cluster_flip(C, rep) + (size_t)colour * plane + off;
+  if (h.valid == 0u) {  // padding word
+    act[0] = 0u;
+    act[plane] = 0u;
+    *flip = 0u;
+    return;
+  }
+  if constexpr (BONDED) apply_bonds(h, B, g, rep, colour, i, w);
+  const uint32_t x = P.state[((size_t)rep * 2 + colour) * plane + off];
+  const int p = (g.row0 + i + colour) & 1;
+  const uint32_t aligned = C.sign > 0 ? 0xffffffffu : 0u;
+  const uint32_t sat_e = (x ^ (p ? h.side : h.c) ^ aligned) & h.valid & ~h.missE;
+  const uint32_t sat_s = h.has_s ? (x ^ h.s ^ aligned) & h.valid : 0u;
+  Coords q;
+  q.colour = (uint32_t)colour;
+  q.sweep = sweep;
+  q.replica = P.replica0 + (uint32_t)rep;
+  q.k0 = P.k0;
+  q.k1 = P.k1;
+  const unsigned long long t = C.thresholds[P.lut_index ? P.lut_index[rep] : 0];
+  const uint32_t row_g = (uint32_t)(g.row0 + i);
+  act[0] = activate_bonds(sat_e, t, q, (uint32_t)w, row_g, TSU_KIND_BOND_E_PLANE0, TSU_KIND_BOND_E_LOW0);
+  act[plane] = activate_bonds(sat_s, t, q, (uint32_t)w, row_g, TSU_KIND_BOND_S_PLANE0, TSU_KIND_BOND_S_LOW0);
+  *flip = lattice_call(q, (uint32_t)w, row_g, TSU_KIND_CLUSTER_FLIP).x & h.valid;
+}
+
+// root of x, halving the path on the way (every site then points at its former grandparent).  A label only ever
+// points at a smaller site of the same cluster, so a stale read or an overwritten link still leads to the root
+// (the pointer jumping of ECL-CC, Jaiganesh & Burtscher 2018).
+__device__ __forceinline__ int cluster_find(int32_t* L, int x) {
+  volatile int32_t* V = L;
+  int y = V[x];
+  while (y != x) {
+    const int z = V[y];
+    if (z != y) V[x] = z;
+    x = y;
+    y = z;
+  }
+  return x;
+}
+
+// joins the trees of a and b, hanging the larger root under the smaller (Playne & Hawick's lock-free union)
+__device__ __forceinline__ void cluster_union(int32_t* L, int a, int b) {
+  while (true) {
+    a = cluster_find(L, a);
+    b = cluster_find(L, b);
+    if (a == b) return;
+    if (a > b) {
+      const int t = a;
+      a = b;
+      b = t;
+    }
+    const int old = atomicMin(L + b, a);
+    if (old == b) return;
+    b = old;  // b was no longer a root: join its parent (b itself now points to min(old, a)) to a
+  }
+}
+
+// Unions in the forest L of one tile every active bond whose two sites both lie in it.  The tile is rows
+// [r0, r0 + nr) and columns [c0, c0 + nc) with c0 = 64 w0; its words are w0 .. w0 + nw - 1 of both colours, and its
+// site (i, col) is L[(i - r0) * nc + col - c0].  Wrapped neighbours count when they lie in the tile.
+__device__ __forceinline__ void cluster_tile_unions(int32_t* L, const uint32_t* act, const Geom& g, int r0, int nr,
+                                                    int w0, int nw, int c0, int nc) {
+  const size_t plane = (size_t)g.rows * g.wpr;
+  for (int t = threadIdx.x; t < 2 * nr * nw; t += blockDim.x) {
+    const int colour = t / (nr * nw), rem = t - colour * nr * nw, r = rem / nw, w = w0 + rem - r * nw, i = r0 + r;
+    const int p = (g.row0 + i + colour) & 1;
+    const uint32_t* a = act + (size_t)colour * 2 * plane + (size_t)i * g.wpr + w;
+    uint32_t e = a[0], s = a[plane];
+    const int ni = i + 1 == g.rows ? 0 : i + 1;
+    if (ni < r0 || ni >= r0 + nr) s = 0u;
+    while (e | s) {
+      const int j = __ffs(e | s) - 1;
+      const uint32_t bit = 1u << j;
+      const int col = 2 * (32 * w + j) + p, x = r * nc + col - c0;
+      if (e & bit) {
+        const int ncol = col + 1 == g.cols ? 0 : col + 1;
+        if (ncol >= c0 && ncol < c0 + nc) cluster_union(L, x, r * nc + ncol - c0);
+      }
+      if (s & bit) cluster_union(L, x, (ni - r0) * nc + col - c0);
+      e &= ~bit;
+      s &= ~bit;
+    }
+  }
+}
+
+// XORs into word (rep, colour, row i, w) the flip bit of every site's cluster root; `L` is the label forest of the
+// whole replica (site index row * cols + col).  Path compression: each site then points at its root.
+__device__ __forceinline__ void cluster_flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int rep,
+                                                  int colour, int i, int w) {
+  const Geom& g = P.g;
+  const int p = (g.row0 + i + colour) & 1;
+  uint32_t m = lane_mask_lt(colour_count(g.cols, p) - 32 * w);
+  if (m == 0u) return;
+  const size_t plane = (size_t)g.rows * g.wpr;
+  const uint32_t* flip = cluster_flip(C, rep);
+  uint32_t out = 0u;
+  while (m) {
+    const int j = __ffs(m) - 1;
+    m &= m - 1u;
+    const int x = i * g.cols + 2 * (32 * w + j) + p;
+    const int root = cluster_find(L, x);
+    if (L[x] != root) L[x] = root;
+    const int ri = root / g.cols, rc = root - ri * g.cols, rk = rc >> 1;
+    out |= ((flip[(size_t)((g.row0 + ri + rc) & 1) * plane + (size_t)ri * g.wpr + (rk >> 5)] >> (rk & 31)) & 1u) << j;
+  }
+  P.state[((size_t)rep * 2 + colour) * plane + (size_t)i * g.wpr + w] ^= out;
+}
+
+// One thread per state word of every replica: activation and flip words of step P.sweep.
+template <bool BONDED>
+__global__ void __launch_bounds__(kClusterThreads) cluster_bonds_kernel(SweepParams P, BondParams B, ClusterParams C) {
+  const Geom& g = P.g;
+  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long per_rep = 2LL * g.rows * g.wpr;
+  if (tid >= per_rep * g.n_replicas) return;
+  const int rep = (int)(tid / per_rep);
+  const int rem = (int)(tid - (long long)rep * per_rep), colour = rem / (g.rows * g.wpr);
+  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr;
+  cluster_bond_word<BONDED>(P, B, C, P.sweep, rep, colour, i, rw - i * g.wpr);
+}
+
+// One block per tile of kClusterTileRows x kClusterTileCols sites: unions in shared memory, then every site's label is
+// the site index of its root within the tile.
+__global__ void __launch_bounds__(kClusterThreads) cluster_local_kernel(SweepParams P, ClusterParams C, int tiles_x,
+                                                                        int tiles_per_rep) {
+  __shared__ int32_t L[kClusterTileRows * kClusterTileCols];
+  const Geom& g = P.g;
+  const int rep = (int)(blockIdx.x / (unsigned)tiles_per_rep), tile = (int)(blockIdx.x % (unsigned)tiles_per_rep);
+  const int ty = tile / tiles_x, tx = tile - ty * tiles_x;
+  const int r0 = ty * kClusterTileRows, nr = min(kClusterTileRows, g.rows - r0);
+  const int c0 = tx * kClusterTileCols, nc = min(kClusterTileCols, g.cols - c0);
+  for (int t = threadIdx.x; t < nr * nc; t += kClusterThreads) L[t] = t;
+  __syncthreads();
+  cluster_tile_unions(L, cluster_act(C, rep), g, r0, nr, tx * kClusterTileWords, kClusterTileWords, c0, nc);
+  __syncthreads();
+  int32_t* labels = cluster_labels(C, rep);
+  for (int t = threadIdx.x; t < nr * nc; t += kClusterThreads) {
+    const int root = cluster_find(L, t), r = t / nc, rr = root / nc;
+    labels[(r0 + r) * g.cols + c0 + t - r * nc] = (r0 + rr) * g.cols + c0 + root - rr * nc;
+  }
+}
+
+// active bond of site (i, col) in direction dir (0 east, 1 south)
+__device__ __forceinline__ bool cluster_bond_active(const uint32_t* act, const Geom& g, int i, int col, int dir) {
+  const int colour = (g.row0 + i + col) & 1, k = col >> 1;
+  return (act[((size_t)colour * 2 + dir) * g.rows * g.wpr + (size_t)i * g.wpr + (k >> 5)] >> (k & 31)) & 1u;
+}
+
+// The bonds between tiles: south bonds of the last row of every tile row (n_brows of them) and east bonds of the last
+// column of every tile column (n_bcols), including the wraps; unions in global memory.
+__global__ void __launch_bounds__(kClusterThreads) cluster_merge_kernel(SweepParams P, ClusterParams C, int n_brows,
+                                                                        int n_bcols) {
+  const Geom& g = P.g;
+  const long long per_rep = (long long)n_brows * g.cols + (long long)g.rows * n_bcols;
+  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (tid >= per_rep * g.n_replicas) return;
+  const int rep = (int)(tid / per_rep);
+  const long long t = tid - (long long)rep * per_rep;
+  int i, col, ni, ncol, dir;
+  if (t < (long long)n_brows * g.cols) {
+    const int b = (int)(t / g.cols);
+    col = (int)(t - (long long)b * g.cols);
+    i = min(b * kClusterTileRows + kClusterTileRows - 1, g.rows - 1);
+    ni = i + 1 == g.rows ? 0 : i + 1;
+    ncol = col;
+    dir = 1;
+    if (ni / kClusterTileRows == i / kClusterTileRows) return;  // one tile row: the local pass took the wrap
+  } else {
+    const long long u = t - (long long)n_brows * g.cols;
+    i = (int)(u / n_bcols);
+    const int b = (int)(u - (long long)i * n_bcols);
+    col = min(b * kClusterTileCols + kClusterTileCols - 1, g.cols - 1);
+    ncol = col + 1 == g.cols ? 0 : col + 1;
+    ni = i;
+    dir = 0;
+    if (ncol / kClusterTileCols == col / kClusterTileCols) return;
+  }
+  if (cluster_bond_active(cluster_act(C, rep), g, i, col, dir))
+    cluster_union(cluster_labels(C, rep), i * g.cols + col, ni * g.cols + ncol);
+}
+
+__global__ void __launch_bounds__(kClusterThreads) cluster_flip_kernel(SweepParams P, ClusterParams C) {
+  const Geom& g = P.g;
+  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long per_rep = 2LL * g.rows * g.wpr;
+  if (tid >= per_rep * g.n_replicas) return;
+  const int rep = (int)(tid / per_rep);
+  const int rem = (int)(tid - (long long)rep * per_rep), colour = rem / (g.rows * g.wpr);
+  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr;
+  cluster_flip_word(P, C, cluster_labels(C, rep), rep, colour, i, rw - i * g.wpr);
+}
+
+// Lattices of at most kClusterResidentSites sites: every step of the call in one launch, one block per replica, the
+// labels in shared memory (the whole lattice is one tile of cluster_tile_unions).  The activation and flip words go
+// through the work buffer; the block's barriers make its own global stores visible to it.
+template <bool BONDED>
+__global__ void __launch_bounds__(kClusterThreads) cluster_resident_kernel(SweepParams P, BondParams B, ClusterParams C,
+                                                                           int n_steps) {
+  extern __shared__ int32_t L[];
+  const Geom& g = P.g;
+  const int rep = blockIdx.x, per_rep = g.rows * g.wpr, n_sites = g.rows * g.cols;
+  for (int s = 0; s < n_steps; ++s) {
+    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
+      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
+      cluster_bond_word<BONDED>(P, B, C, P.sweep + (uint32_t)s, rep, colour, i, rem - i * g.wpr);
+    }
+    for (int t = threadIdx.x; t < n_sites; t += kClusterThreads) L[t] = t;
+    __syncthreads();
+    cluster_tile_unions(L, cluster_act(C, rep), g, 0, g.rows, 0, g.wpr, 0, g.cols);
+    __syncthreads();
+    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
+      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
+      cluster_flip_word(P, C, L, rep, colour, i, rem - i * g.wpr);
+    }
+    __syncthreads();  // the next step's bonds read the flipped words
+  }
+}
+
 // ---- Edwards-Anderson bonds ---------------------------------------------------------------------------------
 // int8 signs[k][2][rows][cols] ([.,0,i,j]: bond (i,j)-(i,j+1 mod cols), [.,1,i,j]: bond (i,j)-(i+1 mod rows,j); < 0
 // = antiferromagnetic) -> bond words[k][colour][N,S,W,E][rows][wpr].  Bonds the wiring does not create (open edges;
@@ -1519,6 +1813,48 @@ int launch_population_reduce(const Lattice& L, const PopParams& Q, const AnnealO
   TSU_RETURN_LAUNCH_STATUS();
 }
 
+// bytes of the Swendsen-Wang work buffer per replica (layout at ClusterParams); 0 for lattices it cannot label
+long long cluster_rep_bytes(int rows, int cols) {
+  if (rows <= 0 || cols <= 0 || (long long)rows * cols > 2147483647LL) return 0;
+  const long long label_bytes = (4LL * rows * cols + 15) / 16 * 16;
+  return label_bytes + 24LL * rows * words_per_row(cols);
+}
+
+// n_steps Swendsen-Wang steps of the replicas of L, which own C.work: one launch for lattices whose labels fit a
+// block's shared memory, otherwise four launches per step (bonds, local labels, merges across tiles, flips)
+int launch_swendsen_wang(const Lattice& L, const ClusterParams& C, uint32_t sweep0, int n_steps, cudaStream_t st) {
+  const Geom& g = L.g;
+  SweepParams P = sweep_params(L, 0, sweep0, nullptr, nullptr);
+  const bool bonded = L.B.words != nullptr;
+  if (tuning().resident != 0 && (long long)g.rows * g.cols <= kClusterResidentSites) {
+    const size_t smem = sizeof(int32_t) * (size_t)g.rows * g.cols;
+    if (bonded)
+      cluster_resident_kernel<true><<<g.n_replicas, kClusterThreads, smem, st>>>(P, L.B, C, n_steps);
+    else
+      cluster_resident_kernel<false><<<g.n_replicas, kClusterThreads, smem, st>>>(P, kNoBonds, C, n_steps);
+    TSU_RETURN_LAUNCH_STATUS();
+  }
+  const unsigned word_grid = blocks_for(2LL * g.rows * g.wpr * g.n_replicas, kClusterThreads);
+  const int tiles_x = (g.cols + kClusterTileCols - 1) / kClusterTileCols;
+  const int tiles_y = (g.rows + kClusterTileRows - 1) / kClusterTileRows;
+  const unsigned merge_grid =
+      blocks_for(((long long)tiles_y * g.cols + (long long)g.rows * tiles_x) * g.n_replicas, kClusterThreads);
+  for (int s = 0; s < n_steps; ++s) {
+    P.sweep = sweep0 + (uint32_t)s;
+    if (bonded)
+      cluster_bonds_kernel<true><<<word_grid, kClusterThreads, 0, st>>>(P, L.B, C);
+    else
+      cluster_bonds_kernel<false><<<word_grid, kClusterThreads, 0, st>>>(P, kNoBonds, C);
+    cluster_local_kernel<<<(unsigned)((long long)tiles_x * tiles_y * g.n_replicas), kClusterThreads, 0, st>>>(
+        P, C, tiles_x, tiles_x * tiles_y);
+    cluster_merge_kernel<<<merge_grid, kClusterThreads, 0, st>>>(P, C, tiles_y, tiles_x);
+    cluster_flip_kernel<<<word_grid, kClusterThreads, 0, st>>>(P, C);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return (int)e;
+  }
+  return TSU_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1811,6 +2147,40 @@ int tsu_ising2d_population_anneal(uint32_t* d_state, uint32_t* d_scratch, int n_
     if (e != cudaSuccess) return (int)e;
   }
   TSU_RETURN_LAUNCH_STATUS();
+}
+
+int64_t tsu_ising2d_cluster_work_bytes(int n_replicas, int rows, int cols) {
+  return n_replicas > 0 ? n_replicas * cluster_rep_bytes(rows, cols) : 0;
+}
+
+int tsu_ising2d_swendsen_wang(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                              const uint64_t* d_thresholds, const int32_t* d_lut_index, int coupling_sign,
+                              const uint32_t* d_bonds, const int32_t* d_bond_index, uint64_t seed, uint32_t sweep0,
+                              int n_steps, uint32_t replica0, void* d_work, size_t work_bytes, uintptr_t stream) {
+  const Lattice L = {d_state, make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, 0), nullptr, d_lut_index,
+                     {d_bonds, d_bond_index}, seed, replica0, JitKernel{nullptr, 0, 0}};
+  TSU_CHECK_ARG(d_state && d_thresholds && d_work && n_steps >= 0 && (coupling_sign == 1 || coupling_sign == -1));
+  TSU_CHECK_ARG(args_ok(L.g, L.B, false, 0, 0, rows));
+  const long long rep_bytes = cluster_rep_bytes(rows, cols);
+  TSU_CHECK_ARG(rep_bytes > 0 && work_bytes >= (size_t)rep_bytes);
+  if (n_steps == 0) return TSU_OK;
+  const long long fit = (long long)(work_bytes / (size_t)rep_bytes);
+  const int chunk = fit < n_replicas ? (int)fit : n_replicas;
+  ClusterParams C;
+  C.thresholds = reinterpret_cast<const unsigned long long*>(d_thresholds);
+  C.sign = coupling_sign;
+  C.work = static_cast<char*>(d_work);
+  C.rep_bytes = (size_t)rep_bytes;
+  C.act_offset = (4 * (size_t)rows * cols + 15) / 16 * 16;
+  C.flip_offset = C.act_offset + 16 * (size_t)rows * L.g.wpr;
+  cudaStream_t st = tsu_stream(stream);
+  // chunks one after the other, each through all its steps: the bits depend on no chunk size
+  for (int r0 = 0; r0 < n_replicas; r0 += chunk) {
+    const int rc = launch_swendsen_wang(L.replicas(r0, r0 + chunk < n_replicas ? r0 + chunk : n_replicas), C, sweep0,
+                                        n_steps, st);
+    if (rc != TSU_OK) return rc;
+  }
+  return TSU_OK;
 }
 
 int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_replicas, double J, double h,

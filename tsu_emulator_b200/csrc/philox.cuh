@@ -104,7 +104,10 @@ __host__ __device__ __forceinline__ tsu_u32x4 tsu_philox4x32_10_keyed(uint32_t c
 //   kind 2    : initial configuration
 //   kind 3    : population annealing, one call per population and step (w = colour = row = 0, replica = the
 //               population's first replica, sweep = the step's first sweep; words x | y << 32 are the 64-bit draw)
+//   kind 4    : Swendsen-Wang cluster flips: bit b of word x of the call of the cluster root's word (as kind 2)
 //   kind 8-15 : low 24 bits, one call per group of 4 lanes (lane b uses word b&3 of call 8+(b>>2))
+//   kind 16,17 / 24-31 : Swendsen-Wang east-bond uniforms (bit-planes / low 24 bits, as kinds 0,1 / 8-15)
+//   kind 18,19 / 32-39 : Swendsen-Wang south-bond uniforms (bit-planes / low 24 bits, as kinds 0,1 / 8-15)
 // Everything that changes between the calls a thread makes while it walks down its rows (row, word within
 // the 4-word group, kind) sits in counter word 1; words 0, 2, 3 are fixed per thread.  Philox round 1 then
 // multiplies only fixed values, and half of rounds 2 and 3 is fixed as well: tsu_lattice_stream keeps those
@@ -115,6 +118,11 @@ __host__ __device__ __forceinline__ tsu_u32x4 tsu_philox4x32_10_keyed(uint32_t c
 #define TSU_KIND_INIT 2u
 #define TSU_KIND_RESAMPLE 3u
 #define TSU_KIND_LOW0 8u
+#define TSU_KIND_CLUSTER_FLIP 4u
+#define TSU_KIND_BOND_E_PLANE0 16u
+#define TSU_KIND_BOND_S_PLANE0 18u
+#define TSU_KIND_BOND_E_LOW0 24u
+#define TSU_KIND_BOND_S_LOW0 32u
 #define TSU_LATTICE_MAX_ROWS (1 << 24)
 #define TSU_LATTICE_C0(w, colour) (((uint32_t)(w) >> 2) | ((uint32_t)(colour) << 24))
 #define TSU_LATTICE_C1(row, w, kind) ((uint32_t)(row) | (((uint32_t)(w) & 3u) << 24) | ((uint32_t)(kind) << 26))

@@ -64,6 +64,19 @@ def build_lut(J: float, h: float, T: float, bias_mode: str = "physical") -> np.n
     return lut
 
 
+def cluster_threshold(J: float, T: float) -> int:
+    """Swendsen-Wang bond activation threshold t = ceil(p 2^32), p = 1 - exp(-2|J|/T) in float64, as a Python int: a
+    satisfied bond with 32-bit uniform u is active iff u < t; t = 2^32 (p rounds to 1) activates every one."""
+    if T <= 0:
+        raise ValueError("Temperature must be positive")
+    p = -math.expm1(-2.0 * abs(float(J)) / float(T))
+    return int(math.ceil(p * 4294967296.0))
+
+
+# Swendsen-Wang workspace per engine: replicas beyond what fits run in chunks (same bits); tests may lower it
+CLUSTER_WORK_BUDGET = 4 << 30
+
+
 def lattice_bond_count(rows: int, cols: int, wrap_rows: bool, wrap_cols: bool) -> int:
     """number of distinct bonds wired by tsu/models/ising.py:343-361"""
     return rows * (cols - 1) + (rows if wrap_cols else 0) + (rows - 1) * cols + (cols if wrap_rows else 0)
@@ -358,7 +371,8 @@ class Ising2DEngine:
             if start < 0 or count <= 0 or start + count > self.n_replicas:
                 raise ValueError("chunk out of range")
             v = object.__new__(Ising2DEngine)
-            v.__dict__.update({k: val for k, val in self.__dict__.items() if k != "_views"})
+            # (a view gets a Swendsen-Wang workspace of its own: views may run concurrently on different streams)
+            v.__dict__.update({k: val for k, val in self.__dict__.items() if k not in ("_views", "_cluster_work")})
             v.n_replicas = int(count)
             v.replica0 = self.replica0 + int(start)
             v.state = self.state[start:start + count]
@@ -366,6 +380,8 @@ class Ising2DEngine:
             v.temperatures = self.temperatures if self.temperatures.size == 1 else self.temperatures[start:start + count]
             cache[key] = v
         v.lut = self.lut
+        if hasattr(self, "_lut_temps"):
+            v._lut_temps = self._lut_temps
         v.lut_index = None if self.lut_index is None else self.lut_index[start:start + count]
         v.bond_index = None if self.bond_index is None else self.bond_index[start:start + count]
         return v
@@ -629,6 +645,59 @@ class Ising2DEngine:
         shift = 62 - (r_pop - 1).bit_length()
         return PopulationResult(energy, family, weight_sum, energy_ref, count_sums, Ts.copy(), T_start, dbeta, r_pop,
                                 shift, self.rows, self.cols, self.coupling, self.field, self.n_bonds, self.n_sites)
+
+    # ------------------------------------------------------------------ cluster updates
+    def swendsen_wang(self, n_steps: int = 1):
+        """n_steps Swendsen-Wang multi-cluster steps of every replica in one call, with no host sync.
+
+        Each replica runs at its current temperature (per-replica temperatures and set_temperature_tables maps
+        included, so replica exchange can alternate with it).  A step activates every satisfied bond
+        (J sigma_ij s_i s_j > 0) with probability p = 1 - exp(-2|J|/T), labels the clusters of active bonds and flips
+        each with probability 1/2; tsu_ising2d_swendsen_wang states the exact random stream.  Near T_c its
+        autocorrelation time grows far more slowly with the lattice size than that of sweep().  Afterwards
+        sweep_index has advanced by n_steps.
+
+        Field 0, bias_mode "physical" and whole lattices only.  The first call allocates a workspace of about 4.4
+        bytes per site for min(n_replicas, CLUSTER_WORK_BUDGET // bytes per replica) replicas, kept with the engine;
+        more replicas run in chunks of that many, with the same bits.
+        """
+        if self.field != 0:
+            raise ValueError("Swendsen-Wang updates need field = 0 (a field needs a ghost spin or a cluster heat bath)")
+        if self.bias_mode != "physical":
+            raise ValueError("Swendsen-Wang updates need bias_mode='physical': the reference bias does not sample "
+                             "exp(-E/T)")
+        if self.is_slab:
+            raise ValueError("Swendsen-Wang updates need whole lattices; row-slab engines cannot run them")
+        if isinstance(n_steps, bool) or not isinstance(n_steps, (int, np.integer)) or n_steps < 0:
+            raise ValueError("n_steps must be a non-negative integer")
+        if self.rows * self.cols >= 1 << 31:
+            raise ValueError("Swendsen-Wang labels are int32: rows * cols must stay below 2^31")
+        n_steps = int(n_steps)
+        if n_steps == 0:
+            return self
+        torch = self._torch
+        with torch.cuda.device(self.device):
+            work = self.__dict__.get("_cluster_work")
+            if work is None:
+                per_rep = int(self.lib.tsu_ising2d_cluster_work_bytes(1, self.rows, self.cols))
+                n_work = min(self.n_replicas, max(1, CLUSTER_WORK_BUDGET // per_rep))
+                work = torch.empty(n_work * per_rep // 8, dtype=torch.int64, device=self.device)
+                self._cluster_work = work
+            key = (self.coupling, np.asarray(self._lut_temps).tobytes())
+            cached = self.__dict__.get("_cluster_tables")
+            if cached is None or cached[0] != key:
+                t = np.array([cluster_threshold(self.coupling, float(T)) for T in self._lut_temps], dtype=np.int64)
+                cached = (key, torch.from_numpy(t).to(self.device))
+                self._cluster_tables = cached
+            _lib.call(
+                "tsu_ising2d_swendsen_wang", ptr(self.state), self.n_replicas, self.rows, self.cols,
+                int(self.wrap_rows), int(self.wrap_cols), ptr(cached[1]), ptr(self.lut_index),
+                -1 if self.coupling < 0 else 1, ptr(self.bonds), ptr(self.bond_index), self.seed,
+                self.sweep_index & 0xFFFFFFFF, n_steps, self.replica0, ptr(work), work.numel() * 8,
+                _lib.current_stream(),
+            )
+        self.sweep_index += n_steps
+        return self
 
     # ------------------------------------------------------------------ observables
     def observables_tensor(self, next_rows=None):
