@@ -294,6 +294,30 @@ int tsu_ising2d_swendsen_wang(uint32_t* d_state, int n_replicas, int rows, int c
                               uint32_t sweep0, int n_steps, uint32_t replica0,
                               void* d_work, size_t work_bytes, uintptr_t stream);
 
+/* Houdayer cluster moves of replica pairs (two replicas of the same couplings at the same temperature); no host sync,
+ * nothing allocated.  One step at sweep index s, for each pair (a, b) of d_pairs (int32 [n_pairs][2] on the device):
+ *   1. differ: d_i = x^a_i xor x^b_i at every site.
+ *   2. active: a bond the wiring creates (right and down of every site, wraps only where wrap_rows / wrap_cols are
+ *      set) is active iff d = 1 at both its ends.  No randomness, temperature or bond sign enters.
+ *   3. clusters: connected components of the active bonds over the sites with d = 1; a cluster's root is its site
+ *      with the smallest row * cols + col.
+ *   4. flip: a cluster flips, in both replicas, iff bit b of word x of the lattice call (w, colour, kind 5, row, s,
+ *      replica0 + a) is 1, (colour, row, w, b) being the root's packed position.  Sites with d = 0 never change.
+ * The move leaves E_a + E_b and q_ab unchanged for any couplings and any uniform field, and keeps the product of the
+ * two Boltzmann distributions.  The caller guarantees that the pairs are disjoint and that the two replicas of a
+ * pair share couplings and temperature; a pair with an index outside [0, n_replicas) or a == b is skipped (its
+ * replicas' words are neither read nor written).
+ * n_steps steps use sweep indices sweep0 .. sweep0 + n_steps - 1; n_steps = 0 is a no-op.  The bits depend on neither
+ * the launch path nor the workspace: the pairs run in chunks of work_bytes / tsu_ising2d_cluster_work_bytes(1, ..)
+ * pairs, each chunk through all its steps, all ordered on `stream`.  Launch paths and the work buffer (one replica's
+ * share per pair) as in tsu_ising2d_swendsen_wang.
+ * TSU_ERR_INVALID_ARG before any CUDA call for: a NULL d_state / d_pairs / d_work, n_steps < 0, n_pairs < 1 or
+ * 2 n_pairs > n_replicas, a work buffer below one pair, rows * cols above 2^31 - 1, and the lattice rules of
+ * tsu_ising2d_sweeps. */
+int tsu_ising2d_houdayer(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                         const int32_t* d_pairs, int n_pairs, uint64_t seed, uint32_t sweep0, int n_steps,
+                         uint32_t replica0, void* d_work, size_t work_bytes, uintptr_t stream);
+
 /* ------------------------------------------------------------------ dense-J Gibbs ----- */
 /*
  * Replaces GibbsSampler.gibbs_sweep / sample_boltzmann / compute_energy and the sweep part of

@@ -96,6 +96,11 @@ SIGNATURES = {
         [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_uint64, c_uint32,
          c_int, c_uint32, c_void_p, ctypes.c_size_t, c_uintptr],
     ),
+    "tsu_ising2d_houdayer": (
+        c_int,
+        [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_uint64, c_uint32, c_int, c_uint32, c_void_p,
+         ctypes.c_size_t, c_uintptr],
+    ),
     "tsu_dense_gibbs_run": (
         c_int,
         [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_void_p, c_int, c_int, c_int,

@@ -1105,16 +1105,11 @@ __device__ __forceinline__ void cluster_tile_unions(int32_t* L, const uint32_t* 
   }
 }
 
-// XORs into word (rep, colour, row i, w) the flip bit of every site's cluster root; `L` is the label forest of the
-// whole replica (site index row * cols + col).  Path compression: each site then points at its root.
-__device__ __forceinline__ void cluster_flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int rep,
-                                                  int colour, int i, int w) {
-  const Geom& g = P.g;
-  const int p = (g.row0 + i + colour) & 1;
-  uint32_t m = lane_mask_lt(colour_count(g.cols, p) - 32 * w);
-  if (m == 0u) return;
-  const size_t plane = (size_t)g.rows * g.wpr;
-  const uint32_t* flip = cluster_flip(C, rep);
+// The flip bits (words `flip`, [colour][rows][wpr]) of the cluster roots of lanes m of the word at row i, word w
+// whose sites sit in columns of parity p; `L` is the label forest of the whole lattice (site index row * cols + col).
+// Path compression: each visited site then points at its root.
+__device__ __forceinline__ uint32_t root_flip_bits(const uint32_t* flip, int32_t* L, const Geom& g, size_t plane, int p,
+                                                   int i, int w, uint32_t m) {
   uint32_t out = 0u;
   while (m) {
     const int j = __ffs(m) - 1;
@@ -1125,6 +1120,19 @@ __device__ __forceinline__ void cluster_flip_word(const SweepParams& P, const Cl
     const int ri = root / g.cols, rc = root - ri * g.cols, rk = rc >> 1;
     out |= ((flip[(size_t)((g.row0 + ri + rc) & 1) * plane + (size_t)ri * g.wpr + (rk >> 5)] >> (rk & 31)) & 1u) << j;
   }
+  return out;
+}
+
+// XORs into word (rep, colour, row i, w) the flip bit of every site's cluster root
+__device__ __forceinline__ void cluster_flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int rep,
+                                                  int colour, int i, int w) {
+  const Geom& g = P.g;
+  const int p = (g.row0 + i + colour) & 1;
+  uint32_t m = lane_mask_lt(colour_count(g.cols, p) - 32 * w);
+  if (m == 0u) return;
+  const size_t plane = (size_t)g.rows * g.wpr;
+  const uint32_t* flip = cluster_flip(C, rep);
+  const uint32_t out = root_flip_bits(flip, L, g, plane, p, i, w, m);
   P.state[((size_t)rep * 2 + colour) * plane + (size_t)i * g.wpr + w] ^= out;
 }
 
@@ -1233,6 +1241,130 @@ __global__ void __launch_bounds__(kClusterThreads) cluster_resident_kernel(Sweep
     for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
       const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
       cluster_flip_word(P, C, L, rep, colour, i, rem - i * g.wpr);
+    }
+    __syncthreads();  // the next step's bonds read the flipped words
+  }
+}
+
+// ---- Houdayer cluster moves (tsu_ising2d_houdayer) ----------------------------------------------------------
+// Pair q of a chunk owns share q of the Swendsen-Wang work buffer (same layout) and runs the same labelling kernels,
+// with the pair index in place of the replica index.  Its activation words hold the bonds whose two sites both have
+// d = x^a xor x^b = 1; its flip words the kind-5 bits.
+struct PairParams {
+  const int32_t* pairs;  // [n][2] replica indices of the chunk's pairs
+  int n_state;           // replicas in the state
+};
+
+// replicas (a, b) of pair q; false for a pair the kernels skip (an index outside the state, or a == b)
+__device__ __forceinline__ bool pair_replicas(const PairParams& Q, int q, int& a, int& b) {
+  a = Q.pairs[2 * q];
+  b = Q.pairs[2 * q + 1];
+  return a >= 0 && a < Q.n_state && b >= 0 && b < Q.n_state && a != b;
+}
+
+// Step `sweep` of word (colour, row i, w) of pair q = (a, b): its east and south activation words and its flip word.
+// The hood is linear in the state words (padding bits are 0), so the XOR of the two replicas' hoods is the hood of d.
+__device__ __forceinline__ void houdayer_bond_word(const SweepParams& P, const ClusterParams& C, uint32_t sweep, int q,
+                                                   int a, int b, int colour, int i, int w) {
+  const Geom& g = P.g;
+  const size_t plane = (size_t)g.rows * g.wpr, off = (size_t)i * g.wpr + w;
+  uint32_t* act = cluster_act(C, q) + (size_t)colour * 2 * plane + off;
+  uint32_t* flip = cluster_flip(C, q) + (size_t)colour * plane + off;
+  const uint32_t d = P.state[((size_t)a * 2 + colour) * plane + off] ^ P.state[((size_t)b * 2 + colour) * plane + off];
+  if (d == 0u) {  // no site of the word is in a cluster (padding words included): nothing to activate or flip
+    act[0] = 0u;
+    act[plane] = 0u;
+    *flip = 0u;
+    return;
+  }
+  Planes pl;
+  pl.halo_top = nullptr;
+  pl.halo_bot = nullptr;
+  pl.opp = P.state + ((size_t)a * 2 + (1 - colour)) * plane;
+  const Hood ha = load_hood(pl, g, colour, i, w);
+  pl.opp = P.state + ((size_t)b * 2 + (1 - colour)) * plane;
+  const Hood hb = load_hood(pl, g, colour, i, w);
+  const int p = (g.row0 + i + colour) & 1;
+  act[0] = d & (p ? ha.side ^ hb.side : ha.c ^ hb.c) & ha.valid & ~ha.missE;
+  act[plane] = d & (ha.s ^ hb.s) & ha.valid;  // a missing south neighbour reads 0 in both
+  Coords c;
+  c.colour = (uint32_t)colour;
+  c.sweep = sweep;
+  c.replica = P.replica0 + (uint32_t)a;
+  c.k0 = P.k0;
+  c.k1 = P.k1;
+  *flip = lattice_call(c, (uint32_t)w, (uint32_t)(g.row0 + i), TSU_KIND_HOUDAYER_FLIP).x & ha.valid;
+}
+
+// XORs the flip bit of the cluster root of every site with d = 1 into word (colour, row i, w) of both replicas
+__device__ __forceinline__ void houdayer_flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int q,
+                                                   int a, int b, int colour, int i, int w) {
+  const Geom& g = P.g;
+  const size_t plane = (size_t)g.rows * g.wpr, off = (size_t)i * g.wpr + w;
+  uint32_t* xa = P.state + ((size_t)a * 2 + colour) * plane + off;
+  uint32_t* xb = P.state + ((size_t)b * 2 + colour) * plane + off;
+  const uint32_t d = *xa ^ *xb;
+  if (d == 0u) return;
+  const uint32_t out = root_flip_bits(cluster_flip(C, q), L, g, plane, (g.row0 + i + colour) & 1, i, w, d);
+  *xa ^= out;
+  *xb ^= out;
+}
+
+// One thread per state word of every pair of the chunk (P.g.n_replicas pairs): activation and flip words of step
+// P.sweep.  A skipped pair reads no state; its share gets no active bond, so the labelling passes leave it alone.
+__global__ void __launch_bounds__(kClusterThreads) houdayer_bonds_kernel(SweepParams P, ClusterParams C, PairParams Q) {
+  const Geom& g = P.g;
+  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long per_pair = 2LL * g.rows * g.wpr;
+  if (tid >= per_pair * g.n_replicas) return;
+  const int q = (int)(tid / per_pair);
+  const int rem = (int)(tid - (long long)q * per_pair), colour = rem / (g.rows * g.wpr);
+  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr, w = rw - i * g.wpr;
+  int a, b;
+  if (!pair_replicas(Q, q, a, b)) {
+    const size_t plane = (size_t)g.rows * g.wpr;
+    uint32_t* act = cluster_act(C, q) + (size_t)colour * 2 * plane + rw;
+    act[0] = 0u;
+    act[plane] = 0u;
+    return;
+  }
+  houdayer_bond_word(P, C, P.sweep, q, a, b, colour, i, w);
+}
+
+__global__ void __launch_bounds__(kClusterThreads) houdayer_flip_kernel(SweepParams P, ClusterParams C, PairParams Q) {
+  const Geom& g = P.g;
+  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long per_pair = 2LL * g.rows * g.wpr;
+  if (tid >= per_pair * g.n_replicas) return;
+  const int q = (int)(tid / per_pair);
+  const int rem = (int)(tid - (long long)q * per_pair), colour = rem / (g.rows * g.wpr);
+  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr;
+  int a, b;
+  if (!pair_replicas(Q, q, a, b)) return;
+  houdayer_flip_word(P, C, cluster_labels(C, q), q, a, b, colour, i, rw - i * g.wpr);
+}
+
+// Lattices of at most kClusterResidentSites sites: every step of the call in one launch, one block per pair, the
+// labels in shared memory, as cluster_resident_kernel.
+__global__ void __launch_bounds__(kClusterThreads) houdayer_resident_kernel(SweepParams P, ClusterParams C, PairParams Q,
+                                                                            int n_steps) {
+  extern __shared__ int32_t L[];
+  const Geom& g = P.g;
+  const int q = blockIdx.x, per_rep = g.rows * g.wpr, n_sites = g.rows * g.cols;
+  int a, b;
+  if (!pair_replicas(Q, q, a, b)) return;
+  for (int s = 0; s < n_steps; ++s) {
+    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
+      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
+      houdayer_bond_word(P, C, P.sweep + (uint32_t)s, q, a, b, colour, i, rem - i * g.wpr);
+    }
+    for (int t = threadIdx.x; t < n_sites; t += kClusterThreads) L[t] = t;
+    __syncthreads();
+    cluster_tile_unions(L, cluster_act(C, q), g, 0, g.rows, 0, g.wpr, 0, g.cols);
+    __syncthreads();
+    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
+      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
+      houdayer_flip_word(P, C, L, q, a, b, colour, i, rem - i * g.wpr);
     }
     __syncthreads();  // the next step's bonds read the flipped words
   }
@@ -1855,6 +1987,49 @@ int launch_swendsen_wang(const Lattice& L, const ClusterParams& C, uint32_t swee
   return TSU_OK;
 }
 
+// the work buffer of tsu_ising2d_cluster_work_bytes carved into rep_bytes shares
+ClusterParams cluster_params(void* work, long long rep_bytes, int rows, int cols) {
+  ClusterParams C;
+  C.thresholds = nullptr;
+  C.sign = 1;
+  C.work = static_cast<char*>(work);
+  C.rep_bytes = (size_t)rep_bytes;
+  C.act_offset = (4 * (size_t)rows * cols + 15) / 16 * 16;
+  C.flip_offset = C.act_offset + 16 * (size_t)rows * words_per_row(cols);
+  return C;
+}
+
+// n_steps Houdayer steps of the n_pairs pairs `pairs` of the replicas of L; pair q owns share q of C.work.  The launch
+// paths of launch_swendsen_wang, with the pairs in place of the replicas.
+int launch_houdayer(const Lattice& L, const ClusterParams& C, const int32_t* pairs, int n_pairs, uint32_t sweep0,
+                    int n_steps, cudaStream_t st) {
+  SweepParams P = sweep_params(L, 0, sweep0, nullptr, nullptr);
+  const PairParams Q = {pairs, L.g.n_replicas};
+  P.g.n_replicas = n_pairs;
+  const Geom& g = P.g;
+  if (tuning().resident != 0 && (long long)g.rows * g.cols <= kClusterResidentSites) {
+    const size_t smem = sizeof(int32_t) * (size_t)g.rows * g.cols;
+    houdayer_resident_kernel<<<n_pairs, kClusterThreads, smem, st>>>(P, C, Q, n_steps);
+    TSU_RETURN_LAUNCH_STATUS();
+  }
+  const unsigned word_grid = blocks_for(2LL * g.rows * g.wpr * n_pairs, kClusterThreads);
+  const int tiles_x = (g.cols + kClusterTileCols - 1) / kClusterTileCols;
+  const int tiles_y = (g.rows + kClusterTileRows - 1) / kClusterTileRows;
+  const unsigned merge_grid =
+      blocks_for(((long long)tiles_y * g.cols + (long long)g.rows * tiles_x) * n_pairs, kClusterThreads);
+  for (int s = 0; s < n_steps; ++s) {
+    P.sweep = sweep0 + (uint32_t)s;
+    houdayer_bonds_kernel<<<word_grid, kClusterThreads, 0, st>>>(P, C, Q);
+    cluster_local_kernel<<<(unsigned)((long long)tiles_x * tiles_y * n_pairs), kClusterThreads, 0, st>>>(
+        P, C, tiles_x, tiles_x * tiles_y);
+    cluster_merge_kernel<<<merge_grid, kClusterThreads, 0, st>>>(P, C, tiles_y, tiles_x);
+    houdayer_flip_kernel<<<word_grid, kClusterThreads, 0, st>>>(P, C, Q);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return (int)e;
+  }
+  return TSU_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2166,18 +2341,37 @@ int tsu_ising2d_swendsen_wang(uint32_t* d_state, int n_replicas, int rows, int c
   if (n_steps == 0) return TSU_OK;
   const long long fit = (long long)(work_bytes / (size_t)rep_bytes);
   const int chunk = fit < n_replicas ? (int)fit : n_replicas;
-  ClusterParams C;
+  ClusterParams C = cluster_params(d_work, rep_bytes, rows, cols);
   C.thresholds = reinterpret_cast<const unsigned long long*>(d_thresholds);
   C.sign = coupling_sign;
-  C.work = static_cast<char*>(d_work);
-  C.rep_bytes = (size_t)rep_bytes;
-  C.act_offset = (4 * (size_t)rows * cols + 15) / 16 * 16;
-  C.flip_offset = C.act_offset + 16 * (size_t)rows * L.g.wpr;
   cudaStream_t st = tsu_stream(stream);
   // chunks one after the other, each through all its steps: the bits depend on no chunk size
   for (int r0 = 0; r0 < n_replicas; r0 += chunk) {
     const int rc = launch_swendsen_wang(L.replicas(r0, r0 + chunk < n_replicas ? r0 + chunk : n_replicas), C, sweep0,
                                         n_steps, st);
+    if (rc != TSU_OK) return rc;
+  }
+  return TSU_OK;
+}
+
+int tsu_ising2d_houdayer(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
+                         const int32_t* d_pairs, int n_pairs, uint64_t seed, uint32_t sweep0, int n_steps,
+                         uint32_t replica0, void* d_work, size_t work_bytes, uintptr_t stream) {
+  const Lattice L = {d_state, make_geom(n_replicas, rows, cols, wrap_rows, wrap_cols, 0), nullptr, nullptr, kNoBonds,
+                     seed, replica0, JitKernel{nullptr, 0, 0}};
+  TSU_CHECK_ARG(d_state && d_pairs && d_work && n_steps >= 0 && n_pairs >= 1 && 2LL * n_pairs <= n_replicas);
+  TSU_CHECK_ARG(args_ok(L.g, L.B, false, 0, 0, rows));
+  const long long rep_bytes = cluster_rep_bytes(rows, cols);
+  TSU_CHECK_ARG(rep_bytes > 0 && work_bytes >= (size_t)rep_bytes);
+  if (n_steps == 0) return TSU_OK;
+  const long long fit = (long long)(work_bytes / (size_t)rep_bytes);
+  const int chunk = fit < n_pairs ? (int)fit : n_pairs;
+  const ClusterParams C = cluster_params(d_work, rep_bytes, rows, cols);
+  cudaStream_t st = tsu_stream(stream);
+  // chunks one after the other, each through all its steps: disjoint pairs give bits that depend on no chunk size
+  for (int q0 = 0; q0 < n_pairs; q0 += chunk) {
+    const int rc = launch_houdayer(L, C, d_pairs + 2 * (size_t)q0, q0 + chunk < n_pairs ? chunk : n_pairs - q0, sweep0,
+                                   n_steps, st);
     if (rc != TSU_OK) return rc;
   }
   return TSU_OK;

@@ -105,6 +105,7 @@ __host__ __device__ __forceinline__ tsu_u32x4 tsu_philox4x32_10_keyed(uint32_t c
 //   kind 3    : population annealing, one call per population and step (w = colour = row = 0, replica = the
 //               population's first replica, sweep = the step's first sweep; words x | y << 32 are the 64-bit draw)
 //   kind 4    : Swendsen-Wang cluster flips: bit b of word x of the call of the cluster root's word (as kind 2)
+//   kind 5    : Houdayer cluster flips, as kind 4 (replica = the pair's first replica)
 //   kind 8-15 : low 24 bits, one call per group of 4 lanes (lane b uses word b&3 of call 8+(b>>2))
 //   kind 16,17 / 24-31 : Swendsen-Wang east-bond uniforms (bit-planes / low 24 bits, as kinds 0,1 / 8-15)
 //   kind 18,19 / 32-39 : Swendsen-Wang south-bond uniforms (bit-planes / low 24 bits, as kinds 0,1 / 8-15)
@@ -119,6 +120,7 @@ __host__ __device__ __forceinline__ tsu_u32x4 tsu_philox4x32_10_keyed(uint32_t c
 #define TSU_KIND_RESAMPLE 3u
 #define TSU_KIND_LOW0 8u
 #define TSU_KIND_CLUSTER_FLIP 4u
+#define TSU_KIND_HOUDAYER_FLIP 5u
 #define TSU_KIND_BOND_E_PLANE0 16u
 #define TSU_KIND_BOND_S_PLANE0 18u
 #define TSU_KIND_BOND_E_LOW0 24u

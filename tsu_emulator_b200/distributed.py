@@ -392,15 +392,30 @@ class LatticeTempering:
     the engine of this rank's replica range; swap_fn(energy, T_slot, slot_replica, lut_index, K, R, step)
     performs the pass in place (tsu_pt_swap on GPUs).  criterion="metropolis" (default) is the detailed-balance
     rule; "reference" reproduces the expression of gibbs.py:317 (see include/tsu_b200.h).
+
+    houdayer_interval = k > 0: every k iterations one Houdayer cluster move (Ising2DEngine.houdayer) runs after the
+    sweeps and before the exchange pass, pairing ladders 2m and 2m+1 at every temperature slot (pairs built on the
+    device from slot_replica, no host sync).  It needs an even n_ladders, one process, and the same bond realisation
+    for every replica of ladders 2m and 2m+1.  0 (default): no cluster moves.
     """
 
     def __init__(self, temperatures: Sequence[float], n_ladders: int, engine_factory, swap_fn=None, group=None,
-                 n_sweeps: int = 10, swap_interval: int = 10, seed: int = 0, criterion: str = "metropolis"):
+                 n_sweeps: int = 10, swap_interval: int = 10, seed: int = 0, criterion: str = "metropolis",
+                 houdayer_interval: int = 0):
         import torch
 
         dist = _dist()
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
+        if (isinstance(houdayer_interval, bool) or not isinstance(houdayer_interval, (int, np.integer))
+                or houdayer_interval < 0):
+            raise ValueError("houdayer_interval must be a non-negative integer")
+        self.houdayer_interval = int(houdayer_interval)
+        if self.houdayer_interval:
+            if int(n_ladders) % 2:
+                raise ValueError("houdayer_interval needs an even n_ladders: ladders 2m and 2m+1 are paired")
+            if self.world != 1:
+                raise ValueError("houdayer_interval needs one process: ladder pairs are not split across ranks")
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.temps = np.asarray(list(temperatures), dtype=np.float64)
         self.R, self.K = len(self.temps), int(n_ladders)
@@ -421,6 +436,13 @@ class LatticeTempering:
         self.swap_fn = swap_fn or self._swap_cuda
         # the engine's LUT tables must be ordered by slot: one table per temperature of the ladder
         self.engine.set_temperature_tables(self.temps, self.lut_index[self.start:self.stop])
+        if self.houdayer_interval:
+            self.engine._houdayer_supported()
+            if self.engine.bond_index is not None:
+                bi = np.asarray(self.engine.bond_index.cpu()).reshape(self.K // 2, 2 * self.R)
+                if np.any(bi != bi[:, :1]):
+                    raise ValueError("houdayer_interval needs one bond realisation for all replicas of ladders 2m "
+                                     "and 2m+1")
 
     def _swap_cuda(self, energy, T_slot, slot_replica, lut_index, K, R, step):
         from . import _lib
@@ -442,9 +464,16 @@ class LatticeTempering:
         return torch.cat(parts)
 
     def step(self):
-        """one iteration: n_sweeps sweeps, then (every swap_interval iterations) the exchange pass"""
+        """one iteration: n_sweeps sweeps, then (every houdayer_interval iterations) one Houdayer move, then (every
+        swap_interval iterations) the exchange pass"""
         self.engine.sweep(self.n_sweeps)
         self.iteration += 1
+        if self.houdayer_interval and self.iteration % self.houdayer_interval == 0:
+            import torch
+
+            sr = self.slot_replica
+            pairs = torch.stack((sr[0::2], sr[1::2]), dim=-1).reshape(-1, 2)  # (ladder 2m, ladder 2m+1) per slot
+            self.engine._houdayer(pairs, pairs.shape[0], 1)
         if self.iteration % self.swap_interval == 0:
             energy = self.gather_energies()
             self.swap_fn(energy, self.T_slot, self.slot_replica, self.lut_index, self.K, self.R, self.iteration)

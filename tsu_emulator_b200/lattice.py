@@ -677,12 +677,7 @@ class Ising2DEngine:
             return self
         torch = self._torch
         with torch.cuda.device(self.device):
-            work = self.__dict__.get("_cluster_work")
-            if work is None:
-                per_rep = int(self.lib.tsu_ising2d_cluster_work_bytes(1, self.rows, self.cols))
-                n_work = min(self.n_replicas, max(1, CLUSTER_WORK_BUDGET // per_rep))
-                work = torch.empty(n_work * per_rep // 8, dtype=torch.int64, device=self.device)
-                self._cluster_work = work
+            work = self._cluster_workspace(self.n_replicas)
             key = (self.coupling, np.asarray(self._lut_temps).tobytes())
             cached = self.__dict__.get("_cluster_tables")
             if cached is None or cached[0] != key:
@@ -695,6 +690,80 @@ class Ising2DEngine:
                 -1 if self.coupling < 0 else 1, ptr(self.bonds), ptr(self.bond_index), self.seed,
                 self.sweep_index & 0xFFFFFFFF, n_steps, self.replica0, ptr(work), work.numel() * 8,
                 _lib.current_stream(),
+            )
+        self.sweep_index += n_steps
+        return self
+
+    def _cluster_workspace(self, n_shares: int):
+        """the cluster workspace shared by swendsen_wang and houdayer: room for min(n_shares, CLUSTER_WORK_BUDGET //
+        bytes per share) replicas or pairs (at least one); reallocated only when a call needs more shares"""
+        per_rep = int(self.lib.tsu_ising2d_cluster_work_bytes(1, self.rows, self.cols))
+        need = min(n_shares, max(1, CLUSTER_WORK_BUDGET // per_rep)) * per_rep
+        work = self.__dict__.get("_cluster_work")
+        if work is None or work.numel() * 8 < need:
+            work = self._torch.empty(need // 8, dtype=self._torch.int64, device=self.device)
+            self._cluster_work = work
+        return work
+
+    def houdayer(self, pairs, n_steps: int = 1):
+        """n_steps Houdayer cluster moves of every replica pair in `pairs` in one call.
+
+        `pairs` is an integer array [n_pairs, 2] of disjoint pairs (a, b) of this engine's replicas; the two replicas
+        of a pair must share the temperature and the bond realisation.  A step takes the sites where the two differ,
+        labels the clusters that bonds between such sites form and flips each cluster in both replicas with
+        probability 1/2 (tsu_ising2d_houdayer states the exact random stream).  E_a + E_b and q_ab are unchanged and
+        the product of the two Boltzmann distributions is kept, for any bonds and any field; each replica's own
+        energy changes, which at low temperature moves a 2-D spin glass between valleys far faster than sweep().
+        The move keeps the set of differing sites, so it is not ergodic alone: alternate it with sweep().  Afterwards
+        sweep_index has advanced by n_steps.
+
+        bias_mode "physical" and whole lattices only; a field is allowed.  Shares the Swendsen-Wang workspace (one
+        replica's share per pair, CLUSTER_WORK_BUDGET at most); more pairs run in chunks, with the same bits.  Every
+        argument is checked on the host before any device work (with bonds, bond_index is read back for that);
+        LatticeTempering(houdayer_interval=k) runs the move with pairs built on the device and no host sync.
+        """
+        self._houdayer_supported()
+        if isinstance(n_steps, bool) or not isinstance(n_steps, (int, np.integer)) or n_steps < 0:
+            raise ValueError("n_steps must be a non-negative integer")
+        pr = np.asarray(pairs)
+        if pr.ndim != 2 or pr.shape[1] != 2 or pr.shape[0] < 1 or not np.issubdtype(pr.dtype, np.integer):
+            raise ValueError("pairs must be integers of shape [n_pairs, 2]")
+        if np.any(pr < 0) or np.any(pr >= self.n_replicas):
+            raise ValueError(f"pair indices must lie in [0, {self.n_replicas})")
+        if np.any(pr[:, 0] == pr[:, 1]):
+            raise ValueError("a pair needs two different replicas")
+        if np.unique(pr).size != pr.size:
+            raise ValueError("pairs must be disjoint: a replica appears twice")
+        temps = np.broadcast_to(np.asarray(self.temperatures, dtype=np.float64), (self.n_replicas,))
+        if np.any(temps[pr[:, 0]] != temps[pr[:, 1]]):
+            raise ValueError("the replicas of a pair need the same temperature")
+        if self.bond_index is not None:
+            bi = np.asarray(self.bond_index.cpu())
+            if np.any(bi[pr[:, 0]] != bi[pr[:, 1]]):
+                raise ValueError("the replicas of a pair need the same bond realisation (bond_index)")
+        if n_steps == 0:
+            return self
+        with self._torch.cuda.device(self.device):
+            dev = self._torch.from_numpy(np.ascontiguousarray(pr.astype(np.int32))).to(self.device)
+        return self._houdayer(dev, int(pr.shape[0]), int(n_steps))
+
+    def _houdayer_supported(self):
+        """the engine rules of houdayer(), also checked once by LatticeTempering(houdayer_interval > 0)"""
+        if self.bias_mode != "physical":
+            raise ValueError("Houdayer moves need bias_mode='physical': the reference bias does not sample exp(-E/T)")
+        if self.is_slab:
+            raise ValueError("Houdayer moves need whole lattices; row-slab engines cannot run them")
+        if self.rows * self.cols >= 1 << 31:
+            raise ValueError("Houdayer cluster labels are int32: rows * cols must stay below 2^31")
+
+    def _houdayer(self, pairs, n_pairs: int, n_steps: int):
+        """houdayer() on validated device pairs (int32 [n_pairs, 2]); no check, no host sync"""
+        with self._torch.cuda.device(self.device):
+            work = self._cluster_workspace(n_pairs)
+            _lib.call(
+                "tsu_ising2d_houdayer", ptr(self.state), self.n_replicas, self.rows, self.cols, int(self.wrap_rows),
+                int(self.wrap_cols), ptr(pairs), n_pairs, self.seed, self.sweep_index & 0xFFFFFFFF, n_steps,
+                self.replica0, ptr(work), work.numel() * 8, _lib.current_stream(),
             )
         self.sweep_index += n_steps
         return self
