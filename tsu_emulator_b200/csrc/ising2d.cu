@@ -946,22 +946,21 @@ __global__ void __launch_bounds__(256) pa_gather_kernel(const uint4* __restrict_
   }
 }
 
-// ---- Swendsen-Wang cluster updates (tsu_ising2d_swendsen_wang) ------------------------------------------------
-// Per replica the caller's work buffer holds (ClusterParams::rep_bytes apart) labels int32 [rows * cols] (site index
-// row * cols + col, padded to 16 bytes), the activation words uint32 [2 colours][east, south][rows][wpr] and the flip
-// words uint32 [2 colours][rows][wpr], both in the layout of the state.  Labels form a union-find forest in which a
-// site's parent never has a larger index; unions always hang the larger root under the smaller, so every tree's root
-// is its cluster's smallest site index, whatever order the unions run in.
+// ---- cluster moves: Swendsen-Wang (tsu_ising2d_swendsen_wang) and Houdayer (tsu_ising2d_houdayer) ------------------
+// A move runs on units (a replica for Swendsen-Wang, a pair of replicas for Houdayer).  Per unit the caller's work
+// buffer holds (ClusterParams::rep_bytes apart) labels int32 [rows * cols] (site index row * cols + col, padded to 16
+// bytes), the activation words uint32 [2 colours][east, south][rows][wpr] and the flip words uint32 [2 colours][rows]
+// [wpr], both in the layout of the state.  Labels form a union-find forest in which a site's parent never has a larger
+// index; unions always hang the larger root under the smaller, so every tree's root is its cluster's smallest site
+// index, whatever order the unions run in.
 constexpr int kClusterThreads = 256;
 constexpr int kClusterTileRows = 32, kClusterTileWords = 4;  // tiles of the local pass: 32 rows x 256 columns
 constexpr int kClusterTileCols = 64 * kClusterTileWords;
-constexpr int kClusterResidentSites = 12288;  // labels of a replica in 48 KB of shared memory: one launch per call
+constexpr int kClusterResidentSites = 12288;  // labels of a unit in 48 KB of shared memory: one launch per call
 
 struct ClusterParams {
-  const unsigned long long* thresholds;  // [n_tables] t = ceil(p 2^32), p = 1 - exp(-2|J|/T); 2^32: always active
-  int sign;                              // sign of J: +1 satisfied = aligned (after the bond sign), -1 anti-aligned
   char* work;
-  size_t rep_bytes, act_offset, flip_offset;  // per replica: its share of the work buffer, where its words start
+  size_t rep_bytes, act_offset, flip_offset;  // per unit: its share of the work buffer, where its words start
 };
 
 __device__ __forceinline__ int32_t* cluster_labels(const ClusterParams& C, int rep) {
@@ -1003,46 +1002,6 @@ __device__ __forceinline__ uint32_t activate_bonds(uint32_t sat, unsigned long l
     lt = (lt & ~(1u << j)) | (bit << j);
   }
   return lt & sat;
-}
-
-// Step `sweep` of word (rep, colour, row i, w): its east and south activation words and its flip word.  The hood's
-// neighbour words carry the bond signs (apply_bonds), so x ^ neighbour is 1 where sigma s_i s_j = -1, as count_word counts.
-template <bool BONDED>
-__device__ __forceinline__ void cluster_bond_word(const SweepParams& P, const BondParams& B, const ClusterParams& C,
-                                                  uint32_t sweep, int rep, int colour, int i, int w) {
-  const Geom& g = P.g;
-  const size_t plane = (size_t)g.rows * g.wpr;
-  Planes pl;
-  pl.opp = P.state + ((size_t)rep * 2 + (1 - colour)) * plane;
-  pl.halo_top = nullptr;
-  pl.halo_bot = nullptr;
-  Hood h = load_hood(pl, g, colour, i, w);
-  const size_t off = (size_t)i * g.wpr + w;
-  uint32_t* act = cluster_act(C, rep) + (size_t)colour * 2 * plane + off;
-  uint32_t* flip = cluster_flip(C, rep) + (size_t)colour * plane + off;
-  if (h.valid == 0u) {  // padding word
-    act[0] = 0u;
-    act[plane] = 0u;
-    *flip = 0u;
-    return;
-  }
-  if constexpr (BONDED) apply_bonds(h, B, g, rep, colour, i, w);
-  const uint32_t x = P.state[((size_t)rep * 2 + colour) * plane + off];
-  const int p = (g.row0 + i + colour) & 1;
-  const uint32_t aligned = C.sign > 0 ? 0xffffffffu : 0u;
-  const uint32_t sat_e = (x ^ (p ? h.side : h.c) ^ aligned) & h.valid & ~h.missE;
-  const uint32_t sat_s = h.has_s ? (x ^ h.s ^ aligned) & h.valid : 0u;
-  Coords q;
-  q.colour = (uint32_t)colour;
-  q.sweep = sweep;
-  q.replica = P.replica0 + (uint32_t)rep;
-  q.k0 = P.k0;
-  q.k1 = P.k1;
-  const unsigned long long t = C.thresholds[P.lut_index ? P.lut_index[rep] : 0];
-  const uint32_t row_g = (uint32_t)(g.row0 + i);
-  act[0] = activate_bonds(sat_e, t, q, (uint32_t)w, row_g, TSU_KIND_BOND_E_PLANE0, TSU_KIND_BOND_E_LOW0);
-  act[plane] = activate_bonds(sat_s, t, q, (uint32_t)w, row_g, TSU_KIND_BOND_S_PLANE0, TSU_KIND_BOND_S_LOW0);
-  *flip = lattice_call(q, (uint32_t)w, row_g, TSU_KIND_CLUSTER_FLIP).x & h.valid;
 }
 
 // root of x, halving the path on the way (every site then points at its former grandparent).  A label only ever
@@ -1123,30 +1082,170 @@ __device__ __forceinline__ uint32_t root_flip_bits(const uint32_t* flip, int32_t
   return out;
 }
 
-// XORs into word (rep, colour, row i, w) the flip bit of every site's cluster root
-__device__ __forceinline__ void cluster_flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int rep,
-                                                  int colour, int i, int w) {
-  const Geom& g = P.g;
-  const int p = (g.row0 + i + colour) & 1;
-  uint32_t m = lane_mask_lt(colour_count(g.cols, p) - 32 * w);
-  if (m == 0u) return;
-  const size_t plane = (size_t)g.rows * g.wpr;
-  const uint32_t* flip = cluster_flip(C, rep);
-  const uint32_t out = root_flip_bits(flip, L, g, plane, p, i, w, m);
-  P.state[((size_t)rep * 2 + colour) * plane + (size_t)i * g.wpr + w] ^= out;
-}
+// The kernels below run a move on units u = 0 .. P.g.n_replicas - 1, unit u owning share u of the work buffer.  A
+// move is passed to them by value and supplies:
+//   unit(u, a, b)        the replicas a, b unit u reads and writes; false for a unit the kernels skip
+//   bond_word(.., sweep, u, a, b, colour, i, w)   step `sweep` of word (colour, row i, w) of unit u: its east and south
+//                        activation words and its flip word
+//   flip_word(.., L, u, a, b, colour, i, w)       XORs into word (colour, row i, w) of the unit's replicas the flip bit
+//                        of every cluster root, L being the unit's label forest
+//   narrow(P, u0)        on the host: P and the move from unit u0 on (the caller sets P.g.n_replicas)
 
-// One thread per state word of every replica: activation and flip words of step P.sweep.
+// Swendsen-Wang: unit rep is replica rep, never skipped.
 template <bool BONDED>
-__global__ void __launch_bounds__(kClusterThreads) cluster_bonds_kernel(SweepParams P, BondParams B, ClusterParams C) {
+struct SwMove {
+  BondParams B;
+  const unsigned long long* thresholds;  // [n_tables] t = ceil(p 2^32), p = 1 - exp(-2|J|/T); 2^32: always active
+  int sign;                              // sign of J: +1 satisfied = aligned (after the bond sign), -1 anti-aligned
+
+  __device__ __forceinline__ bool unit(int rep, int& a, int& b) const {
+    a = b = rep;
+    return true;
+  }
+
+  // The hood's neighbour words carry the bond signs (apply_bonds), so x ^ neighbour is 1 where sigma s_i s_j = -1, as
+  // count_word counts.
+  __device__ __forceinline__ void bond_word(const SweepParams& P, const ClusterParams& C, uint32_t sweep, int rep, int,
+                                            int, int colour, int i, int w) const {
+    const Geom& g = P.g;
+    const size_t plane = (size_t)g.rows * g.wpr;
+    Planes pl;
+    pl.opp = P.state + ((size_t)rep * 2 + (1 - colour)) * plane;
+    pl.halo_top = nullptr;
+    pl.halo_bot = nullptr;
+    Hood h = load_hood(pl, g, colour, i, w);
+    const size_t off = (size_t)i * g.wpr + w;
+    uint32_t* act = cluster_act(C, rep) + (size_t)colour * 2 * plane + off;
+    uint32_t* flip = cluster_flip(C, rep) + (size_t)colour * plane + off;
+    if (h.valid == 0u) {  // padding word
+      act[0] = 0u;
+      act[plane] = 0u;
+      *flip = 0u;
+      return;
+    }
+    if constexpr (BONDED) apply_bonds(h, B, g, rep, colour, i, w);
+    const uint32_t x = P.state[((size_t)rep * 2 + colour) * plane + off];
+    const int p = (g.row0 + i + colour) & 1;
+    const uint32_t aligned = sign > 0 ? 0xffffffffu : 0u;
+    const uint32_t sat_e = (x ^ (p ? h.side : h.c) ^ aligned) & h.valid & ~h.missE;
+    const uint32_t sat_s = h.has_s ? (x ^ h.s ^ aligned) & h.valid : 0u;
+    Coords q;
+    q.colour = (uint32_t)colour;
+    q.sweep = sweep;
+    q.replica = P.replica0 + (uint32_t)rep;
+    q.k0 = P.k0;
+    q.k1 = P.k1;
+    const unsigned long long t = thresholds[P.lut_index ? P.lut_index[rep] : 0];
+    const uint32_t row_g = (uint32_t)(g.row0 + i);
+    act[0] = activate_bonds(sat_e, t, q, (uint32_t)w, row_g, TSU_KIND_BOND_E_PLANE0, TSU_KIND_BOND_E_LOW0);
+    act[plane] = activate_bonds(sat_s, t, q, (uint32_t)w, row_g, TSU_KIND_BOND_S_PLANE0, TSU_KIND_BOND_S_LOW0);
+    *flip = lattice_call(q, (uint32_t)w, row_g, TSU_KIND_CLUSTER_FLIP).x & h.valid;
+  }
+
+  __device__ __forceinline__ void flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int rep, int, int,
+                                            int colour, int i, int w) const {
+    const Geom& g = P.g;
+    const int p = (g.row0 + i + colour) & 1;
+    uint32_t m = lane_mask_lt(colour_count(g.cols, p) - 32 * w);
+    if (m == 0u) return;
+    const size_t plane = (size_t)g.rows * g.wpr;
+    const uint32_t* flip = cluster_flip(C, rep);
+    const uint32_t out = root_flip_bits(flip, L, g, plane, p, i, w, m);
+    P.state[((size_t)rep * 2 + colour) * plane + (size_t)i * g.wpr + w] ^= out;
+  }
+
+  // what Lattice::replicas() narrows
+  void narrow(SweepParams& P, int u0) {
+    P.state += (size_t)u0 * 2 * P.g.rows * P.g.wpr;
+    if (P.lut_index) P.lut_index += u0;
+    if (B.index) B.index += u0;
+    P.replica0 += (uint32_t)u0;
+  }
+};
+
+// Houdayer: unit q is the pair (a, b) = (pairs[2q], pairs[2q + 1]).  Its activation words hold the bonds whose two
+// sites both have d = x^a xor x^b = 1; its flip words the kind-5 bits.
+struct HoudayerMove {
+  const int32_t* pairs;  // [n][2] replica indices of the launch's pairs
+  int n_state;           // replicas in the state
+
+  // false for a pair the kernels skip (an index outside the state, or a == b)
+  __device__ __forceinline__ bool unit(int q, int& a, int& b) const {
+    a = pairs[2 * q];
+    b = pairs[2 * q + 1];
+    return a >= 0 && a < n_state && b >= 0 && b < n_state && a != b;
+  }
+
+  // The hood is linear in the state words (padding bits are 0), so the XOR of the two replicas' hoods is the hood of d.
+  __device__ __forceinline__ void bond_word(const SweepParams& P, const ClusterParams& C, uint32_t sweep, int q, int a,
+                                            int b, int colour, int i, int w) const {
+    const Geom& g = P.g;
+    const size_t plane = (size_t)g.rows * g.wpr, off = (size_t)i * g.wpr + w;
+    uint32_t* act = cluster_act(C, q) + (size_t)colour * 2 * plane + off;
+    uint32_t* flip = cluster_flip(C, q) + (size_t)colour * plane + off;
+    const uint32_t d = P.state[((size_t)a * 2 + colour) * plane + off] ^ P.state[((size_t)b * 2 + colour) * plane + off];
+    if (d == 0u) {  // no site of the word is in a cluster (padding words included): nothing to activate or flip
+      act[0] = 0u;
+      act[plane] = 0u;
+      *flip = 0u;
+      return;
+    }
+    Planes pl;
+    pl.halo_top = nullptr;
+    pl.halo_bot = nullptr;
+    pl.opp = P.state + ((size_t)a * 2 + (1 - colour)) * plane;
+    const Hood ha = load_hood(pl, g, colour, i, w);
+    pl.opp = P.state + ((size_t)b * 2 + (1 - colour)) * plane;
+    const Hood hb = load_hood(pl, g, colour, i, w);
+    const int p = (g.row0 + i + colour) & 1;
+    act[0] = d & (p ? ha.side ^ hb.side : ha.c ^ hb.c) & ha.valid & ~ha.missE;
+    act[plane] = d & (ha.s ^ hb.s) & ha.valid;  // a missing south neighbour reads 0 in both
+    Coords c;
+    c.colour = (uint32_t)colour;
+    c.sweep = sweep;
+    c.replica = P.replica0 + (uint32_t)a;
+    c.k0 = P.k0;
+    c.k1 = P.k1;
+    *flip = lattice_call(c, (uint32_t)w, (uint32_t)(g.row0 + i), TSU_KIND_HOUDAYER_FLIP).x & ha.valid;
+  }
+
+  // only the sites with d = 1 are in a cluster; both replicas flip by the same mask
+  __device__ __forceinline__ void flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int q, int a,
+                                            int b, int colour, int i, int w) const {
+    const Geom& g = P.g;
+    const size_t plane = (size_t)g.rows * g.wpr, off = (size_t)i * g.wpr + w;
+    uint32_t* xa = P.state + ((size_t)a * 2 + colour) * plane + off;
+    uint32_t* xb = P.state + ((size_t)b * 2 + colour) * plane + off;
+    const uint32_t d = *xa ^ *xb;
+    if (d == 0u) return;
+    const uint32_t out = root_flip_bits(cluster_flip(C, q), L, g, plane, (g.row0 + i + colour) & 1, i, w, d);
+    *xa ^= out;
+    *xb ^= out;
+  }
+
+  void narrow(SweepParams&, int q0) { pairs += 2 * (size_t)q0; }
+};
+
+// One thread per state word of every unit: activation and flip words of step P.sweep.  A skipped unit reads no state;
+// its share gets no active bond, so the labelling passes leave it alone.
+template <class Move>
+__global__ void __launch_bounds__(kClusterThreads) cluster_bonds_kernel(SweepParams P, ClusterParams C, Move M) {
   const Geom& g = P.g;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long per_rep = 2LL * g.rows * g.wpr;
-  if (tid >= per_rep * g.n_replicas) return;
-  const int rep = (int)(tid / per_rep);
-  const int rem = (int)(tid - (long long)rep * per_rep), colour = rem / (g.rows * g.wpr);
-  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr;
-  cluster_bond_word<BONDED>(P, B, C, P.sweep, rep, colour, i, rw - i * g.wpr);
+  const long long per_unit = 2LL * g.rows * g.wpr;
+  if (tid >= per_unit * g.n_replicas) return;
+  const int u = (int)(tid / per_unit);
+  const int rem = (int)(tid - (long long)u * per_unit), colour = rem / (g.rows * g.wpr);
+  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr, w = rw - i * g.wpr;
+  int a, b;
+  if (!M.unit(u, a, b)) {
+    const size_t plane = (size_t)g.rows * g.wpr;
+    uint32_t* act = cluster_act(C, u) + (size_t)colour * 2 * plane + rw;
+    act[0] = 0u;
+    act[plane] = 0u;
+    return;
+  }
+  M.bond_word(P, C, P.sweep, u, a, b, colour, i, w);
 }
 
 // One block per tile of kClusterTileRows x kClusterTileCols sites: unions in shared memory, then every site's label is
@@ -1209,162 +1308,44 @@ __global__ void __launch_bounds__(kClusterThreads) cluster_merge_kernel(SweepPar
     cluster_union(cluster_labels(C, rep), i * g.cols + col, ni * g.cols + ncol);
 }
 
-__global__ void __launch_bounds__(kClusterThreads) cluster_flip_kernel(SweepParams P, ClusterParams C) {
+template <class Move>
+__global__ void __launch_bounds__(kClusterThreads) cluster_flip_kernel(SweepParams P, ClusterParams C, Move M) {
   const Geom& g = P.g;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long per_rep = 2LL * g.rows * g.wpr;
-  if (tid >= per_rep * g.n_replicas) return;
-  const int rep = (int)(tid / per_rep);
-  const int rem = (int)(tid - (long long)rep * per_rep), colour = rem / (g.rows * g.wpr);
+  const long long per_unit = 2LL * g.rows * g.wpr;
+  if (tid >= per_unit * g.n_replicas) return;
+  const int u = (int)(tid / per_unit);
+  const int rem = (int)(tid - (long long)u * per_unit), colour = rem / (g.rows * g.wpr);
   const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr;
-  cluster_flip_word(P, C, cluster_labels(C, rep), rep, colour, i, rw - i * g.wpr);
+  int a, b;
+  if (!M.unit(u, a, b)) return;
+  M.flip_word(P, C, cluster_labels(C, u), u, a, b, colour, i, rw - i * g.wpr);
 }
 
-// Lattices of at most kClusterResidentSites sites: every step of the call in one launch, one block per replica, the
+// Lattices of at most kClusterResidentSites sites: every step of the call in one launch, one block per unit, the
 // labels in shared memory (the whole lattice is one tile of cluster_tile_unions).  The activation and flip words go
-// through the work buffer; the block's barriers make its own global stores visible to it.
-template <bool BONDED>
-__global__ void __launch_bounds__(kClusterThreads) cluster_resident_kernel(SweepParams P, BondParams B, ClusterParams C,
+// through the work buffer; the block's barriers make its own global stores visible to it.  A skipped unit's block
+// leaves before its first barrier.
+template <class Move>
+__global__ void __launch_bounds__(kClusterThreads) cluster_resident_kernel(SweepParams P, ClusterParams C, Move M,
                                                                            int n_steps) {
   extern __shared__ int32_t L[];
   const Geom& g = P.g;
-  const int rep = blockIdx.x, per_rep = g.rows * g.wpr, n_sites = g.rows * g.cols;
+  const int u = blockIdx.x, per_unit = g.rows * g.wpr, n_sites = g.rows * g.cols;
+  int a, b;
+  if (!M.unit(u, a, b)) return;
   for (int s = 0; s < n_steps; ++s) {
-    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
-      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
-      cluster_bond_word<BONDED>(P, B, C, P.sweep + (uint32_t)s, rep, colour, i, rem - i * g.wpr);
+    for (int t = threadIdx.x; t < 2 * per_unit; t += kClusterThreads) {
+      const int colour = t / per_unit, rem = t - colour * per_unit, i = rem / g.wpr;
+      M.bond_word(P, C, P.sweep + (uint32_t)s, u, a, b, colour, i, rem - i * g.wpr);
     }
     for (int t = threadIdx.x; t < n_sites; t += kClusterThreads) L[t] = t;
     __syncthreads();
-    cluster_tile_unions(L, cluster_act(C, rep), g, 0, g.rows, 0, g.wpr, 0, g.cols);
+    cluster_tile_unions(L, cluster_act(C, u), g, 0, g.rows, 0, g.wpr, 0, g.cols);
     __syncthreads();
-    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
-      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
-      cluster_flip_word(P, C, L, rep, colour, i, rem - i * g.wpr);
-    }
-    __syncthreads();  // the next step's bonds read the flipped words
-  }
-}
-
-// ---- Houdayer cluster moves (tsu_ising2d_houdayer) ----------------------------------------------------------
-// Pair q of a chunk owns share q of the Swendsen-Wang work buffer (same layout) and runs the same labelling kernels,
-// with the pair index in place of the replica index.  Its activation words hold the bonds whose two sites both have
-// d = x^a xor x^b = 1; its flip words the kind-5 bits.
-struct PairParams {
-  const int32_t* pairs;  // [n][2] replica indices of the chunk's pairs
-  int n_state;           // replicas in the state
-};
-
-// replicas (a, b) of pair q; false for a pair the kernels skip (an index outside the state, or a == b)
-__device__ __forceinline__ bool pair_replicas(const PairParams& Q, int q, int& a, int& b) {
-  a = Q.pairs[2 * q];
-  b = Q.pairs[2 * q + 1];
-  return a >= 0 && a < Q.n_state && b >= 0 && b < Q.n_state && a != b;
-}
-
-// Step `sweep` of word (colour, row i, w) of pair q = (a, b): its east and south activation words and its flip word.
-// The hood is linear in the state words (padding bits are 0), so the XOR of the two replicas' hoods is the hood of d.
-__device__ __forceinline__ void houdayer_bond_word(const SweepParams& P, const ClusterParams& C, uint32_t sweep, int q,
-                                                   int a, int b, int colour, int i, int w) {
-  const Geom& g = P.g;
-  const size_t plane = (size_t)g.rows * g.wpr, off = (size_t)i * g.wpr + w;
-  uint32_t* act = cluster_act(C, q) + (size_t)colour * 2 * plane + off;
-  uint32_t* flip = cluster_flip(C, q) + (size_t)colour * plane + off;
-  const uint32_t d = P.state[((size_t)a * 2 + colour) * plane + off] ^ P.state[((size_t)b * 2 + colour) * plane + off];
-  if (d == 0u) {  // no site of the word is in a cluster (padding words included): nothing to activate or flip
-    act[0] = 0u;
-    act[plane] = 0u;
-    *flip = 0u;
-    return;
-  }
-  Planes pl;
-  pl.halo_top = nullptr;
-  pl.halo_bot = nullptr;
-  pl.opp = P.state + ((size_t)a * 2 + (1 - colour)) * plane;
-  const Hood ha = load_hood(pl, g, colour, i, w);
-  pl.opp = P.state + ((size_t)b * 2 + (1 - colour)) * plane;
-  const Hood hb = load_hood(pl, g, colour, i, w);
-  const int p = (g.row0 + i + colour) & 1;
-  act[0] = d & (p ? ha.side ^ hb.side : ha.c ^ hb.c) & ha.valid & ~ha.missE;
-  act[plane] = d & (ha.s ^ hb.s) & ha.valid;  // a missing south neighbour reads 0 in both
-  Coords c;
-  c.colour = (uint32_t)colour;
-  c.sweep = sweep;
-  c.replica = P.replica0 + (uint32_t)a;
-  c.k0 = P.k0;
-  c.k1 = P.k1;
-  *flip = lattice_call(c, (uint32_t)w, (uint32_t)(g.row0 + i), TSU_KIND_HOUDAYER_FLIP).x & ha.valid;
-}
-
-// XORs the flip bit of the cluster root of every site with d = 1 into word (colour, row i, w) of both replicas
-__device__ __forceinline__ void houdayer_flip_word(const SweepParams& P, const ClusterParams& C, int32_t* L, int q,
-                                                   int a, int b, int colour, int i, int w) {
-  const Geom& g = P.g;
-  const size_t plane = (size_t)g.rows * g.wpr, off = (size_t)i * g.wpr + w;
-  uint32_t* xa = P.state + ((size_t)a * 2 + colour) * plane + off;
-  uint32_t* xb = P.state + ((size_t)b * 2 + colour) * plane + off;
-  const uint32_t d = *xa ^ *xb;
-  if (d == 0u) return;
-  const uint32_t out = root_flip_bits(cluster_flip(C, q), L, g, plane, (g.row0 + i + colour) & 1, i, w, d);
-  *xa ^= out;
-  *xb ^= out;
-}
-
-// One thread per state word of every pair of the chunk (P.g.n_replicas pairs): activation and flip words of step
-// P.sweep.  A skipped pair reads no state; its share gets no active bond, so the labelling passes leave it alone.
-__global__ void __launch_bounds__(kClusterThreads) houdayer_bonds_kernel(SweepParams P, ClusterParams C, PairParams Q) {
-  const Geom& g = P.g;
-  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long per_pair = 2LL * g.rows * g.wpr;
-  if (tid >= per_pair * g.n_replicas) return;
-  const int q = (int)(tid / per_pair);
-  const int rem = (int)(tid - (long long)q * per_pair), colour = rem / (g.rows * g.wpr);
-  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr, w = rw - i * g.wpr;
-  int a, b;
-  if (!pair_replicas(Q, q, a, b)) {
-    const size_t plane = (size_t)g.rows * g.wpr;
-    uint32_t* act = cluster_act(C, q) + (size_t)colour * 2 * plane + rw;
-    act[0] = 0u;
-    act[plane] = 0u;
-    return;
-  }
-  houdayer_bond_word(P, C, P.sweep, q, a, b, colour, i, w);
-}
-
-__global__ void __launch_bounds__(kClusterThreads) houdayer_flip_kernel(SweepParams P, ClusterParams C, PairParams Q) {
-  const Geom& g = P.g;
-  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long per_pair = 2LL * g.rows * g.wpr;
-  if (tid >= per_pair * g.n_replicas) return;
-  const int q = (int)(tid / per_pair);
-  const int rem = (int)(tid - (long long)q * per_pair), colour = rem / (g.rows * g.wpr);
-  const int rw = rem - colour * g.rows * g.wpr, i = rw / g.wpr;
-  int a, b;
-  if (!pair_replicas(Q, q, a, b)) return;
-  houdayer_flip_word(P, C, cluster_labels(C, q), q, a, b, colour, i, rw - i * g.wpr);
-}
-
-// Lattices of at most kClusterResidentSites sites: every step of the call in one launch, one block per pair, the
-// labels in shared memory, as cluster_resident_kernel.
-__global__ void __launch_bounds__(kClusterThreads) houdayer_resident_kernel(SweepParams P, ClusterParams C, PairParams Q,
-                                                                            int n_steps) {
-  extern __shared__ int32_t L[];
-  const Geom& g = P.g;
-  const int q = blockIdx.x, per_rep = g.rows * g.wpr, n_sites = g.rows * g.cols;
-  int a, b;
-  if (!pair_replicas(Q, q, a, b)) return;
-  for (int s = 0; s < n_steps; ++s) {
-    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
-      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
-      houdayer_bond_word(P, C, P.sweep + (uint32_t)s, q, a, b, colour, i, rem - i * g.wpr);
-    }
-    for (int t = threadIdx.x; t < n_sites; t += kClusterThreads) L[t] = t;
-    __syncthreads();
-    cluster_tile_unions(L, cluster_act(C, q), g, 0, g.rows, 0, g.wpr, 0, g.cols);
-    __syncthreads();
-    for (int t = threadIdx.x; t < 2 * per_rep; t += kClusterThreads) {
-      const int colour = t / per_rep, rem = t - colour * per_rep, i = rem / g.wpr;
-      houdayer_flip_word(P, C, L, q, a, b, colour, i, rem - i * g.wpr);
+    for (int t = threadIdx.x; t < 2 * per_unit; t += kClusterThreads) {
+      const int colour = t / per_unit, rem = t - colour * per_unit, i = rem / g.wpr;
+      M.flip_word(P, C, L, u, a, b, colour, i, rem - i * g.wpr);
     }
     __syncthreads();  // the next step's bonds read the flipped words
   }
@@ -1945,53 +1926,16 @@ int launch_population_reduce(const Lattice& L, const PopParams& Q, const AnnealO
   TSU_RETURN_LAUNCH_STATUS();
 }
 
-// bytes of the Swendsen-Wang work buffer per replica (layout at ClusterParams); 0 for lattices it cannot label
+// bytes of the cluster work buffer per unit (layout at ClusterParams); 0 for lattices it cannot label
 long long cluster_rep_bytes(int rows, int cols) {
   if (rows <= 0 || cols <= 0 || (long long)rows * cols > 2147483647LL) return 0;
   const long long label_bytes = (4LL * rows * cols + 15) / 16 * 16;
   return label_bytes + 24LL * rows * words_per_row(cols);
 }
 
-// n_steps Swendsen-Wang steps of the replicas of L, which own C.work: one launch for lattices whose labels fit a
-// block's shared memory, otherwise four launches per step (bonds, local labels, merges across tiles, flips)
-int launch_swendsen_wang(const Lattice& L, const ClusterParams& C, uint32_t sweep0, int n_steps, cudaStream_t st) {
-  const Geom& g = L.g;
-  SweepParams P = sweep_params(L, 0, sweep0, nullptr, nullptr);
-  const bool bonded = L.B.words != nullptr;
-  if (tuning().resident != 0 && (long long)g.rows * g.cols <= kClusterResidentSites) {
-    const size_t smem = sizeof(int32_t) * (size_t)g.rows * g.cols;
-    if (bonded)
-      cluster_resident_kernel<true><<<g.n_replicas, kClusterThreads, smem, st>>>(P, L.B, C, n_steps);
-    else
-      cluster_resident_kernel<false><<<g.n_replicas, kClusterThreads, smem, st>>>(P, kNoBonds, C, n_steps);
-    TSU_RETURN_LAUNCH_STATUS();
-  }
-  const unsigned word_grid = blocks_for(2LL * g.rows * g.wpr * g.n_replicas, kClusterThreads);
-  const int tiles_x = (g.cols + kClusterTileCols - 1) / kClusterTileCols;
-  const int tiles_y = (g.rows + kClusterTileRows - 1) / kClusterTileRows;
-  const unsigned merge_grid =
-      blocks_for(((long long)tiles_y * g.cols + (long long)g.rows * tiles_x) * g.n_replicas, kClusterThreads);
-  for (int s = 0; s < n_steps; ++s) {
-    P.sweep = sweep0 + (uint32_t)s;
-    if (bonded)
-      cluster_bonds_kernel<true><<<word_grid, kClusterThreads, 0, st>>>(P, L.B, C);
-    else
-      cluster_bonds_kernel<false><<<word_grid, kClusterThreads, 0, st>>>(P, kNoBonds, C);
-    cluster_local_kernel<<<(unsigned)((long long)tiles_x * tiles_y * g.n_replicas), kClusterThreads, 0, st>>>(
-        P, C, tiles_x, tiles_x * tiles_y);
-    cluster_merge_kernel<<<merge_grid, kClusterThreads, 0, st>>>(P, C, tiles_y, tiles_x);
-    cluster_flip_kernel<<<word_grid, kClusterThreads, 0, st>>>(P, C);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-  }
-  return TSU_OK;
-}
-
 // the work buffer of tsu_ising2d_cluster_work_bytes carved into rep_bytes shares
 ClusterParams cluster_params(void* work, long long rep_bytes, int rows, int cols) {
   ClusterParams C;
-  C.thresholds = nullptr;
-  C.sign = 1;
   C.work = static_cast<char*>(work);
   C.rep_bytes = (size_t)rep_bytes;
   C.act_offset = (4 * (size_t)rows * cols + 15) / 16 * 16;
@@ -1999,33 +1943,55 @@ ClusterParams cluster_params(void* work, long long rep_bytes, int rows, int cols
   return C;
 }
 
-// n_steps Houdayer steps of the n_pairs pairs `pairs` of the replicas of L; pair q owns share q of C.work.  The launch
-// paths of launch_swendsen_wang, with the pairs in place of the replicas.
-int launch_houdayer(const Lattice& L, const ClusterParams& C, const int32_t* pairs, int n_pairs, uint32_t sweep0,
-                    int n_steps, cudaStream_t st) {
-  SweepParams P = sweep_params(L, 0, sweep0, nullptr, nullptr);
-  const PairParams Q = {pairs, L.g.n_replicas};
-  P.g.n_replicas = n_pairs;
+// n_steps steps of move M from step P.sweep on the P.g.n_replicas units of P, which own C.work: one launch for lattices
+// whose labels fit a block's shared memory, otherwise four launches per step (bonds, local labels, merges across
+// tiles, flips)
+template <class Move>
+int launch_cluster(SweepParams P, const ClusterParams& C, const Move& M, int n_steps, cudaStream_t st) {
   const Geom& g = P.g;
   if (tuning().resident != 0 && (long long)g.rows * g.cols <= kClusterResidentSites) {
     const size_t smem = sizeof(int32_t) * (size_t)g.rows * g.cols;
-    houdayer_resident_kernel<<<n_pairs, kClusterThreads, smem, st>>>(P, C, Q, n_steps);
+    cluster_resident_kernel<Move><<<g.n_replicas, kClusterThreads, smem, st>>>(P, C, M, n_steps);
     TSU_RETURN_LAUNCH_STATUS();
   }
-  const unsigned word_grid = blocks_for(2LL * g.rows * g.wpr * n_pairs, kClusterThreads);
+  const unsigned word_grid = blocks_for(2LL * g.rows * g.wpr * g.n_replicas, kClusterThreads);
   const int tiles_x = (g.cols + kClusterTileCols - 1) / kClusterTileCols;
   const int tiles_y = (g.rows + kClusterTileRows - 1) / kClusterTileRows;
   const unsigned merge_grid =
-      blocks_for(((long long)tiles_y * g.cols + (long long)g.rows * tiles_x) * n_pairs, kClusterThreads);
+      blocks_for(((long long)tiles_y * g.cols + (long long)g.rows * tiles_x) * g.n_replicas, kClusterThreads);
+  const uint32_t sweep0 = P.sweep;
   for (int s = 0; s < n_steps; ++s) {
     P.sweep = sweep0 + (uint32_t)s;
-    houdayer_bonds_kernel<<<word_grid, kClusterThreads, 0, st>>>(P, C, Q);
-    cluster_local_kernel<<<(unsigned)((long long)tiles_x * tiles_y * n_pairs), kClusterThreads, 0, st>>>(
+    cluster_bonds_kernel<Move><<<word_grid, kClusterThreads, 0, st>>>(P, C, M);
+    cluster_local_kernel<<<(unsigned)((long long)tiles_x * tiles_y * g.n_replicas), kClusterThreads, 0, st>>>(
         P, C, tiles_x, tiles_x * tiles_y);
     cluster_merge_kernel<<<merge_grid, kClusterThreads, 0, st>>>(P, C, tiles_y, tiles_x);
-    houdayer_flip_kernel<<<word_grid, kClusterThreads, 0, st>>>(P, C, Q);
+    cluster_flip_kernel<Move><<<word_grid, kClusterThreads, 0, st>>>(P, C, M);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return (int)e;
+  }
+  return TSU_OK;
+}
+
+// n_steps steps of move M on its n_units units of the lattices L, in chunks of units that fit the work buffer
+template <class Move>
+int run_cluster(const Lattice& L, const Move& M, int n_units, void* work, size_t work_bytes, uint32_t sweep0,
+                int n_steps, cudaStream_t st) {
+  const long long rep_bytes = cluster_rep_bytes(L.g.rows, L.g.cols);
+  TSU_CHECK_ARG(rep_bytes > 0 && work_bytes >= (size_t)rep_bytes);
+  if (n_steps == 0) return TSU_OK;
+  const long long fit = (long long)(work_bytes / (size_t)rep_bytes);
+  const int chunk = fit < n_units ? (int)fit : n_units;
+  const ClusterParams C = cluster_params(work, rep_bytes, L.g.rows, L.g.cols);
+  // chunks one after the other, each through all its steps: units do not share replicas (Houdayer pairs are disjoint),
+  // so the bits depend on no chunk size
+  for (int u0 = 0; u0 < n_units; u0 += chunk) {
+    SweepParams P = sweep_params(L, 0, sweep0, nullptr, nullptr);
+    Move Mc = M;
+    Mc.narrow(P, u0);
+    P.g.n_replicas = u0 + chunk < n_units ? chunk : n_units - u0;
+    const int rc = launch_cluster(P, C, Mc, n_steps, st);
+    if (rc != TSU_OK) return rc;
   }
   return TSU_OK;
 }
@@ -2336,22 +2302,13 @@ int tsu_ising2d_swendsen_wang(uint32_t* d_state, int n_replicas, int rows, int c
                      {d_bonds, d_bond_index}, seed, replica0, JitKernel{nullptr, 0, 0}};
   TSU_CHECK_ARG(d_state && d_thresholds && d_work && n_steps >= 0 && (coupling_sign == 1 || coupling_sign == -1));
   TSU_CHECK_ARG(args_ok(L.g, L.B, false, 0, 0, rows));
-  const long long rep_bytes = cluster_rep_bytes(rows, cols);
-  TSU_CHECK_ARG(rep_bytes > 0 && work_bytes >= (size_t)rep_bytes);
-  if (n_steps == 0) return TSU_OK;
-  const long long fit = (long long)(work_bytes / (size_t)rep_bytes);
-  const int chunk = fit < n_replicas ? (int)fit : n_replicas;
-  ClusterParams C = cluster_params(d_work, rep_bytes, rows, cols);
-  C.thresholds = reinterpret_cast<const unsigned long long*>(d_thresholds);
-  C.sign = coupling_sign;
+  const auto* thresholds = reinterpret_cast<const unsigned long long*>(d_thresholds);
   cudaStream_t st = tsu_stream(stream);
-  // chunks one after the other, each through all its steps: the bits depend on no chunk size
-  for (int r0 = 0; r0 < n_replicas; r0 += chunk) {
-    const int rc = launch_swendsen_wang(L.replicas(r0, r0 + chunk < n_replicas ? r0 + chunk : n_replicas), C, sweep0,
-                                        n_steps, st);
-    if (rc != TSU_OK) return rc;
-  }
-  return TSU_OK;
+  if (d_bonds)
+    return run_cluster(L, SwMove<true>{L.B, thresholds, coupling_sign}, n_replicas, d_work, work_bytes, sweep0, n_steps,
+                       st);
+  return run_cluster(L, SwMove<false>{kNoBonds, thresholds, coupling_sign}, n_replicas, d_work, work_bytes, sweep0,
+                     n_steps, st);
 }
 
 int tsu_ising2d_houdayer(uint32_t* d_state, int n_replicas, int rows, int cols, int wrap_rows, int wrap_cols,
@@ -2361,20 +2318,8 @@ int tsu_ising2d_houdayer(uint32_t* d_state, int n_replicas, int rows, int cols, 
                      seed, replica0, JitKernel{nullptr, 0, 0}};
   TSU_CHECK_ARG(d_state && d_pairs && d_work && n_steps >= 0 && n_pairs >= 1 && 2LL * n_pairs <= n_replicas);
   TSU_CHECK_ARG(args_ok(L.g, L.B, false, 0, 0, rows));
-  const long long rep_bytes = cluster_rep_bytes(rows, cols);
-  TSU_CHECK_ARG(rep_bytes > 0 && work_bytes >= (size_t)rep_bytes);
-  if (n_steps == 0) return TSU_OK;
-  const long long fit = (long long)(work_bytes / (size_t)rep_bytes);
-  const int chunk = fit < n_pairs ? (int)fit : n_pairs;
-  const ClusterParams C = cluster_params(d_work, rep_bytes, rows, cols);
-  cudaStream_t st = tsu_stream(stream);
-  // chunks one after the other, each through all its steps: disjoint pairs give bits that depend on no chunk size
-  for (int q0 = 0; q0 < n_pairs; q0 += chunk) {
-    const int rc = launch_houdayer(L, C, d_pairs + 2 * (size_t)q0, q0 + chunk < n_pairs ? chunk : n_pairs - q0, sweep0,
-                                   n_steps, st);
-    if (rc != TSU_OK) return rc;
-  }
-  return TSU_OK;
+  return run_cluster(L, HoudayerMove{d_pairs, n_replicas}, n_pairs, d_work, work_bytes, sweep0, n_steps,
+                     tsu_stream(stream));
 }
 
 int tsu_ising2d_energy_from_observables(const unsigned long long* d_obs, int n_replicas, double J, double h,
