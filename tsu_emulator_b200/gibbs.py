@@ -54,6 +54,14 @@ def _as_square(coupling) -> np.ndarray:
     return J
 
 
+def _host_energy(state: np.ndarray, coupling, bias=None) -> float:
+    """E = -1/2 s^T J s - b^T s (host arithmetic on one configuration)"""
+    energy = -0.5 * state.dot(coupling).dot(state)
+    if bias is not None:
+        energy -= np.asarray(bias).dot(state)
+    return float(energy)
+
+
 # csrc/dense_gibbs.cu keeps a chain's uniforms (and their logits with float64 fields), fields, self couplings and bits
 # in at most 227 KB of shared memory: 33 N + 272 bytes with float64 fields, 17 N + 272 with float32
 DENSE_MAX_N = {"float64": 7035, "float32": 13657}
@@ -62,7 +70,7 @@ DENSE_MAX_N = {"float64": 7035, "float32": 13657}
 class _DenseProblem:
     """coupling matrix + bias resident on the device (transposed, see tsu_b200.h)"""
 
-    def __init__(self, coupling, bias, precision: str, device):
+    def __init__(self, coupling, bias, precision: str, device, update_order: str = "sequential"):
         J = _as_square(coupling)
         self.N = J.shape[0]
         if precision == "bf16":
@@ -78,14 +86,55 @@ class _DenseProblem:
         self.np_dtype = np.float64 if precision == "float64" else np.float32
         self.code = 1 if precision == "float64" else 0
         self.device = device
+        self.update_order = update_order
+        self.host_J, self.host_bias = J, None
         self.Jt = torch.from_numpy(np.ascontiguousarray(J.T.astype(self.np_dtype))).to(device)
         if bias is not None:
             b = np.asarray(bias, dtype=np.float64)
             if b.shape != (self.N,):
                 raise ValueError("bias must have one entry per bit")
             self.bias = torch.from_numpy(np.ascontiguousarray(b.astype(self.np_dtype))).to(device)
+            self.host_bias = b
         else:
             self.bias = None
+
+    def _orders(self, n_sweeps: int, seed: int, sweep0: int):
+        """visiting order per sweep: None for 'sequential', fresh permutations for 'random' (gibbs.py:153-157)"""
+        if self.update_order == "sequential" or n_sweeps == 0:
+            return None
+        torch = _lib.require_cuda()
+        rng = np.random.Generator(np.random.Philox(key=[seed, sweep0]))
+        perms = np.stack([rng.permutation(self.N) for _ in range(n_sweeps)]).astype(np.int32)
+        return torch.from_numpy(perms).to(self.device)
+
+    def run(self, state, *, T: float, seed: int, sweep0: int, chain0: int, n_burnin: int, n_samples: int,
+            sweeps_per_sample: int, T_chain=None, T_sweep=None, uniforms=None, want_samples=False, want_energy=False,
+            track_best=False, order=None, visits_per_sweep: int = 0):
+        """one launch of tsu_dense_gibbs_run on `state` (uint8 tensor [n_chains, N], updated in place); T_sweep is the
+        host float64 temperature of every sweep; without `order` the sweeps follow the problem's update order"""
+        torch = _lib.require_cuda()
+        device = self.device
+        n_chains, N = state.shape
+        if order is None and visits_per_sweep == 0:
+            order = self._orders(n_burnin + n_samples * sweeps_per_sample, seed, sweep0)
+        if T_sweep is not None:
+            T_sweep = torch.from_numpy(T_sweep).to(device)
+        samples = torch.empty((n_samples, n_chains, N), dtype=torch.uint8, device=device) if want_samples else None
+        energy = torch.empty(n_chains, dtype=torch.float64, device=device) if (want_energy or track_best) else None
+        best_state = torch.empty((n_chains, N), dtype=torch.uint8, device=device) if track_best else None
+        best_energy = torch.empty(n_chains, dtype=torch.float64, device=device) if track_best else None
+        with torch.cuda.device(device):
+            _lib.call(
+                "tsu_dense_gibbs_run", ptr(self.Jt), self.code, ptr(self.bias), ptr(state), n_chains, N, float(T),
+                ptr(T_chain), ptr(T_sweep), int(n_burnin), int(n_samples), int(sweeps_per_sample), ptr(order),
+                ptr(uniforms), ptr(samples), ptr(energy), int(track_best), ptr(best_state), ptr(best_energy), seed,
+                sweep0 & 0xFFFFFFFF, chain0 & 0xFFFFFFFF, self.code, int(visits_per_sweep), _lib.current_stream(),
+            )
+        return samples, energy, best_state, best_energy
+
+    def energy(self, state: np.ndarray) -> float:
+        """energy of a host state under the float64 couplings and bias"""
+        return _host_energy(state, self.host_J, self.host_bias)
 
 
 TC_MAX_N = 4096   # csrc/dense_tc.cu keeps the chain bits of a CTA in shared memory
@@ -107,6 +156,7 @@ class _TcProblem:
         if update_order != "sequential":
             raise ValueError("precision='bf16' (tensor-core path) implements the sequential update order only")
         self.device = device
+        self.host_J, self.host_bias = J, None
         # upload as given and round on the device (float64 -> float32 -> bf16, the rounding the oracle applies): the
         # host-side conversion of a 4096 x 4096 matrix used to cost several times the 10 sweeps it was uploaded for
         Jd = torch.from_numpy(np.ascontiguousarray(J)).to(device).to(torch.float32).to(torch.bfloat16)
@@ -123,14 +173,55 @@ class _TcProblem:
             bp = np.zeros(self.Np, dtype=np.float32)
             bp[:self.N] = b
             self.bias = torch.from_numpy(bp).to(device)
+            self.host_bias = b
 
-    def pad_state(self, st):
-        if self.Np == self.N:
-            return st
+    def run(self, state, *, T: float, seed: int, sweep0: int, chain0: int, n_burnin: int, n_samples: int,
+            sweeps_per_sample: int, T_chain=None, T_sweep=None, uniforms=None, want_samples=False, want_energy=False,
+            track_best=False):
+        """the launches of a run on `state` ([n_chains, Np] uint8, updated in place), bf16 couplings, fp32 fields in
+        TMEM.  With T_sweep (host float64): an energy pass on the initial state, then per step one sweep at T_sweep[k]
+        and an energy pass that keeps every chain's best state.  Otherwise n_burnin sweeps, then sweeps_per_sample
+        sweeps before each sample.  With want_energy, one energy pass at the end.  Injected uniforms are a float64 /
+        float32 parity mode: the callers reject them."""
         torch = _lib.require_cuda()
-        out = torch.zeros((st.shape[0], self.Np), dtype=torch.uint8, device=st.device)
-        out[:, :self.N] = st
-        return out
+        n_chains, N, device = int(state.shape[0]), self.N, self.device
+        samples = torch.empty((n_samples, n_chains, N), dtype=torch.uint8, device=device) if want_samples else None
+        energy = torch.empty(n_chains, dtype=torch.float64, device=device) if (want_energy or track_best) else None
+        best_state = torch.empty_like(state) if track_best else None
+        best_energy = torch.full((n_chains,), float("inf"), dtype=torch.float64, device=device) if track_best else None
+
+        def sweeps(n, T, sweep):
+            """n sweeps at T, or at the per-chain T_chain; a count <= 0 launches nothing.  Returns the next offset"""
+            if n <= 0:
+                return sweep
+            _lib.call("tsu_dense_gibbs_tc_run", ptr(self.J), ptr(self.bias), ptr(state), n_chains, self.Np,
+                      1.0 if T_chain is not None else float(T), ptr(T_chain), int(n), seed, sweep & 0xFFFFFFFF,
+                      chain0 & 0xFFFFFFFF, None, _lib.current_stream())
+            return sweep + n
+
+        def energy_pass(best: bool):
+            _lib.call("tsu_dense_tc_energy", ptr(self.J), ptr(self.bias), ptr(state), n_chains, self.Np, ptr(energy),
+                      ptr(best_energy if best else None), ptr(best_state if best else None), _lib.current_stream())
+
+        with torch.cuda.device(device):
+            sweep = sweep0
+            if T_sweep is not None:
+                energy_pass(track_best)   # the initial state is the first best
+                for k in range(n_burnin):
+                    sweep = sweeps(1, T_sweep[k], sweep)
+                    energy_pass(track_best)
+            else:
+                sweep = sweeps(n_burnin, T, sweep)
+                for k in range(n_samples):
+                    sweep = sweeps(sweeps_per_sample, T, sweep)
+                    samples[k] = state[:, :N]
+            if want_energy:
+                energy_pass(False)
+        return samples, energy, None if best_state is None else best_state[:, :N], best_energy
+
+    def energy(self, state: np.ndarray) -> float:
+        """energy of a host state under the float64 couplings and bias (not their bf16 rounding)"""
+        return _host_energy(state, self.host_J, self.host_bias)
 
 
 def annealing_temperatures(T_initial: float, T_final: float, n_steps: int, cooling_schedule: str = "exponential"):
@@ -182,52 +273,38 @@ class GibbsSampler:
 
     def compute_energy(self, state: np.ndarray, coupling: np.ndarray, bias: Optional[np.ndarray] = None) -> float:
         """tsu/gibbs.py:215-236: E = -1/2 s^T J s - b^T s (host arithmetic on one configuration)"""
-        state = np.asarray(state)
-        energy = -0.5 * state.dot(coupling).dot(state)
-        if bias is not None:
-            energy -= np.asarray(bias).dot(state)
-        return float(energy)
+        return _host_energy(np.asarray(state), coupling, bias)
 
     # ------------------------------------------------------------------ device plumbing
     def _dev(self):
         torch = _lib.require_cuda()
         return torch.device(self._device) if self._device is not None else torch.device("cuda", torch.cuda.current_device())
 
-    def _orders(self, n_sweeps: int, N: int, device):
-        """visiting order per sweep: None for 'sequential', fresh permutations for 'random' (gibbs.py:153-157)"""
-        if self.config.update_order == "sequential" or n_sweeps == 0:
-            return None
-        torch = _lib.require_cuda()
-        rng = np.random.Generator(np.random.Philox(key=[self._seed, self._sweep_counter]))
-        perms = np.stack([rng.permutation(N) for _ in range(n_sweeps)]).astype(np.int32)
-        return torch.from_numpy(perms).to(device)
+    def _problem(self, coupling, bias, *, chromatic: bool, tensor_ok: bool):
+        """the couplings on the device for the sampler's back end: chromatic CSR (float64 fields), tensor cores (bf16,
+        for the entry points that serve them) or the float64 / float32 dense kernel"""
+        if chromatic:
+            from .sparse import SparseProblem
 
-    def _run(self, prob: _DenseProblem, state, *, n_burnin: int, n_samples: int, sweeps_per_sample: int,
-             T_chain=None, T_sweep=None, want_samples=False, want_energy=False, track_best=False,
-             order=None, uniforms=None, visits_per_sweep: int = 0):
-        """one launch of tsu_dense_gibbs_run on `state` (uint8 tensor [n_chains, N], updated in place)"""
-        torch = _lib.require_cuda()
-        device = prob.device
-        n_chains, N = state.shape
-        total = n_burnin + n_samples * sweeps_per_sample
-        if order is None and visits_per_sweep == 0:
-            order = self._orders(total, N, device)
-        samples = torch.empty((n_samples, n_chains, N), dtype=torch.uint8, device=device) if want_samples else None
-        energy = torch.empty(n_chains, dtype=torch.float64, device=device) if (want_energy or track_best) else None
-        best_state = torch.empty((n_chains, N), dtype=torch.uint8, device=device) if track_best else None
-        best_energy = torch.empty(n_chains, dtype=torch.float64, device=device) if track_best else None
-        with torch.cuda.device(device):
-            _lib.call(
-                "tsu_dense_gibbs_run", ptr(prob.Jt), prob.code, ptr(prob.bias), ptr(state), n_chains, N,
-                float(self.config.temperature), ptr(T_chain), ptr(T_sweep), int(n_burnin), int(n_samples),
-                int(sweeps_per_sample), ptr(order), ptr(uniforms), ptr(samples), ptr(energy), int(track_best),
-                ptr(best_state), ptr(best_energy), self._seed, self._sweep_counter & 0xFFFFFFFF,
-                self._chain_counter & 0xFFFFFFFF, prob.code, int(visits_per_sweep), _lib.current_stream(),
-            )
-        self._sweep_counter += total
-        return samples, energy, best_state, best_energy
+            if self.precision != "float64":
+                raise ValueError("chromatic=True (sparse couplings) computes float64 fields: use a 'float64' sampler")
+            return SparseProblem(coupling, bias, self._dev())
+        if self.precision == "bf16" and tensor_ok:
+            return _TcProblem(coupling, bias, self._dev(), self.config.update_order)
+        return _DenseProblem(coupling, bias, self.precision, self._dev(), self.config.update_order)
+
+    def _run(self, prob, state, *, n_burnin: int, n_samples: int, sweeps_per_sample: int, **kw):
+        """prob.run on `state` at the sampler's temperature, seed and Philox offsets, which then advance past the sweeps
+        run.  A negative count is an error on the dense and sparse kernels and runs nothing on the tensor cores."""
+        out = prob.run(state, T=float(self.config.temperature), seed=self._seed, sweep0=self._sweep_counter,
+                       chain0=self._chain_counter, n_burnin=n_burnin, n_samples=n_samples,
+                       sweeps_per_sample=sweeps_per_sample, **kw)
+        self._sweep_counter += max(n_burnin, 0) + n_samples * max(sweeps_per_sample, 0)
+        return out
 
     def _initial_states(self, prob, n_chains: int, initial_state=None):
+        """uint8 [n_chains, N] states on the device (given, or Philox draws), padded with zero bits to the tensor-core
+        problem's panel width"""
         torch = _lib.require_cuda()
         if initial_state is not None:
             a = np.asarray(initial_state)
@@ -237,83 +314,72 @@ class GibbsSampler:
                 a = np.broadcast_to(a, (n_chains, prob.N))
             elif a.shape != (n_chains, prob.N):
                 raise ValueError(f"initial_state must have shape ({prob.N},) or ({n_chains}, {prob.N}), got {a.shape}")
-            return torch.from_numpy(np.ascontiguousarray((a != 0).astype(np.uint8))).to(prob.device)
-        state = torch.empty((n_chains, prob.N), dtype=torch.uint8, device=prob.device)
-        with torch.cuda.device(prob.device):
-            _lib.call("tsu_dense_init_random", ptr(state), n_chains, prob.N, self._seed ^ 0x5DEECE66D,
-                      (self._chain_counter + self._sweep_counter) & 0xFFFFFFFF, _lib.current_stream())
-        return state
+            state = torch.from_numpy(np.ascontiguousarray((a != 0).astype(np.uint8))).to(prob.device)
+        else:
+            state = torch.empty((n_chains, prob.N), dtype=torch.uint8, device=prob.device)
+            with torch.cuda.device(prob.device):
+                _lib.call("tsu_dense_init_random", ptr(state), n_chains, prob.N, self._seed ^ 0x5DEECE66D,
+                          (self._chain_counter + self._sweep_counter) & 0xFFFFFFFF, _lib.current_stream())
+        width = getattr(prob, "Np", prob.N)
+        if width == prob.N:
+            return state
+        padded = torch.zeros((n_chains, width), dtype=torch.uint8, device=prob.device)
+        padded[:, :prob.N] = state
+        return padded
+
+    @staticmethod
+    def _injected(prob, uniforms, orders=None) -> dict:
+        """parity mode, as run() arguments on the device: float64 uniforms [sweeps, N] (one chain) or [sweeps, chains,
+        N], in visiting order, and visiting orders [sweeps, N] of the dense kernel"""
+        torch = _lib.require_cuda()
+        kw = {}
+        if uniforms is not None:
+            a = np.asarray(uniforms, dtype=np.float64)
+            if a.ndim == 2:
+                a = a[:, None, :]
+            kw["uniforms"] = torch.from_numpy(np.ascontiguousarray(a)).to(prob.device)
+        if orders is not None:
+            kw["order"] = torch.from_numpy(np.ascontiguousarray(np.asarray(orders, dtype=np.int32))).to(prob.device)
+        return kw
+
+    @staticmethod
+    def _samples_out(samples, n_chains: int, as_tensor: bool):
+        """samples [n_samples, n_chains, N] -> (n_samples, N) for one chain, (n_chains, n_samples, N) host int64 for
+        more; as_tensor keeps them on the device, chain axis second"""
+        if as_tensor:
+            return samples if n_chains > 1 else samples[:, 0]
+        out = _host_int64(samples)
+        return out[:, 0, :] if n_chains == 1 else np.ascontiguousarray(out.transpose(1, 0, 2))
 
     # ------------------------------------------------------------------ reference API
     def sample_conditional(self, i: int, state: np.ndarray, coupling: np.ndarray,
                            bias: Optional[np.ndarray] = None) -> int:
         """tsu/gibbs.py:102-126: resample bit i given the others (one single-site visit on the device)"""
         torch = _lib.require_cuda()
-        prob = _DenseProblem(coupling, bias, self.precision, self._dev())
+        prob = self._problem(coupling, bias, chromatic=False, tensor_ok=False)
         st = self._initial_states(prob, 1, np.asarray(state))
         order = torch.tensor([[int(i)]], dtype=torch.int32, device=prob.device)
         self._run(prob, st, n_burnin=1, n_samples=0, sweeps_per_sample=0, order=order, visits_per_sweep=1)
         return int(st[0, int(i)].item())
 
-    def _inject(self, prob, uniforms, orders):
-        """parity mode: float64 uniforms [sweeps, N] (single chain) / [sweeps, chains, N] and orders [sweeps, N]"""
-        torch = _lib.require_cuda()
-        u = o = None
-        if uniforms is not None:
-            a = np.asarray(uniforms, dtype=np.float64)
-            if a.ndim == 2:
-                a = a[:, None, :]
-            u = torch.from_numpy(np.ascontiguousarray(a)).to(prob.device)
-        if orders is not None:
-            o = torch.from_numpy(np.ascontiguousarray(np.asarray(orders, dtype=np.int32))).to(prob.device)
-        return u, o
-
-    def _sparse(self, coupling, bias):
-        """couplings in CSR form + colour classes on the device (csrc/sparse_gibbs.cu); float64 fields"""
-        from .sparse import SparseProblem
-
-        if self.precision != "float64":
-            raise ValueError("chromatic=True (sparse couplings) computes float64 fields: use a 'float64' sampler")
-        return SparseProblem(coupling, bias, self._dev())
-
-    def _sparse_run(self, prob, state, uniforms=None, **kw):
-        from . import sparse
-
-        torch = _lib.require_cuda()
-        u = None
-        if uniforms is not None:  # parity mode: [sweeps, N] or [sweeps, chains, N] float64 in VISITING order
-            a = np.asarray(uniforms, dtype=np.float64)
-            if a.ndim == 2:
-                a = a[:, None, :]
-            u = torch.from_numpy(np.ascontiguousarray(a)).to(prob.device)
-        total = kw["n_burnin"] + kw["n_samples"] * kw["sweeps_per_sample"]
-        out = sparse.run(prob, state, T=float(self.config.temperature), seed=self._seed, sweep0=self._sweep_counter,
-                         chain0=self._chain_counter, uniforms=u, **kw)
-        self._sweep_counter += total
-        return out
-
     def gibbs_sweep(self, state: np.ndarray, coupling: np.ndarray, bias: Optional[np.ndarray] = None,
                     n_sweeps: int = 1, *, chromatic: bool = False, _uniforms=None, _orders=None) -> np.ndarray:
         """tsu/gibbs.py:128-162: n_sweeps sweeps over all bits; the input is not modified (gibbs.py:150).
         chromatic=True: sparse couplings, sites visited colour class by colour class (csrc/sparse_gibbs.cu)"""
-        if chromatic:
-            prob = self._sparse(coupling, bias)
-            st = self._initial_states(prob, 1, np.asarray(state))
-            self._sparse_run(prob, st, uniforms=_uniforms, n_burnin=int(n_sweeps), n_samples=0, sweeps_per_sample=0)
-            a = np.asarray(state)
-            return st[0].cpu().numpy().astype(a.dtype if a.dtype.kind in "iu" else np.int64)
-        prob = _DenseProblem(coupling, bias, self.precision, self._dev())
+        prob = self._problem(coupling, bias, chromatic=chromatic, tensor_ok=False)
         st = self._initial_states(prob, 1, np.asarray(state))
-        u, o = self._inject(prob, _uniforms, _orders)
-        self._run(prob, st, n_burnin=int(n_sweeps), n_samples=0, sweeps_per_sample=0, uniforms=u, order=o)
-        out = st[0].cpu().numpy().astype(np.asarray(state).dtype if np.asarray(state).dtype.kind in "iu" else np.int64)
-        return out
+        # a chromatic sweep visits the colour classes: injected orders do not apply
+        self._run(prob, st, n_burnin=int(n_sweeps), n_samples=0, sweeps_per_sample=0,
+                  **self._injected(prob, _uniforms, None if chromatic else _orders))
+        a = np.asarray(state)
+        return st[0].cpu().numpy().astype(a.dtype if a.dtype.kind in "iu" else np.int64)
 
     def sample_boltzmann(self, coupling: np.ndarray, bias: Optional[np.ndarray] = None, n_samples: int = 1000,
                          burnin: Optional[int] = None, initial_state: Optional[np.ndarray] = None, *,
                          n_chains: int = 1, as_tensor: bool = False, chromatic: bool = False, _uniforms=None,
                          _orders=None):
-        """tsu/gibbs.py:164-213: burn-in, then n_samples x config.n_sweeps sweeps; one launch.
+        """tsu/gibbs.py:164-213: burn-in, then n_samples x config.n_sweeps sweeps; one launch (one per group of sweeps
+        on the tensor cores).
 
         n_chains == 1 (default): int array (n_samples, n_bits) like the reference.
         n_chains > 1: (n_chains, n_samples, n_bits) - independent chains run concurrently.
@@ -321,118 +387,35 @@ class GibbsSampler:
         a sweep visits the sites colour class by colour class instead of in index order.
         """
         burnin = burnin if burnin is not None else self.config.n_burnin
-        if chromatic:
-            prob = self._sparse(coupling, bias)
-            st = self._initial_states(prob, int(n_chains), initial_state)
-            samples, _, _, _ = self._sparse_run(prob, st, uniforms=_uniforms, n_burnin=int(burnin),
-                                                n_samples=int(n_samples), sweeps_per_sample=self.config.n_sweeps,
-                                                want_samples=True)
-            self._chain_counter += int(n_chains)
-            self.sample_count += int(n_samples)
-            if as_tensor:
-                return samples if n_chains > 1 else samples[:, 0]
-            out = _host_int64(samples)
-            return out[:, 0, :] if n_chains == 1 else np.ascontiguousarray(out.transpose(1, 0, 2))
-        if self.precision == "bf16":
-            if _uniforms is not None or _orders is not None:
-                raise ValueError("injected draws are a float64 / float32 parity mode; precision='bf16' draws Philox")
-            return self._sample_boltzmann_tensor(coupling, bias, int(n_samples), int(burnin), initial_state,
-                                                 int(n_chains), as_tensor)
-        prob = _DenseProblem(coupling, bias, self.precision, self._dev())
+        if self.precision == "bf16" and not chromatic and (_uniforms is not None or _orders is not None):
+            raise ValueError("injected draws are a float64 / float32 parity mode; precision='bf16' draws Philox")
+        prob = self._problem(coupling, bias, chromatic=chromatic, tensor_ok=True)
         st = self._initial_states(prob, int(n_chains), initial_state)
-        u, o = self._inject(prob, _uniforms, _orders)
         samples, _, _, _ = self._run(prob, st, n_burnin=int(burnin), n_samples=int(n_samples),
-                                     sweeps_per_sample=self.config.n_sweeps, want_samples=True, uniforms=u, order=o)
+                                     sweeps_per_sample=self.config.n_sweeps, want_samples=True,
+                                     **self._injected(prob, _uniforms, None if chromatic else _orders))
         self._chain_counter += int(n_chains)
         self.sample_count += int(n_samples)
-        if as_tensor:
-            return samples if n_chains > 1 else samples[:, 0]
-        out = _host_int64(samples)  # (n_samples, n_chains, N)
-        if n_chains == 1:
-            return out[:, 0, :]
-        return np.ascontiguousarray(out.transpose(1, 0, 2))
+        return self._samples_out(samples, int(n_chains), as_tensor)
 
     def sample(self, J: np.ndarray, n_samples: int = 1000, **kwargs) -> np.ndarray:
         """README.md:69-80: `sampler.sample(J, n_samples=1000)` -> (n_samples, n_bits) binary configurations"""
         return self.sample_boltzmann(J, n_samples=n_samples, **kwargs)
-
-    def _tc_sweeps(self, prob: "_TcProblem", st, n_sweeps: int, T, fields=None):
-        """n_sweeps sequential sweeps of all chains of `st` ([n_chains, Np] uint8, in place) on the tensor cores at
-        temperature T: a scalar, or a float64 device tensor [n_chains] of per-chain temperatures"""
-        torch = _lib.require_cuda()
-        if n_sweeps <= 0:
-            return
-        T_chain = T if isinstance(T, torch.Tensor) else None
-        with torch.cuda.device(prob.device):
-            _lib.call("tsu_dense_gibbs_tc_run", ptr(prob.J), ptr(prob.bias), ptr(st), int(st.shape[0]), prob.Np,
-                      1.0 if T_chain is not None else float(T), ptr(T_chain), int(n_sweeps), self._seed,
-                      self._sweep_counter & 0xFFFFFFFF, self._chain_counter & 0xFFFFFFFF, ptr(fields),
-                      _lib.current_stream())
-        self._sweep_counter += int(n_sweeps)
-
-    @staticmethod
-    def _tc_energy(prob: "_TcProblem", st, energy, best_energy=None, best_state=None):
-        """energy[c] = -1/2 s^T J s - b^T s of every chain of `st` on the tensor cores (bf16 J, float64 sums); with
-        best_energy / best_state, chains whose energy is strictly lower than best_energy take it and their state"""
-        torch = _lib.require_cuda()
-        with torch.cuda.device(prob.device):
-            _lib.call("tsu_dense_tc_energy", ptr(prob.J), ptr(prob.bias), ptr(st), int(st.shape[0]), prob.Np,
-                      ptr(energy), ptr(best_energy), ptr(best_state), _lib.current_stream())
-
-    def _sample_boltzmann_tensor(self, coupling, bias, n_samples, burnin, initial_state, n_chains, as_tensor):
-        """tsu/gibbs.py:198-211 on csrc/dense_tc.cu: burn-in sweeps, then n_samples x config.n_sweeps sweeps with the
-        state of every chain recorded after each group; bf16 couplings, fp32 fields accumulated in TMEM"""
-        torch = _lib.require_cuda()
-        prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
-        st = prob.pad_state(self._initial_states(prob, n_chains, initial_state))
-        samples = torch.empty((n_samples, n_chains, prob.N), dtype=torch.uint8, device=prob.device)
-        T = self.config.temperature
-        self._tc_sweeps(prob, st, burnin, T)
-        for k in range(n_samples):
-            self._tc_sweeps(prob, st, self.config.n_sweeps, T)
-            samples[k] = st[:, :prob.N]
-        self._chain_counter += n_chains
-        self.sample_count += n_samples
-        if as_tensor:
-            return samples if n_chains > 1 else samples[:, 0]
-        out = _host_int64(samples)
-        if n_chains == 1:
-            return out[:, 0, :]
-        return np.ascontiguousarray(out.transpose(1, 0, 2))
-
-    def _sample_chains_tensor(self, coupling, bias, n_chains, n_sweeps, initial_state, as_tensor, return_energy):
-        """tensor-core path (csrc/dense_tc.cu): bf16 couplings, fp32 fields accumulated in TMEM"""
-        torch = _lib.require_cuda()
-        prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
-        device, N = prob.device, prob.N
-        st = prob.pad_state(self._initial_states(prob, int(n_chains), initial_state))
-        self._tc_sweeps(prob, st, int(n_sweeps), self.config.temperature)
-        self._chain_counter += int(n_chains)
-        energy = None
-        if return_energy:  # E = -1/2 s^T J s - b^T s: one more tensor-core field evaluation, summed on the device
-            energy = torch.empty(int(n_chains), dtype=torch.float64, device=device)
-            self._tc_energy(prob, st, energy)
-        st = st[:, :N]
-        out = st if as_tensor else _host_int64(st)
-        if return_energy:
-            return out, (energy if as_tensor else energy.cpu().numpy())
-        return out
 
     def sample_chains(self, coupling, bias=None, n_chains: int = 1024, n_sweeps: Optional[int] = None,
                       initial_state=None, as_tensor: bool = False, return_energy: bool = False):
         """batched entry point: n_chains independent chains, n_sweeps sweeps each, final states returned.
 
         This is the shape of BASELINE config 3 (dense J, N=4096, 2048 chains, 10 sweeps).  With
-        precision="bf16" the fields are evaluated on the tensor cores (tcgen05, csrc/dense_tc.cu)."""
-        if self.precision == "bf16":
-            n_sw = self.config.n_sweeps if n_sweeps is None else int(n_sweeps)
-            return self._sample_chains_tensor(coupling, bias, n_chains, n_sw, initial_state, as_tensor, return_energy)
-        prob = _DenseProblem(coupling, bias, self.precision, self._dev())
+        precision="bf16" the fields are evaluated on the tensor cores (tcgen05, csrc/dense_tc.cu) and the energy
+        E = -1/2 s^T J s - b^T s is one more tensor-core field evaluation, summed on the device."""
         n_sweeps = self.config.n_sweeps if n_sweeps is None else int(n_sweeps)
+        prob = self._problem(coupling, bias, chromatic=False, tensor_ok=True)
         st = self._initial_states(prob, int(n_chains), initial_state)
         _, energy, _, _ = self._run(prob, st, n_burnin=n_sweeps, n_samples=0, sweeps_per_sample=0,
                                     want_energy=return_energy)
         self._chain_counter += int(n_chains)
+        st = st[:, :prob.N]
         out = st if as_tensor else _host_int64(st)
         if return_energy:
             return out, (energy if as_tensor else energy.cpu().numpy())
@@ -463,13 +446,9 @@ class GibbsSampler:
             raise ValueError("n_ladders must be at least 1")
         if criterion not in ("metropolis", "reference"):
             raise ValueError("criterion must be 'metropolis' or 'reference'")
-        tc = self.precision == "bf16"
-        if _inject is not None and (tc or K > 1):
+        if _inject is not None and (self.precision == "bf16" or K > 1):
             raise ValueError("injected draws are a float64 / float32 parity mode of one ladder")
-        if tc:
-            prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
-        else:
-            prob = _DenseProblem(coupling, bias, self.precision, self._dev())
+        prob = self._problem(coupling, bias, chromatic=False, tensor_ok=True)
         device = prob.device
         temps = np.asarray(list(temperatures), dtype=np.float64)
         R = temps.size
@@ -482,32 +461,23 @@ class GibbsSampler:
         stats = torch.zeros(2, dtype=torch.int64, device=device)
         inj = _inject
         states = self._initial_states(prob, K * R, None if inj is None else np.asarray(inj["inits"]))
-        if tc:
-            states = prob.pad_state(states)
-            e = torch.empty(K * R, dtype=torch.float64, device=device)
-            self._tc_sweeps(prob, states, self.config.n_burnin, T_chain)
-        else:
-            bu = None
-            if inj is not None:  # parity mode: draws are given per temperature slot; slot i starts on replica i
-                bu = torch.from_numpy(np.ascontiguousarray(np.asarray(inj["burn_uniforms"]).transpose(1, 0, 2))).to(device)
-            self._run(prob, states, n_burnin=self.config.n_burnin, n_samples=0, sweeps_per_sample=0, T_chain=T_chain,
-                      uniforms=bu)
+        bu = None
+        if inj is not None:  # parity mode: draws are given per temperature slot; slot i starts on replica i
+            bu = torch.from_numpy(np.ascontiguousarray(np.asarray(inj["burn_uniforms"]).transpose(1, 0, 2))).to(device)
+        self._run(prob, states, n_burnin=self.config.n_burnin, n_samples=0, sweeps_per_sample=0, T_chain=T_chain,
+                  uniforms=bu)
         samples = torch.empty((n_samples, K, prob.N), dtype=torch.uint8, device=device)
         energies = torch.empty((n_samples, K, R), dtype=torch.float64, device=device)
         for it in range(n_samples):
-            if tc:
-                self._tc_sweeps(prob, states, n_sweeps, T_chain)
-                self._tc_energy(prob, states, e)
-            else:
-                su = None
-                if inj is not None:
-                    sr_host = slot_replica[0].cpu().numpy()
-                    u_slot = np.asarray(inj["sweep_uniforms"][it])            # [slot, sweep, N]
-                    u_rep = np.empty_like(u_slot)
-                    u_rep[sr_host] = u_slot                                    # replica sr_host[i] sits at slot i
-                    su = torch.from_numpy(np.ascontiguousarray(u_rep.transpose(1, 0, 2))).to(device)
-                _, e, _, _ = self._run(prob, states, n_burnin=n_sweeps, n_samples=0, sweeps_per_sample=0,
-                                       T_chain=T_chain, want_energy=True, uniforms=su)
+            su = None
+            if inj is not None:
+                sr_host = slot_replica[0].cpu().numpy()
+                u_slot = np.asarray(inj["sweep_uniforms"][it])            # [slot, sweep, N]
+                u_rep = np.empty_like(u_slot)
+                u_rep[sr_host] = u_slot                                    # replica sr_host[i] sits at slot i
+                su = torch.from_numpy(np.ascontiguousarray(u_rep.transpose(1, 0, 2))).to(device)
+            _, e, _, _ = self._run(prob, states, n_burnin=n_sweeps, n_samples=0, sweeps_per_sample=0, T_chain=T_chain,
+                                   want_energy=True, uniforms=su)
             energies[it] = e[slot_replica.long()]          # history is kept per temperature slot (gibbs.py:302-303)
             if (it + 1) % swap_interval == 0:
                 wu = None
@@ -534,8 +504,7 @@ class GibbsSampler:
             "energies": energy_lists[0] if K == 1 else energy_lists,
             "final_states": final_states[0] if K == 1 else final_states,
         }
-        out = _host_int64(samples)                         # (n_samples, K, N)
-        return (out[:, 0, :], info) if K == 1 else (np.ascontiguousarray(out.transpose(1, 0, 2)), info)
+        return self._samples_out(samples, K, False), info
 
     def simulated_annealing(self, coupling: np.ndarray, bias: Optional[np.ndarray] = None, T_initial: float = 10.0,
                             T_final: float = 0.1, n_steps: int = 1000, cooling_schedule: str = "exponential", *,
@@ -551,60 +520,22 @@ class GibbsSampler:
         (the model this path samples); the returned energy is that state's energy under the caller's float64
         couplings and bias.  The two coincide when the couplings are exact in bf16.
         """
-        torch = _lib.require_cuda()
-        tc = self.precision == "bf16" and not chromatic
-        if tc:
-            if _uniforms is not None:
-                raise ValueError("injected draws are a float64 / float32 parity mode; precision='bf16' draws Philox")
-            prob = _TcProblem(coupling, bias, self._dev(), self.config.update_order)
-        elif chromatic:
-            prob = self._sparse(coupling, bias)
-        else:
-            prob = _DenseProblem(coupling, bias, self.precision, self._dev())
+        _lib.require_cuda()
+        if self.precision == "bf16" and not chromatic and _uniforms is not None:
+            raise ValueError("injected draws are a float64 / float32 parity mode; precision='bf16' draws Philox")
+        prob = self._problem(coupling, bias, chromatic=chromatic, tensor_ok=True)
         Ts = annealing_temperatures(T_initial, T_final, n_steps, cooling_schedule)
         st = self._initial_states(prob, int(n_chains), _initial_state)
-        if tc and n_steps > 0:
-            st = prob.pad_state(st)
-            energy = torch.empty(int(n_chains), dtype=torch.float64, device=prob.device)
-            best_energy = torch.full((int(n_chains),), float("inf"), dtype=torch.float64, device=prob.device)
-            best_state = torch.empty_like(st)
-            self._tc_energy(prob, st, energy, best_energy, best_state)   # the initial state is the first best
-            for k in range(int(n_steps)):
-                self._tc_sweeps(prob, st, 1, float(Ts[k]))
-                self._tc_energy(prob, st, energy, best_energy, best_state)
-            self.config.temperature = float(Ts[-1])
-            k = int(np.argmin(best_energy.cpu().numpy()))
-            state = _host_int64(best_state[k, :prob.N])
-        elif n_steps > 0:
-            T_sweep = torch.from_numpy(Ts).to(prob.device)
+        if n_steps > 0:
             self.config.temperature = float(Ts[-1])  # the reference leaves the last T in the config (gibbs.py:382)
-            if chromatic:
-                _, _, best_state, best_energy = self._sparse_run(prob, st, uniforms=_uniforms, n_burnin=int(n_steps),
-                                                                 n_samples=0, sweeps_per_sample=0, T_sweep=T_sweep,
-                                                                 track_best=True)
-            else:
-                u, _ = self._inject(prob, _uniforms, None)
-                _, _, best_state, best_energy = self._run(prob, st, n_burnin=int(n_steps), n_samples=0,
-                                                          sweeps_per_sample=0, T_sweep=T_sweep, track_best=True,
-                                                          uniforms=u)
-            be = best_energy.cpu().numpy()
-            k = int(np.argmin(be))
+            _, _, best_state, best_energy = self._run(prob, st, n_burnin=int(n_steps), n_samples=0, sweeps_per_sample=0,
+                                                      T_sweep=Ts, track_best=True, **self._injected(prob, _uniforms))
+            k = int(np.argmin(best_energy.cpu().numpy()))
             state = _host_int64(best_state[k])
         else:
-            state = _host_int64(st[0])
+            state = _host_int64(st[0, :prob.N])
         self._chain_counter += int(n_chains)
-        if chromatic:
-            from .sparse import to_csr
-
-            rowptr, col, val, _ = to_csr(coupling)
-            sb = state.astype(np.float64)
-            row = np.repeat(np.arange(len(sb)), np.diff(rowptr))
-            e = -0.5 * float(np.sum(val * sb[row] * sb[col]))
-            if bias is not None:
-                e -= float(np.dot(np.asarray(bias, dtype=np.float64), sb))
-            return state, e
-        J = np.asarray(coupling, dtype=np.float64)
-        return state, self.compute_energy(state, J, None if bias is None else np.asarray(bias, dtype=np.float64))
+        return state, prob.energy(state)
 
 
 def _bf16_exact(coupling) -> bool:

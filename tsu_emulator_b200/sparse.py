@@ -79,6 +79,7 @@ class SparseProblem:
         rowptr, col, val, N = to_csr(coupling)
         self.N, self.nnz = N, int(val.size)
         self.device = device
+        self.csr = (rowptr, col, val)  # host copy of the couplings (energy of a returned state)
         colour = greedy_colouring(rowptr, col, N)
         cptr, sites = colour_classes(colour)
         self.n_colours = len(cptr) - 1
@@ -86,32 +87,44 @@ class SparseProblem:
         t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(device)
         self.rowptr, self.col, self.val = t(rowptr), t(col if col.size else np.zeros(1, np.int32)), t(val if val.size else np.zeros(1))
         self.cptr, self.sites = t(cptr), t(sites)
-        self.bias = None
+        self.bias = self.host_bias = None
         if bias is not None:
             b = np.asarray(bias, dtype=np.float64)
             if b.shape != (N,):
                 raise ValueError("bias must have one entry per bit")
-            self.bias = t(b)
+            self.bias, self.host_bias = t(b), b
 
+    def run(self, state, *, T: float, seed: int, sweep0: int, chain0: int, n_burnin: int, n_samples: int,
+            sweeps_per_sample: int, T_chain=None, T_sweep=None, uniforms=None, want_samples=False, want_energy=False,
+            track_best=False):
+        """one launch of tsu_sparse_gibbs_run on `state` (uint8 tensor [n_chains, N], updated in place); T_sweep is
+        the host float64 temperature of every sweep"""
+        torch = _lib.require_cuda()
+        n_chains, N = state.shape
+        dev = self.device
+        if T_sweep is not None:
+            T_sweep = torch.from_numpy(T_sweep).to(dev)
+        samples = torch.empty((n_samples, n_chains, N), dtype=torch.uint8, device=dev) if want_samples else None
+        energy = torch.empty(n_chains, dtype=torch.float64, device=dev) if (want_energy or track_best) else None
+        best_state = torch.empty((n_chains, N), dtype=torch.uint8, device=dev) if track_best else None
+        best_energy = torch.empty(n_chains, dtype=torch.float64, device=dev) if track_best else None
+        with torch.cuda.device(dev):
+            _lib.call("tsu_sparse_gibbs_run", ptr(self.rowptr), ptr(self.col), ptr(self.val), ptr(self.bias),
+                      ptr(self.cptr), ptr(self.sites), self.n_colours, ptr(state), int(n_chains), int(N), float(T),
+                      ptr(T_chain), ptr(T_sweep), int(n_burnin), int(n_samples), int(sweeps_per_sample), ptr(uniforms),
+                      ptr(samples), ptr(energy), int(track_best), ptr(best_state), ptr(best_energy), int(seed),
+                      sweep0 & 0xFFFFFFFF, chain0 & 0xFFFFFFFF, _lib.current_stream())
+        return samples, energy, best_state, best_energy
 
-def run(prob: SparseProblem, state, *, T: float, seed: int, sweep0: int, chain0: int, n_burnin: int, n_samples: int,
-        sweeps_per_sample: int, T_chain=None, T_sweep=None, uniforms=None, want_samples=False, want_energy=False,
-        track_best=False):
-    """one launch of tsu_sparse_gibbs_run on `state` (uint8 tensor [n_chains, N], updated in place)"""
-    torch = _lib.require_cuda()
-    n_chains, N = state.shape
-    dev = prob.device
-    samples = torch.empty((n_samples, n_chains, N), dtype=torch.uint8, device=dev) if want_samples else None
-    energy = torch.empty(n_chains, dtype=torch.float64, device=dev) if (want_energy or track_best) else None
-    best_state = torch.empty((n_chains, N), dtype=torch.uint8, device=dev) if track_best else None
-    best_energy = torch.empty(n_chains, dtype=torch.float64, device=dev) if track_best else None
-    with torch.cuda.device(dev):
-        _lib.call("tsu_sparse_gibbs_run", ptr(prob.rowptr), ptr(prob.col), ptr(prob.val), ptr(prob.bias), ptr(prob.cptr),
-                  ptr(prob.sites), prob.n_colours, ptr(state), int(n_chains), int(N), float(T), ptr(T_chain), ptr(T_sweep),
-                  int(n_burnin), int(n_samples), int(sweeps_per_sample), ptr(uniforms), ptr(samples), ptr(energy),
-                  int(track_best), ptr(best_state), ptr(best_energy), int(seed), sweep0 & 0xFFFFFFFF,
-                  chain0 & 0xFFFFFFFF, _lib.current_stream())
-    return samples, energy, best_state, best_energy
+    def energy(self, state: np.ndarray) -> float:
+        """E = -1/2 s^T J s - b^T s of a host state under the float64 CSR couplings and bias"""
+        rowptr, col, val = self.csr
+        sb = state.astype(np.float64)
+        row = np.repeat(np.arange(len(sb)), np.diff(rowptr))
+        e = -0.5 * float(np.sum(val * sb[row] * sb[col]))
+        if self.host_bias is not None:
+            e -= float(np.dot(self.host_bias, sb))
+        return e
 
 
 def is_sparse_enough(coupling, max_density: float = 0.05, min_n: int = 64) -> bool:
