@@ -263,6 +263,35 @@ int tsu_ising2d_population_anneal(uint32_t* d_state, uint32_t* d_scratch, int n_
                                   unsigned long long* d_count_sums, unsigned long long* d_obs, double* d_energy,
                                   void* d_work, size_t work_bytes, uintptr_t stream);
 
+/* One resampling step of population annealing on the chain states of any back end (GibbsSampler.population_annealing):
+ * n_chains rows of row_bytes bytes (d_state, read only), forming n_populations equal contiguous populations of
+ * R_p = n_chains / n_populations chains, each resampled on its own; no host sync.  Steps 2-4 of
+ * tsu_ising2d_population_anneal with E_i = d_energy[i] (float64):
+ *   E_ref = min_i E_i of the population -> d_energy_ref[p];
+ *   q_i = floor(exp(-x_i) 2^s), x_i = *d_dbeta (E_i - E_ref), s = 62 - ceil(log2 R_p), exp as spelled out there;
+ *   W = sum q_i -> d_weight_sum[p];
+ *   u = one 64-bit draw of the lattice stream (kind 3, replica chain0 + p R_p (mod 2^32), sweep `sweep`),
+ *   U = floor(u W / 2^64); the parent of child j is the smallest i with R_p C_i > j W + U (C: inclusive prefix sums);
+ *   gather: d_state_out[j] = d_state[parent(j)], d_family_out[j] = d_family[parent(j)] (int32).
+ * Rows of a multiple of 16 bytes at 16-byte aligned bases are copied in 16-byte vectors, others byte by byte; only
+ * the n_chains rows of d_state_out and entries of d_family_out are written.  A block of whole populations run on its
+ * own (its chain0, its slices of every buffer) equals that block of the whole call.
+ * d_work: at least tsu_ising2d_population_work_bytes(n_chains, n_populations) bytes, 8-byte aligned.
+ * TSU_ERR_INVALID_ARG before any CUDA call for: a NULL pointer, n_chains < 1, n_populations outside [1, 65535] or not
+ * dividing n_chains, row_bytes < 1, d_state_out == d_state, d_family_out == d_family, and a work buffer below the
+ * size or not 8-byte aligned. */
+int tsu_population_resample(const void* d_state, void* d_state_out, const int32_t* d_family, int32_t* d_family_out,
+                            const double* d_energy, const double* d_dbeta, int n_chains, int n_populations,
+                            long long row_bytes, uint64_t seed, uint32_t sweep, uint32_t chain0,
+                            unsigned long long* d_weight_sum, double* d_energy_ref, void* d_work, size_t work_bytes,
+                            uintptr_t stream);
+/* Per population p of n_populations equal contiguous populations of d_energy [n_chains]:
+ * d_moments[p][0] = sum E, d_moments[p][1] = sum E^2, in float64 with one fixed summation order per population, so a
+ * block of whole populations run on its own gives the same bits.  TSU_ERR_INVALID_ARG before any CUDA call for a NULL
+ * pointer, n_chains < 1, and n_populations outside [1, 65535] or not dividing n_chains. */
+int tsu_population_moments(const double* d_energy, int n_chains, int n_populations, double* d_moments,
+                           uintptr_t stream);
+
 /* Swendsen-Wang cluster updates of whole lattices at h = 0 ("physical" bias); no host sync, nothing allocated.
  * One step at sweep index s, for replica r with threshold t = d_thresholds[d_lut_index ? d_lut_index[r] : 0]:
  *   1. satisfied bonds: J sigma_ij s_i s_j > 0 (sigma = +-1 bond sign, +1 without bonds; J's sign is

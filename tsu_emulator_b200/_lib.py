@@ -90,6 +90,12 @@ SIGNATURES = {
          c_void_p, c_uint64, c_uint32, c_uint32, c_double, c_double, c_int64, c_int64, c_void_p, c_void_p, c_void_p,
          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_size_t, c_uintptr],
     ),
+    "tsu_population_resample": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.c_longlong, c_uint64,
+         c_uint32, c_uint32, c_void_p, c_void_p, c_void_p, ctypes.c_size_t, c_uintptr],
+    ),
+    "tsu_population_moments": (c_int, [c_void_p, c_int, c_int, c_void_p, c_uintptr]),
     "tsu_ising2d_cluster_work_bytes": (c_int64, [c_int, c_int, c_int]),
     "tsu_ising2d_swendsen_wang": (
         c_int,

@@ -12,6 +12,7 @@ Differences that are deliberate and documented:
     dimension the reference only emulates serially (gibbs.py:475-479).
 """
 
+import math
 from dataclasses import dataclass
 from typing import List, Optional, Tuple
 
@@ -19,6 +20,9 @@ import numpy as np
 
 from . import _lib
 from ._lib import ptr
+from .population import PopulationEstimates
+
+M32 = 0xFFFFFFFF
 
 
 @dataclass
@@ -233,6 +237,44 @@ def annealing_temperatures(T_initial: float, T_final: float, n_steps: int, cooli
     return T_initial + (T_final - T_initial) * steps / n_steps  # linear
 
 
+class DensePopulationResult(PopulationEstimates):
+    """What GibbsSampler.population_annealing returns; pass it back as `previous=` to continue the run.
+
+    Device tensors (P = n_populations, n = len(temperatures)):
+      energy          float64 [n_chains], E of every chain's final state (on bf16: under the bf16-rounded couplings)
+      family          int32 [n_chains], the initial chain (chain0 + j, mod 2^32) each chain descends from
+      weight_sum      int64 [n, P], W of step k; energy_ref float64 [n, P], E_ref of the population entering step k
+      energy_moments  float64 [n + 1, P, 2], (sum E, sum E^2) over the population entering step k; entry n: the final
+                      states
+      states          uint8 [n_chains, N], the final states
+    Host: temperatures, T_start, dbeta, r_pop (R_p), shift (s), n_sites (N), chain0, backend ("float64", "float32",
+    "bf16" or "chromatic").  ln Z ratios, free energies and rho_t: PopulationEstimates.
+    """
+
+    def __init__(self, state, energy, family, weight_sum, energy_ref, energy_moments, temperatures, T_start, dbeta,
+                 r_pop, shift, N, chain0, backend):
+        self._state = state  # rows padded to the tensor-core panel width: what previous= continues from
+        self.energy, self.family = energy, family
+        self.weight_sum, self.energy_ref, self.energy_moments = weight_sum, energy_ref, energy_moments
+        self.temperatures, self.T_start, self.dbeta = temperatures, float(T_start), dbeta
+        self.r_pop, self.shift, self.n_sites = int(r_pop), int(shift), int(N)
+        self.chain0, self.backend = int(chain0), backend
+
+    @property
+    def states(self):
+        return self._state[:, :self.n_sites]
+
+    def mean_energy(self) -> np.ndarray:
+        """[n, P]: population mean of E at temperatures[k] (after step k's sweeps), from energy_moments[1:]"""
+        return self.energy_moments[1:, :, 0].cpu().numpy() / self.r_pop
+
+    def specific_heat(self) -> np.ndarray:
+        """[n, P]: specific heat per spin at temperatures[k], (<E^2> - <E>^2) / (T_k^2 N) over each population"""
+        m = self.energy_moments[1:].cpu().numpy() / self.r_pop
+        beta = 1.0 / self.temperatures[:, None]
+        return beta * beta * (m[..., 1] - m[..., 0] * m[..., 0]) / self.n_sites
+
+
 class GibbsSampler:
     """tsu/gibbs.py:39-393 on the GPU.
 
@@ -293,12 +335,14 @@ class GibbsSampler:
             return _TcProblem(coupling, bias, self._dev(), self.config.update_order)
         return _DenseProblem(coupling, bias, self.precision, self._dev(), self.config.update_order)
 
-    def _run(self, prob, state, *, n_burnin: int, n_samples: int, sweeps_per_sample: int, **kw):
-        """prob.run on `state` at the sampler's temperature, seed and Philox offsets, which then advance past the sweeps
-        run.  A negative count is an error on the dense and sparse kernels and runs nothing on the tensor cores."""
-        out = prob.run(state, T=float(self.config.temperature), seed=self._seed, sweep0=self._sweep_counter,
-                       chain0=self._chain_counter, n_burnin=n_burnin, n_samples=n_samples,
-                       sweeps_per_sample=sweeps_per_sample, **kw)
+    def _run(self, prob, state, *, n_burnin: int, n_samples: int, sweeps_per_sample: int, T: Optional[float] = None,
+             chain0: Optional[int] = None, **kw):
+        """prob.run on `state` at the sampler's temperature (or T), seed and Philox offsets (the chain offset, or
+        chain0), which then advance past the sweeps run.  A negative count is an error on the dense and sparse kernels
+        and runs nothing on the tensor cores."""
+        out = prob.run(state, T=float(self.config.temperature if T is None else T), seed=self._seed,
+                       sweep0=self._sweep_counter, chain0=self._chain_counter if chain0 is None else chain0,
+                       n_burnin=n_burnin, n_samples=n_samples, sweeps_per_sample=sweeps_per_sample, **kw)
         self._sweep_counter += max(n_burnin, 0) + n_samples * max(sweeps_per_sample, 0)
         return out
 
@@ -536,6 +580,98 @@ class GibbsSampler:
             state = _host_int64(st[0, :prob.N])
         self._chain_counter += int(n_chains)
         return state, prob.energy(state)
+
+    def population_annealing(self, coupling, temperatures, bias=None, *, n_chains: int = 1024, n_populations: int = 1,
+                             sweeps_per_step: int = 10, T_start: float = math.inf, chromatic: bool = False,
+                             previous: Optional[DensePopulationResult] = None) -> DensePopulationResult:
+        """Population annealing (Hukushima-Iba, Machta) of n_chains chains in one call, with no host sync.
+
+        The chains form n_populations equal contiguous populations of R_p chains, each resampled on its own.  A fresh
+        run starts from the sampler's random initial states, which are equilibrium states at T_start = inf.  Step k:
+        the energies of the current states, their moments (energy_moments[k]), a resampling of every population in
+        proportion to exp(-dbeta_k E) with dbeta_k = 1/T_k - 1/T_{k-1} (T_{-1} = T_start), keeping R_p fixed
+        (tsu_population_resample states the exact rule), then sweeps_per_step sweeps at T_k.  The chain at position j
+        draws the Philox stream of chain0 + j, and the sweep indices continue from the sampler's counter.  The result
+        gives ln Z ratios, free energies, mean energies, specific heats and the family statistic rho_t; see
+        DensePopulationResult.
+
+        The back end is the sampler's: precision="bf16" runs the tensor-core sweeps and energy pass, "float64" /
+        "float32" the dense kernel, chromatic=True the chromatic CSR kernel (float64 sampler).  On bf16 the energies,
+        and so the weights, are those of the bf16-rounded couplings: the model this path samples.
+
+        temperatures must be non-increasing and at most T_start.  previous: the result of an earlier run with the same
+        couplings, back end, chain count and populations; its last temperature becomes T_start and its states, family
+        and chain0 are continued, so a run split into calls equals one call.  Afterwards the sweep counter has advanced
+        by len(temperatures) * sweeps_per_step, the chain counter by n_chains (fresh runs only), and config.temperature
+        is temperatures[-1].
+
+        The call holds two state buffers of n_chains rows while it runs (a third when it continues `previous`, whose
+        tensors it leaves as they were).
+        """
+        Ts = np.asarray(temperatures, dtype=np.float64)
+        if Ts.ndim != 1 or Ts.size == 0:
+            raise ValueError("temperatures must be a non-empty 1-D schedule")
+        if not np.all(np.isfinite(Ts)) or np.any(Ts <= 0):
+            raise ValueError("temperatures must be positive and finite")
+        if np.any(np.diff(Ts) > 0):
+            raise ValueError("temperatures must be non-increasing")
+        theta, P, C = int(sweeps_per_step), int(n_populations), int(n_chains)
+        if theta < 1:
+            raise ValueError("sweeps_per_step must be >= 1")
+        if C < 1:
+            raise ValueError("n_chains must be at least 1")
+        if P < 1 or P > 65535 or C % P:
+            raise ValueError(f"n_populations must divide n_chains = {C} (and lie in [1, 65535])")
+        r_pop = C // P
+        N = int(coupling[3]) if isinstance(coupling, tuple) and len(coupling) == 4 else int(np.shape(coupling)[0])
+        backend = "chromatic" if chromatic else self.precision
+        if previous is not None:
+            if (not isinstance(previous, DensePopulationResult) or previous.n_sites != N or previous.backend != backend
+                    or tuple(previous.family.shape) != (C,) or previous.n_populations != P or previous.r_pop != r_pop):
+                raise ValueError(f"previous must come from a run of {P} populations of {r_pop} chains of {N} bits on "
+                                 f"the {backend} back end")
+            T_start = float(previous.temperatures[-1])
+        T_start = float(T_start)
+        if not T_start > 0 or Ts[0] > T_start:
+            raise ValueError("T_start must be positive and at least temperatures[0]")
+        beta = 1.0 / Ts
+        dbeta = np.diff(np.concatenate([[0.0 if math.isinf(T_start) else 1.0 / T_start], beta]))
+        prob = self._problem(coupling, bias, chromatic=chromatic, tensor_ok=True)
+        torch = _lib.require_cuda()
+        dev, n = prob.device, int(Ts.size)
+        with torch.cuda.device(dev):
+            if previous is None:
+                chain0 = self._chain_counter
+                state = self._initial_states(prob, C)
+                family = (torch.arange(C, dtype=torch.int64, device=dev) + (chain0 & M32)).to(torch.int32)
+                _, energy, _, _ = self._run(prob, state, n_burnin=0, n_samples=0, sweeps_per_sample=0, T=Ts[0],
+                                            chain0=chain0, want_energy=True)
+            else:
+                chain0, state, family, energy = previous.chain0, previous._state, previous.family, previous.energy
+            other, family_other = torch.empty_like(state), torch.empty_like(family)
+            work_bytes = int(_lib.load().tsu_ising2d_population_work_bytes(C, P))
+            work = torch.empty(work_bytes // 8, dtype=torch.int64, device=dev)
+            d_dbeta = torch.from_numpy(dbeta).to(dev)
+            weight_sum = torch.empty((n, P), dtype=torch.int64, device=dev)
+            energy_ref = torch.empty((n, P), dtype=torch.float64, device=dev)
+            moments = torch.empty((n + 1, P, 2), dtype=torch.float64, device=dev)
+            for k in range(n):
+                _lib.call("tsu_population_moments", ptr(energy), C, P, ptr(moments[k]), _lib.current_stream())
+                _lib.call("tsu_population_resample", ptr(state), ptr(other), ptr(family), ptr(family_other),
+                          ptr(energy), ptr(d_dbeta[k]), C, P, int(state.shape[1]), self._seed,
+                          self._sweep_counter & M32, chain0 & M32, ptr(weight_sum[k]), ptr(energy_ref[k]), ptr(work),
+                          work_bytes, _lib.current_stream())
+                state, other, family, family_other = other, state, family_other, family
+                if k == 0 and previous is not None:  # previous's tensors stay as they were
+                    other, family_other = torch.empty_like(state), torch.empty_like(family)
+                _, energy, _, _ = self._run(prob, state, n_burnin=theta, n_samples=0, sweeps_per_sample=0, T=Ts[k],
+                                            chain0=chain0, want_energy=True)
+            _lib.call("tsu_population_moments", ptr(energy), C, P, ptr(moments[n]), _lib.current_stream())
+        if previous is None:
+            self._chain_counter += C
+        self.config.temperature = float(Ts[-1])
+        return DensePopulationResult(state, energy, family, weight_sum, energy_ref, moments, Ts.copy(), T_start, dbeta,
+                                     r_pop, 62 - (r_pop - 1).bit_length(), N, chain0, backend)
 
 
 def _bf16_exact(coupling) -> bool:

@@ -17,6 +17,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import c_void_p, ptr
+from .population import PopulationEstimates
 
 LUT_WORDS = 32
 
@@ -142,7 +143,7 @@ class AnnealResult:
         return out
 
 
-class PopulationResult:
+class PopulationResult(PopulationEstimates):
     """What Ising2DEngine.population_annealing returns; pass it back as `previous=` to continue the run.
 
     Device tensors (P = n_populations, n = len(temperatures)):
@@ -153,6 +154,7 @@ class PopulationResult:
       count_sums  int64 [n + 1, P, 2], (sum of up spins, sum of anti-aligned / unsatisfied bonds) of the states
                   entering step k; entry n: the final states
     Host: temperatures, T_start, dbeta, r_pop (R_p), shift (s), rows, cols, J, h, n_bonds, n_sites.
+    ln Z ratios, free energies and rho_t: PopulationEstimates.
     """
 
     def __init__(self, energy, family, weight_sum, energy_ref, count_sums, temperatures, T_start, dbeta, r_pop, shift,
@@ -164,40 +166,10 @@ class PopulationResult:
         self.rows, self.cols, self.J, self.h = int(rows), int(cols), float(J), float(h)
         self.n_bonds, self.n_sites = int(n_bonds), int(n_sites)
 
-    @property
-    def n_populations(self) -> int:
-        return int(self.weight_sum.shape[1])
-
-    def log_q(self) -> np.ndarray:
-        """[n, P] float64: ln Q_k = ln Z(T_k) / Z(T_{k-1}) ~ ln(W / (R_p 2^s)) - dbeta_k E_ref"""
-        W = self.weight_sum.cpu().numpy().astype(np.float64)
-        e_ref = self.energy_ref.cpu().numpy()
-        return np.log(W) - math.log(self.r_pop) - self.shift * math.log(2.0) - self.dbeta[:, None] * e_ref
-
-    def log_z_ratio(self) -> np.ndarray:
-        """[n, P]: ln Z(T_k) / Z(T_start), the cumulative sum of log_q"""
-        return np.cumsum(self.log_q(), axis=0)
-
-    def free_energy(self) -> np.ndarray:
-        """[n, P]: free energy per site -T_k ln Z(T_k) / N, with ln Z(T_start = inf) = N ln 2"""
-        if not math.isinf(self.T_start):
-            raise ValueError("free_energy needs a run from T_start = inf (ln Z is known only at infinite temperature)")
-        N = self.n_sites
-        return -self.temperatures[:, None] * (N * math.log(2.0) + self.log_z_ratio()) / N
-
     def mean_energy(self) -> np.ndarray:
         """[n, P]: population mean of E at temperatures[k] (after step k's sweeps), from count_sums[1:]"""
         c = self.count_sums[1:].cpu().numpy().astype(np.float64) / self.r_pop
         return -self.J * (self.n_bonds - 2.0 * c[..., 1]) - self.h * (2.0 * c[..., 0] - self.n_sites)
-
-    def rho_t(self) -> np.ndarray:
-        """[P]: R_p sum_f (n_f / R_p)^2 over the families f of each population (1 when every family has one member)"""
-        fam = self.family.cpu().numpy().reshape(self.n_populations, self.r_pop)
-        out = np.empty(self.n_populations)
-        for p in range(self.n_populations):
-            n_f = np.unique(fam[p], return_counts=True)[1].astype(np.float64)
-            out[p] = (n_f * n_f).sum() / self.r_pop
-        return out
 
 
 class Ising2DEngine:
