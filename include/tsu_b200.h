@@ -443,6 +443,38 @@ int tsu_sparse_gibbs_run(const int32_t* d_rowptr, const int32_t* d_col, const do
                          int track_best, uint8_t* d_best_state, double* d_best_energy, uint64_t seed,
                          uint32_t sweep0, uint32_t chain0, uintptr_t stream);
 
+/* Houdayer cluster moves of chain pairs on SPARSE couplings (csrc/sparse_houdayer.cu), the overlap-cluster move of
+ * ICM (Zhu, Ochoa & Katzgraber 2015) on any graph.  d_state is the [n_chains][N] uint8 state of tsu_sparse_gibbs_run,
+ * couplings in its CSR form (d_rowptr, d_col, d_val, d_bias may be NULL).  No host sync, nothing allocated.  One step
+ * at index s, for each pair (a, b) of d_pairs (int32 [n_pairs][2] on the device):
+ *   1. differ: d_i = x^a_i xor x^b_i.
+ *   2. graph: edge {i, j} for every stored entry J_ij != 0 of row i with j > i (self couplings never join); for the
+ *      symmetric couplings the move is meant for, that is every coupled pair.
+ *   3. clusters: connected components of the graph restricted to the sites with d = 1; a cluster's root is its
+ *      smallest site index.
+ *   4. flip: a cluster flips, x^a_i ^= 1 and x^b_i ^= 1 on all its sites (the two chains swap their bits there), iff
+ *      bit 0 of word 0 of Philox(counter = (root, chain0 + a, s, 'HOUD'), key = seed) is 1.  Sites with d = 0 never
+ *      change.
+ * For symmetric J the move leaves E_a + E_b and the overlap unchanged, for any bias and self couplings, and keeps the
+ * product of the two Boltzmann distributions.  The caller guarantees that the pairs are disjoint and that the two
+ * chains of a pair share couplings and temperature; a pair with an index outside [0, n_chains) or a == b is skipped
+ * (its rows are neither read nor written).  n_steps steps use the indices step0 .. step0 + n_steps - 1; n_steps = 0 is
+ * a no-op.  With d_energy, every processed chain gets E = -1/2 s^T J s - b^T s of its final state, bit for bit the
+ * value tsu_sparse_gibbs_run reports for that state.  Rows are written back as 0 / 1 bytes.
+ * One CTA per pair runs all steps.  Up to N = 32768 the rows and labels stay in shared memory and d_work is unused;
+ * above that (to the sweep kernel's N <= 204800) the labels go to d_work, tsu_sparse_houdayer_work_bytes(1, N) bytes
+ * per pair (16-byte aligned), and the pairs run in chunks of work_bytes / that, each chunk through all its steps, all
+ * ordered on `stream`.  The bits depend on neither path nor chunking.
+ * TSU_ERR_INVALID_ARG before any CUDA call for: a NULL d_rowptr / d_col / d_val / d_state / d_pairs, N outside
+ * [1, 204800], n_steps < 0, n_pairs < 1 or 2 n_pairs > n_chains, and (above N = 32768) a NULL or not 16-byte aligned
+ * d_work or a work buffer below one pair.  tsu_sparse_houdayer_work_bytes returns 0 when no workspace is needed or the arguments cannot be
+ * served. */
+int64_t tsu_sparse_houdayer_work_bytes(int n_pairs, int N);
+int tsu_sparse_houdayer(const int32_t* d_rowptr, const int32_t* d_col, const double* d_val, const double* d_bias,
+                        uint8_t* d_state, int n_chains, int N, const int32_t* d_pairs, int n_pairs,
+                        uint64_t seed, uint32_t step0, int n_steps, uint32_t chain0, double* d_energy,
+                        void* d_work, size_t work_bytes, uintptr_t stream);
+
 /* Replica-exchange pass (tsu/gibbs.py:308-323): for each ladder, pairs i = 0..R-2 in order;
  * delta = (1/T_i - 1/T_{i+1}) (E_{i+1} - E_i); accept if delta >= 0 or u < exp(delta) (u drawn
  * only when delta < 0).  Configurations stay in place; d_slot_replica[ladder][i] (the replica

@@ -119,6 +119,12 @@ SIGNATURES = {
          c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_uint64, c_uint32,
          c_uint32, c_uintptr],
     ),
+    "tsu_sparse_houdayer_work_bytes": (c_int64, [c_int, c_int]),
+    "tsu_sparse_houdayer": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_uint64, c_uint32, c_int,
+         c_uint32, c_void_p, c_void_p, ctypes.c_size_t, c_uintptr],
+    ),
     "tsu_dense_energy": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_uintptr]),
     "tsu_dense_init_random": (c_int, [c_void_p, c_int, c_int, c_uint64, c_uint32, c_uintptr]),
     "tsu_dense_gibbs_tc_run": (

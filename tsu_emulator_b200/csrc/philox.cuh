@@ -206,3 +206,4 @@ __host__ __device__ __forceinline__ tsu_u32x4 tsu_lattice_stream_call_x0(const t
 #define TSU_STREAM_LANGEVIN 0x4C414E47u  // 'LANG'
 #define TSU_STREAM_LANGEVIN_INIT 0x4C494E49u  // 'LINI'
 #define TSU_STREAM_PT_SWAP 0x50545357u   // 'PTSW'
+#define TSU_STREAM_HOUDAYER 0x484F5544u  // 'HOUD': sparse Houdayer flips, counter = (root, chain0 + a, step, tag)

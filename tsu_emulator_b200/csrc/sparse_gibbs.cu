@@ -17,6 +17,7 @@
 
 #include "common.cuh"
 #include "philox.cuh"
+#include "sparse_energy.cuh"
 
 namespace {
 
@@ -47,31 +48,6 @@ __device__ __forceinline__ double sigmoid_clamped_d(double x) {  // tsu/gibbs.py
   return 1.0 / (1.0 + exp(-x));
 }
 
-__device__ __forceinline__ double block_sum_d(double v, double* red) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = (blockDim.x + 31) >> 5;
-  __syncthreads();
-  if (lane == 0) red[warp] = v;
-  __syncthreads();
-  double t = 0.0;
-  for (int w = 0; w < nw; ++w) t += red[w];
-  return t;
-}
-
-// E = -1/2 s^T J s - b^T s (tsu/gibbs.py:215-236)
-__device__ double sparse_energy(const SparseParams& P, const uint8_t* s, double* red) {
-  double acc = 0.0;
-  for (int i = threadIdx.x; i < P.N; i += blockDim.x) {
-    if (!s[i]) continue;
-    double h = 0.0;
-    for (int k = P.rowptr[i]; k < P.rowptr[i + 1]; ++k)
-      if (s[P.col[k]]) h += P.val[k];
-    acc += -0.5 * h - (P.bias ? P.bias[i] : 0.0);
-  }
-  return block_sum_d(acc, red);
-}
-
 __global__ void __launch_bounds__(256) sparse_gibbs_kernel(SparseParams P) {
   extern __shared__ unsigned char smem_s[];
   __shared__ double red[32];
@@ -83,7 +59,7 @@ __global__ void __launch_bounds__(256) sparse_gibbs_kernel(SparseParams P) {
 
   double best_e = 0.0;
   if (P.track_best) {
-    best_e = sparse_energy(P, s, red);
+    best_e = sparse_energy(P.rowptr, P.col, P.val, P.bias, P.N, s, red);
     for (int j = threadIdx.x; j < N; j += blockDim.x) P.best_state[(size_t)chain * N + j] = s[j];
   }
   const int total = P.n_burnin + P.n_samples * P.sweeps_per_sample;
@@ -114,7 +90,7 @@ __global__ void __launch_bounds__(256) sparse_gibbs_kernel(SparseParams P) {
       __syncthreads();
     }
     if (P.track_best) {  // gibbs.py:387-391
-      const double e = sparse_energy(P, s, red);
+      const double e = sparse_energy(P.rowptr, P.col, P.val, P.bias, P.N, s, red);
       if (e < best_e) {
         best_e = e;
         for (int j = threadIdx.x; j < N; j += blockDim.x) P.best_state[(size_t)chain * N + j] = s[j];
@@ -132,7 +108,7 @@ __global__ void __launch_bounds__(256) sparse_gibbs_kernel(SparseParams P) {
   }
   for (int j = threadIdx.x; j < N; j += blockDim.x) gstate[j] = s[j];
   if (P.energy) {
-    const double e = sparse_energy(P, s, red);
+    const double e = sparse_energy(P.rowptr, P.col, P.val, P.bias, P.N, s, red);
     if (threadIdx.x == 0) P.energy[chain] = e;
   }
   if (P.track_best && threadIdx.x == 0) P.best_energy[chain] = best_e;
@@ -186,9 +162,6 @@ extern "C" int tsu_sparse_gibbs_run(const int32_t* d_rowptr, const int32_t* d_co
   P.k1 = (uint32_t)(seed >> 32);
   P.sweep0 = sweep0;
   P.chain0 = chain0;
-  int threads = (N + 3) / 4;
-  threads = (threads + 31) / 32 * 32;
-  threads = threads < 32 ? 32 : (threads > 256 ? 256 : threads);
-  sparse_gibbs_kernel<<<n_chains, threads, smem, tsu_stream(stream)>>>(P);
+  sparse_gibbs_kernel<<<n_chains, sparse_threads(N), smem, tsu_stream(stream)>>>(P);
   TSU_RETURN_LAUNCH_STATUS();
 }

@@ -70,6 +70,8 @@ def _host_energy(state: np.ndarray, coupling, bias=None) -> float:
 # in at most 227 KB of shared memory: 33 N + 272 bytes with float64 fields, 17 N + 272 with float32
 DENSE_MAX_N = {"float64": 7035, "float32": 13657}
 
+CHROMATIC_NEEDS_FLOAT64 = "chromatic=True (sparse couplings) computes float64 fields: use a 'float64' sampler"
+
 
 class _DenseProblem:
     """coupling matrix + bias resident on the device (transposed, see tsu_b200.h)"""
@@ -294,6 +296,7 @@ class GibbsSampler:
         self._sweep_counter = 0  # Philox offset: advances with every sweep executed
         self._chain_counter = 0
         self._swap_counter = 0   # Philox offset of the replica-exchange draws: advances with every swap pass
+        self._houdayer_counter = 0  # step index of the Houdayer moves of parallel_tempering: advances with every move
         self._device = device
 
     # ------------------------------------------------------------------ scalar helpers
@@ -329,7 +332,7 @@ class GibbsSampler:
             from .sparse import SparseProblem
 
             if self.precision != "float64":
-                raise ValueError("chromatic=True (sparse couplings) computes float64 fields: use a 'float64' sampler")
+                raise ValueError(CHROMATIC_NEEDS_FLOAT64)
             return SparseProblem(coupling, bias, self._dev())
         if self.precision == "bf16" and tensor_ok:
             return _TcProblem(coupling, bias, self._dev(), self.config.update_order)
@@ -467,7 +470,8 @@ class GibbsSampler:
 
     def parallel_tempering(self, coupling: np.ndarray, temperatures: List[float], bias: Optional[np.ndarray] = None,
                            n_samples: int = 1000, swap_interval: int = 10, *, n_ladders: int = 1,
-                           criterion: str = "reference", _inject=None) -> Tuple[np.ndarray, dict]:
+                           criterion: str = "reference", chromatic: bool = False, houdayer_interval: int = 0,
+                           houdayer_max_temperature: float = math.inf, _inject=None) -> Tuple[np.ndarray, dict]:
         """tsu/gibbs.py:238-338: replicas at `temperatures`, n_sweeps sweeps per iteration, adjacent-pair
         Metropolis swaps every swap_interval iterations, samples from temperature slot 0.
 
@@ -483,16 +487,45 @@ class GibbsSampler:
         criterion="reference" keeps the swap expression of gibbs.py:317, which favours moving high-energy
         configurations to cold slots; "metropolis" is the detailed-balance rule, under which slot 0 samples the
         Boltzmann distribution at temperatures[0].
+
+        chromatic=True: sparse couplings (dense array, scipy.sparse matrix or CSR tuple) on the chromatic CSR kernel
+        (float64 sampler); a sweep visits the sites colour class by colour class.
+
+        houdayer_interval = k > 0 (chromatic=True, even n_ladders, symmetric couplings): every k iterations, after the
+        sweeps and before the energy record and the exchange pass, one Houdayer move (ICM, Zhu, Ochoa & Katzgraber
+        2015; tsu_sparse_houdayer states the exact rule) acts on the replicas of ladders 2m and 2m + 1 at every slot
+        whose temperature is at most houdayer_max_temperature.  Hot slots, where difference clusters percolate and the
+        move only exchanges configurations, can be left out that way.  The pairs are built on the device; the move
+        keeps E_a + E_b and the product of the two Boltzmann distributions, and its step index is the sampler's
+        Houdayer counter, which advances by one per move.
         """
-        torch = _lib.require_cuda()
         K = int(n_ladders)
+        hk = houdayer_interval
+        if isinstance(hk, bool) or not isinstance(hk, (int, np.integer)) or hk < 0:
+            raise ValueError("houdayer_interval must be a non-negative integer")
+        if chromatic and self.precision != "float64":
+            raise ValueError(CHROMATIC_NEEDS_FLOAT64)
+        if chromatic and _inject is not None:
+            raise ValueError("injected draws are a float64 / float32 parity mode of one ladder on the dense kernel")
+        if hk > 0:
+            from .sparse import is_symmetric_csr, to_csr
+
+            if not chromatic:
+                raise ValueError("Houdayer moves run on the chromatic back end: pass chromatic=True")
+            if K % 2:
+                raise ValueError("Houdayer moves pair ladders 2m and 2m + 1: n_ladders must be even")
+            if not float(houdayer_max_temperature) > 0:
+                raise ValueError("houdayer_max_temperature must be positive")
+            if not is_symmetric_csr(*to_csr(coupling)):
+                raise ValueError("Houdayer moves need symmetric couplings (J equal to its transpose)")
+        torch = _lib.require_cuda()
         if K < 1:
             raise ValueError("n_ladders must be at least 1")
         if criterion not in ("metropolis", "reference"):
             raise ValueError("criterion must be 'metropolis' or 'reference'")
         if _inject is not None and (self.precision == "bf16" or K > 1):
             raise ValueError("injected draws are a float64 / float32 parity mode of one ladder")
-        prob = self._problem(coupling, bias, chromatic=False, tensor_ok=True)
+        prob = self._problem(coupling, bias, chromatic=chromatic, tensor_ok=True)
         device = prob.device
         temps = np.asarray(list(temperatures), dtype=np.float64)
         R = temps.size
@@ -510,6 +543,10 @@ class GibbsSampler:
             bu = torch.from_numpy(np.ascontiguousarray(np.asarray(inj["burn_uniforms"]).transpose(1, 0, 2))).to(device)
         self._run(prob, states, n_burnin=self.config.n_burnin, n_samples=0, sweeps_per_sample=0, T_chain=T_chain,
                   uniforms=bu)
+        chain0, h_slots, n_pairs = self._chain_counter, None, 0
+        if hk > 0:
+            h_slots = torch.from_numpy(np.nonzero(temps <= float(houdayer_max_temperature))[0]).to(device)
+            n_pairs = (K // 2) * int(h_slots.numel())
         samples = torch.empty((n_samples, K, prob.N), dtype=torch.uint8, device=device)
         energies = torch.empty((n_samples, K, R), dtype=torch.float64, device=device)
         for it in range(n_samples):
@@ -522,6 +559,12 @@ class GibbsSampler:
                 su = torch.from_numpy(np.ascontiguousarray(u_rep.transpose(1, 0, 2))).to(device)
             _, e, _, _ = self._run(prob, states, n_burnin=n_sweeps, n_samples=0, sweeps_per_sample=0, T_chain=T_chain,
                                    want_energy=True, uniforms=su)
+            if n_pairs and (it + 1) % hk == 0:  # ladders 2m and 2m + 1 at the selected slots
+                sel = slot_replica[:, h_slots]
+                pairs = torch.stack((sel[0::2], sel[1::2]), -1).reshape(-1, 2).contiguous()
+                prob.houdayer(states, pairs, n_pairs, seed=self._seed, step0=self._houdayer_counter, n_steps=1,
+                              chain0=chain0, energy=e)
+                self._houdayer_counter += 1
             energies[it] = e[slot_replica.long()]          # history is kept per temperature slot (gibbs.py:302-303)
             if (it + 1) % swap_interval == 0:
                 wu = None

@@ -15,6 +15,19 @@ import numpy as np
 from . import _lib
 from ._lib import ptr
 
+HOUDAYER_WORK_BUDGET = 1 << 30  # bytes of Houdayer labels a SparseProblem keeps (N > 32768: 4 N bytes per pair)
+
+
+def is_symmetric_csr(rowptr: np.ndarray, col: np.ndarray, val: np.ndarray, N: int) -> bool:
+    """the CSR matrix (columns ascending within a row) equals its transpose in structure and values"""
+    from scipy.sparse import csr_matrix
+
+    A = csr_matrix((val, col, rowptr), shape=(N, N))
+    T = A.T.tocsr()
+    T.sort_indices()
+    return (np.array_equal(A.indptr, T.indptr) and np.array_equal(A.indices, T.indices)
+            and np.array_equal(A.data, T.data))
+
 
 def to_csr(coupling) -> Tuple[np.ndarray, np.ndarray, np.ndarray, int]:
     """(rowptr int32[N+1], col int32[nnz], val float64[nnz], N) of a square coupling matrix given as a dense array,
@@ -88,6 +101,7 @@ class SparseProblem:
         self.rowptr, self.col, self.val = t(rowptr), t(col if col.size else np.zeros(1, np.int32)), t(val if val.size else np.zeros(1))
         self.cptr, self.sites = t(cptr), t(sites)
         self.bias = self.host_bias = None
+        self._houdayer_work = None  # Houdayer label workspace (N > 32768), allocated by the first call that needs it
         if bias is not None:
             b = np.asarray(bias, dtype=np.float64)
             if b.shape != (N,):
@@ -115,6 +129,27 @@ class SparseProblem:
                       ptr(samples), ptr(energy), int(track_best), ptr(best_state), ptr(best_energy), int(seed),
                       sweep0 & 0xFFFFFFFF, chain0 & 0xFFFFFFFF, _lib.current_stream())
         return samples, energy, best_state, best_energy
+
+    def houdayer(self, state, pairs, n_pairs: int, *, seed: int, step0: int, n_steps: int, chain0: int, energy=None):
+        """one launch of tsu_sparse_houdayer on `state` (uint8 tensor [n_chains, N], updated in place): n_steps
+        Houdayer moves, step indices step0 .. step0 + n_steps - 1, of the disjoint chain pairs `pairs` (int32 device
+        tensor [n_pairs, 2]); with `energy` (float64 [n_chains]) every processed chain's energy is written there.  The
+        label workspace of N > 32768 is owned here and grows to what a call needs, at most HOUDAYER_WORK_BUDGET (then
+        the pairs run in chunks, with the same bits)."""
+        torch = _lib.require_cuda()
+        lib = _lib.load()
+        n_pairs = int(n_pairs)
+        per_pair = int(lib.tsu_sparse_houdayer_work_bytes(1, self.N))
+        need = min(n_pairs, max(1, HOUDAYER_WORK_BUDGET // per_pair)) * per_pair if per_pair else 0
+        work = self._houdayer_work
+        if need and (work is None or work.numel() * 8 < need):
+            work = torch.empty(need // 8, dtype=torch.int64, device=self.device)
+            self._houdayer_work = work
+        with torch.cuda.device(self.device):
+            _lib.call("tsu_sparse_houdayer", ptr(self.rowptr), ptr(self.col), ptr(self.val), ptr(self.bias), ptr(state),
+                      int(state.shape[0]), self.N, ptr(pairs), n_pairs, int(seed), step0 & 0xFFFFFFFF, int(n_steps),
+                      chain0 & 0xFFFFFFFF, ptr(energy), ptr(work if need else None), work.numel() * 8 if need else 0,
+                      _lib.current_stream())
 
     def energy(self, state: np.ndarray) -> float:
         """E = -1/2 s^T J s - b^T s of a host state under the float64 CSR couplings and bias"""
